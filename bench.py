@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's algorithm on host cores (oracle port)
+    python bench.py ... --dump-outputs DIR                   # + a seeded sample of the last timed step's outputs as .npy
 
 A "step" is one pass of LinearTFTPoseEstimation (+ ReprError) over one batch of synthetic trials
 of BASELINE.json config 3: experiments.m's noise sweep, n = 20 points, `--trials` (default
@@ -329,6 +330,9 @@ def run_gpu(args, rank, local_rank, world):
     ms, prof = timed(step_tft, args.steps, profile=True)
     launches = lib.tvf_launch_count(h._h) - l0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:            # before the other legs reuse the output buffers
+        dump_outputs(args.dump_outputs, B, n, {"R_t_2": d_Rt2, "R_t_3": d_Rt3, "Reconst": d_rec, "T": d_T,
+                                                "repr_err": d_rep, "status": d_st})
     flagged = int(torch.count_nonzero(d_st).item())
     flagged_detail = None
     if flagged:
@@ -646,6 +650,26 @@ def run_gpu(args, rank, local_rank, world):
         dist.destroy_process_group()
 
 
+DUMP_MAX_TRIALS = 32768
+DUMP_MAX_BYTES = 60 * 10 ** 6
+
+
+def dump_outputs(out_dir, B, n, outputs):
+    """Write what the last timed step handed its caller (`outputs`: name -> device tensor with one row per trial) as
+    out_dir/<name>.npy in float64, for a fixed sample of trials drawn with a fixed seed (`trial.npy`: their indices),
+    so that two builds run with the same arguments can be compared output for output.  At most DUMP_MAX_BYTES."""
+    import torch
+    per_trial = 8 * (sum(t[0].numel() for t in outputs.values()) + 1)
+    S = min(B, DUMP_MAX_TRIALS, DUMP_MAX_BYTES // per_trial)
+    idx = np.sort(np.random.default_rng(0).choice(B, size=S, replace=False))
+    sel = torch.from_numpy(idx).to(next(iter(outputs.values())).device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "trial.npy"), idx.astype(np.float64))
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.index_select(0, sel).cpu().numpy().astype(np.float64))
+    print("bench: wrote %d of %d trials' outputs (n = %d) to %s" % (S, B, n, out_dir), file=sys.stderr)
+
+
 # ---- BASELINE config 5: large-n triplets (HBM-oriented Gram formation) ------------------------------
 def large_n_scenes(B, n, dev, seed=1):
     """B scenes of generateSyntheticScene's geometry (f = 50, angle = 0), n points each, 1 px Gaussian noise, generated on
@@ -760,7 +784,7 @@ def run_large_n(args, local_rank):
     torch.cuda.set_device(local_rank)
     h = _lib.Handle(local_rank)
     sampler = ClockSampler(local_rank)
-    blk = large_n_measure(h, h.lib, local_rank, args.trials, args.n, max(1, min(args.steps, 5)), max(1, args.warmup))
+    blk = large_n_measure(h, h.lib, local_rank, args.trials, args.n, args.steps, max(1, args.warmup))
     clocks = sampler.stop()
     line = {"metric": blk["metric"], "unit": blk["unit"], "value": blk["value"], "n_gpus": 1, "steps": blk["steps"],
             "warmup": max(1, args.warmup), "ms_per_step": blk["ms_per_step"], "higher_is_better": True, "scaling": "weak",
@@ -808,7 +832,14 @@ def main():
                     help="scenes of the config-5 block inside the default line (n = 10000; 0 = skip; N = 1 only)")
     ap.add_argument("--workload", default="sweep", choices=["sweep", "large-n"],
                     help="sweep = BASELINE config 3/4 (headline); large-n = config 5 (use with --n 10000 --trials 65536)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed, seeded sample of the last step's outputs as DIR/<name>.npy "
+                         "(sweep workload of the CUDA path, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "sweep"):
+        ap.error("--dump-outputs applies to the sweep workload of the CUDA path (--impl b200 --workload sweep)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -11,8 +11,6 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
-REFERENCE = "/root/reference"
-
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
@@ -46,6 +44,37 @@ def tvf(libtvf_path):
     import tft_vs_fund_b200 as pkg
     pkg.handle()          # raises loudly when there is no CUDA device / library
     return pkg
+
+
+@pytest.fixture(scope="session")
+def epfl_data(tmp_path_factory):
+    """Directory with fountain-P11/ and Herz-Jesu-P8/ laid out as the reference's Data/ folders (Corresp_triplets.mat
+    and one .camera file per image), written from tests/golden/epfl_inputs.npz: indexes_sorted and the match lists of
+    the tested triplets, and the calibration and orientation of every image.  Image names and sizes are not stored
+    there, so the images are named 0000, 0001, ... and given the EPFL size 3072 x 2048."""
+    import scipy.io as sio
+    inp = np.load(os.path.join(ROOT, "tests", "golden", "epfl_inputs.npz"))
+    root = tmp_path_factory.mktemp("epfl_data")
+    for ds in ("fountain-P11", "Herz-Jesu-P8"):
+        key = ds.replace("-", "_")
+        K, R, t = inp[key + "_K"], inp[key + "_R"], inp[key + "_t"]
+        idx, offs, matches = inp[key + "_indexes_sorted"], inp[key + "_offsets"], inp[key + "_matches"]
+        names = ["%04d" % i for i in range(len(K))]
+        path = root / ds
+        path.mkdir()
+        for name, Ki, Ri, ti in zip(names, K, R, t):
+            # readCalibrationOrientation_EPFL.m:8-20: K, a skipped line, R' row by row, camera centre C (t = -R*C), size.
+            # The stored R are orthonormal only to the digits of the data files, so C solves R*C = -t (not C = -R'*t).
+            rows = list(Ki) + [np.zeros(3)] + list(Ri.T) + [np.linalg.solve(Ri, -ti), [3072.0, 2048.0]]
+            (path / (name + ".camera")).write_text("".join(" ".join(repr(float(v)) for v in r) + "\n" for r in rows))
+        cells = np.empty((len(K),) * 3, dtype=object)
+        for ijk in np.ndindex(cells.shape):
+            cells[ijk] = np.zeros((0, 6))
+        for r, (i, j, k, _) in enumerate(idx):
+            cells[i - 1, j - 1, k - 1] = matches[offs[r]:offs[r + 1]]
+        sio.savemat(str(path / "Corresp_triplets.mat"), {"indexes_sorted": idx.astype(np.float64), "Corresp": cells,
+                                                         "im_names": np.array(names, dtype=object).reshape(1, -1)})
+    return str(root)
 
 
 # ---- comparison helpers shared by the tests --------------------------------------------------

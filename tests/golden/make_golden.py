@@ -76,7 +76,10 @@ def sweep():
         CalM, R_t0, C, _ = o.experiments_subsample(20, noise, seed)
         cases.append(dict(Corresp=C, CalM=CalM, res=run_both(C, CalM), noise=noise, seed=seed,
                           Rt0_2=R_t0[0], Rt0_3=R_t0[1]))
-    np.savez_compressed(os.path.join(HERE, "sweep_n20.npz"), **pack(cases))
+    d = pack(cases)
+    # the ref_* arrays go to a companion file, which keeps each file under 1 MB
+    np.savez_compressed(os.path.join(HERE, "sweep_n20.npz"), **{k: v for k, v in d.items() if not k.startswith("ref_")})
+    np.savez_compressed(os.path.join(HERE, "sweep_n20_ref.npz"), **{k: v for k, v in d.items() if k.startswith("ref_")})
 
 
 def example():

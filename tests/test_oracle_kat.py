@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 
 import oracle as o
-from conftest import REFERENCE, rel_frob_up_to_sign, rot_angle, vec_angle
+from conftest import rel_frob_up_to_sign, rot_angle, vec_angle
 
 
 @pytest.mark.parametrize("seed", [1, 2, 3])
@@ -101,10 +101,9 @@ def test_triangulation_and_reprerror_forms():
     assert o.triangulation3D(Ps[:1], C[:2]) is None and o.triangulation3D(Ps, C[:5]) is None
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference data not present on this box")
-def test_epfl_fountain_top_triplet_prints():
+def test_epfl_fountain_top_triplet_prints(epfl_data):
     """experiments_real.m:94-101 prints 1360 valid correspondences with reprojection error 0.2586 (SURVEY.md 4)."""
-    path = os.path.join(REFERENCE, "Data", "fountain-P11")
+    path = os.path.join(epfl_data, "fountain-P11")
     idx, cor, names = o.load_corresp_triplets(path)
     d = o.epfl_triplet(path, idx, cor, names, 1)
     assert d["triplet"] == (5, 6, 7)

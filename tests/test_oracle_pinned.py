@@ -1,19 +1,27 @@
 """Pins the oracle restatement against the reference's own source.
 
 tests/golden/*.npz hold `ref_*` arrays produced by executing the UNMODIFIED reference .m files
-(/root/reference/TFT_methods, F_methods, auxiliar_functions) with oracle/mini_matlab.py, a minimal
-MATLAB-subset interpreter whose built-ins are NumPy/LAPACK.  The oracle (oracle/reference_port.py)
-must reproduce them; where /root/reference is mounted the interpreter is also run live."""
+(TFT_methods, F_methods, auxiliar_functions of the original project) with oracle/mini_matlab.py, a
+minimal MATLAB-subset interpreter whose built-ins are NumPy/LAPACK.  The oracle
+(oracle/reference_port.py) must reproduce them."""
 import os
 
 import numpy as np
 import pytest
 
 import oracle as o
-from conftest import REFERENCE, ROOT, rel_frob_up_to_sign, votes8_equal
+from conftest import ROOT, rel_frob_up_to_sign, votes8_equal
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-HAVE_REF = os.path.isdir(REFERENCE)
+
+
+def _load_golden(name):
+    """A golden file together with its `_ref` companion (the ref_* arrays, kept apart where one file would exceed 1 MB)."""
+    d = dict(np.load(os.path.join(GOLDEN, name)))
+    ref = os.path.join(GOLDEN, name.replace(".npz", "_ref.npz"))
+    if os.path.exists(ref):
+        d.update(np.load(ref))
+    return d
 
 
 def _run_oracle(method, C, CalM):
@@ -26,8 +34,8 @@ def _run_oracle(method, C, CalM):
 @pytest.mark.parametrize("name,stride", [("sweep_n20.npz", 7), ("example_n100.npz", 1), ("epfl_triplets.npz", 3)])
 @pytest.mark.parametrize("method", ["tft", "f"])
 def test_oracle_reproduces_reference_source_outputs(name, stride, method):
-    g = np.load(os.path.join(GOLDEN, name))
-    assert "ref_%s_T" % method in g.files, "golden file lacks interpreter outputs: regenerate with make_golden.py"
+    g = _load_golden(name)
+    assert "ref_%s_T" % method in g, "golden file lacks interpreter outputs: regenerate with make_golden.py"
     for b in range(0, g["Corresp"].shape[0], stride):
         got = _run_oracle(method, g["Corresp"][b], g["CalM"][b])
         for k, key in enumerate(("Rt2", "Rt3", "Reconst", "T", "repr")):
@@ -61,34 +69,21 @@ def test_gauss_helmert_port_reproduces_reference_source_outputs(name, stride):
         assert rel_frob_up_to_sign(g["optf_T"][b], g["ref_optf_T"][b]) < 1e-10
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference sources not present on this box")
-def test_faugpapa_constraint_function_and_why_it_is_not_a_parity_target():
-    """SURVEY 8 f4, second step (FaugPapaTFTPoseEstimation): the oracle restates its constraint function exactly
-    (f, g, A, B, C equal to the reference's own constrGH run by the interpreter) -- and documents why the method has no
-    well-defined oracle at the north-star tolerances: the reference's analytic Jacobian C of constraints 4..12 is not
-    the derivative of its g (the minors are taken as if reshape([..],3,3) stacked the vectors as columns; MATLAB stacks
-    them as rows), and the 39 x 39 KKT matrix is rank deficient (12 constraints of rank 9) with pinv keeping the
-    1e-12-shifted singular values.  Two LAPACK-based executions of the same .m text then differ by ~1e-5 in T."""
-    from oracle.gauss_helmert_port import constrGH_FaugPapa, FaugPapaTFTPoseEstimation
-    from oracle.mini_matlab import reference_interpreter
-    I = reference_interpreter(REFERENCE, rng_factory=o.SceneRNG)
-    loc = I.load("FaugPapaTFTPoseEstimation")[1]
+def test_faugpapa_constraint_jacobian_is_not_the_derivative():
+    """SURVEY 8 f4, second step (FaugPapaTFTPoseEstimation): why the method has no well-defined oracle at the north-star
+    tolerances.  The analytic Jacobian C of constraints 4..12 in the restated constrGH is not the derivative of its g
+    (the minors are taken as if reshape([..],3,3) stacked the vectors as columns; MATLAB stacks them as rows), and the
+    39 x 39 KKT matrix is rank deficient (12 constraints of rank 9) with pinv keeping the 1e-12-shifted singular
+    values.  Two LAPACK-based executions of the same .m text then differ by ~1e-5 in T (DESIGN.md 8)."""
+    from oracle.gauss_helmert_port import constrGH_FaugPapa
     rs = np.random.RandomState(1)
     obs = rs.standard_normal(30); x = rs.standard_normal(27)
-    ref = I.call("constrGH", [obs.reshape(-1, 1).copy(), x.reshape(-1, 1).copy(), np.zeros((0, 1))], 6, loc)
     got = constrGH_FaugPapa(obs, x)
-    for r, g in zip(ref[:5], got[:5]):
-        assert np.abs(np.asarray(r).reshape(np.asarray(g).shape) - g).max() < 1e-12
     eps = 1e-6
     Cfd = np.stack([(constrGH_FaugPapa(obs, x + eps * e)[1] - constrGH_FaugPapa(obs, x - eps * e)[1]) / (2 * eps)
                     for e in np.eye(27)], axis=1)
     assert np.abs(Cfd[:3] - got[4][:3]).max() < 1e-6            # det(T_i) rows: consistent
     assert np.abs(Cfd[3:] - got[4][3:]).max() > 1e-2            # rows 4..12: NOT the Jacobian of g
-    CalM, _, C, _ = o.experiments_subsample(20, 2.25, 1)
-    a = I.call("FaugPapaTFTPoseEstimation", [C.copy(), CalM.copy()], 5)
-    b = FaugPapaTFTPoseEstimation(C, CalM)
-    assert rel_frob_up_to_sign(a[3], b[3]) < 1e-3               # same method ...
-    # ... but not reproducible to 1e-9 between two float64/LAPACK executions -> no parity target (DESIGN.md 8)
 
 
 def test_matlab_pinv_definition():
@@ -100,76 +95,6 @@ def test_matlab_pinv_definition():
     D = np.diag([4.0, 1e-18, 2.0])
     assert np.array_equal(o.matlab_pinv(D), np.diag([0.25, 0.0, 0.5]))     # entries below max(size)*eps(norm) vanish
     assert o.matlab_pinv(np.zeros((0, 3))).shape == (3, 0)
-
-
-@pytest.mark.skipif(not HAVE_REF, reason="reference sources not present on this box")
-def test_interpreter_live_small_functions():
-    from oracle.mini_matlab import reference_interpreter, Cell, MatlabError
-    I = reference_interpreter(REFERENCE, rng_factory=o.SceneRNG)
-    f = lambda x: np.array([[float(x)]])
-    rs = np.random.RandomState(3)
-    # generateSyntheticScene.m (matrix products there are BLAS-ordered: projections agree to rounding only)
-    CalM, R_t, C, X = I.call("generateSyntheticScene", [f(60), f(2), f(5), f(50), f(0)], 4)
-    a = o.generateSyntheticScene(60, 2, 5, 50, 0)
-    assert np.array_equal(CalM, a[0]) and np.array_equal(X, a[3])
-    assert np.abs(C - a[2]).max() < 1e-10 and max(np.abs(R_t[i] - a[1][i]).max() for i in range(2)) < 1e-13
-    # collinear-centres branch (angle in [70,180])
-    CalM2, R_t2, C2, _ = I.call("generateSyntheticScene", [f(30), f(0), f(2), f(100), f(175)], 4)
-    b = o.generateSyntheticScene(30, 0, 2, 100, 175)
-    assert np.abs(C2 - b[2]).max() < 1e-9 and max(np.abs(R_t2[i] - b[1][i]).max() for i in range(2)) < 1e-12
-    # Normalize2Ddata, transform_TFT (both directions), TFT_from_P, crossM, project3Dpoints
-    p, N = I.call("Normalize2Ddata", [C[0:2]], 2)
-    po, No = o.Normalize2Ddata(C[0:2])
-    assert np.abs(p - po).max() < 1e-14 and np.abs(N - No).max() < 1e-15 * np.abs(No).max() + 1e-18
-    T = rs.standard_normal((3, 3, 3)); Ms = [rs.standard_normal((3, 3)) + 2 * np.eye(3) for _ in range(3)]
-    for inv in (0, 1):
-        assert np.abs(I.call("transform_TFT", [T] + Ms + [f(inv)], 1)[0] - o.transform_TFT(T, *Ms, inv)).max() < 1e-14
-    assert np.abs(I.call("transform_TFT", [T] + Ms, 1)[0] - o.transform_TFT(T, *Ms, 0)).max() < 1e-14   # nargin<5
-    K = a[0][:3]
-    Ps = [K @ np.eye(3, 4), K @ a[1][0], K @ a[1][1]]
-    assert np.abs(I.call("TFT_from_P", Ps, 1)[0] - o.TFT_from_P(*Ps)).max() < 1e-14
-    assert np.array_equal(I.call("crossM", [np.array([[1.0], [2.0], [3.0]])], 1)[0], o.crossM([1, 2, 3]))
-    Xe = a[3]
-    assert np.abs(I.call("project3Dpoints", [Xe, Cell(Ps)], 1)[0] - o.project3Dpoints(Xe, Ps)).max() < 1e-9
-    # linearTFT with all four outputs, 2xN and 3xN inputs
-    xs = [o.Normalize2Ddata(a[2][2 * v:2 * v + 2])[0] for v in range(3)]
-    r = I.call("linearTFT", xs, 4)
-    ro = o.linearTFT(*xs)
-    for x, y in zip(r, ro):
-        assert np.abs(x - y).max() < 1e-10
-    hs = [np.vstack([x * 2.0, 2.0 * np.ones((1, x.shape[1]))]) for x in xs]
-    assert np.abs(I.call("linearTFT", hs, 1)[0] - ro[0]).max() < 1e-10
-    # linearF and its error text (linearF.m:35-37)
-    assert rel_frob_up_to_sign(I.call("linearF", [a[2][0:2], a[2][2:4]], 1)[0], o.linearF(a[2][0:2], a[2][2:4])) < 1e-12
-    with pytest.raises(MatlabError, match="At least 8 correspondences are necessary"):
-        I.call("linearF", [a[2][0:2, :7], a[2][2:4, :7]], 1)
-    # triangulation3D + ReprError (with / without 3-D points), AngError
-    X4 = I.call("triangulation3D", [Cell(Ps), a[2]], 1)[0]
-    assert np.abs(np.abs(X4) - np.abs(o.triangulation3D(Ps, a[2]))).max() < 1e-12
-    for pts in ([X4[:3] / X4[3]], [X4], []):
-        assert abs(I.call("ReprError", [Cell(Ps), a[2]] + pts, 1)[0].item() - o.ReprError(Ps, a[2], *pts)) < 1e-11
-    R2, R3 = o.LinearTFTPoseEstimation(a[2], a[0])[:2]
-    ri, ti = I.call("AngError", [a[1][0], R2], 2)
-    ro_, to_ = o.AngError(a[1][0], R2)
-    assert abs(ri.item() - ro_) < 1e-10 and abs(ti.item() - to_) < 1e-10
-    # R_t_from_TFT with the oracle's tensor
-    To = o.LinearTFTPoseEstimation(a[2], a[0])[3]
-    g2, g3 = I.call("R_t_from_TFT", [To, a[0], a[2]], 2)
-    o2, o3 = o.R_t_from_TFT(To, a[0], a[2])
-    assert np.abs(g2 - o2).max() < 1e-12 and np.abs(g3 - o3).max() < 1e-11
-
-
-@pytest.mark.skipif(not HAVE_REF, reason="reference sources not present on this box")
-def test_interpreter_live_pose_methods():
-    from oracle.mini_matlab import reference_interpreter
-    I = reference_interpreter(REFERENCE, rng_factory=o.SceneRNG)
-    for n, noise, seed in ((12, 0.5, 3), (20, 3.0, 11), (33, 1.0, 2)):
-        CalM, _, C, _ = o.experiments_subsample(n, noise, seed)
-        for method, fn in (("tft", "LinearTFTPoseEstimation"), ("f", "LinearFPoseEstimation")):
-            r = I.call(fn, [C.copy(), CalM.copy()], 5)
-            got = _run_oracle(method, C, CalM)
-            for x, y in zip(r[:4], got[:4]):
-                assert np.max(np.abs(np.asarray(x) - y)) <= 1e-9 * max(1.0, np.max(np.abs(y)))
 
 
 def test_epfl_all_triplets_golden_is_pinned_by_the_reference_sources():
@@ -192,24 +117,6 @@ def test_epfl_all_triplets_golden_is_pinned_by_the_reference_sources():
         assert rel_frob_up_to_sign(o.LinearTFTPoseEstimation(C, CalM)[3], g["tft_T"][b]) < 1e-12
         tv, fv = oracle_votes(C, CalM)
         assert votes8_equal(tv, g["tft_votes"][b]) and votes8_equal(fv, g["f_votes"][b])      # labels: see conftest
-
-
-@pytest.mark.skipif(not HAVE_REF, reason="reference data not present on this box")
-def test_epfl_inputs_fixture_equals_the_reference_data_files():
-    """tests/golden/epfl_inputs.npz is the reference's own data (match lists, cameras, indexes_sorted), bit for bit."""
-    inp = np.load(os.path.join(GOLDEN, "epfl_inputs.npz"))
-    for ds, ntrip in (("fountain-P11", 70), ("Herz-Jesu-P8", 50)):
-        key = ds.replace("-", "_")
-        path = os.path.join(REFERENCE, "Data", ds)
-        idx, cor, names = o.load_corresp_triplets(path)
-        assert np.array_equal(inp[key + "_indexes_sorted"], idx[:ntrip])
-        for it in (1, 2, ntrip // 2, ntrip):
-            im = [int(v) for v in idx[it - 1, :3]]
-            lo, hi = inp[key + "_offsets"][it - 1], inp[key + "_offsets"][it]
-            assert np.array_equal(inp[key + "_matches"][lo:hi], np.asarray(cor[im[0] - 1, im[1] - 1, im[2] - 1], dtype=np.float64))
-        for k, nm in enumerate(names):
-            K, R, t, _ = o.readCalibrationOrientation_EPFL(path, nm)
-            assert np.array_equal(K, inp[key + "_K"][k]) and np.array_equal(R, inp[key + "_R"][k]) and np.array_equal(t, inp[key + "_t"][k])
 
 
 @pytest.mark.parametrize("name", ["sweep_n20.npz", "example_n100.npz", "epfl_triplets.npz"])

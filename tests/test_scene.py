@@ -47,14 +47,11 @@ def test_sweep_batch_workers_identical():
     assert np.array_equal(a["Corresp"], b["Corresp"])
 
 
-def test_epfl_loaders_match_oracle():
-    """Product-side .camera / .mat loaders == oracle restatement (skipped where the reference data is absent)."""
+def test_epfl_loaders_match_oracle(epfl_data):
+    """Product-side .camera / .mat loaders == oracle restatement, on files in the reference's format."""
     import os
-    from conftest import REFERENCE
-    if not os.path.isdir(REFERENCE):
-        pytest.skip("reference data not present on this box")
     from tft_vs_fund_b200 import epfl
-    path = os.path.join(REFERENCE, "Data", "Herz-Jesu-P8")
+    path = os.path.join(epfl_data, "Herz-Jesu-P8")
     a = epfl.load_corresp_triplets(path); b = o.load_corresp_triplets(path)
     assert np.array_equal(a[0], b[0]) and a[2] == b[2]
     for name in a[2][:3]:
