@@ -47,6 +47,7 @@ typedef struct tvf_context* tvf_handle_t;
 #define TVF_ST_NO_POSE_2 4     /* all 4 cheirality votes < 0 or NaN: MATLAB leaves R_f undefined (:91-104)    */
 #define TVF_ST_NO_POSE_3 8
 #define TVF_ST_NONFINITE 16    /* non-finite value in R_t / reprojection error                                */
+#define TVF_ST_BA_NOCONV 32    /* tvf_bundle_adjust: iteration cap reached before the stopping rule held          */
 
 /* the message linearF.m:36 raises; gateways re-raise it verbatim */
 #define TVF_LINEARF_ERRMSG \
@@ -196,6 +197,41 @@ int tvf_project3d(tvf_handle_t h, const double* points3d, const double* P, int M
  * Rt_true 3x4 (true_batched = 0) or 3x4xB. */
 int tvf_ang_error(tvf_handle_t h, const double* Rt_true, int true_batched, const double* Rt_est, int64_t B,
                   double* rot_err, double* t_err);
+
+/* ---- bundle adjustment of the three-view poses ------------------------------------------------------------------
+ * Minimises  sum over views m = 1..3 and points i of |pi(K_m (R_m X_i + t_m)) - x_{m,i}|^2  (pixels, no data
+ * normalisation; = 3n ReprError^2, auxiliar_functions/ReprError.m:65) over R2, t2, R3, t3 and the points, with camera 1
+ * fixed at K1[I|0] and the scale gauge |t2| = 1 (11 + 3n unknowns).  A start with |t2| != 1 is first scaled by 1/|t2|
+ * (t2, t3 and the points; the reprojection is unchanged).  This is NOT the reference's BundleAdjustment.m, whose source
+ * is not available to check: it normalises the image data first (Normalize2Ddata), which may weight the views
+ * differently and then has another minimiser (DESIGN.md section 8).
+ *
+ * Inputs per problem: corresp 6 x n, calm 9 x 3 (calm_batched = 0: shared) or 9 x 3 x B, the start poses Rt2_0, Rt3_0
+ * (3 x 4 x B) and optionally reconst0 (3 x n x B, Euclidean); reconst0 = NULL triangulates the start points with
+ * triangulation3D({K1[I|0], K2 Rt2_0, K3 Rt3_0}, corresp), as the pose methods compute Reconst.  n < 4 -> TVF_ERR_ARG.
+ * Outputs: Rt2, Rt3 (required), reconst (3 x n x B, Euclidean), repr_err = ReprError of the result, iter = number of
+ * linearisations, status (each may be NULL).  Outputs must not overlap inputs.
+ *
+ * Solver: Levenberg-Marquardt, one warp per problem, the points eliminated by the Schur complement (11 x 11 reduced
+ * camera system, Cholesky).  Local chart at every iterate: R <- exp([w]x) R for R2 and R3, t2 moved in its tangent
+ * plane and renormalised, t3 and the points additively.  Damping H + mu diag(H), mu_0 = 1e-3; an accepted step (gain
+ * ratio rho) sets mu *= max(1/3, 1 - (2 rho - 1)^3), nu = 2; a rejected step (cost not lower, or a damped system that
+ * is not positive definite) sets mu *= nu, nu *= 2 and re-solves at the same linearisation.  Only steps that lower the
+ * cost are accepted, so repr_err never exceeds the start's.  Stops with status 0 when
+ *   |g|_inf <= 1e-12 |g_start|_inf (g = J'r over all 11 + 3n unknowns), or
+ *   |step|_2 <= 1e-12 sqrt(sum |X_i|^2 + |t3|^2 + 1), or
+ *   an accepted step lowered the cost by at most 1e-15 of it;
+ * TVF_ST_BA_NOCONV after 100 linearisations or 400 damped solves without that.  A non-finite input, start point or
+ * start cost, or |t2| = 0, gives TVF_ST_NONFINITE with the inputs copied through (reconst = the start points) and
+ * iter = 0.  Every sum and test depends on the problem alone: a result is bit-identical whatever its batch, chunk
+ * (tvf_set_chunk) or shard.  The host form runs in chunks and shards B over a group handle like tvf_pose; the _dev form
+ * takes device pointers (corresp 16-byte aligned) and is asynchronous on the handle's stream. */
+int tvf_bundle_adjust(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
+                      const double* Rt2_0, const double* Rt3_0, const double* reconst0, double* Rt2, double* Rt3,
+                      double* reconst, double* repr_err, int32_t* iter, int32_t* status);
+int tvf_bundle_adjust_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
+                          const double* Rt2_0, const double* Rt3_0, const double* reconst0, double* Rt2, double* Rt3,
+                          double* reconst, double* repr_err, int32_t* iter, int32_t* status);
 
 /* ---- inputs of the measured configurations, generated where they are consumed ------------------------
  * Trials [first_trial, first_trial+B) of experiments.m's sweep: trial j uses noise_levels[j mod L] and

@@ -1,0 +1,312 @@
+"""tvf_bundle_adjust on the GPU against the CPU oracle (oracle/bundle_adjust.py), its invariances and its edge cases."""
+import ctypes as C
+import os
+
+import numpy as np
+import pytest
+from scipy.spatial.transform import Rotation
+
+import oracle as o
+from oracle import bundle_adjust as oba
+from conftest import ROOT, rot_angle, vec_angle
+
+pytestmark = pytest.mark.gpu
+
+TOL_ANG = 1e-6       # rad, R and t directions
+TOL_REL = 1e-7       # |t3| and Reconst, relative
+TOL_REPR = 1e-8      # px
+
+
+def golden(name):
+    return np.load(os.path.join(ROOT, "tests", "golden", name))
+
+
+def start_repr(Cr, CalM, Rt2, Rt3, X):
+    Ks = [CalM[0:3], CalM[3:6], CalM[6:9]]
+    return oba.repr_error(Ks, Rt2[:, :3], Rt2[:, 3], Rt3[:, :3], Rt3[:, 3], X, Cr)
+
+
+def check_against_oracle(tvf, Cr, CalM, Rt2, Rt3, X, label):
+    """Batch (B,6,n) through the library, each problem with a start ReprError below 10 px through the oracle."""
+    res = tvf.bundle_adjust(Cr, CalM, Rt2, Rt3, X)
+    checked = 0
+    for b in range(Cr.shape[0]):
+        cb = CalM if CalM.ndim == 2 else CalM[b]
+        if not start_repr(Cr[b], cb, Rt2[b], Rt3[b], X[b]) < 10.0:
+            continue
+        r2, r3, rX, rep = oba.bundle_adjust(Cr[b], cb, Rt2[b], Rt3[b], X[b])
+        g2, g3, gX = res[0][b], res[1][b], res[2][b]
+        tag = "%s problem %d" % (label, b)
+        assert res.status[b] == 0, tag
+        for a, c in ((r2, g2), (r3, g3)):
+            assert rot_angle(a[:, :3], c[:, :3]) < TOL_ANG, tag
+            assert vec_angle(a[:, 3], c[:, 3]) < TOL_ANG, tag
+        assert abs(np.linalg.norm(g2[:, 3]) - 1.0) < 1e-14, tag
+        assert abs(np.linalg.norm(g3[:, 3]) - np.linalg.norm(r3[:, 3])) <= TOL_REL * np.linalg.norm(r3[:, 3]), tag
+        assert np.abs(gX - rX).max() <= TOL_REL * np.abs(rX).max(), tag
+        assert abs(res.repr_err[b] - rep) <= TOL_REPR, (tag, res.repr_err[b], rep)
+        checked += 1
+    return res, checked
+
+
+def library_starts(tvf, Cr, CalM, method):
+    fn = tvf.LinearTFTPoseEstimation if method == 1 else tvf.LinearFPoseEstimation
+    r = fn(Cr, CalM)
+    return r[0], r[1], r[2], r
+
+
+@pytest.mark.parametrize("method", [1, 7])
+def test_matches_oracle_on_the_sweep_trials(tvf, method):
+    g = golden("sweep_n20.npz")
+    Cr, CalM = g["Corresp"], g["CalM"]
+    Rt2, Rt3, X, _ = library_starts(tvf, Cr, CalM, method)
+    res, checked = check_against_oracle(tvf, Cr, CalM, Rt2, Rt3, X, "sweep method %d" % method)
+    print("method %d: %d of 260 sweep trials compared with the oracle; iter mean %.1f max %d"
+          % (method, checked, np.mean(res[3]), np.max(res[3])))
+    assert checked >= 80
+
+
+@pytest.mark.parametrize("name", ["example_n100.npz", "epfl_triplets.npz"])
+def test_matches_oracle_on_example_and_epfl(tvf, name):
+    g = golden(name)
+    Cr, CalM = g["Corresp"], g["CalM"]
+    for method in (1, 7):
+        Rt2, Rt3, X, _ = library_starts(tvf, Cr, CalM, method)
+        _, checked = check_against_oracle(tvf, Cr, CalM, Rt2, Rt3, X, "%s method %d" % (name, method))
+        assert checked >= 1
+
+
+def noisy_scene(n, seed, noise=1.0):
+    CalM, R_t0, Cr, _ = o.experiments_subsample(n, noise, seed)
+    return CalM, R_t0, Cr
+
+
+def truth_start(CalM, R_t0, Cr, rs, rot=2e-3, rel=2e-3):
+    """The true poses (|t2| = 1) and their triangulated points, perturbed."""
+    K = CalM[:3]
+    Xh = o.triangulation3D([K @ np.eye(3, 4), K @ R_t0[0], K @ R_t0[1]], Cr)
+    s = 1.0 / np.linalg.norm(R_t0[0][:, 3])
+    dR = lambda: Rotation.from_rotvec(rs.standard_normal(3) * rot / np.sqrt(3)).as_matrix()
+    Rt2 = np.column_stack([dR() @ R_t0[0][:, :3], R_t0[0][:, 3] * s + rel * rs.standard_normal(3)])
+    Rt3 = np.column_stack([dR() @ R_t0[1][:, :3], R_t0[1][:, 3] * s * (1 + rel * rs.standard_normal(3))])
+    X = Xh[:3] / Xh[3] * s
+    return Rt2, Rt3, X * (1 + rel * rs.standard_normal(X.shape))
+
+
+@pytest.mark.parametrize("n", [4, 7, 20, 33, 100, 500])
+def test_matches_oracle_at_several_sizes(tvf, n):
+    rs = np.random.RandomState(n)
+    seeds = (1, 2) if n <= 100 else (1,)
+    Cs, Ms, S2, S3, SX = [], [], [], [], []
+    for seed in seeds:
+        CalM, R_t0, Cr = noisy_scene(n, seed)
+        starts = [truth_start(CalM, R_t0, Cr, rs)]
+        if n >= 8:
+            r = tvf.LinearTFTPoseEstimation(Cr, CalM)
+            starts.append((r[0], r[1], r[2]))
+        for s2, s3, sx in starts:
+            Cs.append(Cr); Ms.append(CalM); S2.append(s2); S3.append(s3); SX.append(sx)
+    _, checked = check_against_oracle(tvf, np.stack(Cs), np.stack(Ms), np.stack(S2), np.stack(S3), np.stack(SX), "n=%d" % n)
+    assert checked >= 1
+
+
+def test_large_batch_properties(tvf):
+    """1e5 device-generated trials at n = 20 from method-1 starts: ReprError never rises; the oracle's gradient at
+    the result is <= 1e-6 of its value at the start wherever the solver did not hit its cap."""
+    B, n = 100000, 20
+    d = tvf.scene.sweep_batch_device(B, n)
+    Cr, CalM = d["Corresp"], d["CalM"]
+    start = tvf.LinearTFTPoseEstimation(Cr, CalM)
+    res = tvf.bundle_adjust(Cr, CalM, start[0], start[1], start[2])
+    st = np.asarray(res.status)
+    finite = (st & tvf._lib.ST_NONFINITE) == 0
+    assert np.all(res.repr_err[finite] <= start.repr_err[finite] * (1 + 1e-12) + 1e-300)
+    g0 = np.abs(oba.gradient_batch(Cr, CalM, start[0], start[1], start[2])).max(1)
+    g1 = np.abs(oba.gradient_batch(Cr, CalM, res[0], res[1], res[2])).max(1)
+    # a noise-free trial's start (every 13th: noise level 0) is already the minimiser to rounding (ReprError ~1e-12 px):
+    # its gradient is rounding noise before and after, and the ratio says nothing; those are held to "never rises" only
+    conv = (st == 0) & (start.repr_err > 1e-9)
+    worst = np.max(g1[conv] / g0[conv])
+    print("1e5 trials, n = 20: %d NONFINITE, %d BA_NOCONV, %d starts already at the minimum; iter mean %.2f max %d; "
+          "worst gradient ratio %.2e" % (int(np.sum(~finite)), int(np.sum((st & tvf._lib.ST_BA_NOCONV) != 0)),
+                                          int(np.sum(start.repr_err <= 1e-9)), np.mean(res[3]), np.max(res[3]), worst))
+    assert worst <= 1e-6
+
+
+def test_perturbed_ground_truth_returns_the_ground_truth(tvf):
+    rs = np.random.RandomState(11)
+    for seed in (1, 2, 3):
+        CalM, R_t0, Cr = noisy_scene(20, seed, noise=0.0)
+        K = CalM[:3]
+        Xh = o.triangulation3D([K @ np.eye(3, 4), K @ R_t0[0], K @ R_t0[1]], Cr)
+        s = 1.0 / np.linalg.norm(R_t0[0][:, 3])
+        X = Xh[:3] / Xh[3] * s
+        dR = lambda: Rotation.from_rotvec(rs.standard_normal(3) * 1e-3 / np.sqrt(3)).as_matrix()
+        Rt2 = np.column_stack([dR() @ R_t0[0][:, :3], R_t0[0][:, 3] * s])
+        Rt3 = np.column_stack([dR() @ R_t0[1][:, :3], R_t0[1][:, 3] * s])
+        res = tvf.bundle_adjust(Cr, CalM, Rt2, Rt3, X)
+        assert res.status == 0 and res.repr_err < 1e-9, (seed, res.repr_err)
+        for true, got in ((R_t0[0], res[0]), (R_t0[1], res[1])):
+            assert rot_angle(true[:, :3], got[:, :3]) < 1e-9 and vec_angle(true[:, 3], got[:, 3]) < 1e-9
+        assert abs(np.linalg.norm(res[1][:, 3]) - np.linalg.norm(R_t0[1][:, 3]) * s) < 1e-9 * np.linalg.norm(res[1][:, 3])
+        assert np.abs(res[2] - X).max() < 1e-9 * np.abs(X).max()
+
+
+def test_start_with_t2_of_norm_5_gives_the_normalised_answer(tvf):
+    g = golden("sweep_n20.npz")
+    b = 30
+    Cr, CalM = g["Corresp"][b], g["CalM"][b]
+    Rt2, Rt3, X = g["tft_Rt2"][b], g["tft_Rt3"][b], g["tft_Reconst"][b]
+    ref = tvf.bundle_adjust(Cr, CalM, Rt2, Rt3, X)
+    big = tvf.bundle_adjust(Cr, CalM, np.column_stack([Rt2[:, :3], 5 * Rt2[:, 3]]), np.column_stack([Rt3[:, :3], 5 * Rt3[:, 3]]), 5 * X)
+    assert abs(np.linalg.norm(big[0][:, 3]) - 1.0) < 1e-14
+    for a, c in ((ref[0], big[0]), (ref[1], big[1])):
+        assert rot_angle(a[:, :3], c[:, :3]) < 1e-9 and vec_angle(a[:, 3], c[:, 3]) < 1e-9
+    assert abs(np.linalg.norm(big[1][:, 3]) / np.linalg.norm(ref[1][:, 3]) - 1) < 1e-9
+    assert np.abs(big[2] - ref[2]).max() < 1e-9 * np.abs(ref[2]).max()
+    assert abs(big.repr_err - ref.repr_err) < 1e-10
+
+
+def _bits_equal(a, b):
+    return all(np.array_equal(np.asarray(x), np.asarray(y)) for x, y in zip(a, b))
+
+
+def test_bit_identity_across_batch_chunk_group_and_device_pointers(tvf):
+    import torch
+    from tft_vs_fund_b200 import _lib
+    g = golden("sweep_n20.npz")
+    Cr, CalM = g["Corresp"][:60], g["CalM"][:60]
+    Rt2, Rt3, X = g["f_Rt2"][:60], g["f_Rt3"][:60], g["f_Reconst"][:60]
+    full = tvf.bundle_adjust(Cr, CalM, Rt2, Rt3, X)
+    outs = lambda r: (r[0], r[1], r[2], r[3], r.repr_err, r.status)
+    # a batch of one == its element in the larger batch
+    for b in (0, 17, 59):
+        one = tvf.bundle_adjust(Cr[b:b + 1], CalM[b:b + 1], Rt2[b:b + 1], Rt3[b:b + 1], X[b:b + 1])
+        assert _bits_equal([x[b:b + 1] for x in outs(full)], outs(one)), b
+    # chunk size
+    h = _lib.handle()
+    try:
+        h.call("tvf_set_chunk", 7)
+        chunked = tvf.bundle_adjust(Cr, CalM, Rt2, Rt3, X)
+    finally:
+        h.call("tvf_set_chunk", 0)
+    assert _bits_equal(outs(full), outs(chunked))
+    # group handle with two members on one GPU
+    grouped = tvf.api.bundle_adjust(Cr, CalM, Rt2, Rt3, X, device=(0, 0))
+    assert _bits_equal(outs(full), outs(grouped))
+    # _dev == host
+    dev = torch.device("cuda", 0)
+    cm = lambda a, nd: torch.from_numpy(tvf.api._cm(a, nd)[0]).to(dev)
+    B, n = Cr.shape[0], Cr.shape[2]
+    d_c, d_m = cm(Cr, 2), cm(CalM, 2)
+    d_r2, d_r3, d_x = cm(Rt2, 2), cm(Rt3, 2), cm(X, 2)
+    o_r2 = torch.empty((B, 12), dtype=torch.float64, device=dev); o_r3 = torch.empty_like(o_r2)
+    o_x = torch.empty((B, 3 * n), dtype=torch.float64, device=dev); o_rep = torch.empty(B, dtype=torch.float64, device=dev)
+    o_it = torch.zeros(B, dtype=torch.int32, device=dev); o_st = torch.zeros(B, dtype=torch.int32, device=dev)
+    p = lambda t: C.c_void_p(t.data_ptr())
+    torch.cuda.synchronize()
+    h.call("tvf_bundle_adjust_dev", p(d_c), p(d_m), 1, n, B, p(d_r2), p(d_r3), p(d_x), p(o_r2), p(o_r3), p(o_x), p(o_rep),
+           p(o_it), p(o_st))
+    h.call("tvf_synchronize")
+    back = lambda t, dims: tvf.api._from_cm(t.cpu().numpy().ravel(), B, dims, True)
+    assert np.array_equal(back(o_r2, (3, 4)), full[0]) and np.array_equal(back(o_r3, (3, 4)), full[1])
+    assert np.array_equal(back(o_x, (3, n)), full[2])
+    assert np.array_equal(o_rep.cpu().numpy(), full.repr_err) and np.array_equal(o_it.cpu().numpy(), full[3])
+    assert np.array_equal(o_st.cpu().numpy(), full.status)
+
+
+def test_without_reconst0_the_points_are_triangulated(tvf):
+    g = golden("sweep_n20.npz")
+    idx = np.arange(1, 260, 20)
+    Cr, CalM = g["Corresp"][idx], g["CalM"][idx]
+    Rt2, Rt3, _, _ = library_starts(tvf, Cr, CalM, 1)
+    K = CalM[:, :3]
+    P1 = K @ np.eye(3, 4)
+    Xh = tvf.triangulation3D([P1, K @ Rt2, K @ Rt3], Cr)
+    X0 = Xh[:, :3] / Xh[:, 3:4]
+    a = tvf.bundle_adjust(Cr, CalM, Rt2, Rt3)
+    b = tvf.bundle_adjust(Cr, CalM, Rt2, Rt3, X0)
+    for k in range(len(idx)):
+        for x, y in ((a[0][k], b[0][k]), (a[1][k], b[1][k])):
+            assert rot_angle(x[:, :3], y[:, :3]) < 1e-9 and vec_angle(x[:, 3], y[:, 3]) < 1e-9, k
+        assert np.abs(a[2][k] - b[2][k]).max() < 1e-9 * np.abs(b[2][k]).max(), k
+        assert abs(a.repr_err[k] - b.repr_err[k]) < 1e-10, k
+
+
+def test_nan_problem_is_flagged_and_neighbours_unchanged(tvf):
+    g = golden("sweep_n20.npz")
+    Cr, CalM = g["Corresp"][:6].copy(), g["CalM"][:6]
+    Rt2, Rt3, X = g["tft_Rt2"][:6], g["tft_Rt3"][:6], g["tft_Reconst"][:6]
+    clean = tvf.bundle_adjust(Cr, CalM, Rt2, Rt3, X)
+    Cr[2, 3, 5] = np.nan
+    dirty = tvf.bundle_adjust(Cr, CalM, Rt2, Rt3, X)
+    assert dirty.status[2] == tvf._lib.ST_NONFINITE and dirty[3][2] == 0
+    assert np.array_equal(dirty[0][2], Rt2[2]) and np.array_equal(dirty[1][2], Rt3[2]) and np.array_equal(dirty[2][2], X[2])
+    keep = [0, 1, 3, 4, 5]
+    for a, b in zip((clean[0], clean[1], clean[2], clean[3], clean.repr_err, clean.status),
+                    (dirty[0], dirty[1], dirty[2], dirty[3], dirty.repr_err, dirty.status)):
+        assert np.array_equal(np.asarray(a)[keep], np.asarray(b)[keep])
+    # |t2| = 0 is flagged the same way
+    z = Rt2.copy(); z[4, :, 3] = 0.0
+    res = tvf.bundle_adjust(g["Corresp"][:6], CalM, z, Rt3, X)
+    assert res.status[4] == tvf._lib.ST_NONFINITE and res[3][4] == 0
+
+
+def test_n3_is_an_argument_error(tvf):
+    from tft_vs_fund_b200 import _lib
+    h = _lib.handle()
+    n, B = 3, 1
+    c = np.zeros(6 * n); m = np.tile(np.eye(3), (3, 1)).T.copy(); r = np.zeros(12); x = np.zeros(3 * n)
+    dp = lambda a: a.ctypes.data_as(_lib.c_double_p)
+    rc = h.lib.tvf_bundle_adjust(h._h, dp(c), dp(m), 0, n, B, dp(r), dp(r), None, dp(r.copy()), dp(r.copy()), None, None,
+                                 None, None)
+    assert rc == _lib.TVF_ERR_ARG
+    with pytest.raises(_lib.TvfError):
+        tvf.bundle_adjust(np.zeros((6, 3)), np.tile(np.eye(3), (3, 1)), np.eye(3, 4), np.eye(3, 4))
+
+
+def test_api_single_problem_and_batch(tvf):
+    g = golden("sweep_n20.npz")
+    Cr, CalM = g["Corresp"][:5], g["CalM"][0]
+    Rt2, Rt3, X = g["tft_Rt2"][:5], g["tft_Rt3"][:5], g["tft_Reconst"][:5]
+    batch = tvf.bundle_adjust(Cr, CalM, Rt2, Rt3, X)
+    assert batch[0].shape == (5, 3, 4) and batch[2].shape == (5, 3, 20) and batch.repr_err.shape == (5,)
+    one = tvf.bundle_adjust(Cr[3], CalM, Rt2[3], Rt3[3], X[3])
+    assert one[0].shape == (3, 4) and one[2].shape == (3, 20)
+    assert isinstance(one[3], int) and isinstance(one.repr_err, float) and isinstance(one.status, int)
+    assert np.array_equal(one[0], batch[0][3]) and np.array_equal(one[2], batch[2][3]) and one.repr_err == batch.repr_err[3]
+
+
+def test_run_sweep_with_bundle_adjust_matches_a_host_loop(tvf):
+    from tft_vs_fund_b200 import experiments, scene
+    total, L = 52, 13
+    out = experiments.run_sweep(total, n=20, methods=(1, 7), bundle_adjust=True)
+    plain = experiments.run_sweep(total, n=20, methods=(1, 7))
+    d = scene.sweep_batch(total, 20)
+    lvl = np.arange(total) % L
+    for m, fn in ((1, tvf.LinearTFTPoseEstimation), (7, tvf.LinearFPoseEstimation)):
+        assert out[m].shape == (L, 6) and np.array_equal(out[m][:, :3], plain[m])
+        sums = np.zeros((L, 3)); cnt = np.zeros(L)
+        for j in range(total):
+            r = fn(d["Corresp"][j], d["CalM"])
+            ba = tvf.bundle_adjust(d["Corresp"][j], d["CalM"], r[0], r[1], r[2])
+            r2, t2 = tvf.AngError(d["R_t0"][0], ba[0]); r3, t3 = tvf.AngError(d["R_t0"][1], ba[1])
+            sums[lvl[j]] += [ba.repr_err, (r2 + r3) / 2, (t2 + t3) / 2]; cnt[lvl[j]] += 1
+        assert np.allclose(out[m][:, 3:], sums / cnt[:, None], rtol=1e-12, atol=1e-14), m
+
+
+def test_n5000_properties(tvf):
+    CalM, R_t0, Cr = noisy_scene(5000, 1)
+    start = tvf.LinearTFTPoseEstimation(Cr, CalM)
+    res = tvf.bundle_adjust(Cr, CalM, start[0], start[1], start[2])
+    assert res.status == 0
+    assert res.repr_err <= start.repr_err
+    assert abs(np.linalg.norm(res[0][:, 3]) - 1.0) < 1e-14
+    for R in (res[0][:, :3], res[1][:, :3]):
+        assert np.abs(R.T @ R - np.eye(3)).max() < 1e-13
+    g0 = np.abs(oba.gradient_batch(Cr[None], CalM, start[0][None], start[1][None], start[2][None])).max()
+    g1 = np.abs(oba.gradient_batch(Cr[None], CalM, res[0][None], res[1][None], res[2][None])).max()
+    assert g1 <= 1e-6 * g0
+    rot, _ = tvf.AngError(R_t0[0], res[0])
+    assert rot < 0.1          # degrees: 5000 points at 1 px
+    print("n = 5000: ReprError %.4f -> %.4f px in %d linearisations" % (start.repr_err, res.repr_err, res[3]))

@@ -8,7 +8,7 @@ no CPU fallback; importing is cheap, the library is loaded on first use.
 from .api import (  # noqa: F401
     LinearTFTPoseEstimation, LinearFPoseEstimation, OptimFPoseEstimation, linearTFT, linearF, optimF,
     Normalize2Ddata, transform_TFT, R_t_from_TFT, TFT_from_P, triangulation3D,
-    ReprError, AngError, crossM, project3Dpoints, PoseResult,
+    ReprError, AngError, crossM, project3Dpoints, PoseResult, bundle_adjust, BundleAdjustResult,
 )
 from ._lib import TvfError, Handle, handle, load, LIB_PATH  # noqa: F401
 from .scene import generateSyntheticScene, sweep_batch, SceneRNG  # noqa: F401
@@ -17,6 +17,6 @@ from . import experiments, sharding, epfl  # noqa: F401
 __all__ = [
     "LinearTFTPoseEstimation", "LinearFPoseEstimation", "OptimFPoseEstimation", "linearTFT", "linearF", "optimF",
     "Normalize2Ddata", "transform_TFT", "R_t_from_TFT", "TFT_from_P",
-    "triangulation3D", "ReprError", "AngError", "crossM", "project3Dpoints",
+    "triangulation3D", "ReprError", "AngError", "crossM", "project3Dpoints", "bundle_adjust",
     "generateSyntheticScene", "sweep_batch", "Handle", "handle", "TvfError",
 ]

@@ -289,6 +289,44 @@ def AngError(R_t_true, R_t_est, device=None):
     return (rot, tr) if batched else (float(rot[0]), float(tr[0]))
 
 
+class BundleAdjustResult(tuple):
+    """(R_t_2, R_t_3, Reconst, iter) of bundle_adjust, plus .repr_err and .status."""
+    repr_err = None
+    status = None
+
+
+def bundle_adjust(Corresp, CalM, R_t_2, R_t_3, Reconst=None, device=None):
+    """Three-view bundle adjustment of a pose (tvf_bundle_adjust, include/tvf.h): minimises the pixel reprojection error
+    over R2, t2 (|t2| = 1), R3, t3 and the points, camera 1 fixed at K1[I|0], from the start (R_t_2, R_t_3, Reconst).
+    Reconst None: the start points are triangulated from the start poses.  Not the reference's BundleAdjustment.m (which
+    normalises the image data first; DESIGN.md section 8).  Returns (R_t_2, R_t_3, Reconst, iter) with .repr_err (the
+    result's ReprError) and .status (TVF_ST_* bits: NONFINITE, BA_NOCONV)."""
+    c, batched, B = _cm(Corresp, 2)
+    if c.shape[2] != 6:
+        raise ValueError("Corresp must be 6xN")
+    n = c.shape[1]
+    calm, cb = _calm(CalM, B)
+    r2, _, _ = _cm(np.broadcast_to(R_t_2, (B, 3, 4)) if batched else R_t_2, 2)
+    r3, _, _ = _cm(np.broadcast_to(R_t_3, (B, 3, 4)) if batched else R_t_3, 2)
+    x0 = None
+    if Reconst is not None:
+        x0, _, _ = _cm(Reconst, 2)
+        if x0.shape != (B, n, 3):
+            raise ValueError("Reconst must be 3xN (with the batch axis of Corresp)")
+    if r2.shape != (B, 4, 3) or r3.shape != (B, 4, 3):
+        raise ValueError("R_t_2, R_t_3 must be 3x4 (with the batch axis of Corresp)")
+    h = _lib.handle(device)
+    Rt2 = np.empty((B, 12)); Rt3 = np.empty((B, 12)); Rec = np.empty((B, 3 * n)); rep = np.empty(B)
+    its = np.zeros(B, dtype=np.int32); st = np.zeros(B, dtype=np.int32)
+    h.call("tvf_bundle_adjust", _p(c), _p(calm), cb, n, B, _p(r2), _p(r3), _p(x0), _p(Rt2), _p(Rt3), _p(Rec), _p(rep),
+           its.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
+    out = BundleAdjustResult((_from_cm(Rt2, B, (3, 4), batched), _from_cm(Rt3, B, (3, 4), batched),
+                              _from_cm(Rec, B, (3, n), batched), its if batched else int(its[0])))
+    out.repr_err = rep if batched else float(rep[0])
+    out.status = st if batched else int(st[0])
+    return out
+
+
 def crossM(v):
     """M=crossM(v) (auxiliar_functions/crossM.m:22) -- pure data placement, no arithmetic."""
     v = np.asarray(v, dtype=np.float64).ravel()

@@ -536,6 +536,172 @@ int pose_dev(tvf_handle_t h, Method method, const double* corresp, const double*
     return TVF_OK;
 }
 
+// ---- bundle adjustment (tvf_bundle_adjust[_dev]) ----------------------------------------------------------------------
+// one call's arrays (host or device pointers); outputs may be null except Rt2 / Rt3
+struct BaIo {
+    const double* corresp; const double* calm; int calm_batched; int n;
+    const double* Rt2_0; const double* Rt3_0; const double* X0;
+    double* Rt2; double* Rt3; double* X; double* repr; int32_t* iter; int32_t* status;
+    BaIo shifted(int64_t lo) const {           // problems [lo, ...)
+        BaIo s = *this;
+        s.corresp += lo * 6 * n;
+        if (calm_batched) s.calm += lo * 27;
+        s.Rt2_0 += lo * 12; s.Rt3_0 += lo * 12; s.Rt2 += lo * 12; s.Rt3 += lo * 12;
+        if (s.X0) s.X0 += lo * 3 * n;
+        if (s.X) s.X += lo * 3 * n;
+        if (s.repr) s.repr += lo;
+        if (s.iter) s.iter += lo;
+        if (s.status) s.status += lo;
+        return s;
+    }
+};
+
+int check_ba_args(tvf_handle_t h, const BaIo& io, int64_t B) {
+    if (!h) return TVF_ERR_ARG;
+    if (!io.corresp || !io.calm || !io.Rt2_0 || !io.Rt3_0 || !io.Rt2 || !io.Rt3)
+        return fail(h, TVF_ERR_ARG, "bundle_adjust: corresp, calm, Rt2_0, Rt3_0, Rt2 and Rt3 must not be NULL");
+    if (B < 0) return fail(h, TVF_ERR_ARG, "bundle_adjust: B >= 0");
+    if (io.n < 4) return fail(h, TVF_ERR_ARG, "bundle_adjust: needs n >= 4 points (11 + 3n unknowns, 6n residuals)");
+    return TVF_OK;
+}
+
+// per-problem device bytes of a chunk: host_io -> inputs and outputs too; always the two point buffers
+size_t ba_bytes_per_problem(int n, bool host_io) {
+    size_t b = (size_t)2 * 3 * n * sizeof(double);
+    if (host_io) b += (size_t)(6 * n + 27 + 24 + 3 * n + 24 + 1) * sizeof(double) + 2 * sizeof(int32_t);
+    return b;
+}
+
+int64_t pick_chunk_ba(tvf_handle_t h, int n, int64_t B, bool host_io) {
+    int64_t c = h->chunk_user > 0 ? h->chunk_user : (host_io ? DEFAULT_CHUNK : DEFAULT_CHUNK_DEV);
+    if (h->chunk_user <= 0) {
+        const int64_t fit = (int64_t)((host_io ? ARENA_BUDGET : 8 * ARENA_BUDGET) / ba_bytes_per_problem(n, host_io));
+        if (c > fit) c = fit;
+    }
+    if (c < 1) c = 1;
+    if (c > B) c = B;
+    return c;
+}
+
+// device copies of one host chunk of C problems in a slot arena (base = nullptr: size only)
+size_t carve_ba(char* base, int n, int64_t C, int calm_batched, BaIo* d, double** Xc) {
+    Carver c(base);
+    d->corresp = c.take<double>((size_t)6 * n * C); d->calm = c.take<double>(calm_batched ? 27 * C : 27);
+    d->calm_batched = calm_batched; d->n = n;
+    d->Rt2_0 = c.take<double>(12 * C); d->Rt3_0 = c.take<double>(12 * C); d->X0 = c.take<double>((size_t)3 * n * C);
+    d->Rt2 = c.take<double>(12 * C); d->Rt3 = c.take<double>(12 * C); d->X = c.take<double>((size_t)3 * n * C);
+    *Xc = c.take<double>((size_t)3 * n * C);
+    d->repr = c.take<double>(C); d->iter = c.take<int32_t>(C); d->status = c.take<int32_t>(C);
+    return c.off;
+}
+
+int ba_launch(tvf_handle_t h, cudaStream_t st, const BaIo& d, int64_t Bc, double* Xc) {
+    BaArgs a{d.corresp, d.calm, d.calm_batched, d.n, Bc, d.Rt2_0, d.Rt3_0, d.X0, d.Rt2, d.Rt3, d.X, Xc, d.repr, d.iter, d.status};
+    const int ok = launch_bundle_adjust(a, st);
+    h->launches += 1;
+    if (!ok) { cudaError_t e = cudaGetLastError(); return fail(h, TVF_ERR_CUDA, std::string("bundle_adjust_kernel: ") + cudaGetErrorString(e)); }
+    return TVF_OK;
+}
+
+int ba_host_one(tvf_handle_t h, const BaIo& io, int64_t B) {
+    if (B == 0) return TVF_OK;
+    TVF_CK(cudaSetDevice(h->device));
+    const int n = io.n;
+    const int64_t C = pick_chunk_ba(h, n, B, true);
+    std::vector<int32_t> st_tmp;
+    int32_t* st_host = io.status;
+    if (!st_host) { st_tmp.resize((size_t)B); st_host = st_tmp.data(); }
+    TVF_CK(cudaStreamSynchronize(h->slot[0].stream));
+    if (h->use_user_stream) TVF_CK(cudaStreamSynchronize(h->user_stream));
+    int64_t done = 0; int ci = 0; int rc;
+    while (done < B) {
+        const int64_t Bc = (B - done < C) ? (B - done) : C;
+        Slot& s = h->slot[ci % NSLOT];
+        TVF_CK(cudaStreamSynchronize(s.stream));            // the slot's previous chunk (with its copies back) is done
+        BaIo d{}; double* Xc;
+        rc = ensure_arena(h, s, carve_ba(nullptr, n, C, io.calm_batched, &d, &Xc)); if (rc) return rc;
+        carve_ba(s.arena, n, C, io.calm_batched, &d, &Xc);
+        double* x0 = const_cast<double*>(d.X0);
+        if (!io.X0) d.X0 = nullptr;
+        double* in = const_cast<double*>(d.corresp); double* calm = const_cast<double*>(d.calm);
+        double* r2 = const_cast<double*>(d.Rt2_0); double* r3 = const_cast<double*>(d.Rt3_0);
+        const BaIo hio = io.shifted(done);
+        auto up = [&](void* dst, const void* src, size_t bytes) { return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, s.stream); };
+        auto down = [&](void* dst, const void* src, size_t bytes) {
+            return dst ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, s.stream) : cudaSuccess;
+        };
+        TVF_CK(up(in, hio.corresp, (size_t)Bc * 6 * n * sizeof(double)));
+        TVF_CK(up(calm, hio.calm, (size_t)(io.calm_batched ? Bc * 27 : 27) * sizeof(double)));
+        TVF_CK(up(r2, hio.Rt2_0, (size_t)Bc * 12 * sizeof(double)));
+        TVF_CK(up(r3, hio.Rt3_0, (size_t)Bc * 12 * sizeof(double)));
+        if (io.X0) TVF_CK(up(x0, hio.X0, (size_t)Bc * 3 * n * sizeof(double)));
+        rc = ba_launch(h, s.stream, d, Bc, Xc); if (rc) return rc;
+        TVF_CK(down(hio.Rt2, d.Rt2, (size_t)Bc * 12 * sizeof(double)));
+        TVF_CK(down(hio.Rt3, d.Rt3, (size_t)Bc * 12 * sizeof(double)));
+        TVF_CK(down(hio.X, d.X, (size_t)Bc * 3 * n * sizeof(double)));
+        TVF_CK(down(hio.repr, d.repr, (size_t)Bc * sizeof(double)));
+        TVF_CK(down(hio.iter, d.iter, (size_t)Bc * sizeof(int32_t)));
+        TVF_CK(down(st_host + done, d.status, (size_t)Bc * sizeof(int32_t)));
+        done += Bc; ++ci;
+    }
+    for (int i = 0; i < NSLOT; ++i) TVF_CK(cudaStreamSynchronize(h->slot[i].stream));
+    return count_flagged(st_host, B);
+}
+
+// host pointers; a group handle shards B exactly as pose_host does (results bit-identical to one device)
+int ba_host(tvf_handle_t h, const BaIo& io, int64_t B) {
+    int rc = check_ba_args(h, io, B);
+    if (rc != TVF_OK) return rc;
+    if (B == 0) return TVF_OK;
+    const int G = 1 + (int)h->peers.size();
+    if (G == 1 || B < G) return ba_host_one(h, io, B);
+    std::vector<int> rcs((size_t)G, TVF_OK);
+    auto run = [&](int g) {
+        tvf_handle_t m = (g == 0) ? h : h->peers[(size_t)g - 1];
+        int64_t lo, hi; shard_of(B, g, G, &lo, &hi);
+        m->chunk_user = h->chunk_user;
+        rcs[(size_t)g] = ba_host_one(m, io.shifted(lo), hi - lo);
+    };
+    std::vector<std::thread> th;
+    for (int g = 1; g < G; ++g) th.emplace_back(run, g);
+    run(0);
+    for (auto& t : th) t.join();
+    int64_t flagged = 0;
+    for (int g = 0; g < G; ++g) {
+        if (rcs[(size_t)g] < 0) {
+            if (g > 0) h->err = "device " + std::to_string(h->peers[(size_t)g - 1]->device) + ": " + h->peers[(size_t)g - 1]->err;
+            return rcs[(size_t)g];
+        }
+        flagged += rcs[(size_t)g];
+    }
+    cudaSetDevice(h->device);
+    return (int)(flagged > 0x7fffffff ? 0x7fffffff : flagged);
+}
+
+// device pointers, asynchronous on the handle's stream
+int ba_dev(tvf_handle_t h, const BaIo& io, int64_t B) {
+    int rc = check_ba_args(h, io, B);
+    if (rc != TVF_OK) return rc;
+    if ((reinterpret_cast<uintptr_t>(io.corresp) & 15u) != 0) return fail(h, TVF_ERR_ARG, "device pointer `corresp` must be 16-byte aligned");
+    if (B == 0) return TVF_OK;
+    TVF_CK(cudaSetDevice(h->device));
+    Slot& s = h->slot[0];
+    cudaStream_t st = h->use_user_stream ? h->user_stream : s.stream;
+    const int64_t C = pick_chunk_ba(h, io.n, B, false);
+    const size_t pts = (size_t)3 * io.n * C;
+    rc = ensure_arena(h, s, 2 * pts * sizeof(double) + 512); if (rc) return rc;
+    Carver c(s.arena);
+    double* Xc = c.take<double>(pts);
+    double* Xw = c.take<double>(pts);
+    for (int64_t done = 0; done < B; done += C) {
+        const int64_t Bc = (B - done < C) ? (B - done) : C;
+        BaIo d = io.shifted(done);
+        if (!io.X) d.X = Xw;
+        rc = ba_launch(h, st, d, Bc, Xc); if (rc) return rc;
+    }
+    return TVF_OK;
+}
+
 // small helper for the stand-alone functions: upload, run, download on slot 0
 struct Up {
     tvf_handle_t h; cudaStream_t st; int rc = TVF_OK; int next = 1;
@@ -582,7 +748,7 @@ __global__ void __launch_bounds__(256) fp64_peak_kernel(double* out, int iters, 
 // =========================================================================== C ABI
 extern "C" {
 
-int tvf_version(void) { return 200; }
+int tvf_version(void) { return 201; }
 
 int tvf_device_count(void) {
     int n = 0;
@@ -1288,6 +1454,18 @@ int tvf_sweep_run_levels(tvf_handle_t h, int method, int64_t first_trial, int64_
     for (int l = 0; l < L; ++l)
         if (skipped[(size_t)l]) { table[5 * l] = inf; table[5 * l + 1] = inf; table[5 * l + 2] = inf; table[5 * l + 3] = 0.0; table[5 * l + 4] = 0.0; }
     return TVF_OK;
+}
+
+int tvf_bundle_adjust(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
+                      const double* Rt2_0, const double* Rt3_0, const double* reconst0, double* Rt2, double* Rt3,
+                      double* reconst, double* repr_err, int32_t* iter, int32_t* status) {
+    return ba_host(h, BaIo{corresp, calm, calm_batched, n, Rt2_0, Rt3_0, reconst0, Rt2, Rt3, reconst, repr_err, iter, status}, B);
+}
+
+int tvf_bundle_adjust_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
+                          const double* Rt2_0, const double* Rt3_0, const double* reconst0, double* Rt2, double* Rt3,
+                          double* reconst, double* repr_err, int32_t* iter, int32_t* status) {
+    return ba_dev(h, BaIo{corresp, calm, calm_batched, n, Rt2_0, Rt3_0, reconst0, Rt2, Rt3, reconst, repr_err, iter, status}, B);
 }
 
 int tvf_ang_error(tvf_handle_t h, const double* Rt_true, int true_batched, const double* Rt_est, int64_t B,

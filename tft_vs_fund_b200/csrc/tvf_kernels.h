@@ -45,6 +45,27 @@ int launch_optimf_gh(const double* corresp, int n, long long B, const double* ws
                      int sm_count, cudaStream_t stream);
 void launch_sum_pairs(const int* in2, long long B, int* out, cudaStream_t stream);
 
+// ---- three-view bundle adjustment (tvf_ba_kernels.cu).  Device pointers; X receives the result and holds the current
+// iterate, Xc (3 x n x B) is work space; repr_err, iter, status may be null.  Returns 0 if the launch failed.
+struct BaArgs {
+    const double* corresp;     // 6 x n x B, 16-byte aligned
+    const double* calm;        // 9 x 3 (shared) or 9 x 3 x B
+    int calm_batched;
+    int n;
+    long long B;
+    const double* Rt2_0;       // 12 x B
+    const double* Rt3_0;       // 12 x B
+    const double* X0;          // 3 x n x B, or null: triangulated from the start poses
+    double* Rt2;               // 12 x B
+    double* Rt3;               // 12 x B
+    double* X;                 // 3 x n x B
+    double* Xc;                // 3 x n x B
+    double* repr_err;          // B
+    int* iter;                 // B
+    int* status;               // B
+};
+int launch_bundle_adjust(const BaArgs& a, cudaStream_t stream);
+
 // ---- pose tail -----------------------------------------------------------------------------
 struct PoseTailArgs {
     const double* corresp;     // 6 x n x B

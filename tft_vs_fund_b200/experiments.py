@@ -38,10 +38,16 @@ def level_sums(level_idx, n_levels, *columns, bad=None):
 
 
 def run_sweep(total_trials, n=20, methods=(1, 7), noise_levels=NOISE_LEVELS, focalL=50, angle=0, device=None,
-              solver=None, workers=1):
+              solver=None, workers=1, bundle_adjust=False):
     """Sharded sweep.  Returns on rank 0 a dict method -> (n_levels, 3) array of mean [repr_err, rot_err,
     t_err] per noise level (the `(:,m,1)` slices of experiments.m:68-70), None on the other ranks.
-    `solver(method_id, Corresp, CalM)` may replace the GPU call (used by the CPU plumbing tests)."""
+    `solver(method_id, Corresp, CalM)` may replace the GPU call (used by the CPU plumbing tests).
+    bundle_adjust=True: every method's pose is then refined by api.bundle_adjust (what experiments.m:127-141 do with
+    the reference's own BundleAdjustment, which this is not: DESIGN.md section 8) and each entry is (n_levels, 6):
+    the three means above, then the same three after the adjustment.  Trials without a pose or with a non-finite
+    adjustment are left out of the adjusted means."""
+    if bundle_adjust and solver is not None:
+        raise ValueError("bundle_adjust needs the library's pose methods (solver must be None)")
     rank, size = sharding.world()
     lo, hi = sharding.shard_range(total_trials, rank, size)
     d = scene.sweep_batch(hi - lo, n, first_trial=lo, noise_levels=noise_levels, focalL=focalL, angle=angle,
@@ -59,8 +65,14 @@ def run_sweep(total_trials, n=20, methods=(1, 7), noise_levels=NOISE_LEVELS, foc
             repr_err, rot_err, t_err = evaluate(res, d["R_t0"], device=device)
             bad = (np.asarray(res.status) & (_lib.ST_NO_POSE_2 | _lib.ST_NO_POSE_3 | _lib.ST_NONFINITE)) != 0
         total = sharding.sum_in_rank_order(level_sums(level_idx, L, repr_err, rot_err, t_err, bad=bad))
+        if bundle_adjust:
+            ba = api.bundle_adjust(d["Corresp"], d["CalM"], res[0], res[1], res[2], device=device)
+            bad_ba = bad | ((np.asarray(ba.status) & _lib.ST_NONFINITE) != 0)
+            total_ba = sharding.sum_in_rank_order(level_sums(level_idx, L, *evaluate(ba, d["R_t0"], device=device), bad=bad_ba))
         if total is not None:
             out[m] = total[:, :3] / total[:, 3:4]
+            if bundle_adjust:
+                out[m] = np.hstack([out[m], total_ba[:, :3] / total_ba[:, 3:4]])
             skipped[m] = total[:, 4].astype(np.int64)
     if rank == 0:
         run_sweep.last_skipped = skipped        # trials without a pose per (method, level); all zero in the reference's sweeps
