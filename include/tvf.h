@@ -273,6 +273,19 @@ typedef struct tvf_sweep_level {
 int tvf_sweep_run_levels(tvf_handle_t h, int method, int64_t first_trial, int64_t B, const tvf_sweep_level* levels, int L,
                          double hi_x, double hi_y, double* table);
 
+/* tvf_sweep_run_levels followed, trial by trial, by the library's bundle adjustment (tvf_bundle_adjust, started from the
+ * method's R_t_2, R_t_3 and Reconst, the level's CalM shared): the two column groups of experiments.m:127-141.  Arguments,
+ * trial mapping, checks and skipped levels as tvf_sweep_run_levels.  table: L x 11 row-major =
+ *   0-4   the method, exactly as tvf_sweep_run_levels;
+ *   5-7   after adjustment: sum repr_err (the adjusted ReprError over the trial's n points), sum rot_err, sum t_err;
+ *   8     trials counted after adjustment;
+ *   9     trials skipped after adjustment (the method's pose skipped, or the adjustment TVF_ST_NONFINITE);
+ *   10    sum of the adjustment's `iter` over the trials of column 8.
+ * Trials ending with TVF_ST_BA_NOCONV are counted.  A level the reference skips gets +inf in 0-2 and 5-7, 0 elsewhere.
+ * Each trial's adjustment is bit-identical to tvf_bundle_adjust's on the same start, whatever the chunk or range. */
+int tvf_sweep_run_levels_ba(tvf_handle_t h, int method, int64_t first_trial, int64_t B, const tvf_sweep_level* levels,
+                            int L, double hi_x, double hi_y, double* table);
+
 /* ---- device-pointer forms (inputs/outputs already in HBM; asynchronous on the handle's stream,
  *      return 0 without synchronising -- read `status` after tvf_synchronize).  `corresp` must be
  *      16-byte aligned (any cudaMalloc'ed buffer, and any problem boundary inside one, is); otherwise

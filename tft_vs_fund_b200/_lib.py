@@ -87,6 +87,7 @@ SIGNATURES = {
     "tvf_generate_sweep": (_I, [_H, _L, _L, _I, _D, _I, _D, C.c_double, C.c_double, _D]),
     "tvf_sweep_run": (_I, [_H, _I, _L, _L, _I, _D, _I, _D, C.c_double, C.c_double, _D, _D, _D, _D]),
     "tvf_sweep_run_levels": (_I, [_H, _I, _L, _L, C.POINTER(SweepLevel), _I, C.c_double, C.c_double, _D]),
+    "tvf_sweep_run_levels_ba": (_I, [_H, _I, _L, _L, C.POINTER(SweepLevel), _I, C.c_double, C.c_double, _D]),
     "tvf_generate_sweep_dev": (_I, [_H, _L, _L, _I, _D, _I, _D, C.c_double, C.c_double, C.c_void_p]),
     "tvf_linear_tft_pose_dev": (_I, [_H, C.c_void_p, C.c_void_p, _I, _I, _L] + [C.c_void_p] * 6),
     "tvf_linear_f_pose_dev": (_I, [_H, C.c_void_p, C.c_void_p, _I, _I, _L] + [C.c_void_p] * 8),

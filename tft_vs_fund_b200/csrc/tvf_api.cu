@@ -127,9 +127,14 @@ struct Carver {
 struct ChunkBufs {
     double* in; double* calm; double* T; double* F; double* core; double* cand; int* votes; double* scale;
     double* Rt2; double* Rt3; double* reconst; double* repr; int* status; int* iters; int* iter_sum;
+    // ba: the bundle adjustment of the chunk's poses (tvf_sweep_run_levels_ba)
+    double* ba_Rt2; double* ba_Rt3; double* ba_X; double* ba_Xc; double* ba_repr; int* ba_iter; int* ba_status;
 };
 
-size_t carve(char* base, int n, int64_t C, bool host_io, bool calm_batched, ChunkBufs* out) {
+// per-problem bytes of the ba buffers: Rt2, Rt3, X, Xc, repr (+ iter, status in the last double)
+inline size_t ba_chunk_bytes(int n) { return (size_t)(24 + 6 * n + 3) * sizeof(double); }
+
+size_t carve(char* base, int n, int64_t C, bool host_io, bool calm_batched, bool ba, ChunkBufs* out) {
     Carver c(base);
     ChunkBufs b{};
     b.T = c.take<double>(27 * C);
@@ -149,15 +154,25 @@ size_t carve(char* base, int n, int64_t C, bool host_io, bool calm_batched, Chun
         b.reconst = c.take<double>((size_t)3 * n * C);
         b.repr = c.take<double>(C);
     }
+    if (ba) {
+        b.ba_Rt2 = c.take<double>(12 * C);
+        b.ba_Rt3 = c.take<double>(12 * C);
+        b.ba_X = c.take<double>((size_t)3 * n * C);
+        b.ba_Xc = c.take<double>((size_t)3 * n * C);
+        b.ba_repr = c.take<double>(C);
+        b.ba_iter = c.take<int>(C);
+        b.ba_status = c.take<int>(C);
+    }
     if (out) *out = b;
     return c.off;
 }
 
-int64_t pick_chunk(tvf_handle_t h, int n, int64_t B, bool host_io) {
+int64_t pick_chunk(tvf_handle_t h, int n, int64_t B, bool host_io, bool ba) {
     int64_t c = h->chunk_user > 0 ? h->chunk_user : (host_io ? DEFAULT_CHUNK : DEFAULT_CHUNK_DEV);
     if (h->chunk_user <= 0) {   // automatic: keep one slot's work space near ARENA_BUDGET
         size_t payload = (27 + 18 + CORE_WS_TFT + CAND_SIZE + 2) * 8 + 14 * 4;
         if (host_io) payload += (size_t)(6 * n + 27 + 24 + 3 * n + 1) * 8;
+        if (ba) payload += ba_chunk_bytes(n);
         const int64_t fit = (int64_t)((host_io ? ARENA_BUDGET : 8 * ARENA_BUDGET) / payload);
         if (c > fit) c = fit;
     }
@@ -326,8 +341,8 @@ int pose_host_one(tvf_handle_t h, Method method, const double* corresp, const do
                   int64_t B, const PoseOut& o) {
     if (B == 0) return TVF_OK;
     TVF_CK(cudaSetDevice(h->device));
-    const int64_t C = pick_chunk(h, n, B, true);
-    const size_t need = carve(nullptr, n, C, true, calm_batched != 0, nullptr);
+    const int64_t C = pick_chunk(h, n, B, true, false);
+    const size_t need = carve(nullptr, n, C, true, calm_batched != 0, false, nullptr);
     std::vector<int32_t> st_tmp;
     int32_t* st_host = o.status;
     if (!st_host) { st_tmp.resize((size_t)B); st_host = st_tmp.data(); }
@@ -380,7 +395,7 @@ int pose_host_one(tvf_handle_t h, Method method, const double* corresp, const do
         Slot& s = h->slot[si];
         TVF_CK(cudaStreamSynchronize(s.stream));        // slot reuse: its previous chunk (incl. D2H) is finished
         rc = ensure_arena(h, s, need); if (rc) return rc;
-        ChunkBufs b; carve(s.arena, n, C, true, calm_batched != 0, &b);
+        ChunkBufs b; carve(s.arena, n, C, true, calm_batched != 0, false, &b);
         const double* src_in = corresp + done * 6 * n;
         const double* src_calm = calm + (calm_batched ? done * 27 : 0);
         char* stage_out = nullptr;
@@ -511,11 +526,11 @@ int pose_dev(tvf_handle_t h, Method method, const double* corresp, const double*
     TVF_CK(cudaSetDevice(h->device));
     Slot& s = h->slot[0];
     cudaStream_t st = h->use_user_stream ? h->user_stream : s.stream;
-    const int64_t C = pick_chunk(h, n, B, false);
+    const int64_t C = pick_chunk(h, n, B, false, false);
     // internal buffers only; Rt2/Rt3 are needed internally by the F method's TFT_from_P, so stage them if absent
-    const size_t need = carve(nullptr, n, C, false, false, nullptr) + (size_t)(24 * C) * sizeof(double) + 512;
+    const size_t need = carve(nullptr, n, C, false, false, false, nullptr) + (size_t)(24 * C) * sizeof(double) + 512;
     rc = ensure_arena(h, s, need); if (rc) return rc;
-    ChunkBufs b; const size_t used = carve(s.arena, n, C, false, false, &b);
+    ChunkBufs b; const size_t used = carve(s.arena, n, C, false, false, false, &b);
     double* tmpRt2 = reinterpret_cast<double*>(s.arena + used);
     double* tmpRt3 = tmpRt2 + 12 * C;
     for (int64_t done = 0; done < B; done += C) {
@@ -1342,10 +1357,10 @@ int tvf_sweep_run(tvf_handle_t h, int method, int64_t first_trial, int64_t B, in
     const int Q = 512;
     // nothing crosses the bus here, so the solver runs its large device-path launches (the per-problem output buffers of
     // the host-path layout are still needed: the evaluation kernels read them)
-    const int64_t C = pick_chunk(h, n, B > 0 ? B : 1, false);
-    const size_t need = carve(nullptr, n, C, true, false, nullptr);
+    const int64_t C = pick_chunk(h, n, B > 0 ? B : 1, false, false);
+    const size_t need = carve(nullptr, n, C, true, false, false, nullptr);
     rc = ensure_arena(h, s, need); if (rc) return rc;
-    ChunkBufs b; carve(s.arena, n, C, true, false, &b);
+    ChunkBufs b; carve(s.arena, n, C, true, false, false, &b);
     void *pc, *pr, *pp, *pt;
     rc = ensure_scratch(h, 0, 27 * sizeof(double), &pc); if (rc) return rc;
     rc = ensure_scratch(h, NSCRATCH - 4, 24 * sizeof(double), &pr); if (rc) return rc;
@@ -1384,8 +1399,10 @@ int tvf_sweep_run(tvf_handle_t h, int method, int64_t first_trial, int64_t B, in
 // experiments.m:74-124 for any of its four options ('noise', 'focal', 'points', 'angle', :38-47): every level carries its
 // own noise, point count, cameras, calibration and ground truth.  Level by level: the level's trials (one per seed) are
 // generated with its cameras, solved with its n and CalM, and reduced into its row of the table -- all on the device.
-int tvf_sweep_run_levels(tvf_handle_t h, int method, int64_t first_trial, int64_t B, const tvf_sweep_level* levels, int L,
-                         double hi_x, double hi_y, double* table) {
+// ba: each chunk's poses are then bundle-adjusted (experiments.m:127-141 with the library's adjustment) and reduced into
+// columns 5-10 of an L x 11 table; without it the table is L x 5 and the chunk size, and so every sum, is unchanged.
+static int sweep_levels(tvf_handle_t h, int method, int64_t first_trial, int64_t B, const tvf_sweep_level* levels, int L,
+                        double hi_x, double hi_y, double* table, bool ba) {
     if (!h) return TVF_ERR_ARG;
     if (!levels || !table || L < 1 || B < 0 || first_trial < 0) return fail(h, TVF_ERR_ARG, "NULL argument or bad size");
     if (method != 1 && method != 7 && method != 8) return fail(h, TVF_ERR_ARG, "method must be 1 (linear TFT), 7 (linear F) or 8 (optimal F)");
@@ -1399,17 +1416,19 @@ int tvf_sweep_run_levels(tvf_handle_t h, int method, int64_t first_trial, int64_
     Slot& s = h->slot[0];
     cudaStream_t st = s.stream;
     const int Q = 512;
+    const int W = ba ? 11 : 5;                 // table columns
     const Method m = method == 1 ? METHOD_TFT : (method == 7 ? METHOD_F : METHOD_OPTF);
     const int64_t per_level = B / L + 1;
-    const int64_t C = pick_chunk(h, n_max, per_level, false);
-    const size_t need = carve(nullptr, n_max, C, true, false, nullptr);
+    const int64_t C = pick_chunk(h, n_max, per_level, false, ba);
+    const size_t need = carve(nullptr, n_max, C, true, false, ba, nullptr);
     int rc = ensure_arena(h, s, need); if (rc) return rc;
-    ChunkBufs b; carve(s.arena, n_max, C, true, false, &b);
-    void *pc, *pr, *pp, *pt, *pg;
+    ChunkBufs b; carve(s.arena, n_max, C, true, false, ba, &b);
+    void *pc, *pr, *pp, *pt, *pg, *pb = nullptr;
     rc = ensure_scratch(h, NSCRATCH - 8, (size_t)L * 27 * sizeof(double), &pc); if (rc) return rc;
     rc = ensure_scratch(h, NSCRATCH - 9, (size_t)L * 24 * sizeof(double), &pr); if (rc) return rc;
     rc = ensure_scratch(h, NSCRATCH - 5, (size_t)L * Q * 5 * sizeof(double), &pp); if (rc) return rc;
-    rc = ensure_scratch(h, NSCRATCH - 6, (size_t)L * 5 * sizeof(double), &pt); if (rc) return rc;
+    rc = ensure_scratch(h, NSCRATCH - 6, (size_t)L * W * sizeof(double), &pt); if (rc) return rc;
+    if (ba) { rc = ensure_scratch(h, NSCRATCH - 10, (size_t)L * Q * 6 * sizeof(double), &pb); if (rc) return rc; }
     const int64_t G = (per_level < 4 * C) ? per_level : 4 * C;
     rc = ensure_scratch(h, NSCRATCH - 7, (size_t)G * 6 * n_max * sizeof(double), &pg); if (rc) return rc;
     std::vector<double> hc((size_t)L * 27), hr((size_t)L * 24);
@@ -1421,7 +1440,8 @@ int tvf_sweep_run_levels(tvf_handle_t h, int method, int64_t first_trial, int64_
     TVF_CK(cudaMemcpyAsync(pc, hc.data(), hc.size() * sizeof(double), cudaMemcpyHostToDevice, st));
     TVF_CK(cudaMemcpyAsync(pr, hr.data(), hr.size() * sizeof(double), cudaMemcpyHostToDevice, st));
     TVF_CK(cudaMemsetAsync(pp, 0, (size_t)L * Q * 5 * sizeof(double), st));
-    TVF_CK(cudaMemsetAsync(pt, 0, (size_t)L * 5 * sizeof(double), st));
+    TVF_CK(cudaMemsetAsync(pt, 0, (size_t)L * W * sizeof(double), st));
+    if (ba) TVF_CK(cudaMemsetAsync(pb, 0, (size_t)L * Q * 6 * sizeof(double), st));
     std::vector<char> skipped((size_t)L, 0);
     for (int l = 0; l < L; ++l) {
         // trials j = l + L*q of [first_trial, first_trial + B): 0-based seed index q in [q_lo, q_hi), seed = q + 1
@@ -1431,29 +1451,59 @@ int tvf_sweep_run_levels(tvf_handle_t h, int method, int64_t first_trial, int64_
         const int n = levels[l].n;
         if ((method != 1 && n < 8) || n < 7) { skipped[(size_t)l] = 1; continue; }          // experiments.m:99-104: "not enough matches"
         if (Bl <= 0) continue;
+        const double* calm_l = (const double*)pc + (size_t)l * 27;
+        const double* gt_l = (const double*)pr + (size_t)l * 24;
         for (int64_t gdone = 0; gdone < Bl; gdone += G) {
             const int64_t Gc = (Bl - gdone < G) ? (Bl - gdone) : G;
             rc = sweep_common(h, q_lo + gdone, Gc, n, &levels[l].noise, 1, levels[l].P, hi_x, hi_y, (double*)pg, st); if (rc) return rc;
             for (int64_t off = 0; off < Gc; off += C) {
                 const int64_t Bc = (Gc - off < C) ? (Gc - off) : C;
-                rc = run_pose_chunk(h, st, m, (const double*)pg + off * 6 * n, (const double*)pc + (size_t)l * 27, 0, n, Bc, b.T, b.F, b.core,
+                const double* d_in = (const double*)pg + off * 6 * n;
+                rc = run_pose_chunk(h, st, m, d_in, calm_l, 0, n, Bc, b.T, b.F, b.core,
                                     b.cand, b.votes, b.scale, b.Rt2, b.Rt3, b.reconst, b.repr, b.status, b.iters, nullptr);
                 if (rc) return rc;
-                launch_sweep_eval_accumulate(b.Rt2, b.Rt3, b.repr, b.status, q_lo + gdone + off, Bc, 1, Q, (const double*)pr + (size_t)l * 24,
+                launch_sweep_eval_accumulate(b.Rt2, b.Rt3, b.repr, b.status, q_lo + gdone + off, Bc, 1, Q, gt_l,
                                              (double*)pp + (size_t)l * Q * 5, st);
+                h->launches += 1;
+                if (!ba) continue;
+                // a trial without a pose starts from NaN: the kernel copies it through with TVF_ST_NONFINITE and iter = 0
+                rc = ba_launch(h, st, BaIo{d_in, calm_l, 0, n, b.Rt2, b.Rt3, b.reconst, b.ba_Rt2, b.ba_Rt3, b.ba_X, b.ba_repr,
+                                           b.ba_iter, b.ba_status}, Bc, b.ba_Xc);
+                if (rc) return rc;
+                launch_sweep_eval_accumulate(b.ba_Rt2, b.ba_Rt3, b.ba_repr, b.status, q_lo + gdone + off, Bc, 1, Q, gt_l,
+                                             (double*)pb + (size_t)l * Q * 6, st, b.ba_status, b.ba_iter);
                 h->launches += 1;
             }
         }
-        launch_sweep_eval_finish((const double*)pp + (size_t)l * Q * 5, 1, Q, (double*)pt + (size_t)l * 5, st);
+        launch_sweep_eval_finish((const double*)pp + (size_t)l * Q * 5, 1, Q, (double*)pt + (size_t)l * W, st);
         h->launches += 1;
+        if (ba) {
+            launch_sweep_eval_finish((const double*)pb + (size_t)l * Q * 6, 1, Q, (double*)pt + (size_t)l * W + 5, st, 6);
+            h->launches += 1;
+        }
     }
     TVF_CK(cudaGetLastError());
-    TVF_CK(cudaMemcpyAsync(table, pt, (size_t)L * 5 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    TVF_CK(cudaMemcpyAsync(table, pt, (size_t)L * W * sizeof(double), cudaMemcpyDeviceToHost, st));
     TVF_CK(cudaStreamSynchronize(st));
     const double inf = __builtin_huge_val();
-    for (int l = 0; l < L; ++l)
-        if (skipped[(size_t)l]) { table[5 * l] = inf; table[5 * l + 1] = inf; table[5 * l + 2] = inf; table[5 * l + 3] = 0.0; table[5 * l + 4] = 0.0; }
+    for (int l = 0; l < L; ++l) {
+        if (!skipped[(size_t)l]) continue;
+        double* row = table + (size_t)W * l;
+        for (int c = 0; c < W; ++c) row[c] = 0.0;
+        row[0] = row[1] = row[2] = inf;
+        if (ba) row[5] = row[6] = row[7] = inf;
+    }
     return TVF_OK;
+}
+
+int tvf_sweep_run_levels(tvf_handle_t h, int method, int64_t first_trial, int64_t B, const tvf_sweep_level* levels, int L,
+                         double hi_x, double hi_y, double* table) {
+    return sweep_levels(h, method, first_trial, B, levels, L, hi_x, hi_y, table, false);
+}
+
+int tvf_sweep_run_levels_ba(tvf_handle_t h, int method, int64_t first_trial, int64_t B, const tvf_sweep_level* levels, int L,
+                            double hi_x, double hi_y, double* table) {
+    return sweep_levels(h, method, first_trial, B, levels, L, hi_x, hi_y, table, true);
 }
 
 int tvf_bundle_adjust(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,

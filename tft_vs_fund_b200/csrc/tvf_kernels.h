@@ -112,11 +112,13 @@ void launch_project3d(const double* pts3d, const double* P, int M, int cams_batc
 void launch_ang_error(const double* Rt_true, int true_batched, const double* Rt_est, long long B, double* rot,
                       double* tr, cudaStream_t s);
 
-// ---- per-noise-level evaluation sums (f3): partial is (L*Q) x 5, table L x 5 = [sum repr, sum rot, sum t, count, skipped]
+// ---- per-noise-level evaluation sums (f3): partial is (L*Q) x 5, table L x 5 = [sum repr, sum rot, sum t, count, skipped].
+// status2 != null (bundle adjustment's status, with its iter per trial): a trial flagged in either status word is skipped,
+// and partial / table get a sixth column, the sum of iter over the counted trials (finish with ncol = 6).
 void launch_sweep_eval_accumulate(const double* Rt2, const double* Rt3, const double* repr, const int* status,
                                   long long first_trial, long long B, int L, int Q, const double* d_Rt0, double* d_partial,
-                                  cudaStream_t s);
-void launch_sweep_eval_finish(const double* d_partial, int L, int Q, double* d_table, cudaStream_t s);
+                                  cudaStream_t s, const int* status2 = nullptr, const int* iter = nullptr);
+void launch_sweep_eval_finish(const double* d_partial, int L, int Q, double* d_table, cudaStream_t s, int ncol = 5);
 
 // ---- synthetic sweep trials generated on the device (f1) -----------------------------------------------
 constexpr int SWEEP_MAX_N = 60;      // n + 100 points per scene must fit the per-thread scratch

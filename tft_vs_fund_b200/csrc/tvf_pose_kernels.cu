@@ -797,10 +797,16 @@ __global__ void ang_error_kernel(const double* __restrict__ Rt_true, int true_ba
 // Per-trial ReprError / AngError accumulated per noise level.  Thread g owns level g % L and a fixed,
 // strided subset of that level's trials, so its four partial sums are updated by one thread in a fixed
 // order (chunk after chunk); sweep_eval_finish adds the per-thread partials in index order.  Bit-stable.
+// NC = 6 (the after-adjustment columns of tvf_sweep_run_levels_ba): a trial is also skipped when its second status word
+// (the adjustment's) is flagged, and its `iter` is summed into a sixth column.  NC = 5 never reads status2 / iter.
+template <int NC>
 __global__ void __launch_bounds__(256)
 sweep_eval_accumulate_kernel(const double* __restrict__ Rt2, const double* __restrict__ Rt3, const double* __restrict__ repr,
-                             const int* __restrict__ status, long long first_trial, long long B, int L, int Q,
-                             const double* __restrict__ Rt0, double* __restrict__ partial) {
+                             const int* __restrict__ status, const int* __restrict__ status2, const int* __restrict__ iter,
+                             long long first_trial, long long B, int L, int Q, const double* __restrict__ Rt0,
+                             double* __restrict__ partial) {
+    static_assert(NC == 5 || NC == 6, "sweep_eval: 5 or 6 columns");
+    constexpr int SKIP = ST_NO_POSE_2 | ST_NO_POSE_3 | ST_NONFINITE;
     const int g = blockIdx.x * blockDim.x + threadIdx.x;
     if (g >= L * Q) return;
     const int level = g % L, q = g / L;
@@ -808,9 +814,12 @@ sweep_eval_accumulate_kernel(const double* __restrict__ Rt2, const double* __res
     double gt2[12], gt3[12];
 #pragma unroll
     for (int i = 0; i < 12; ++i) { gt2[i] = Rt0[i]; gt3[i] = Rt0[12 + i]; }
-    double s_rep = 0.0, s_rot = 0.0, s_t = 0.0, cnt = 0.0, bad = 0.0;
+    double s_rep = 0.0, s_rot = 0.0, s_t = 0.0, cnt = 0.0, bad = 0.0, s_it = 0.0;
     for (long long b = r + (long long)L * q; b < B; b += (long long)L * Q) {
-        if (status != nullptr && (status[b] & (ST_NO_POSE_2 | ST_NO_POSE_3 | ST_NONFINITE))) { bad += 1.0; continue; }
+        if (status != nullptr && (status[b] & SKIP)) { bad += 1.0; continue; }
+        if constexpr (NC == 6) {
+            if (status2[b] & SKIP) { bad += 1.0; continue; }
+        }
         double e2[12], e3[12];
 #pragma unroll
         for (int i = 0; i < 12; ++i) { e2[i] = Rt2[b * 12 + i]; e3[i] = Rt3[b * 12 + i]; }
@@ -818,29 +827,38 @@ sweep_eval_accumulate_kernel(const double* __restrict__ Rt2, const double* __res
         ang_error(gt2, e2, &r2, &t2);                                   // experiments.m:117-118
         ang_error(gt3, e3, &r3, &t3);
         s_rep += repr[b]; s_rot += (r2 + r3) * 0.5; s_t += (t2 + t3) * 0.5; cnt += 1.0;   // :112-120
+        if constexpr (NC == 6) s_it += (double)iter[b];
     }
-    double* p = partial + (size_t)g * 5;
+    double* p = partial + (size_t)g * NC;
     p[0] += s_rep; p[1] += s_rot; p[2] += s_t; p[3] += cnt; p[4] += bad;
+    if constexpr (NC == 6) p[5] += s_it;
 }
 
+template <int NC>
 __global__ void sweep_eval_finish_kernel(const double* __restrict__ partial, int L, int Q, double* __restrict__ table) {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= L * 5) return;
-    const int level = e / 5, c = e % 5;
+    if (e >= L * NC) return;
+    const int level = e / NC, c = e % NC;
     double a = 0.0;
-    for (int q = 0; q < Q; ++q) a += partial[((size_t)q * L + level) * 5 + c];
+    for (int q = 0; q < Q; ++q) a += partial[((size_t)q * L + level) * NC + c];
     table[e] = a;
 }
 
 void launch_sweep_eval_accumulate(const double* Rt2, const double* Rt3, const double* repr, const int* status,
                                   long long first_trial, long long B, int L, int Q, const double* d_Rt0, double* d_partial,
-                                  cudaStream_t s) {
+                                  cudaStream_t s, const int* status2, const int* iter) {
     if (B <= 0) return;
-    sweep_eval_accumulate_kernel<<<(L * Q + 255) / 256, 256, 0, s>>>(Rt2, Rt3, repr, status, first_trial, B, L, Q, d_Rt0, d_partial);
+    if (status2 != nullptr)
+        sweep_eval_accumulate_kernel<6><<<(L * Q + 255) / 256, 256, 0, s>>>(Rt2, Rt3, repr, status, status2, iter, first_trial,
+                                                                             B, L, Q, d_Rt0, d_partial);
+    else
+        sweep_eval_accumulate_kernel<5><<<(L * Q + 255) / 256, 256, 0, s>>>(Rt2, Rt3, repr, status, nullptr, nullptr, first_trial,
+                                                                             B, L, Q, d_Rt0, d_partial);
 }
 
-void launch_sweep_eval_finish(const double* d_partial, int L, int Q, double* d_table, cudaStream_t s) {
-    sweep_eval_finish_kernel<<<(L * 5 + 63) / 64, 64, 0, s>>>(d_partial, L, Q, d_table);
+void launch_sweep_eval_finish(const double* d_partial, int L, int Q, double* d_table, cudaStream_t s, int ncol) {
+    if (ncol == 6) sweep_eval_finish_kernel<6><<<(L * 6 + 63) / 64, 64, 0, s>>>(d_partial, L, Q, d_table);
+    else sweep_eval_finish_kernel<5><<<(L * 5 + 63) / 64, 64, 0, s>>>(d_partial, L, Q, d_table);
 }
 
 // ------------------------------------------------------------------- launchers

@@ -101,19 +101,32 @@ def prepare_triplet(data, it, repr_err_th=1.0, device=None):
     return dict(triplet=tuple(im), CalM=CalM, R_t0=R_t0, Corresp=Corresp, Corresp_inliers=inl, inlier_mask=mask, REr=REr)
 
 
-def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), device=None, details=None):
+def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), device=None, details=None,
+             bundle_adjust=False):
     """The linear-method part of experiments_real.m:75-138.  `data`: a Dataset or the path of a dataset directory;
     `triplets_to_test`: rows of indexes_sorted (1-based; the reference uses 1:70 / 1:50, :31-36).  Per loop index `it`:
     pre-filter (:94-101), sample min(100, N) inliers with rng(it) (:103-105; documented stand-in for MATLAB's
     randsample: scene.SceneRNG(it).randsample), run methods 1 / 7 on the sample (:126), evaluate ReprError over ALL
     inliers (triangulating them, :130-131) and AngError against the ground truth (:133-136).
     Returns dict method -> array (len(triplets_to_test), 3) of [repr_err, rot_err, t_err]; `details` (a list) receives
-    one dict per triplet (inlier count, ground-truth RMS, sample, per-method poses / T / votes)."""
+    one dict per triplet (inlier count, ground-truth RMS, sample, per-method poses / T / votes).
+    bundle_adjust=True: each method's pose is then refined by api.bundle_adjust on the same sample, from the method's
+    R_t_2, R_t_3 and Reconst -- the library's three-view adjustment, not the reference's BundleAdjustment.m (DESIGN.md
+    section 8) -- and the adjusted cameras are evaluated exactly as the method's.  Each entry is then (T, 6): the three
+    errors of the method, then the same three after the adjustment; details[k]["ba"][m] holds the adjusted result."""
     from .scene import SceneRNG
     from .experiments import METHODS
     if not isinstance(data, Dataset):
         data = load_dataset(data)
-    out = {m: np.zeros((len(triplets_to_test), 3)) for m in methods}
+    out = {m: np.zeros((len(triplets_to_test), 6 if bundle_adjust else 3)) for m in methods}
+
+    def errors(R2, R3, CalM, inl, R_t0):
+        Ps = [CalM[0:3] @ np.eye(3, 4), CalM[3:6] @ R2, CalM[6:9] @ R3]
+        rep = api.ReprError(Ps, inl, device=device)                                                     # :130-131
+        r2, t2 = api.AngError(R_t0[0], R2, device=device)
+        r3, t3 = api.AngError(R_t0[1], R3, device=device)
+        return [rep, (r2 + r3) / 2, (t2 + t3) / 2]                                                      # :133-136
+
     for row, trip in enumerate(triplets_to_test):
         it = row + 1                                                                                    # :75 loop index
         d = prepare_triplet(data, trip, device=device)
@@ -123,18 +136,19 @@ def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), de
         C0 = inl[:, sample]
         CalM = d["CalM"]
         rec = dict(triplet=d["triplet"], n_inliers=N, REr=d["REr"], sample=sample, res={})
+        if bundle_adjust:
+            rec["ba"] = {}
         for m in methods:
             if (m > 6 and N < 8) or N < 7:                                                              # :117-122
                 out[m][row] = np.inf
                 continue
             res = METHODS[m][1](C0, CalM, device=device)                                                # :126
-            R2, R3 = res[0], res[1]
-            Ps = [CalM[0:3] @ np.eye(3, 4), CalM[3:6] @ R2, CalM[6:9] @ R3]
-            rep = api.ReprError(Ps, inl, device=device)                                                 # :130-131
-            r2, t2 = api.AngError(d["R_t0"][0], R2, device=device)
-            r3, t3 = api.AngError(d["R_t0"][1], R3, device=device)
-            out[m][row] = [rep, (r2 + r3) / 2, (t2 + t3) / 2]                                           # :133-136
+            out[m][row, :3] = errors(res[0], res[1], CalM, inl, d["R_t0"])
             rec["res"][m] = res
+            if bundle_adjust:
+                ba = api.bundle_adjust(C0, CalM, res[0], res[1], res[2], device=device)
+                out[m][row, 3:] = errors(ba[0], ba[1], CalM, inl, d["R_t0"])
+                rec["ba"][m] = ba
         if details is not None:
             details.append(rec)
     return out

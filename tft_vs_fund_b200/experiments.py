@@ -79,9 +79,17 @@ def run_sweep(total_trials, n=20, methods=(1, 7), noise_levels=NOISE_LEVELS, foc
     return out if rank == 0 else None
 
 
-def run_sweep_device(total_trials, n=20, methods=(1, 7), noise_levels=NOISE_LEVELS, focalL=50, angle=0, device=None):
+def run_sweep_device(total_trials, n=20, methods=(1, 7), noise_levels=NOISE_LEVELS, focalL=50, angle=0, device=None,
+                     bundle_adjust=False):
     """run_sweep with everything on the device (tvf_sweep_run): trials are generated, solved and reduced per
-    noise level in HBM; each rank moves one L x 5 table.  Per-rank sums are added in rank order on rank 0."""
+    noise level in HBM; each rank moves one L x 5 table.  Per-rank sums are added in rank order on rank 0.
+    bundle_adjust=True: the device-resident twin of run_sweep(bundle_adjust=True) -- the noise levels become L levels of
+    tvf_sweep_run_levels_ba with the same n, cameras, CalM and ground truth, and each entry is (n_levels, 6) as there.
+    run_sweep_device.last_skipped_ba and .last_ba_iter then hold, per method and level, the trials left out of the
+    adjusted means and the mean number of adjustment iterations."""
+    if bundle_adjust:
+        params = [dict(N=int(n), noise=float(v), f=focalL, angle=angle) for v in np.asarray(noise_levels, dtype=np.float64).ravel()]
+        return _run_levels(run_sweep_device, params, total_trials, methods, device, True)
     rank, size = sharding.world()
     lo, hi = sharding.shard_range(total_trials, rank, size)
     noise_levels = np.ascontiguousarray(noise_levels, dtype=np.float64)
@@ -107,6 +115,54 @@ def run_sweep_device(total_trials, n=20, methods=(1, 7), noise_levels=NOISE_LEVE
     return out if rank == 0 else None
 
 
+def _sweep_levels(params):
+    """tvf_sweep_level array of the per-level parameters (N, noise, f, angle)."""
+    levels = (_lib.SweepLevel * len(params))()
+    for lv, p in zip(levels, params):
+        K, Ps, R_t0 = scene.scene_cameras(p["f"], p["angle"])
+        lv.noise, lv.n = p["noise"], p["N"]
+        lv.P[:] = np.ascontiguousarray(np.stack(Ps)).ravel()
+        lv.calm[:] = np.tile(K, (3, 1)).T.ravel()
+        lv.Rt0_2[:] = R_t0[0].T.ravel(); lv.Rt0_3[:] = R_t0[1].T.ravel()
+    return levels
+
+
+def _run_levels(driver, params, total_trials, methods, device, bundle_adjust):
+    """tvf_sweep_run_levels[_ba] over the global trials [0, total_trials), sharded; per-rank tables added in rank order.
+    Returns on rank 0 dict method -> (L, 3) means, or (L, 6) with the adjusted means; inf on the levels the reference
+    skips.  Sets driver.last_skipped (and with bundle_adjust .last_skipped_ba, .last_ba_iter) on rank 0."""
+    L = len(params)
+    levels = _sweep_levels(params)
+    W, fn = (11, "tvf_sweep_run_levels_ba") if bundle_adjust else (5, "tvf_sweep_run_levels")
+    rank, size = sharding.world()
+    lo, hi = sharding.shard_range(total_trials, rank, size)
+    h = _lib.handle(device)
+    out, skipped, skipped_ba, ba_iter = {}, {}, {}, {}
+    for m in methods:
+        table = np.zeros((L, W))
+        h.call(fn, int(m), lo, hi - lo, levels, L, 36 * scene.PIX, 24 * scene.PIX, table.ctypes.data_as(_lib.c_double_p))
+        unavailable = np.isinf(table[:, 0])
+        table[unavailable, :3] = 0.0
+        if bundle_adjust:
+            table[unavailable, 5:8] = 0.0
+        total = sharding.sum_in_rank_order(table)
+        if total is not None:
+            with np.errstate(divide="ignore", invalid="ignore"):
+                out[m] = total[:, :3] / total[:, 3:4]
+                if bundle_adjust:
+                    out[m] = np.hstack([out[m], total[:, 5:8] / total[:, 8:9]])
+                    ba_iter[m] = total[:, 10] / total[:, 8]
+            out[m][unavailable] = np.inf
+            skipped[m] = total[:, 4].astype(np.int64)
+            if bundle_adjust:
+                skipped_ba[m] = total[:, 9].astype(np.int64)
+    if rank == 0:
+        driver.last_skipped = skipped
+        if bundle_adjust:
+            driver.last_skipped_ba, driver.last_ba_iter = skipped_ba, ba_iter
+    return out if rank == 0 else None
+
+
 # ---- the four experiments of experiments.m:23-47 -------------------------------------------------------------
 INTERVALS = {                                                                     # experiments.m:38-47
     "noise": [0.25 * k for k in range(13)],                                      # 0:0.25:3
@@ -127,49 +183,36 @@ def experiment_levels(option, N=12, noise=1.0, f=50, angle=0, interval=None):
     return interval, out
 
 
-def run_experiment(option, n_sim=20, methods=(1, 7), N=12, noise=1.0, f=50, angle=0, interval=None, device=None):
+def run_experiment(option, n_sim=20, methods=(1, 7), N=12, noise=1.0, f=50, angle=0, interval=None, device=None,
+                   bundle_adjust=False):
     """experiments.m for one `option`, device-resident (tvf_sweep_run_levels): level i x seeds 1..n_sim x methods.  Sharded
     like run_sweep (contiguous ranges of the global trial index j = (seed-1)*L + level).  Returns on rank 0
     (interval, dict method -> (L, 3) mean [repr_err, rot_err, t_err]; inf where the reference skips the method for lack
-    of matches, experiments.m:99-104), None elsewhere."""
-    import ctypes as C
+    of matches, experiments.m:99-104), None elsewhere.
+    bundle_adjust=True (tvf_sweep_run_levels_ba): every pose is then refined by the library's bundle adjustment (not the
+    reference's BundleAdjustment.m, DESIGN.md section 8) on the device, and each entry is (L, 6): the three means, then the
+    same three after the adjustment, as run_sweep(bundle_adjust=True).  run_experiment.last_skipped_ba (trials left out of
+    the adjusted means: no pose, or a non-finite adjustment) and .last_ba_iter (mean adjustment iterations) are per level."""
+    interval, params = experiment_levels(option, N, noise, f, angle, interval)
+    out = _run_levels(run_experiment, params, len(params) * n_sim, methods, device, bundle_adjust)
+    return (interval, out) if out is not None else None
+
+
+def run_experiment_host(option, n_sim=20, methods=(1, 7), N=12, noise=1.0, f=50, angle=0, interval=None, device=None,
+                        bundle_adjust=False):
+    """The same experiment driven from the host (inputs from scene.sweep_batch, one batched solver call per level and
+    method, NumPy reduction): the twin the tests hold run_experiment against.  bundle_adjust=True: api.bundle_adjust from
+    each method's (R_t_2, R_t_3, Reconst), evaluated as the method; entries (L, 6) and, as for run_experiment,
+    run_experiment_host.last_skipped, .last_skipped_ba and .last_ba_iter per method and level."""
     interval, params = experiment_levels(option, N, noise, f, angle, interval)
     L = len(params)
-    levels = (_lib.SweepLevel * L)()
-    for lv, p in zip(levels, params):
-        K, Ps, R_t0 = scene.scene_cameras(p["f"], p["angle"])
-        lv.noise, lv.n = p["noise"], p["N"]
-        lv.P[:] = np.ascontiguousarray(np.stack(Ps)).ravel()
-        lv.calm[:] = np.tile(K, (3, 1)).T.ravel()
-        lv.Rt0_2[:] = R_t0[0].T.ravel(); lv.Rt0_3[:] = R_t0[1].T.ravel()
-    rank, size = sharding.world()
-    lo, hi = sharding.shard_range(L * n_sim, rank, size)
-    h = _lib.handle(device)
-    out, skipped = {}, {}
-    for m in methods:
-        table = np.zeros((L, 5))
-        h.call("tvf_sweep_run_levels", int(m), lo, hi - lo, levels, L, 36 * scene.PIX, 24 * scene.PIX,
-               table.ctypes.data_as(_lib.c_double_p))
-        unavailable = np.isinf(table[:, 0])
-        table[unavailable, :3] = 0.0
-        total = sharding.sum_in_rank_order(table)
-        if total is not None:
-            with np.errstate(divide="ignore", invalid="ignore"):
-                out[m] = total[:, :3] / total[:, 3:4]
-            out[m][unavailable] = np.inf
-            skipped[m] = total[:, 4].astype(np.int64)
-    if rank == 0:
-        run_experiment.last_skipped = skipped
-    return (interval, out) if rank == 0 else None
-
-
-def run_experiment_host(option, n_sim=20, methods=(1, 7), N=12, noise=1.0, f=50, angle=0, interval=None, device=None):
-    """The same experiment driven from the host (inputs from scene.sweep_batch, one batched solver call per level and
-    method, NumPy reduction): the twin the tests hold run_experiment against."""
-    interval, params = experiment_levels(option, N, noise, f, angle, interval)
-    out = {m: np.zeros((len(params), 3)) for m in methods}
+    out = {m: np.zeros((L, 6 if bundle_adjust else 3)) for m in methods}
+    skipped = {m: np.zeros(L, dtype=np.int64) for m in methods}
+    skipped_ba = {m: np.zeros(L, dtype=np.int64) for m in methods}
+    ba_iter = {m: np.full(L, np.nan) for m in methods}
     for i, p in enumerate(params):
         d = scene.sweep_batch(n_sim, p["N"], noise_levels=[p["noise"]], focalL=p["f"], angle=p["angle"])
+        lvl = np.zeros(n_sim, dtype=np.int64)
         for m in methods:
             if (m > 6 and p["N"] < 8) or p["N"] < 7:                                                 # experiments.m:99-104
                 out[m][i] = np.inf
@@ -177,6 +220,19 @@ def run_experiment_host(option, n_sim=20, methods=(1, 7), N=12, noise=1.0, f=50,
             res = METHODS[m][1](d["Corresp"], d["CalM"], device=device)
             repr_err, rot_err, t_err = evaluate(res, d["R_t0"], device=device)
             bad = (np.asarray(res.status) & (_lib.ST_NO_POSE_2 | _lib.ST_NO_POSE_3 | _lib.ST_NONFINITE)) != 0
-            sums = level_sums(np.zeros(n_sim, dtype=np.int64), 1, repr_err, rot_err, t_err, bad=bad)
-            out[m][i] = sums[0, :3] / sums[0, 3]
+            sums = level_sums(lvl, 1, repr_err, rot_err, t_err, bad=bad)
+            out[m][i, :3] = sums[0, :3] / sums[0, 3]
+            skipped[m][i] = int(sums[0, 4])
+            if bundle_adjust:
+                ba = api.bundle_adjust(d["Corresp"], d["CalM"], res[0], res[1], res[2], device=device)
+                bad_ba = bad | ((np.asarray(ba.status) & _lib.ST_NONFINITE) != 0)
+                sums = level_sums(lvl, 1, *evaluate(ba, d["R_t0"], device=device), np.asarray(ba[3], dtype=np.float64),
+                                  bad=bad_ba)
+                with np.errstate(divide="ignore", invalid="ignore"):
+                    out[m][i, 3:] = sums[0, :3] / sums[0, 4]
+                    ba_iter[m][i] = sums[0, 3] / sums[0, 4]
+                skipped_ba[m][i] = int(sums[0, 5])
+    run_experiment_host.last_skipped = skipped
+    if bundle_adjust:
+        run_experiment_host.last_skipped_ba, run_experiment_host.last_ba_iter = skipped_ba, ba_iter
     return interval, out
