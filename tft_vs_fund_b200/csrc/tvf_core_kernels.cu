@@ -225,10 +225,10 @@ __device__ __forceinline__ double f_apply_AtA(const CoreInput& in, long long pro
 }
 
 // G(r,c) -> moment index (96 = structural zero), one table per CTA
-__device__ __forceinline__ void build_gidx(unsigned char* gidx, int zero_slot = 96) {
+__device__ __forceinline__ void build_gidx(unsigned char* gidx) {
     for (int e = threadIdx.x; e < 32 * 27; e += blockDim.x) {
         const int r = e / 27, c = e % 27;
-        int idx = zero_slot;                 // structural zeros of the Gram (and rows >= 27) read a slot that holds 0.0
+        int idx = 96;                        // structural zeros of the Gram (and rows >= 27) read a slot that holds 0.0
         if (r < 27) {
             const int j = r % 3, k = (r / 3) % 3, i = r / 9;
             const int j2 = c % 3, k2 = (c / 3) % 3, i2 = c / 9;
@@ -799,10 +799,64 @@ tft_epipoles_kernel(double* __restrict__ ws, long long B) {
 }
 
 // =========================================================================== TFT stage 2
+// The projected Gram H = Up' G Up of linearTFT.m:84, straight from the 96 moments (DESIGN.md §3.4).  Column (i,a) of Up is
+// e_i (x) vec(p_a q_a') with p_a in (e21, e21, e21, u1, u2) and q_a in (e31, v1, v2, e31, e31), the basis of range(E) per
+// slice.  G = sum (p1 p1') (x) M(x3,y3) (x) M(x2,y2) and M = sum_g m4_g N_g with four constant N_g, so
+//   H[(i,a),(i',b)] = sum_{beta,gamma} mom[16 sym6(i,i') + 4 beta + gamma] c_beta(q_a,q_b) c_gamma(p_a,p_b)
+// with the quadratic forms c(p,q) = (p0 q0 + p1 q1, p0 q2 + p2 q0, p1 q2 + p2 q1, p2 q2) of the N_g.  The entry is symmetric in
+// a <-> b and in i <-> i': 6 x 15 distinct values.  Lane r < 15 of the 16 calling lanes takes the pair {a,b} number r, forms
+// its 6 values (96 + 24 multiply-adds: first over gamma, then over beta) and stores each at its (up to) 4 places in hs, the
+// full 15 x 15 matrix with row stride H15_LD.  pb / qb: (e21, u1, u2) / (e31, v1, v2), 9 doubles each.
+constexpr int H15_LD = 18;       // rows 16-byte aligned, and the row reads of 8 lanes hit 8 different bank quads
+__device__ __forceinline__ void cforms(const double* p, const double* q, double* c) {
+    c[0] = fma(p[0], q[0], p[1] * q[1]);
+    c[1] = fma(p[0], q[2], p[2] * q[0]);
+    c[2] = fma(p[1], q[2], p[2] * q[1]);
+    c[3] = p[2] * q[2];
+}
+__device__ __forceinline__ void form_h15(const double* mom, const double* pb, const double* qb, int r, double* hs) {
+    if (r >= 15) return;
+    // pair r -> (a, b), a <= b: (0,0) (0,1) .. (0,4) (1,1) .. (1,4) (2,2) .. (2,4) (3,3) (3,4) (4,4)
+    const int a = (int)((0x433222111100000ull >> (4 * r)) & 15), b = (int)((0x443432432143210ull >> (4 * r)) & 15);
+    double cp[4], cq[4];
+    cforms(pb + 3 * (a < 3 ? 0 : a - 2), pb + 3 * (b < 3 ? 0 : b - 2), cp);
+    cforms(qb + 3 * (a < 3 ? a : 0), qb + 3 * (b < 3 ? b : 0), cq);
+    double* hab = hs + H15_LD * a + b;      // (row a, column b) of a 5 x 5 block
+    double* hba = hs + H15_LD * b + a;
+#pragma unroll
+    for (int al = 0; al < 6; ++al) {
+        const int i = (al < 3) ? 0 : ((al < 5) ? 1 : 2), i2 = (al < 3) ? al : ((al < 5) ? al - 2 : 2);   // sym6(i,i2) = al
+        const double* m = mom + 16 * al;
+        double hv = 0.0;
+#pragma unroll
+        for (int be = 0; be < 4; ++be) {
+            const double y = fma(m[4 * be], cp[0], fma(m[4 * be + 1], cp[1], fma(m[4 * be + 2], cp[2], m[4 * be + 3] * cp[3])));
+            hv = fma(cq[be], y, hv);
+        }
+        const int o = 5 * H15_LD * i + 5 * i2, ot = 5 * H15_LD * i2 + 5 * i;
+        hab[o] = hv; hba[o] = hv;
+        if (i != i2) { hab[ot] = hv; hba[ot] = hv; }
+    }
+}
+// row r of H (zeros for r >= 15, as the eigenvector solvers want them)
+__device__ __forceinline__ void load_h15_row(const double* hs, int r, double (&g)[15]) {
+    const double* row = hs + H15_LD * (r < 15 ? r : 0);
+    const double2* row2 = reinterpret_cast<const double2*>(row);
+#pragma unroll
+    for (int m2 = 0; m2 < 7; ++m2) { const double2 v = row2[m2]; g[2 * m2] = v.x; g[2 * m2 + 1] = v.y; }
+    g[14] = row[14];
+    if (r >= 15) {
+#pragma unroll
+        for (int c = 0; c < 15; ++c) g[c] = 0.0;
+    }
+}
+
 struct __align__(16) Stage2Scratch {
     double sbuf[64];
-    double W[27 * FEAT_STRIDE + 3];  // G*Up, 27 x 15 (row stride 15)
-    double mom[98];
+    double H[15 * H15_LD];           // Up' G Up
+    double ax[64];                   // refinement: the 27-vector Up tp at [0, 27), A'A times it at [32, 59)
+    double mom[96];
+    double bas[18];                  // e21, u1, u2, e31, v1, v2
     double T[28];
     double tp[16];
     double Nm[28];                   // N1, inv(N2), inv(N3)
@@ -815,10 +869,7 @@ tft_stage2_kernel(CoreInput in, const double* __restrict__ ws, double* __restric
     const int normalize = in.normalize;
     const long long B = in.B;
     __shared__ Stage2Scratch scratch[CORE_WARPS];
-    __shared__ unsigned char gidx[32 * 27];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    build_gidx(gidx);
-    __syncthreads();
     Stage2Scratch& sc = scratch[warp];
     const int jr = lane % 3, kr = (lane / 3) % 3, ir = (lane < 27) ? lane / 9 : 0;
 
@@ -828,41 +879,23 @@ tft_stage2_kernel(CoreInput in, const double* __restrict__ ws, double* __restric
         if (prob >= B) continue;
         const double* rec = ws + prob * CORE_WS_TFT;
         sc.mom[lane] = rec[CW_MOM + lane]; sc.mom[lane + 32] = rec[CW_MOM + 32 + lane]; sc.mom[lane + 64] = rec[CW_MOM + 64 + lane];
-        if (lane == 0) { sc.mom[96] = 0.0; sc.mom[97] = 0.0; }
         const double e21[3] = {rec[CW_EPI], rec[CW_EPI + 1], rec[CW_EPI + 2]};
         const double e31[3] = {rec[CW_EPI + 3], rec[CW_EPI + 4], rec[CW_EPI + 5]};
         double u1[3], u2[3], v1[3], v2[3];
         onb3(e21, u1, u2);
         onb3(e31, v1, v2);
-        __syncwarp();
         // basis of range(E) per slice: B0=e21 e31', B1=e21 v1', B2=e21 v2', B3=u1 e31', B4=u2 e31'
-        // W = G*Up: first contract j' with {e21,u1,u2}, then k' with {e31,v1,v2}
-        {
-            double Ze[9], Zu1[9], Zu2[9];
+        if (lane == 0) {
 #pragma unroll
-            for (int q = 0; q < 9; ++q) {
-                const double g0 = sc.mom[gidx[lane * 27 + 3 * q]];
-                const double g1 = sc.mom[gidx[lane * 27 + 3 * q + 1]];
-                const double g2 = sc.mom[gidx[lane * 27 + 3 * q + 2]];
-                Ze[q] = g0 * e21[0] + g1 * e21[1] + g2 * e21[2];
-                Zu1[q] = g0 * u1[0] + g1 * u1[1] + g2 * u1[2];
-                Zu2[q] = g0 * u2[0] + g1 * u2[1] + g2 * u2[2];
+            for (int q = 0; q < 3; ++q) {
+                sc.bas[q] = e21[q]; sc.bas[3 + q] = u1[q]; sc.bas[6 + q] = u2[q];
+                sc.bas[9 + q] = e31[q]; sc.bas[12 + q] = v1[q]; sc.bas[15 + q] = v2[q];
             }
-            if (lane < 27) {
-                double* W = sc.W + lane * FEAT_STRIDE;
-#pragma unroll
-                for (int i2 = 0; i2 < 3; ++i2) {
-                    const double* ze = Ze + 3 * i2; const double* zu1 = Zu1 + 3 * i2; const double* zu2 = Zu2 + 3 * i2;
-                    W[5 * i2 + 0] = ze[0] * e31[0] + ze[1] * e31[1] + ze[2] * e31[2];
-                    W[5 * i2 + 1] = ze[0] * v1[0] + ze[1] * v1[1] + ze[2] * v1[2];
-                    W[5 * i2 + 2] = ze[0] * v2[0] + ze[1] * v2[1] + ze[2] * v2[2];
-                    W[5 * i2 + 3] = zu1[0] * e31[0] + zu1[1] * e31[1] + zu1[2] * e31[2];
-                    W[5 * i2 + 4] = zu2[0] * e31[0] + zu2[1] * e31[1] + zu2[2] * e31[2];
-                }
-            }
-            __syncwarp();
         }
-        // G15 = Up' W, lane (i,a) owns row 5i+a; then its smallest eigenvector (linearTFT.m:84)
+        __syncwarp();
+        form_h15(sc.mom, sc.bas, sc.bas + 9, lane, sc.H);
+        __syncwarp();
+        // lane (i,a) owns row 5i+a of H; then its smallest eigenvector (linearTFT.m:84)
         double tl2;
         int st = 0;
         {
@@ -874,17 +907,7 @@ tft_stage2_kernel(CoreInput in, const double* __restrict__ ws, double* __restric
                 qa[q] = (aa == 1) ? v1[q] : ((aa == 2) ? v2[q] : e31[q]);
             }
             double g15[15];
-#pragma unroll
-            for (int c = 0; c < 15; ++c) g15[c] = 0.0;
-#pragma unroll
-            for (int k = 0; k < 3; ++k)
-#pragma unroll
-                for (int j = 0; j < 3; ++j) {
-                    const double coef = (lane < 15) ? pa[j] * qa[k] : 0.0;
-                    const double* W = sc.W + (9 * ia + 3 * k + j) * FEAT_STRIDE;
-#pragma unroll
-                    for (int c = 0; c < 15; ++c) g15[c] = fma(coef, W[c], g15[c]);
-                }
+            load_h15_row(sc.H, lane, g15);
             const double pe = sel3(e21, jr), pu1 = sel3(u1, jr), pu2 = sel3(u2, jr);
             const double qe = sel3(e31, kr), qv1 = sel3(v1, kr), qv2 = sel3(v2, kr);
             const double st_s[3] = {rec[CW_STATS], rec[CW_STATS + 1], rec[CW_STATS + 2]};
@@ -898,17 +921,17 @@ tft_stage2_kernel(CoreInput in, const double* __restrict__ ws, double* __restric
                     a27 = pe * (qe * tp[0] + qv1 * tp[1] + qv2 * tp[2]) + qe * (pu1 * tp[3] + pu2 * tp[4]);
                 }
                 __syncwarp();
-                if (lane < 27) sc.W[lane] = a27;
+                if (lane < 27) sc.ax[lane] = a27;
                 __syncwarp();
-                const double g27 = tft_apply_AtA<PACKED>(in, prob, lane, st_s, st_t, sc.W);
+                const double g27 = tft_apply_AtA<PACKED>(in, prob, lane, st_s, st_t, sc.ax);
                 __syncwarp();
-                if (lane < 27) sc.W[32 + lane] = g27;
+                if (lane < 27) sc.ax[32 + lane] = g27;
                 __syncwarp();
                 double r = 0.0;
 #pragma unroll
                 for (int k = 0; k < 3; ++k)
 #pragma unroll
-                    for (int j = 0; j < 3; ++j) r = fma(pa[j] * qa[k], sc.W[32 + 9 * ia + 3 * k + j], r);
+                    for (int j = 0; j < 3; ++j) r = fma(pa[j] * qa[k], sc.ax[32 + 9 * ia + 3 * k + j], r);
                 return (lane < 15) ? r : 0.0;
             };
             bool conv2;
@@ -980,9 +1003,9 @@ tft_stage2_kernel(CoreInput in, const double* __restrict__ ws, double* __restric
     }
 }
 
-// ---- two problems per warp (n >= REFINE_N_MAX): the 27-lane parts run once per problem, the 15-lane parts (the
-// projected Gram Up'(G Up), its Gauss-Jordan inverse and the power iteration: half of this kernel's instructions) run
-// for both problems at once on the two half-warps (smallest_eigvec_spd_half).
+// ---- two problems per warp (n >= REFINE_N_MAX), one per half-warp from the staged record to the last store: half h = problem
+// 2 pair + h forms its H (form_h15 on its 16 lanes), solves it (smallest_eigvec_spd_half) and runs the back end with two
+// entries of T per lane.
 // The pair's two work-space records are adjacent in global memory (2 x 1120 bytes): lane 0 fetches the NEXT pair's with one
 // bulk asynchronous copy per warp (own mbarrier) as soon as the current pair's moments have been consumed (the epipoles
 // and statistics are copied aside first), so no pair waits for its loads.
@@ -991,43 +1014,36 @@ tft_stage2_kernel(CoreInput in, const double* __restrict__ ws, double* __restric
 #endif
 struct __align__(16) Stage2DualScratch {
     double sbuf[64];
-    double W[2][27 * FEAT_STRIDE + 3];   // G*Up of the two problems
+    double H[2][15 * H15_LD];            // Up' G Up of the two problems
 #if TVF_S2_TMA
     double rec2[2 * CORE_WS_TFT];        // the two work-space records as they lie in global memory (one bulk copy)
 #else
-    double mom2[2][98];                  // moments of the two problems (+ zero sentinel)
+    double mom2[2][96];                  // moments of the two problems
 #endif
-    double es[2][16];                    // epipoles (6) + normalisation statistics (9) of the two problems
-    double T[28];
+    double es[2][28];                    // e21, u1, u2 (0..8), e31, v1, v2 (9..17), normalisation statistics (18..26)
+    double T[2][28];
     double tp[2][16];
-    double Nm[28];
 };
 
 #ifndef TVF_STAGE2_DUAL
 #define TVF_STAGE2_DUAL 1
 #endif
 
-// resident CTAs per SM the kernel is compiled for: 4 (128 registers, no spills) measured 24.8 ms per 10 M against 26.0 at 5 (96
-// registers, 92 bytes spilled) and 27.4 at 6
+// resident CTAs per SM the kernel is compiled for: 5 (96 registers, 12 bytes spilled) measured 14.7 ms per 10 M against 15.1 at 4
+// (128 registers, 4 bytes spilled) and 16.2 at 3 (profiles/r03_stage2_factored_h.md)
 #ifndef TVF_S2D_MINB
-#define TVF_S2D_MINB 4
+#define TVF_S2D_MINB 5
 #endif
 __global__ void __launch_bounds__(CORE_WARPS * 32, TVF_S2D_MINB)
 tft_stage2_dual_kernel(int normalize, long long B, const double* __restrict__ ws, double* __restrict__ Tout,
                        double* __restrict__ P2out, double* __restrict__ P3out, int* __restrict__ status) {
     __shared__ Stage2DualScratch scratch[CORE_WARPS];
-    __shared__ unsigned char gidx[32 * 27];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#if TVF_S2_TMA
-    build_gidx(gidx, CW_STATS + 9);         // the unused pad slot of the staged record, zeroed after every copy
-#else
-    build_gidx(gidx);
-#endif
-    __syncthreads();
     Stage2DualScratch& sc = scratch[warp];
-    const int jr = lane % 3, kr = (lane / 3) % 3, ir = (lane < 27) ? lane / 9 : 0;
     const int h = lane >> 4, r15 = lane & 15;
-    const int ia = (r15 < 15) ? r15 / 5 : 0, aa = (r15 < 15) ? r15 % 5 : 0;
+    // entries e0 = r15 and e1 = r15 + 16 of T (index j + 3k + 9i); e1 exists for r15 < 11 (the clamped index is never stored)
+    const bool has1 = r15 < 11;
+    const int e0 = r15, e1 = has1 ? r15 + 16 : 26;
     const long long npairs = (B + 1) / 2;
 #if TVF_S2_TMA
     __shared__ unsigned long long wbar[CORE_WARPS];
@@ -1050,20 +1066,22 @@ tft_stage2_dual_kernel(int normalize, long long B, const double* __restrict__ ws
         if (pair >= npairs) continue;
         const long long prob0 = 2 * pair;
         const int nprob = (prob0 + 1 < B) ? 2 : 1;
+        const bool live = h < nprob;            // odd batch: the idle half works on problem prob0 and stores nothing
+        const int hp = live ? h : 0;
+        // lane 16 p + q: epipoles (q < 6) and normalisation statistics (6 <= q < 15) of problem p, set aside
+        const int es_slot = (r15 < 3) ? r15 : ((r15 < 6) ? r15 + 6 : r15 + 12);
 #if TVF_S2_TMA
         mbar_wait(&wbar[warp], parity);
         parity ^= 1u;
+        const double* mom = sc.rec2 + hp * CORE_WS_TFT + CW_MOM;
         {
-            // lane 16 p + q: epipoles (q < 6) and normalisation statistics (6 <= q < 15) of problem p, set aside
-            const int pq = lane >> 4, q15 = lane & 15;
-            const double* recq = sc.rec2 + ((pq < nprob) ? pq : 0) * CORE_WS_TFT;
-            sc.es[pq][q15] = (q15 < 6) ? recq[CW_EPI + q15] : ((q15 < 15) ? recq[CW_STATS + q15 - 6] : 0.0);
-            if (q15 == 15) sc.rec2[pq * CORE_WS_TFT + CW_STATS + 9] = 0.0;          // the Gram gather's zero slot
-            __syncwarp();
+            const double* recq = sc.rec2 + hp * CORE_WS_TFT;
+            if (r15 < 15) sc.es[h][es_slot] = (r15 < 6) ? recq[CW_EPI + r15] : recq[CW_STATS + r15 - 6];
         }
 #else
-        // ---- every global load of the pair is issued up front (moments, epipoles, normalisation statistics): one exposed
-        //      memory latency per pair instead of five; the epipoles stay in registers for all three phases
+        // every global load of the pair is issued up front (moments, epipoles, normalisation statistics): one exposed memory
+        // latency per pair
+        const double* mom = sc.mom2[hp];
         {
             double mm[2][3];
 #pragma unroll
@@ -1071,87 +1089,37 @@ tft_stage2_dual_kernel(int normalize, long long B, const double* __restrict__ ws
                 const double* rec = ws + (prob0 + ((p < nprob) ? p : 0)) * CORE_WS_TFT;
                 mm[p][0] = rec[CW_MOM + lane]; mm[p][1] = rec[CW_MOM + 32 + lane]; mm[p][2] = rec[CW_MOM + 64 + lane];
             }
-            // lane 16 p + q: epipoles (q < 6) and normalisation statistics (6 <= q < 15) of problem p -> shared memory
-            const int pq = lane >> 4, q15 = lane & 15;
-            const double* recq = ws + (prob0 + ((pq < nprob) ? pq : 0)) * CORE_WS_TFT;
-            const double ev = (q15 < 6) ? recq[CW_EPI + q15] : ((q15 < 15) ? recq[CW_STATS + q15 - 6] : 0.0);
-            __syncwarp();
+            const double* recq = ws + (prob0 + hp) * CORE_WS_TFT;
+            const double ev = (r15 < 6) ? recq[CW_EPI + r15] : ((r15 < 15) ? recq[CW_STATS + r15 - 6] : 0.0);
 #pragma unroll
             for (int p = 0; p < 2; ++p) {
                 sc.mom2[p][lane] = mm[p][0]; sc.mom2[p][lane + 32] = mm[p][1]; sc.mom2[p][lane + 64] = mm[p][2];
             }
-            if (lane < 4) { sc.mom2[lane >> 1][96 + (lane & 1)] = 0.0; }
-            sc.es[pq][q15] = ev;
+            if (r15 < 15) sc.es[h][es_slot] = ev;
+        }
+#endif
+        __syncwarp();
+        {
+            // orthonormal completions, once per problem: lane 0 of the half -> u1, u2; lane 1 -> v1, v2
+            double* e = sc.es[h] + 9 * (r15 & 1);
+            double u1[3], u2[3];
+            onb3(e, u1, u2);
+            if (r15 < 2) {
+#pragma unroll
+                for (int q = 0; q < 3; ++q) { e[3 + q] = u1[q]; e[6 + q] = u2[q]; }
+            }
             __syncwarp();
         }
-#endif
-        // ---- 27-lane part, problem by problem: W = G*Up (linearTFT.m:82-84 without svd(E), see tft_stage2_kernel) ----
-        for (int p = 0; p < nprob; ++p) {
-#if TVF_S2_TMA
-            const double* mom = sc.rec2 + p * CORE_WS_TFT + CW_MOM;
-#else
-            const double* mom = sc.mom2[p];
-#endif
-            const double e21[3] = {sc.es[p][0], sc.es[p][1], sc.es[p][2]};
-            const double e31[3] = {sc.es[p][3], sc.es[p][4], sc.es[p][5]};
-            double u1[3], u2[3], v1[3], v2[3];
-            onb3(e21, u1, u2);
-            onb3(e31, v1, v2);
-            double Ze[9], Zu1[9], Zu2[9];
-#pragma unroll
-            for (int q = 0; q < 9; ++q) {
-                const double g0 = mom[gidx[lane * 27 + 3 * q]];
-                const double g1 = mom[gidx[lane * 27 + 3 * q + 1]];
-                const double g2 = mom[gidx[lane * 27 + 3 * q + 2]];
-                Ze[q] = g0 * e21[0] + g1 * e21[1] + g2 * e21[2];
-                Zu1[q] = g0 * u1[0] + g1 * u1[1] + g2 * u1[2];
-                Zu2[q] = g0 * u2[0] + g1 * u2[1] + g2 * u2[2];
-            }
-            if (lane < 27) {
-                double* W = sc.W[p] + lane * FEAT_STRIDE;
-#pragma unroll
-                for (int i2 = 0; i2 < 3; ++i2) {
-                    const double* ze = Ze + 3 * i2; const double* zu1 = Zu1 + 3 * i2; const double* zu2 = Zu2 + 3 * i2;
-                    W[5 * i2 + 0] = ze[0] * e31[0] + ze[1] * e31[1] + ze[2] * e31[2];
-                    W[5 * i2 + 1] = ze[0] * v1[0] + ze[1] * v1[1] + ze[2] * v1[2];
-                    W[5 * i2 + 2] = ze[0] * v2[0] + ze[1] * v2[1] + ze[2] * v2[2];
-                    W[5 * i2 + 3] = zu1[0] * e31[0] + zu1[1] * e31[1] + zu1[2] * e31[2];
-                    W[5 * i2 + 4] = zu2[0] * e31[0] + zu2[1] * e31[1] + zu2[2] * e31[2];
-                }
-            }
-        }
+        const double* bh = sc.es[h];
+        form_h15(mom, bh, bh + 9, r15, sc.H[h]);
         __syncwarp();
 #if TVF_S2_TMA
         if (lane == 0 && pair + pstride < npairs) fetch(pair + pstride);       // every lane is done with sc.rec2
 #endif
-        // ---- 15-lane part, both problems at once: half h = problem prob0 + h ------------------------------------
+        // ---- the smallest eigenvector of H (linearTFT.m:84), both problems at once
         {
-            const bool live = h < nprob;
-            const double* eh = sc.es[live ? h : 0];
-            const double e21[3] = {eh[0], eh[1], eh[2]};
-            const double e31[3] = {eh[3], eh[4], eh[5]};
-            double u1[3], u2[3], v1[3], v2[3];
-            onb3(e21, u1, u2);
-            onb3(e31, v1, v2);
-            double pa[3], qa[3];
-#pragma unroll
-            for (int q = 0; q < 3; ++q) {
-                pa[q] = (aa < 3) ? e21[q] : ((aa == 3) ? u1[q] : u2[q]);
-                qa[q] = (aa == 1) ? v1[q] : ((aa == 2) ? v2[q] : e31[q]);
-            }
             double g15[15];
-#pragma unroll
-            for (int c = 0; c < 15; ++c) g15[c] = 0.0;
-            const double* Wh = sc.W[live ? h : 0];
-#pragma unroll
-            for (int k = 0; k < 3; ++k)
-#pragma unroll
-                for (int j = 0; j < 3; ++j) {
-                    const double coef = (r15 < 15) ? pa[j] * qa[k] : 0.0;
-                    const double* W = Wh + (9 * ia + 3 * k + j) * FEAT_STRIDE;
-#pragma unroll
-                    for (int c = 0; c < 15; ++c) g15[c] = fma(coef, W[c], g15[c]);
-                }
+            load_h15_row(sc.H[h], r15, g15);
             if (!live) {                                   // odd batch: the idle half solves the identity
 #pragma unroll
                 for (int c = 0; c < 15; ++c) g15[c] = (c == r15) ? 1.0 : 0.0;
@@ -1163,71 +1131,75 @@ tft_stage2_dual_kernel(int normalize, long long B, const double* __restrict__ ws
             if (live && !conv2 && r15 == 0 && status != nullptr) status[prob0 + h] |= ST_EIG_NOCONV;
         }
         __syncwarp();
-        // ---- back to 27 lanes, problem by problem: t = Up*tp, P2/P3, undo the normalisation -----------------------
-        for (int p = 0; p < nprob; ++p) {
-            const long long prob = prob0 + p;
-            const double e21[3] = {sc.es[p][0], sc.es[p][1], sc.es[p][2]};
-            const double e31[3] = {sc.es[p][3], sc.es[p][4], sc.es[p][5]};
-            const double* st9p = sc.es[p] + 6;
-            double u1[3], u2[3], v1[3], v2[3];
-            onb3(e21, u1, u2);
-            onb3(e31, v1, v2);
-            const double pe = sel3(e21, jr), pu1 = sel3(u1, jr), pu2 = sel3(u2, jr);
-            const double qe = sel3(e31, kr), qv1 = sel3(v1, kr), qv2 = sel3(v2, kr);
-            double acc = 0.0;                                                   // t = Up*tp  (linearTFT.m:85)
-            if (lane < 27) {
-                const double* tp = sc.tp[p] + 5 * ir;
-                acc = pe * (qe * tp[0] + qv1 * tp[1] + qv2 * tp[2]) + qe * (pu1 * tp[3] + pu2 * tp[4]);
-            }
-            const double tl2 = acc * rsqrt_(warp_sum(acc * acc));
-            __syncwarp();
-            if (lane < 27) sc.T[lane] = tl2;
-            __syncwarp();
-            if (P2out != nullptr && P3out != nullptr) {                          // linearTFT.m:86-90, a = pinv(E) t in closed form
-                if (lane < 3) {
-                    const double* Ti = sc.T + 9 * lane;
-                    double a[3], b[3];
-                    mat3_vec(Ti, e31, a);
-                    mat3_tvec(Ti, e21, b);
-                    const double tau = e21[0] * a[0] + e21[1] * a[1] + e21[2] * a[2];
+        // ---- back end, both problems at once: t = Up*tp, P2/P3, undo the normalisation
+        const long long prob = prob0 + h;
+        const double* tp = sc.tp[h];
+        auto up_tp = [&](int e) {                                               // t = Up*tp  (linearTFT.m:85)
+            const int j = e % 3, k = (e / 3) % 3, i = e / 9;
+            const double pe = bh[j], pu1 = bh[3 + j], pu2 = bh[6 + j], qe = bh[9 + k], qv1 = bh[12 + k], qv2 = bh[15 + k];
+            const double* t5 = tp + 5 * i;
+            return pe * (qe * t5[0] + qv1 * t5[1] + qv2 * t5[2]) + qe * (pu1 * t5[3] + pu2 * t5[4]);
+        };
+        double t0 = up_tp(e0), t1 = has1 ? up_tp(e1) : 0.0;
+        {
+            const double nrm = rsqrt_(half_sum(fma(t0, t0, t1 * t1)));
+            t0 *= nrm; t1 *= nrm;
+        }
+        double* Th = sc.T[h];
+        Th[e0] = t0;
+        if (has1) Th[e1] = t1;
+        __syncwarp();
+        if (live && P2out != nullptr && P3out != nullptr) {                      // linearTFT.m:86-90, a = pinv(E) t in closed form
+            const double* e21 = bh;
+            const double* e31 = bh + 9;
+            if (r15 < 3) {
+                const double* Ti = Th + 9 * r15;
+                double a[3], b[3];
+                mat3_vec(Ti, e31, a);
+                mat3_tvec(Ti, e21, b);
+                const double tau = e21[0] * a[0] + e21[1] * a[1] + e21[2] * a[2];
 #pragma unroll
-                    for (int q = 0; q < 3; ++q) {
-                        P2out[prob * 12 + 3 * lane + q] = a[q] - 0.5 * tau * e21[q];
-                        P3out[prob * 12 + 3 * lane + q] = 0.5 * tau * e31[q] - b[q];
-                    }
-                } else if (lane == 3) {
-#pragma unroll
-                    for (int q = 0; q < 3; ++q) { P2out[prob * 12 + 9 + q] = e21[q]; P3out[prob * 12 + 9 + q] = e31[q]; }
+                for (int q = 0; q < 3; ++q) {
+                    P2out[prob * 12 + 3 * r15 + q] = a[q] - 0.5 * tau * e21[q];
+                    P3out[prob * 12 + 3 * r15 + q] = 0.5 * tau * e31[q] - b[q];
                 }
+            } else if (r15 == 3) {
+#pragma unroll
+                for (int q = 0; q < 3; ++q) { P2out[prob * 12 + 9 + q] = e21[q]; P3out[prob * 12 + 9 + q] = e31[q]; }
             }
-            double tout = tl2;
-            if (normalize) {
-                // LinearTFTPoseEstimation.m:53 -> transform_TFT.m:43-49 with the three Normalize2Ddata matrices
-                // N_v = [s 0 tx; 0 s ty; 0 0 1]: T_new(:,:,i) = inv(N2) * (sum_r N1(r,i) T(:,:,r)) * inv(N3).'.  The matrices
-                // are similarities, so the sum over r has at most three terms, inv(N) = [1/s 0 -tx/s; 0 1/s -ty/s; 0 0 1] is
-                // known in closed form, and element (j,k) of the product touches rows {j, 2} and columns {k, 2} only.
-                const double s1 = st9p[0], i2 = rcp_(st9p[1]), i3 = rcp_(st9p[2]);
-                const double t1x = st9p[3], t1y = st9p[4];
+        }
+        if (normalize) {
+            // LinearTFTPoseEstimation.m:53 -> transform_TFT.m:43-49 with the three Normalize2Ddata matrices
+            // N_v = [s 0 tx; 0 s ty; 0 0 1]: T_new(:,:,i) = inv(N2) * (sum_r N1(r,i) T(:,:,r)) * inv(N3).'.  The matrices
+            // are similarities, so the sum over r has at most three terms, inv(N) = [1/s 0 -tx/s; 0 1/s -ty/s; 0 0 1] is
+            // known in closed form, and element (j,k) of the product touches rows {j, 2} and columns {k, 2} only.
+            const double* st9p = bh + 18;
+            const double s1 = st9p[0], i2 = rcp_(st9p[1]), i3 = rcp_(st9p[2]);
+            const double t1x = st9p[3], t1y = st9p[4];
+            auto unnorm = [&](int e) {
+                const int jr = e % 3, kr = (e / 3) % 3, ir = e / 9;
                 // row j of inv(N2): (a2, .., b2): out(j,:) = a2 * S(j,:) + b2 * S(2,:)   (j = 2: a2 = 1, b2 = 0)
                 const double a2 = (jr == 2) ? 1.0 : i2, b2 = (jr == 0) ? -st9p[5] * i2 : ((jr == 1) ? -st9p[6] * i2 : 0.0);
                 const double a3 = (kr == 2) ? 1.0 : i3, b3 = (kr == 0) ? -st9p[7] * i3 : ((kr == 1) ? -st9p[8] * i3 : 0.0);
-                double acc2 = 0.0;
-                if (lane < 27) {
-                    // S(j',k') of slice i: i = 0,1: s1 * T_i;  i = 2: t1x T_0 + t1y T_1 + T_2
-                    auto S = [&](int jj, int kk) -> double {
-                        const int e = jj + 3 * kk;
-                        if (ir == 2) return fma(t1x, sc.T[e], fma(t1y, sc.T[9 + e], sc.T[18 + e]));
-                        return s1 * sc.T[9 * ir + e];
-                    };
-                    const double sjk = S(jr, kr), s2k = S(2, kr), sj2 = S(jr, 2), s22 = S(2, 2);
-                    // out(j,k) = sum_{j',k'} inv2(j,j') S(j',k') inv3(k,k') over j' in {j,2}, k' in {k,2}
-                    acc2 = a3 * (a2 * sjk + b2 * s2k) + b3 * (a2 * sj2 + b2 * s22);
-                }
-                tout = acc2 * rsqrt_(warp_sum(acc2 * acc2));                       // :49
-            }
-            if (lane < 27) Tout[prob * 27 + lane] = tout;
-            __syncwarp();                                                        // sc.T is reused by the next problem
+                // S(j',k') of slice i: i = 0,1: s1 * T_i;  i = 2: t1x T_0 + t1y T_1 + T_2
+                auto S = [&](int jj, int kk) -> double {
+                    const int x = jj + 3 * kk;
+                    if (ir == 2) return fma(t1x, Th[x], fma(t1y, Th[9 + x], Th[18 + x]));
+                    return s1 * Th[9 * ir + x];
+                };
+                const double sjk = S(jr, kr), s2k = S(2, kr), sj2 = S(jr, 2), s22 = S(2, 2);
+                // out(j,k) = sum_{j',k'} inv2(j,j') S(j',k') inv3(k,k') over j' in {j,2}, k' in {k,2}
+                return a3 * (a2 * sjk + b2 * s2k) + b3 * (a2 * sj2 + b2 * s22);
+            };
+            t0 = unnorm(e0); t1 = has1 ? unnorm(e1) : 0.0;
+            const double nrm = rsqrt_(half_sum(fma(t0, t0, t1 * t1)));                // :49
+            t0 *= nrm; t1 *= nrm;
         }
+        if (live) {
+            Tout[prob * 27 + e0] = t0;
+            if (has1) Tout[prob * 27 + e1] = t1;
+        }
+        __syncwarp();                                                            // sc.es, sc.T are reused by the next pair
     }
 }
 
