@@ -48,6 +48,8 @@ typedef struct tvf_context* tvf_handle_t;
 #define TVF_ST_NO_POSE_3 8
 #define TVF_ST_NONFINITE 16    /* non-finite value in R_t / reprojection error                                */
 #define TVF_ST_BA_NOCONV 32    /* tvf_bundle_adjust: iteration cap reached before the stopping rule held          */
+#define TVF_ST_COV_SINGULAR 64 /* tvf_ba_covariance: reduced camera system or a point block not positive definite:
+                                  covariance undefined                                                            */
 
 /* the message linearF.m:36 raises; gateways re-raise it verbatim */
 #define TVF_LINEARF_ERRMSG \
@@ -232,6 +234,36 @@ int tvf_bundle_adjust(tvf_handle_t h, const double* corresp, const double* calm,
 int tvf_bundle_adjust_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                           const double* Rt2_0, const double* Rt3_0, const double* reconst0, double* Rt2, double* Rt3,
                           double* reconst, double* repr_err, int32_t* iter, int32_t* status);
+
+/* ---- first-order covariance of the bundle adjustment at a state ------------------------------------------------
+ * The uncertainty of tvf_bundle_adjust's result: the inverse of the Gauss-Newton matrix H = J'J of the adjustment's
+ * model (pixel residuals, camera 1 = K1[I|0], |t2| = 1), taken at the given state without damping.  The state (Rt2, Rt3
+ * 3 x 4 x B, reconst 3 x n x B Euclidean, all required) is usually tvf_bundle_adjust's output, but any state is accepted;
+ * it is first put into the adjustment's gauge exactly as tvf_bundle_adjust does (t2, t3 and the points scaled by
+ * 1/|t2|).  corresp, calm, calm_batched and n as for tvf_bundle_adjust; n < 4 -> TVF_ERR_ARG.
+ *
+ * Chart: the adjustment's 11 camera unknowns at the state, R2 <- exp([w2]x) R2, t2 moved by a in its tangent plane
+ * (basis u1, u2), R3 <- exp([w3]x) R3, t3 <- t3 + dt3, and the points additively.  The camera block of H^-1 is S^-1,
+ * S the 11 x 11 reduced camera system (the points eliminated); the chart covariance C = S^-1 is expanded with
+ * G = blkdiag(I3, [u1 u2], I3, I3) to
+ *   cov_cam (12 x 12 x B, column-major, may be NULL) = G C G' over [w2 (3), dt2 (3, ambient), w3 (3), dt3 (3)]:
+ *           rank 11, null direction (0, t2, 0, 0); independent of the tangent basis;
+ *   cov_pts (3 x 3 x n x B, may be NULL): the marginal covariance of each point in the gauge-normalised frame,
+ *           V_i^-1 + V_i^-1 W_i' S^-1 W_i V_i^-1 (V_i = the point's 3 x 3 block of H, W_i its 11 x 3 camera block);
+ *   sigma2  (B, may be NULL): the a-posteriori noise variance sum r^2 / (3n - 11) (6n residuals, 11 + 3n unknowns).
+ * Both covariances are for UNIT pixel noise: multiply by sigma^2 (for example sigma2) for another noise level.
+ * status (B, may be NULL): TVF_ST_NONFINITE for a non-finite input, residual or |t2| = 0; TVF_ST_COV_SINGULAR when a
+ * point block V_i or S is not positive definite, where a Cholesky pivot counts as positive only above 1e-12 times the
+ * matrix's own diagonal entry.  Either way every output of that problem is NaN.  Every sum depends on the problem alone:
+ * a result is bit-identical whatever its batch, chunk (tvf_set_chunk), group-handle shard or _dev form.  The host form
+ * chunks and shards like tvf_bundle_adjust; the _dev form takes device pointers (corresp 16-byte aligned) and is
+ * asynchronous on the handle's stream. */
+int tvf_ba_covariance(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
+                      const double* Rt2, const double* Rt3, const double* reconst, double* cov_cam, double* cov_pts,
+                      double* sigma2, int32_t* status);
+int tvf_ba_covariance_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
+                          const double* Rt2, const double* Rt3, const double* reconst, double* cov_cam, double* cov_pts,
+                          double* sigma2, int32_t* status);
 
 /* ---- inputs of the measured configurations, generated where they are consumed ------------------------
  * Trials [first_trial, first_trial+B) of experiments.m's sweep: trial j uses noise_levels[j mod L] and

@@ -290,9 +290,13 @@ def AngError(R_t_true, R_t_est, device=None):
 
 
 class BundleAdjustResult(tuple):
-    """(R_t_2, R_t_3, Reconst, iter) of bundle_adjust, plus .repr_err and .status."""
+    """(R_t_2, R_t_3, Reconst, iter) of bundle_adjust, plus .repr_err and .status.  epfl.run_real(covariance=True) also
+    sets .sigma2 and the predicted RMS errors .pred_rot_err, .pred_t_err (degrees, mean of views 2 and 3)."""
     repr_err = None
     status = None
+    sigma2 = None
+    pred_rot_err = None
+    pred_t_err = None
 
 
 def bundle_adjust(Corresp, CalM, R_t_2, R_t_3, Reconst=None, device=None):
@@ -325,6 +329,67 @@ def bundle_adjust(Corresp, CalM, R_t_2, R_t_3, Reconst=None, device=None):
     out.repr_err = rep if batched else float(rep[0])
     out.status = st if batched else int(st[0])
     return out
+
+
+class CovarianceResult(tuple):
+    """(cov_cam, sigma2) of ba_covariance, plus .cov_pts (None unless points=True) and .status."""
+    cov_pts = None
+    status = None
+
+
+def ba_covariance(Corresp, CalM, R_t_2, R_t_3, Reconst, points=False, device=None):
+    """First-order covariance of the bundle adjustment at the state (R_t_2, R_t_3, Reconst), usually bundle_adjust's
+    result (tvf_ba_covariance, include/tvf.h).  The state is first scaled to |t2| = 1 as bundle_adjust does.  Returns
+    (cov_cam, sigma2): cov_cam 12x12 over [w2, dt2, w3, dt3] (rotation vectors R <- exp([w]x) R and translation
+    perturbations, rank 11, null direction (0, t2, 0, 0)), for UNIT pixel noise -- multiply by sigma2, the a-posteriori
+    noise variance sum r^2 / (3N - 11), or by any other sigma^2.  points=True also fills .cov_pts, 3x3xN (the marginal
+    covariance of each point in the gauge-normalised frame, unit noise).  .status: TVF_ST_* bits (NONFINITE,
+    COV_SINGULAR); a flagged problem's outputs are NaN.  Batched like bundle_adjust: cov_cam (B,12,12), sigma2 (B,),
+    cov_pts (B,3,3,N)."""
+    c, batched, B = _cm(Corresp, 2)
+    if c.shape[2] != 6:
+        raise ValueError("Corresp must be 6xN")
+    n = c.shape[1]
+    calm, cb = _calm(CalM, B)
+    r2, _, _ = _cm(np.broadcast_to(R_t_2, (B, 3, 4)) if batched else R_t_2, 2)
+    r3, _, _ = _cm(np.broadcast_to(R_t_3, (B, 3, 4)) if batched else R_t_3, 2)
+    x, _, _ = _cm(Reconst, 2)
+    if r2.shape != (B, 4, 3) or r3.shape != (B, 4, 3):
+        raise ValueError("R_t_2, R_t_3 must be 3x4 (with the batch axis of Corresp)")
+    if x.shape != (B, n, 3):
+        raise ValueError("Reconst must be 3xN (with the batch axis of Corresp)")
+    h = _lib.handle(device)
+    cc = np.empty((B, 144)); s2 = np.empty(B); st = np.zeros(B, dtype=np.int32)
+    cp = np.empty((B, 9 * n)) if points else None
+    h.call("tvf_ba_covariance", _p(c), _p(calm), cb, n, B, _p(r2), _p(r3), _p(x), _p(cc), _p(cp), _p(s2),
+           st.ctypes.data_as(_ip))
+    out = CovarianceResult((_from_cm(cc, B, (12, 12), batched), s2 if batched else float(s2[0])))
+    if points:
+        out.cov_pts = _from_cm(cp, B, (3, 3, n), batched)
+    out.status = st if batched else int(st[0])
+    return out
+
+
+def pose_rms_errors(cov_cam, R_t_2, R_t_3, sigma2=1.0):
+    """First-order RMS of the errors AngError measures (auxiliar_functions/AngError.m), in degrees, from a 12x12
+    cov_cam of ba_covariance (unit noise) scaled by sigma2: returns (rot_err, t_err), each [view 2, view 3] (shape (2,),
+    or (B,2) for batched inputs).  Rotation: sqrt(trace Sigma_w); t2 direction: sqrt(trace Sigma_t2) (|t2| = 1 in the
+    covariance's gauge); t3 direction: the t3 block projected on the tangent plane of t3/|t3|, over |t3|^2.  R_t_2 and
+    R_t_3 are the state the covariance was taken at (any scale: t3 is taken relative to |t2|)."""
+    cov = np.asarray(cov_cam, dtype=np.float64)
+    batched = cov.ndim == 3
+    cov = cov if batched else cov[None]
+    s2 = np.broadcast_to(np.asarray(sigma2, dtype=np.float64), cov.shape[:1])
+    t2 = np.asarray(R_t_2, dtype=np.float64).reshape(-1, 3, 4)[:, :, 3]
+    t3 = np.asarray(R_t_3, dtype=np.float64).reshape(-1, 3, 4)[:, :, 3] / np.linalg.norm(t2, axis=1)[:, None]
+    d3 = t3 / np.linalg.norm(t3, axis=1)[:, None]
+    P = np.eye(3) - d3[:, :, None] * d3[:, None, :]
+    tr = lambda k: np.trace(cov[:, k:k + 3, k:k + 3], axis1=1, axis2=2)
+    t3v = np.trace(P @ cov[:, 9:12, 9:12] @ P, axis1=1, axis2=2) / np.sum(t3 * t3, axis=1)
+    deg = 180.0 / np.pi
+    rot = np.sqrt(s2[:, None] * np.stack([tr(0), tr(6)], 1)) * deg
+    tdir = np.sqrt(s2[:, None] * np.stack([tr(3), t3v], 1)) * deg
+    return (rot, tdir) if batched else (rot[0], tdir[0])
 
 
 def crossM(v):

@@ -551,46 +551,59 @@ int pose_dev(tvf_handle_t h, Method method, const double* corresp, const double*
     return TVF_OK;
 }
 
-// ---- bundle adjustment (tvf_bundle_adjust[_dev]) ----------------------------------------------------------------------
-// one call's arrays (host or device pointers); outputs may be null except Rt2 / Rt3
+// ---- bundle adjustment (tvf_bundle_adjust[_dev]) and its covariance (tvf_ba_covariance[_dev]) ------------------------
+// one call's arrays (host or device pointers).  Adjustment: outputs may be null except Rt2 / Rt3.  Covariance (cov):
+// the state is Rt2_0, Rt3_0, X0 (all required) and the outputs cov_cam, cov_pts, sigma2, status may be null.
 struct BaIo {
     const double* corresp; const double* calm; int calm_batched; int n;
     const double* Rt2_0; const double* Rt3_0; const double* X0;
     double* Rt2; double* Rt3; double* X; double* repr; int32_t* iter; int32_t* status;
+    bool cov; double* cov_cam; double* cov_pts; double* sigma2;
     BaIo shifted(int64_t lo) const {           // problems [lo, ...)
         BaIo s = *this;
         s.corresp += lo * 6 * n;
         if (calm_batched) s.calm += lo * 27;
-        s.Rt2_0 += lo * 12; s.Rt3_0 += lo * 12; s.Rt2 += lo * 12; s.Rt3 += lo * 12;
+        s.Rt2_0 += lo * 12; s.Rt3_0 += lo * 12;
+        if (s.Rt2) s.Rt2 += lo * 12;
+        if (s.Rt3) s.Rt3 += lo * 12;
         if (s.X0) s.X0 += lo * 3 * n;
         if (s.X) s.X += lo * 3 * n;
         if (s.repr) s.repr += lo;
         if (s.iter) s.iter += lo;
         if (s.status) s.status += lo;
+        if (s.cov_cam) s.cov_cam += lo * 144;
+        if (s.cov_pts) s.cov_pts += lo * 9 * n;
+        if (s.sigma2) s.sigma2 += lo;
         return s;
     }
 };
 
 int check_ba_args(tvf_handle_t h, const BaIo& io, int64_t B) {
     if (!h) return TVF_ERR_ARG;
-    if (!io.corresp || !io.calm || !io.Rt2_0 || !io.Rt3_0 || !io.Rt2 || !io.Rt3)
+    if (io.cov) {
+        if (!io.corresp || !io.calm || !io.Rt2_0 || !io.Rt3_0 || !io.X0)
+            return fail(h, TVF_ERR_ARG, "ba_covariance: corresp, calm, Rt2, Rt3 and reconst must not be NULL");
+    } else if (!io.corresp || !io.calm || !io.Rt2_0 || !io.Rt3_0 || !io.Rt2 || !io.Rt3) {
         return fail(h, TVF_ERR_ARG, "bundle_adjust: corresp, calm, Rt2_0, Rt3_0, Rt2 and Rt3 must not be NULL");
+    }
     if (B < 0) return fail(h, TVF_ERR_ARG, "bundle_adjust: B >= 0");
     if (io.n < 4) return fail(h, TVF_ERR_ARG, "bundle_adjust: needs n >= 4 points (11 + 3n unknowns, 6n residuals)");
     return TVF_OK;
 }
 
-// per-problem device bytes of a chunk: host_io -> inputs and outputs too; always the two point buffers
-size_t ba_bytes_per_problem(int n, bool host_io) {
+// per-problem device bytes of a chunk: host_io -> inputs and outputs too; the adjustment always has its two point buffers
+size_t ba_bytes_per_problem(int n, bool host_io, bool cov) {
+    if (cov) return host_io ? (size_t)(6 * n + 27 + 24 + 3 * n + 144 + 9 * n + 1 + 1) * sizeof(double) : 0;
     size_t b = (size_t)2 * 3 * n * sizeof(double);
     if (host_io) b += (size_t)(6 * n + 27 + 24 + 3 * n + 24 + 1) * sizeof(double) + 2 * sizeof(int32_t);
     return b;
 }
 
-int64_t pick_chunk_ba(tvf_handle_t h, int n, int64_t B, bool host_io) {
+int64_t pick_chunk_ba(tvf_handle_t h, int n, int64_t B, bool host_io, bool cov = false) {
     int64_t c = h->chunk_user > 0 ? h->chunk_user : (host_io ? DEFAULT_CHUNK : DEFAULT_CHUNK_DEV);
-    if (h->chunk_user <= 0) {
-        const int64_t fit = (int64_t)((host_io ? ARENA_BUDGET : 8 * ARENA_BUDGET) / ba_bytes_per_problem(n, host_io));
+    const size_t per = ba_bytes_per_problem(n, host_io, cov);
+    if (h->chunk_user <= 0 && per > 0) {
+        const int64_t fit = (int64_t)((host_io ? ARENA_BUDGET : 8 * ARENA_BUDGET) / per);
         if (c > fit) c = fit;
     }
     if (c < 1) c = 1;
@@ -599,11 +612,21 @@ int64_t pick_chunk_ba(tvf_handle_t h, int n, int64_t B, bool host_io) {
 }
 
 // device copies of one host chunk of C problems in a slot arena (base = nullptr: size only)
-size_t carve_ba(char* base, int n, int64_t C, int calm_batched, BaIo* d, double** Xc) {
+// (the covariance's chunk: inputs, cov_cam and cov_pts when the caller wants them, sigma2, status)
+size_t carve_ba(char* base, int n, int64_t C, const BaIo& io, BaIo* d, double** Xc) {
     Carver c(base);
-    d->corresp = c.take<double>((size_t)6 * n * C); d->calm = c.take<double>(calm_batched ? 27 * C : 27);
-    d->calm_batched = calm_batched; d->n = n;
+    *d = BaIo{};
+    d->cov = io.cov;
+    d->corresp = c.take<double>((size_t)6 * n * C); d->calm = c.take<double>(io.calm_batched ? 27 * C : 27);
+    d->calm_batched = io.calm_batched; d->n = n;
     d->Rt2_0 = c.take<double>(12 * C); d->Rt3_0 = c.take<double>(12 * C); d->X0 = c.take<double>((size_t)3 * n * C);
+    if (io.cov) {
+        d->cov_cam = io.cov_cam ? c.take<double>(144 * C) : nullptr;
+        d->cov_pts = io.cov_pts ? c.take<double>((size_t)9 * n * C) : nullptr;
+        d->sigma2 = c.take<double>(C); d->status = c.take<int32_t>(C);
+        *Xc = nullptr;
+        return c.off;
+    }
     d->Rt2 = c.take<double>(12 * C); d->Rt3 = c.take<double>(12 * C); d->X = c.take<double>((size_t)3 * n * C);
     *Xc = c.take<double>((size_t)3 * n * C);
     d->repr = c.take<double>(C); d->iter = c.take<int32_t>(C); d->status = c.take<int32_t>(C);
@@ -611,10 +634,19 @@ size_t carve_ba(char* base, int n, int64_t C, int calm_batched, BaIo* d, double*
 }
 
 int ba_launch(tvf_handle_t h, cudaStream_t st, const BaIo& d, int64_t Bc, double* Xc) {
-    BaArgs a{d.corresp, d.calm, d.calm_batched, d.n, Bc, d.Rt2_0, d.Rt3_0, d.X0, d.Rt2, d.Rt3, d.X, Xc, d.repr, d.iter, d.status};
-    const int ok = launch_bundle_adjust(a, st);
+    int ok;
+    if (d.cov) {
+        BaCovArgs a{d.corresp, d.calm, d.calm_batched, d.n, Bc, d.Rt2_0, d.Rt3_0, d.X0, d.cov_cam, d.cov_pts, d.sigma2, d.status};
+        ok = launch_ba_covariance(a, st);
+    } else {
+        BaArgs a{d.corresp, d.calm, d.calm_batched, d.n, Bc, d.Rt2_0, d.Rt3_0, d.X0, d.Rt2, d.Rt3, d.X, Xc, d.repr, d.iter, d.status};
+        ok = launch_bundle_adjust(a, st);
+    }
     h->launches += 1;
-    if (!ok) { cudaError_t e = cudaGetLastError(); return fail(h, TVF_ERR_CUDA, std::string("bundle_adjust_kernel: ") + cudaGetErrorString(e)); }
+    if (!ok) {
+        cudaError_t e = cudaGetLastError();
+        return fail(h, TVF_ERR_CUDA, std::string(d.cov ? "ba_covariance_kernel: " : "bundle_adjust_kernel: ") + cudaGetErrorString(e));
+    }
     return TVF_OK;
 }
 
@@ -622,7 +654,7 @@ int ba_host_one(tvf_handle_t h, const BaIo& io, int64_t B) {
     if (B == 0) return TVF_OK;
     TVF_CK(cudaSetDevice(h->device));
     const int n = io.n;
-    const int64_t C = pick_chunk_ba(h, n, B, true);
+    const int64_t C = pick_chunk_ba(h, n, B, true, io.cov);
     std::vector<int32_t> st_tmp;
     int32_t* st_host = io.status;
     if (!st_host) { st_tmp.resize((size_t)B); st_host = st_tmp.data(); }
@@ -634,8 +666,8 @@ int ba_host_one(tvf_handle_t h, const BaIo& io, int64_t B) {
         Slot& s = h->slot[ci % NSLOT];
         TVF_CK(cudaStreamSynchronize(s.stream));            // the slot's previous chunk (with its copies back) is done
         BaIo d{}; double* Xc;
-        rc = ensure_arena(h, s, carve_ba(nullptr, n, C, io.calm_batched, &d, &Xc)); if (rc) return rc;
-        carve_ba(s.arena, n, C, io.calm_batched, &d, &Xc);
+        rc = ensure_arena(h, s, carve_ba(nullptr, n, C, io, &d, &Xc)); if (rc) return rc;
+        carve_ba(s.arena, n, C, io, &d, &Xc);
         double* x0 = const_cast<double*>(d.X0);
         if (!io.X0) d.X0 = nullptr;
         double* in = const_cast<double*>(d.corresp); double* calm = const_cast<double*>(d.calm);
@@ -651,11 +683,17 @@ int ba_host_one(tvf_handle_t h, const BaIo& io, int64_t B) {
         TVF_CK(up(r3, hio.Rt3_0, (size_t)Bc * 12 * sizeof(double)));
         if (io.X0) TVF_CK(up(x0, hio.X0, (size_t)Bc * 3 * n * sizeof(double)));
         rc = ba_launch(h, s.stream, d, Bc, Xc); if (rc) return rc;
-        TVF_CK(down(hio.Rt2, d.Rt2, (size_t)Bc * 12 * sizeof(double)));
-        TVF_CK(down(hio.Rt3, d.Rt3, (size_t)Bc * 12 * sizeof(double)));
-        TVF_CK(down(hio.X, d.X, (size_t)Bc * 3 * n * sizeof(double)));
-        TVF_CK(down(hio.repr, d.repr, (size_t)Bc * sizeof(double)));
-        TVF_CK(down(hio.iter, d.iter, (size_t)Bc * sizeof(int32_t)));
+        if (io.cov) {
+            TVF_CK(down(hio.cov_cam, d.cov_cam, (size_t)Bc * 144 * sizeof(double)));
+            TVF_CK(down(hio.cov_pts, d.cov_pts, (size_t)Bc * 9 * n * sizeof(double)));
+            TVF_CK(down(hio.sigma2, d.sigma2, (size_t)Bc * sizeof(double)));
+        } else {
+            TVF_CK(down(hio.Rt2, d.Rt2, (size_t)Bc * 12 * sizeof(double)));
+            TVF_CK(down(hio.Rt3, d.Rt3, (size_t)Bc * 12 * sizeof(double)));
+            TVF_CK(down(hio.X, d.X, (size_t)Bc * 3 * n * sizeof(double)));
+            TVF_CK(down(hio.repr, d.repr, (size_t)Bc * sizeof(double)));
+            TVF_CK(down(hio.iter, d.iter, (size_t)Bc * sizeof(int32_t)));
+        }
         TVF_CK(down(st_host + done, d.status, (size_t)Bc * sizeof(int32_t)));
         done += Bc; ++ci;
     }
@@ -702,16 +740,19 @@ int ba_dev(tvf_handle_t h, const BaIo& io, int64_t B) {
     TVF_CK(cudaSetDevice(h->device));
     Slot& s = h->slot[0];
     cudaStream_t st = h->use_user_stream ? h->user_stream : s.stream;
-    const int64_t C = pick_chunk_ba(h, io.n, B, false);
-    const size_t pts = (size_t)3 * io.n * C;
-    rc = ensure_arena(h, s, 2 * pts * sizeof(double) + 512); if (rc) return rc;
-    Carver c(s.arena);
-    double* Xc = c.take<double>(pts);
-    double* Xw = c.take<double>(pts);
+    const int64_t C = pick_chunk_ba(h, io.n, B, false, io.cov);
+    double* Xc = nullptr; double* Xw = nullptr;
+    if (!io.cov) {                                           // the adjustment's work space; the covariance needs none
+        const size_t pts = (size_t)3 * io.n * C;
+        rc = ensure_arena(h, s, 2 * pts * sizeof(double) + 512); if (rc) return rc;
+        Carver c(s.arena);
+        Xc = c.take<double>(pts);
+        Xw = c.take<double>(pts);
+    }
     for (int64_t done = 0; done < B; done += C) {
         const int64_t Bc = (B - done < C) ? (B - done) : C;
         BaIo d = io.shifted(done);
-        if (!io.X) d.X = Xw;
+        if (!io.cov && !io.X) d.X = Xw;
         rc = ba_launch(h, st, d, Bc, Xc); if (rc) return rc;
     }
     return TVF_OK;
@@ -1516,6 +1557,20 @@ int tvf_bundle_adjust_dev(tvf_handle_t h, const double* corresp, const double* c
                           const double* Rt2_0, const double* Rt3_0, const double* reconst0, double* Rt2, double* Rt3,
                           double* reconst, double* repr_err, int32_t* iter, int32_t* status) {
     return ba_dev(h, BaIo{corresp, calm, calm_batched, n, Rt2_0, Rt3_0, reconst0, Rt2, Rt3, reconst, repr_err, iter, status}, B);
+}
+
+int tvf_ba_covariance(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
+                      const double* Rt2, const double* Rt3, const double* reconst, double* cov_cam, double* cov_pts,
+                      double* sigma2, int32_t* status) {
+    return ba_host(h, BaIo{corresp, calm, calm_batched, n, Rt2, Rt3, reconst, nullptr, nullptr, nullptr, nullptr, nullptr,
+                           status, true, cov_cam, cov_pts, sigma2}, B);
+}
+
+int tvf_ba_covariance_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
+                          const double* Rt2, const double* Rt3, const double* reconst, double* cov_cam, double* cov_pts,
+                          double* sigma2, int32_t* status) {
+    return ba_dev(h, BaIo{corresp, calm, calm_batched, n, Rt2, Rt3, reconst, nullptr, nullptr, nullptr, nullptr, nullptr,
+                          status, true, cov_cam, cov_pts, sigma2}, B);
 }
 
 int tvf_ang_error(tvf_handle_t h, const double* Rt_true, int true_batched, const double* Rt_est, int64_t B,

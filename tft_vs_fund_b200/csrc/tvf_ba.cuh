@@ -305,4 +305,109 @@ TVF_HD bool ba_solve_reduced(double* red, double mu, double* dc) {
     return finite;
 }
 
+// ---- first-order covariance at a state (tvf_ba_covariance, tvf_ba_cov_kernels.cu) -------------------------------
+// H = J'J at mu = 0.  The camera block of H^-1 is S^-1 (S = the reduced matrix of ba_point_accumulate); point i's block
+// is V_i^-1 + V_i^-1 H_pc,i S^-1 H_cp,i V_i^-1 = L^-T (I + W S^-1 W') L^-1 with V_i = L L' and W = L^-1 H_pc,i.
+// A pivot of a Cholesky factorisation (of a V_i or of S) counts as positive only if it exceeds BA_COV_PIVOT times the
+// matrix's own diagonal entry: below that, 1/pivot carries fewer than ~4 correct digits and the covariance is undefined.
+constexpr double BA_COV_PIVOT = 1e-12;
+constexpr int ST_COV_SINGULAR = 64;       // TVF_ST_COV_SINGULAR
+
+// the point block V = H_pp of ba_point_eliminate(p, 0, e) passes the relative pivot floor (e.L[0]^2 = e.d[0])
+TVF_HD bool ba_cov_point_ok(const BaElim& e) {
+    return (e.L[0] > 0.0) && (e.L[2] * e.L[2] > BA_COV_PIVOT * e.d[1]) && (e.L[5] * e.L[5] > BA_COV_PIVOT * e.d[2]);
+}
+
+// Cholesky S = U'U in place on the 66 upper-triangle entries of the reduced matrix; false if a pivot is not above
+// BA_COV_PIVOT times S's diagonal entry (or is NaN)
+TVF_HD bool ba_cov_factor(double* U) {
+#pragma unroll 1
+    for (int i = 0; i < BA_NC; ++i) {
+#pragma unroll 1
+        for (int j = 0; j <= i; ++j) {
+            double s = U[ba_tri(j, i)];
+            for (int k = 0; k < j; ++k) s -= U[ba_tri(k, i)] * U[ba_tri(k, j)];
+            if (i == j) {
+                if (!(s > 0.0 && s > BA_COV_PIVOT * U[ba_tri(i, i)])) return false;
+                U[ba_tri(i, i)] = sqrt(s);
+            } else {
+                U[ba_tri(j, i)] = s / U[ba_tri(j, j)];
+            }
+        }
+    }
+    return true;
+}
+
+// column j of S^-1 from the factor of ba_cov_factor: U'y = e_j, U x = y
+TVF_HD void ba_cov_column(const double* U, int j, double* x) {
+    double y[BA_NC];
+#pragma unroll 1
+    for (int i = 0; i < BA_NC; ++i) {
+        double s = (i == j) ? 1.0 : 0.0;
+        for (int k = 0; k < i; ++k) s -= U[ba_tri(k, i)] * y[k];
+        y[i] = s / U[ba_tri(i, i)];
+    }
+#pragma unroll 1
+    for (int i = BA_NC - 1; i >= 0; --i) {
+        double s = y[i];
+        for (int k = i + 1; k < BA_NC; ++k) s -= U[ba_tri(i, k)] * x[k];
+        x[i] = s / U[ba_tri(i, i)];
+    }
+}
+
+// entry (i, j) of G C G', G = blkdiag(I3, [u1 u2], I3, I3) (12 x 11): the chart covariance C (11 x 11, column-major)
+// in the basis-free coordinates [w2, dt2 (ambient), w3, dt3].  Callers form i <= j and mirror, so the result is
+// symmetric bit for bit.
+TVF_HD double ba_cov_expand(const double* C, const double* u1, const double* u2, int i, int j) {
+    double gi[2], gj[2];
+    int ci = i < 3 ? i : (i < 6 ? 3 : i - 1), cj = j < 3 ? j : (j < 6 ? 3 : j - 1);   // first chart column of the row
+    const int ni = (i >= 3 && i < 6) ? 2 : 1, nj = (j >= 3 && j < 6) ? 2 : 1;
+    gi[0] = ni == 2 ? u1[i - 3] : 1.0; gi[1] = ni == 2 ? u2[i - 3] : 0.0;
+    gj[0] = nj == 2 ? u1[j - 3] : 1.0; gj[1] = nj == 2 ? u2[j - 3] : 0.0;
+    double s = 0.0;
+    for (int a = 0; a < ni; ++a)
+        for (int b = 0; b < nj; ++b) s += gi[a] * C[(ci + a) + BA_NC * (cj + b)] * gj[b];
+    return s;
+}
+
+// point i's 3 x 3 marginal covariance (column-major, symmetric bit for bit) from its elimination at mu = 0 and the
+// camera covariance C = S^-1 (11 x 11, column-major): L^-T (I + W C W') L^-1
+TVF_HD void ba_cov_point(const BaElim& e, const double* C, double* cov) {
+    double T[3][BA_NC], M[3][3], Li[3][3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k)
+#pragma unroll 1
+        for (int b = 0; b < BA_NC; ++b) {
+            double s = 0.0;
+            for (int a = 0; a < BA_NC; ++a) s += e.W[k][a] * C[a + BA_NC * b];
+            T[k][b] = s;
+        }
+#pragma unroll
+    for (int k = 0; k < 3; ++k)
+#pragma unroll
+        for (int l = k; l < 3; ++l) {
+            double s = (k == l) ? 1.0 : 0.0;
+#pragma unroll 1
+            for (int b = 0; b < BA_NC; ++b) s += T[k][b] * e.W[l][b];
+            M[k][l] = s; M[l][k] = s;
+        }
+    const double l00 = e.L[0], l10 = e.L[1], l11 = e.L[2], l20 = e.L[3], l21 = e.L[4], l22 = e.L[5];
+    Li[0][0] = 1.0 / l00; Li[1][1] = 1.0 / l11; Li[2][2] = 1.0 / l22;
+    Li[1][0] = -l10 * Li[0][0] * Li[1][1];
+    Li[2][1] = -l21 * Li[1][1] * Li[2][2];
+    Li[2][0] = -(l20 * Li[0][0] + l21 * Li[1][0]) * Li[2][2];
+    Li[0][1] = 0.0; Li[0][2] = 0.0; Li[1][2] = 0.0;
+#pragma unroll
+    for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int b = a; b < 3; ++b) {
+            double s = 0.0;
+#pragma unroll
+            for (int k = 0; k < 3; ++k)
+#pragma unroll
+                for (int l = 0; l < 3; ++l) s += Li[k][a] * M[k][l] * Li[l][b];
+            cov[a + 3 * b] = s; cov[b + 3 * a] = s;
+        }
+}
+
 }  // namespace tvf

@@ -66,6 +66,24 @@ struct BaArgs {
 };
 int launch_bundle_adjust(const BaArgs& a, cudaStream_t stream);
 
+// ---- covariance of the bundle adjustment at a state (tvf_ba_cov_kernels.cu).  Device pointers; cov_cam, cov_pts,
+// sigma2 and status may be null.  Returns 0 if the launch failed.
+struct BaCovArgs {
+    const double* corresp;     // 6 x n x B, 16-byte aligned
+    const double* calm;        // 9 x 3 (shared) or 9 x 3 x B
+    int calm_batched;
+    int n;
+    long long B;
+    const double* Rt2;         // 12 x B
+    const double* Rt3;         // 12 x B
+    const double* X;           // 3 x n x B
+    double* cov_cam;           // 144 x B
+    double* cov_pts;           // 9 x n x B
+    double* sigma2;            // B
+    int* status;               // B
+};
+int launch_ba_covariance(const BaCovArgs& a, cudaStream_t stream);
+
 // ---- pose tail -----------------------------------------------------------------------------
 struct PoseTailArgs {
     const double* corresp;     // 6 x n x B

@@ -102,7 +102,7 @@ def prepare_triplet(data, it, repr_err_th=1.0, device=None):
 
 
 def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), device=None, details=None,
-             bundle_adjust=False):
+             bundle_adjust=False, covariance=False):
     """The linear-method part of experiments_real.m:75-138.  `data`: a Dataset or the path of a dataset directory;
     `triplets_to_test`: rows of indexes_sorted (1-based; the reference uses 1:70 / 1:50, :31-36).  Per loop index `it`:
     pre-filter (:94-101), sample min(100, N) inliers with rng(it) (:103-105; documented stand-in for MATLAB's
@@ -113,7 +113,11 @@ def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), de
     bundle_adjust=True: each method's pose is then refined by api.bundle_adjust on the same sample, from the method's
     R_t_2, R_t_3 and Reconst -- the library's three-view adjustment, not the reference's BundleAdjustment.m (DESIGN.md
     section 8) -- and the adjusted cameras are evaluated exactly as the method's.  Each entry is then (T, 6): the three
-    errors of the method, then the same three after the adjustment; details[k]["ba"][m] holds the adjusted result."""
+    errors of the method, then the same three after the adjustment; details[k]["ba"][m] holds the adjusted result.
+    covariance=True (with bundle_adjust): api.ba_covariance is also taken at each adjusted pose, and
+    details[k]["ba"][m] gets .sigma2 (the a-posteriori pixel noise variance of the sample) and the predicted RMS
+    rotation / translation errors .pred_rot_err, .pred_t_err (degrees, api.pose_rms_errors scaled by sigma2, the mean
+    of the two views as :133-136).  The returned error columns are unchanged."""
     from .scene import SceneRNG
     from .experiments import METHODS
     if not isinstance(data, Dataset):
@@ -148,6 +152,11 @@ def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), de
             if bundle_adjust:
                 ba = api.bundle_adjust(C0, CalM, res[0], res[1], res[2], device=device)
                 out[m][row, 3:] = errors(ba[0], ba[1], CalM, inl, d["R_t0"])
+                if covariance:
+                    cov = api.ba_covariance(C0, CalM, ba[0], ba[1], ba[2], device=device)
+                    rot, tdir = api.pose_rms_errors(cov[0], ba[0], ba[1], sigma2=cov[1])
+                    ba.sigma2 = cov[1]
+                    ba.pred_rot_err, ba.pred_t_err = float(np.mean(rot)), float(np.mean(tdir))
                 rec["ba"][m] = ba
         if details is not None:
             details.append(rec)
