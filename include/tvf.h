@@ -14,7 +14,7 @@
  *     0 success, > 0 number of problems whose status word is non-zero;
  *   - `status` (int32 per problem, may be NULL) is a bit set, see TVF_ST_*;
  *   - one handle per host thread; a handle drives one GPU (tvf_create) or several
- *     (tvf_create_multi: the host-pointer pose entry points shard the batch over the
+ *     (tvf_create_multi: the host-pointer batched calls shard the batch over the
  *     devices); calls on a handle are serialised by the caller (MATLAB calls MEX on
  *     its interpreter thread only);
  *   - there is no CPU fallback: without a CUDA device tvf_create() fails.
@@ -60,8 +60,9 @@ int tvf_version(void);
 int tvf_device_count(void);
 int tvf_create(tvf_handle_t* out, int device);
 /* Group handle over n_dev devices (ids may repeat: two members on one GPU are legal).  Member 0 serves every entry
- * point; the host-pointer pose entry points (tvf_pose, tvf_linear_tft_pose, tvf_linear_f_pose, tvf_optim_f_pose)
- * split B into n_dev contiguous ranges, one host thread + one device per range, no exchange between them -- the batched
+ * point; the host-pointer batched calls -- pose (tvf_pose, tvf_linear_tft_pose, tvf_linear_f_pose, tvf_optim_f_pose),
+ * bundle adjustment (tvf_bundle_adjust) and covariance (tvf_ba_covariance) -- split B into n_dev contiguous ranges,
+ * one host thread + one device per range, no exchange between them -- the batched
  * form of the trial loop experiments.m:91-143 / experiments_real.m:75-163.  Results are bit-identical to a one-device call. */
 int tvf_create_multi(tvf_handle_t* out, const int* devices, int n_dev);
 int tvf_num_devices(tvf_handle_t h);
@@ -80,12 +81,13 @@ int tvf_synchronize(tvf_handle_t h);
 void* tvf_host_alloc(size_t bytes);
 void tvf_host_free(void* p);
 /* on != 0: caller buffers >= 1 MiB that are pageable (an mxArray's data) are page-locked with cudaHostRegister for the
- * duration of each host-pointer pose call and released before it returns; off (default): pageable buffers take the
- * CUDA runtime's staged copies */
+ * duration of each host-pointer batched call (pose, bundle adjustment, covariance) and released before it returns;
+ * off (default): pageable buffers are staged as tvf_set_host_threads describes */
 int tvf_set_host_register(tvf_handle_t h, int on);
-/* Pageable caller buffers are otherwise staged chunk by chunk through pinned per-slot buffers, filled and drained by
- * `threads` host threads (0 = automatic: hardware threads / devices of the handle, clamped to 2..8), so the copies still
- * overlap the kernels.  Pinned buffers (tvf_host_alloc, cudaHostRegister) are used in place. */
+/* Pageable caller buffers of the host-pointer batched calls (pose, bundle adjustment, covariance) are otherwise staged
+ * chunk by chunk through pinned per-slot buffers, filled and drained by `threads` host threads (0 = automatic: hardware
+ * threads / devices of the handle, clamped to 2..8), so the copies still overlap the kernels.  Pinned buffers
+ * (tvf_host_alloc, cudaHostRegister) are used in place. */
 int tvf_set_host_threads(tvf_handle_t h, int threads);
 
 /* ---- method entry points (host pointers; copies are inside the call) ------------------- */

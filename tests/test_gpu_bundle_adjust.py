@@ -215,6 +215,67 @@ def test_bit_identity_across_batch_chunk_group_and_device_pointers(tvf):
     assert np.array_equal(o_st.cpu().numpy(), full.status)
 
 
+def test_pageable_staged_path_equals_pinned_path(tvf):
+    """Pageable caller buffers (NumPy arrays) of tvf_bundle_adjust and tvf_ba_covariance go through the pinned per-slot
+    staging buffers, like the pose calls' (tests/test_gpu_parity_r2.py); pinned buffers (tvf_host_alloc) are used in
+    place.  Same bits either way, for any host thread count, with tvf_set_host_register and through a group handle."""
+    from tft_vs_fund_b200 import _lib
+    B, n = 60_001, 20                      # > 4 MB per call: staged; 9 chunks of 7 000 reuse every slot
+    d = tvf.scene.sweep_batch_device(B, n, first_trial=3)
+    start = tvf.LinearTFTPoseEstimation(d["Corresp"], d["CalM"])
+    cm = lambda a: tvf.api._cm(a, 2)[0]
+    inputs = [cm(d["Corresp"]), np.ascontiguousarray(np.broadcast_to(d["CalM"].T, (B, 3, 9))), cm(start[0]), cm(start[1]),
+              cm(start[2])]
+    shapes = [(B, 12), (B, 12), (B, 3 * n), (B,), (B,), (B,), (B, 144), (B, 9 * n), (B,), (B,)]
+    dtypes = [np.float64] * 4 + [np.int32] * 2 + [np.float64] * 3 + [np.int32]
+
+    def run(h, alloc):
+        """bundle_adjust from the start poses, then the covariance at its result, every array from `alloc`"""
+        ins = [alloc(a.shape, a.dtype) for a in inputs]
+        for a, b in zip(ins, inputs):
+            a[...] = b
+        o = [alloc(s, t) for s, t in zip(shapes, dtypes)]
+        p = lambda a: a.ctypes.data_as(_lib.c_int32_p if a.dtype == np.int32 else _lib.c_double_p)
+        h.call("tvf_bundle_adjust", p(ins[0]), p(ins[1]), 1, n, B, p(ins[2]), p(ins[3]), p(ins[4]), *[p(a) for a in o[:6]])
+        h.call("tvf_ba_covariance", p(ins[0]), p(ins[1]), 1, n, B, p(o[0]), p(o[1]), p(o[2]), *[p(a) for a in o[6:]])
+        return [a.copy() for a in o]
+
+    pins = []
+
+    def pinned(shape, dtype):
+        nbytes = int(np.prod(shape)) * np.dtype(dtype).itemsize
+        ptr = _lib.load().tvf_host_alloc(nbytes)
+        assert ptr
+        pins.append(ptr)
+        return np.frombuffer((C.c_char * nbytes).from_address(ptr), dtype=dtype).reshape(shape)
+    pageable = lambda shape, dtype: np.empty(shape, dtype)
+    h, grp = _lib.handle(), _lib.handle((0, 0))
+    try:
+        for x in (h, grp):
+            x.call("tvf_set_chunk", 7000)
+        ref = run(h, pinned)
+        assert np.count_nonzero(ref[5] == 0) > B // 2 and np.count_nonzero(ref[9] == 0) > B // 2
+        runs = {}
+        for threads in (1, 3):
+            h.call("tvf_set_host_threads", threads)
+            runs["threads %d" % threads] = run(h, pageable)
+        h.call("tvf_set_host_threads", 0)
+        h.call("tvf_set_host_register", 1)
+        runs["registered"] = run(h, pageable)
+        h.call("tvf_set_host_register", 0)
+        runs["group (0, 0)"] = run(grp, pageable)
+    finally:
+        for x in (h, grp):
+            x.call("tvf_set_chunk", 0)
+            x.call("tvf_set_host_threads", 0)
+            x.call("tvf_set_host_register", 0)
+        for ptr in pins:
+            _lib.load().tvf_host_free(C.c_void_p(ptr))
+    for name, got in runs.items():
+        for k, (a, b) in enumerate(zip(ref, got)):
+            assert np.array_equal(a, b, equal_nan=True), (name, k)
+
+
 def test_without_reconst0_the_points_are_triangulated(tvf):
     g = golden("sweep_n20.npz")
     idx = np.arange(1, 260, 20)

@@ -29,7 +29,18 @@ namespace {
 #define TVF_RAMP 0
 #endif
 constexpr int NSLOT = TVF_NSLOT;
-constexpr int NSCRATCH = 24;
+// per-handle device scratch buffers (ensure_scratch): Up's count up from SCR_UP, the named ones lie above them
+constexpr int UP_SLOTS = 12;                    // Up: one buffer per array of a stand-alone call (tvf_rt_from_tft has 9)
+enum Scratch {
+    SCR_UP = 0,
+    SCR_FP64_PEAK = SCR_UP + UP_SLOTS,          // tvf_fp64_peak_tflops' output
+    SCR_SWEEP_NOISE, SCR_SWEEP_CAMS,            // the scene generator's noise levels and cameras
+    SCR_SWEEP_CALM, SCR_SWEEP_GT,               // a sweep's calibrations and ground-truth poses
+    SCR_SWEEP_PARTIAL, SCR_SWEEP_BA_PARTIAL,    // its per-level partial sums, of the poses and of their adjustment
+    SCR_SWEEP_TABLE, SCR_SWEEP_TRIALS,          // its table and one generator call's trials
+    NSCRATCH
+};
+static_assert(SCR_UP + UP_SLOTS <= SCR_FP64_PEAK && SCR_FP64_PEAK < NSCRATCH, "Up's scratch range meets the named ones");
 constexpr int64_t DEFAULT_CHUNK = 65536;        // host-pointer entry points: chunks are the H2D / kernels / D2H pipeline stages
 constexpr int64_t DEFAULT_CHUNK_DEV = 1 << 20;  // device-pointer entry points: fewer, larger launches (less launch and wave-tail
                                                 // overhead: 8.32e7 / 8.48e7 / 8.58e7 / 8.63e7 solves/s at 262 144 / 524 288 / 1 M /
@@ -65,10 +76,10 @@ struct tvf_context {
     std::vector<cudaEvent_t> free_events;
     double prof_ms[TVF_NUM_KERNELS] = {};
     int64_t prof_n[TVF_NUM_KERNELS] = {};
-    // tvf_create_multi: further devices of a group handle (this context is member 0); the host-pointer pose entry points
-    // shard B over the members, one host thread per device (experiments.m:91-143 is the loop that fans out)
+    // tvf_create_multi: further devices of a group handle (this context is member 0); the host-pointer batched calls
+    // (host_call) shard B over the members, one host thread per device (experiments.m:91-143 is the loop that fans out)
     std::vector<tvf_context*> peers;
-    // tvf_set_host_register: pin caller buffers that are pageable for the duration of a host-pointer pose call
+    // tvf_set_host_register: pin caller buffers that are pageable for the duration of a host-pointer batched call
     int host_register = 0;
     // pageable caller buffers (an mxArray's data): chunks travel through per-slot pinned staging buffers filled / drained by
     // a few host threads, so the DMA engines see pinned memory and the three-slot pipeline keeps overlapping
@@ -124,17 +135,15 @@ struct Carver {
     }
 };
 
+// the buffers of one pose chunk (run_pose_chunk; in and calm are the chunk's inputs)
 struct ChunkBufs {
-    double* in; double* calm; double* T; double* F; double* core; double* cand; int* votes; double* scale;
+    const double* in; const double* calm; double* T; double* F; double* core; double* cand; int* votes; double* scale;
     double* Rt2; double* Rt3; double* reconst; double* repr; int* status; int* iters; int* iter_sum;
     // ba: the bundle adjustment of the chunk's poses (tvf_sweep_run_levels_ba)
     double* ba_Rt2; double* ba_Rt3; double* ba_X; double* ba_Xc; double* ba_repr; int* ba_iter; int* ba_status;
 };
 
-// per-problem bytes of the ba buffers: Rt2, Rt3, X, Xc, repr (+ iter, status in the last double)
-inline size_t ba_chunk_bytes(int n) { return (size_t)(24 + 6 * n + 3) * sizeof(double); }
-
-size_t carve(char* base, int n, int64_t C, bool host_io, bool calm_batched, bool ba, ChunkBufs* out) {
+size_t carve_pose(char* base, int n, int64_t C, bool host_io, bool calm_batched, bool ba, ChunkBufs* out) {
     Carver c(base);
     ChunkBufs b{};
     b.T = c.take<double>(27 * C);
@@ -167,13 +176,20 @@ size_t carve(char* base, int n, int64_t C, bool host_io, bool calm_batched, bool
     return c.off;
 }
 
-int64_t pick_chunk(tvf_handle_t h, int n, int64_t B, bool host_io, bool ba) {
+// per-problem bytes of carve_pose's buffers, for the automatic chunk size (a batched calm counted either way)
+size_t pose_budget(int n, bool host_io, bool ba) {
+    size_t payload = (27 + 18 + CORE_WS_TFT + CAND_SIZE + 2) * 8 + 14 * 4;
+    if (host_io) payload += (size_t)(6 * n + 27 + 24 + 3 * n + 1) * 8;
+    if (ba) payload += (size_t)(24 + 6 * n + 3) * sizeof(double);   // Rt2, Rt3, X, Xc, repr (+ iter, status in the last double)
+    return payload;
+}
+
+// problems per chunk: tvf_set_chunk's, else the default cut so that `per` bytes per problem stay within one slot's
+// arena budget (eight budgets on the device-pointer path); per = 0: no cut
+int64_t pick_chunk(tvf_handle_t h, int64_t B, bool host_io, size_t per) {
     int64_t c = h->chunk_user > 0 ? h->chunk_user : (host_io ? DEFAULT_CHUNK : DEFAULT_CHUNK_DEV);
-    if (h->chunk_user <= 0) {   // automatic: keep one slot's work space near ARENA_BUDGET
-        size_t payload = (27 + 18 + CORE_WS_TFT + CAND_SIZE + 2) * 8 + 14 * 4;
-        if (host_io) payload += (size_t)(6 * n + 27 + 24 + 3 * n + 1) * 8;
-        if (ba) payload += ba_chunk_bytes(n);
-        const int64_t fit = (int64_t)((host_io ? ARENA_BUDGET : 8 * ARENA_BUDGET) / payload);
+    if (h->chunk_user <= 0 && per > 0) {
+        const int64_t fit = (int64_t)((host_io ? ARENA_BUDGET : 8 * ARENA_BUDGET) / per);
         if (c > fit) c = fit;
     }
     if (c < 1) c = 1;
@@ -214,47 +230,45 @@ int drain_events(tvf_handle_t h) {
     return TVF_OK;
 }
 
-// kernels of one chunk; all pointers are device pointers
-int run_pose_chunk(tvf_handle_t h, cudaStream_t st, Method method, const double* d_corresp, const double* d_calm,
-                   int calm_batched, int n, int64_t Bc, double* d_T, double* d_F, double* d_core, double* d_cand, int* d_votes,
-                   double* d_scale, double* d_Rt2, double* d_Rt3, double* d_reconst, double* d_repr, int* d_status,
-                   int* d_iters = nullptr, int* d_iter_sum = nullptr) {
+// kernels of one chunk of Bc problems; all pointers are device pointers.  b.T null: T is not wanted (the F methods
+// then skip TFT_from_P); b.reconst, b.repr and b.iter_sum may be null.
+int run_pose_chunk(tvf_handle_t h, cudaStream_t st, Method method, int calm_batched, int n, int64_t Bc, const ChunkBufs& b) {
     CoreInput in{};
-    in.p1 = d_corresp; in.p2 = nullptr; in.p3 = nullptr; in.packed = 1; in.rows = 2; in.n = n; in.B = Bc; in.normalize = 1;
+    in.p1 = b.in; in.p2 = nullptr; in.p3 = nullptr; in.packed = 1; in.rows = 2; in.n = n; in.B = Bc; in.normalize = 1;
     PoseTailArgs a{};
-    a.corresp = d_corresp; a.calm = d_calm; a.calm_batched = calm_batched; a.n = n; a.B = Bc;
-    a.cand = d_cand; a.votes = d_votes; a.scale = d_scale;
-    a.Rt2 = d_Rt2; a.Rt3 = d_Rt3; a.reconst = d_reconst; a.repr_err = d_repr; a.status = d_status;
+    a.corresp = b.in; a.calm = b.calm; a.calm_batched = calm_batched; a.n = n; a.B = Bc;
+    a.cand = b.cand; a.votes = b.votes; a.scale = b.scale;
+    a.Rt2 = b.Rt2; a.Rt3 = b.Rt3; a.reconst = b.reconst; a.repr_err = b.repr; a.status = b.status;
     const int sm = h->sm_count;
     if (method == METHOD_TFT) {
         bool large_done = false;
         if (n >= LARGE_N_MIN) {
             timed_launch(h, TVF_K_TFT_MOMENTS_LARGE, st, [&] {
-                large_done = launch_tft_moments_large(d_corresp, n, Bc, 1, d_core, sm, st) != 0;
+                large_done = launch_tft_moments_large(b.in, n, Bc, 1, b.core, sm, st) != 0;
             });
             if (large_done)
-                timed_launch(h, TVF_K_TFT_STAGE1_SOLVE, st, [&] { launch_tft_stage1_solve(Bc, d_core, d_status, sm, st); });
+                timed_launch(h, TVF_K_TFT_STAGE1_SOLVE, st, [&] { launch_tft_stage1_solve(Bc, b.core, b.status, sm, st); });
         }
         if (!large_done) {
             int need_solve = 0;
-            timed_launch(h, TVF_K_TFT_STAGE1, st, [&] { need_solve = launch_tft_stage1(in, d_core, d_status, sm, st); });
+            timed_launch(h, TVF_K_TFT_STAGE1, st, [&] { need_solve = launch_tft_stage1(in, b.core, b.status, sm, st); });
             if (need_solve)
-                timed_launch(h, TVF_K_TFT_STAGE1_SOLVE, st, [&] { launch_tft_stage1_solve(Bc, d_core, d_status, sm, st); });
+                timed_launch(h, TVF_K_TFT_STAGE1_SOLVE, st, [&] { launch_tft_stage1_solve(Bc, b.core, b.status, sm, st); });
         }
-        timed_launch(h, TVF_K_TFT_EPIPOLES, st, [&] { launch_tft_epipoles(d_core, Bc, st); });
-        timed_launch(h, TVF_K_TFT_STAGE2, st, [&] { launch_tft_stage2(in, d_core, d_T, nullptr, nullptr, d_status, sm, st); });
-        timed_launch(h, TVF_K_CANDIDATES, st, [&] { launch_candidates(0, d_T, a, st); });
+        timed_launch(h, TVF_K_TFT_EPIPOLES, st, [&] { launch_tft_epipoles(b.core, Bc, st); });
+        timed_launch(h, TVF_K_TFT_STAGE2, st, [&] { launch_tft_stage2(in, b.core, b.T, nullptr, nullptr, b.status, sm, st); });
+        timed_launch(h, TVF_K_CANDIDATES, st, [&] { launch_candidates(0, b.T, a, st); });
     } else if (method == METHOD_F) {
-        timed_launch(h, TVF_K_F_STAGE1, st, [&] { launch_f_stage1(in, d_core, d_status, sm, st); });
-        timed_launch(h, TVF_K_F_FINISH, st, [&] { launch_f_finish(d_core, 1, Bc, d_F, st); });
-        timed_launch(h, TVF_K_CANDIDATES, st, [&] { launch_candidates(1, d_F, a, st); });
+        timed_launch(h, TVF_K_F_STAGE1, st, [&] { launch_f_stage1(in, b.core, b.status, sm, st); });
+        timed_launch(h, TVF_K_F_FINISH, st, [&] { launch_f_finish(b.core, 1, Bc, b.F, st); });
+        timed_launch(h, TVF_K_CANDIDATES, st, [&] { launch_candidates(1, b.F, a, st); });
     } else {    // OptimFPoseEstimation.m:47-53: linearF start, Gauss-Helmert refinement, then the F pose tail
-        timed_launch(h, TVF_K_F_STAGE1, st, [&] { launch_f_stage1(in, d_core, d_status, sm, st); });
+        timed_launch(h, TVF_K_F_STAGE1, st, [&] { launch_f_stage1(in, b.core, b.status, sm, st); });
         int ok = 1;
-        timed_launch(h, TVF_K_OPTIMF_GH, st, [&] { ok = launch_optimf_gh(d_corresp, n, Bc, d_core, d_F, d_iters, d_status, sm, st); });
+        timed_launch(h, TVF_K_OPTIMF_GH, st, [&] { ok = launch_optimf_gh(b.in, n, Bc, b.core, b.F, b.iters, b.status, sm, st); });
         if (!ok) return fail(h, TVF_ERR_ARG, "optimF: too many correspondences for the Gauss-Helmert kernel (see tvf_optim_f_max_n)");
-        if (d_iter_sum) launch_sum_pairs(d_iters, Bc, d_iter_sum, st);
-        timed_launch(h, TVF_K_CANDIDATES, st, [&] { launch_candidates(1, d_F, a, st); });
+        if (b.iter_sum) launch_sum_pairs(b.iters, Bc, b.iter_sum, st);
+        timed_launch(h, TVF_K_CANDIDATES, st, [&] { launch_candidates(1, b.F, a, st); });
     }
     if (n >= TAIL_FUSED_MIN_N && n <= TAIL_FUSED_MAX_N) {
         timed_launch(h, TVF_K_TAIL_FUSED, st, [&] { launch_pose_tail_fused(a, sm, st); });
@@ -263,8 +277,8 @@ int run_pose_chunk(tvf_handle_t h, cudaStream_t st, Method method, const double*
         timed_launch(h, TVF_K_SCALE, st, [&] { launch_scale(a, sm, st); });
         timed_launch(h, TVF_K_FINAL, st, [&] { launch_final(a, sm, st); });
     }
-    if (method != METHOD_TFT && d_T != nullptr)
-        timed_launch(h, TVF_K_TFT_FROM_POSE, st, [&] { launch_tft_from_pose(d_calm, calm_batched, d_Rt2, d_Rt3, Bc, d_T, st); });
+    if (method != METHOD_TFT && b.T != nullptr)
+        timed_launch(h, TVF_K_TFT_FROM_POSE, st, [&] { launch_tft_from_pose(b.calm, calm_batched, b.Rt2, b.Rt3, Bc, b.T, st); });
     TVF_CK(cudaGetLastError());
     return TVF_OK;
 }
@@ -316,45 +330,64 @@ int ensure_stage(tvf_handle_t h, int slot, size_t bytes) {
     return TVF_OK;
 }
 
-// outputs of a pose call (any may be null); `votes` = 10 int32 per problem: the 4 + 4 cheirality votes of
-// R_t_from_TFT.m:91-104 in the reference's candidate order for the pairs (1,2) and (1,3), then the two NaN masks
-struct PoseOut {
-    double* Rt2; double* Rt3; double* reconst; double* T; double* repr_err; double* F21; double* F31;
-    int32_t* iter; int32_t* votes; int32_t* status;
-};
-
 // caller buffers that are pageable get pinned for the duration of a call (tvf_set_host_register); RAII
 struct HostPins {
     std::vector<void*> pinned;
     void add(const void* p, size_t bytes) {
-        if (!p || bytes < (1u << 20)) return;
-        cudaPointerAttributes at;
-        if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return; }
-        if (at.type != cudaMemoryTypeUnregistered) return;
+        if (bytes < (1u << 20) || !is_pageable(p)) return;
         if (cudaHostRegister(const_cast<void*>(p), bytes, cudaHostRegisterPortable) == cudaSuccess) pinned.push_back(const_cast<void*>(p));
         else cudaGetLastError();
     }
     ~HostPins() { for (void* p : pinned) cudaHostUnregister(p); }
 };
 
-int pose_host_one(tvf_handle_t h, Method method, const double* corresp, const double* calm, int calm_batched, int n,
-                  int64_t B, const PoseOut& o) {
+inline size_t align256(size_t bytes) { return (bytes + 255) & ~size_t(255); }
+
+// ---- host-pointer calls -------------------------------------------------------------------------------------------
+// A host-pointer entry point is a Call: its caller arrays, the device buffers of the chunk in flight (`d`), and
+//   size_t budget(bool host_io)          per-problem bytes of a chunk, for pick_chunk
+//   size_t carve(char* base, int64_t C)  lays `d` out in a slot arena (base = nullptr: size only)
+//   void arrays(F f)                     f(caller pointer, Arr) for every caller array: the one place their layout is written
+//   int launch(h, stream, Bc)            the kernels of one chunk on `d`
+//   int check(h, B), int32_t*& status()  argument checks; the per-problem status array
+
+// One caller array beside its device buffer in the chunk's arena
+struct Arr {
+    bool out;         // false: host -> device before the chunk's kernels; true: device -> host after them
+    size_t per;       // bytes per problem; 0: one copy of `pitch` bytes that every problem shares (a 9 x 3 calm)
+    const void* dev;  // the chunk's device buffer
+    size_t pitch;     // bytes per problem in `dev` (F21 / F31: 72 bytes out of each 144-byte F record)
+    size_t bytes(int64_t k) const { return per ? (size_t)k * per : pitch; }   // of k problems
+    static Arr input(size_t per, const void* dev, bool shared = false) { return Arr{false, shared ? 0 : per, dev, per}; }
+    static Arr output(size_t per, const void* dev, size_t pitch = 0) { return Arr{true, per, dev, pitch ? pitch : per}; }
+};
+
+// the caller arrays of `c` from problem `lo` on
+template <class Call> void shift(Call& c, int64_t lo) {
+    c.arrays([&](auto& p, const Arr& a) { if (p) p += lo * (int64_t)(a.per / sizeof(*p)); });
+}
+
+// One host-pointer call on one device.  Chunk i runs on slot i mod NSLOT (stream + arena), so its H2D, kernels and D2H
+// overlap those of its neighbours.
+template <class Call> int host_pipeline(tvf_handle_t h, Call c, int64_t B) {
     if (B == 0) return TVF_OK;
     TVF_CK(cudaSetDevice(h->device));
-    const int64_t C = pick_chunk(h, n, B, true, false);
-    const size_t need = carve(nullptr, n, C, true, calm_batched != 0, false, nullptr);
-    std::vector<int32_t> st_tmp;
-    int32_t* st_host = o.status;
-    if (!st_host) { st_tmp.resize((size_t)B); st_host = st_tmp.data(); }
-    // earlier asynchronous *_dev / sweep work of this handle may still be using slot 0's arena
-    TVF_CK(cudaStreamSynchronize(h->slot[0].stream));
-    if (h->use_user_stream) TVF_CK(cudaStreamSynchronize(h->user_stream));
-
+    const int64_t C = pick_chunk(h, B, true, c.budget(true));
+    const size_t need = c.carve(nullptr, C);
     // Pageable caller memory (what a MEX gateway receives): cudaMemcpyAsync would fall back to synchronous copies through
     // the runtime's own bounce buffer and serialise the pipeline (measured 6.6e6 solves/s against 4.5e7 with pinned
     // buffers).  Instead every chunk goes through a pinned per-slot staging buffer that a few host threads fill and drain.
-    const bool staged = !h->host_register && (size_t)B * 6 * n * sizeof(double) >= (size_t(4) << 20) &&
-                        (is_pageable(corresp) || is_pageable(o.Rt2) || is_pageable(o.reconst) || is_pageable(o.T) || is_pageable(o.repr_err));
+    // A shared array is one small copy and stays where it is.
+    size_t moved = 0;
+    bool pageable = false;
+    c.arrays([&](const void* p, const Arr& a) {
+        if (p && a.per) { moved += a.bytes(B); pageable = pageable || is_pageable(p); }
+    });
+    const bool staged = pageable && !h->host_register && moved >= (size_t(4) << 20);
+    std::vector<int32_t> st_tmp;
+    if (!c.status()) { st_tmp.resize((size_t)B); c.status() = st_tmp.data(); }
+    size_t stage_bytes = 0;
+    c.arrays([&](const void* p, const Arr& a) { if (p && a.per) stage_bytes += align256(a.bytes(C)); });
     int nthreads = h->host_threads;
     if (nthreads <= 0) {
         const int hw = (int)std::thread::hardware_concurrency();
@@ -367,8 +400,9 @@ int pose_host_one(tvf_handle_t h, Method method, const double* corresp, const do
         for (const Drain& d : pending[slot]) par_memcpy(d.dst, d.src, d.bytes, nthreads);
         pending[slot].clear();
     };
-    const size_t in_bytes_max = (size_t)C * 6 * n * sizeof(double) + (calm_batched ? (size_t)C * 27 * sizeof(double) : 0);
-    const size_t out_bytes_max = (size_t)C * ((24 + 3 * n + 27 + 1 + 18) * sizeof(double) + 12 * sizeof(int32_t)) + 16 * 256;   // + region alignment
+    // earlier asynchronous *_dev / sweep work of this handle may still be using slot 0's arena
+    TVF_CK(cudaStreamSynchronize(h->slot[0].stream));
+    if (h->use_user_stream) TVF_CK(cudaStreamSynchronize(h->user_stream));
 
     // Chunk schedule.  The call is bound by the host link (H2D of chunk i+1, kernels of chunk i and D2H of chunk i-1
     // overlap).  Quarter- and half-size chunks at both ends, meant to shorten the pipeline's fill and drain, were
@@ -395,56 +429,39 @@ int pose_host_one(tvf_handle_t h, Method method, const double* corresp, const do
         Slot& s = h->slot[si];
         TVF_CK(cudaStreamSynchronize(s.stream));        // slot reuse: its previous chunk (incl. D2H) is finished
         rc = ensure_arena(h, s, need); if (rc) return rc;
-        ChunkBufs b; carve(s.arena, n, C, true, calm_batched != 0, false, &b);
-        const double* src_in = corresp + done * 6 * n;
-        const double* src_calm = calm + (calm_batched ? done * 27 : 0);
-        char* stage_out = nullptr;
+        c.carve(s.arena, C);
+        char* stage = nullptr;
         if (staged) {
             drain(si);                                   // the slot's previous outputs leave the staging buffer first
-            rc = ensure_stage(h, si, in_bytes_max + out_bytes_max); if (rc) return rc;
-            char* st_in = (char*)h->stage[si];
-            par_memcpy(st_in, src_in, (size_t)Bc * 6 * n * sizeof(double), nthreads);
-            src_in = (const double*)st_in;
-            if (calm_batched) {
-                char* st_calm = st_in + (size_t)C * 6 * n * sizeof(double);
-                memcpy(st_calm, src_calm, (size_t)Bc * 27 * sizeof(double));
-                src_calm = (const double*)st_calm;
-            }
-            stage_out = st_in + in_bytes_max;
+            rc = ensure_stage(h, si, stage_bytes); if (rc) return rc;
+            stage = (char*)h->stage[si];
         }
-        TVF_CK(cudaMemcpyAsync(b.in, src_in, (size_t)Bc * 6 * n * sizeof(double), cudaMemcpyHostToDevice, s.stream));
-        // CalM travels on the chunk's own stream (ordered before the kernels that read it), shared 9x3 included
-        TVF_CK(cudaMemcpyAsync(b.calm, src_calm, (size_t)(calm_batched ? Bc * 27 : 27) * sizeof(double), cudaMemcpyHostToDevice, s.stream));
-        rc = run_pose_chunk(h, s.stream, method, b.in, b.calm, calm_batched, n, Bc,
-                            (method == METHOD_TFT || o.T) ? b.T : nullptr, b.F, b.core, b.cand, b.votes, b.scale, b.Rt2, b.Rt3,
-                            b.reconst, b.repr, b.status, b.iters, b.iter_sum);
-        if (rc) return rc;
-        // device -> host: straight into the caller's array, or into the staging buffer with a drain entry
-        size_t soff = 0;
-        auto back = [&](void* host_base, size_t per, const void* dev, size_t dev_pitch) -> cudaError_t {
-            if (!host_base) return cudaSuccess;
-            char* dst = (char*)host_base + (size_t)done * per;
+        // straight from / into the caller's array, or through the slot's staging buffer (outputs with a drain entry)
+        cudaError_t e = cudaSuccess;
+        c.arrays([&](const void* p, const Arr& a) {
+            if (!p || a.out || e != cudaSuccess) return;
+            const char* src = (const char*)p + (size_t)done * a.per;
+            if (staged && a.per) {
+                par_memcpy(stage, src, a.bytes(Bc), nthreads);
+                src = stage;
+                stage += align256(a.bytes(C));
+            }
+            e = cudaMemcpyAsync(const_cast<void*>(a.dev), src, a.bytes(Bc), cudaMemcpyHostToDevice, s.stream);
+        });
+        if (e != cudaSuccess) return fail(h, TVF_ERR_CUDA, std::string("cudaMemcpyAsync(host to device): ") + cudaGetErrorString(e));
+        rc = c.launch(h, s.stream, Bc); if (rc) return rc;
+        c.arrays([&](const void* p, const Arr& a) {
+            if (!p || !a.out || e != cudaSuccess) return;
+            char* dst = (char*)const_cast<void*>(p) + (size_t)done * a.per;
             if (staged) {
-                char* stg = stage_out + soff;
-                soff += ((size_t)C * per + 255) & ~size_t(255);
-                pending[si].push_back(Drain{dst, stg, (size_t)Bc * per});
-                dst = stg;
+                pending[si].push_back(Drain{dst, stage, a.bytes(Bc)});
+                dst = stage;
+                stage += align256(a.bytes(C));
             }
-            if (dev_pitch == per) return cudaMemcpyAsync(dst, dev, (size_t)Bc * per, cudaMemcpyDeviceToHost, s.stream);
-            return cudaMemcpy2DAsync(dst, per, dev, dev_pitch, per, (size_t)Bc, cudaMemcpyDeviceToHost, s.stream);
-        };
-        if (method == METHOD_OPTF) TVF_CK(back(o.iter, sizeof(int32_t), b.iter_sum, sizeof(int32_t)));
-        TVF_CK(back(o.Rt2, 12 * sizeof(double), b.Rt2, 12 * sizeof(double)));
-        TVF_CK(back(o.Rt3, 12 * sizeof(double), b.Rt3, 12 * sizeof(double)));
-        TVF_CK(back(o.reconst, (size_t)3 * n * sizeof(double), b.reconst, (size_t)3 * n * sizeof(double)));
-        TVF_CK(back(o.T, 27 * sizeof(double), b.T, 27 * sizeof(double)));
-        TVF_CK(back(o.repr_err, sizeof(double), b.repr, sizeof(double)));
-        TVF_CK(back(o.votes, 10 * sizeof(int32_t), b.votes, 10 * sizeof(int32_t)));
-        if (method != METHOD_TFT) {
-            TVF_CK(back(o.F21, 72, b.F, 144));
-            TVF_CK(back(o.F31, 72, b.F + 9, 144));
-        }
-        TVF_CK(back(st_host, sizeof(int32_t), b.status, sizeof(int32_t)));
+            e = (a.pitch == a.per) ? cudaMemcpyAsync(dst, a.dev, a.bytes(Bc), cudaMemcpyDeviceToHost, s.stream)
+                                   : cudaMemcpy2DAsync(dst, a.per, a.dev, a.pitch, a.per, (size_t)Bc, cudaMemcpyDeviceToHost, s.stream);
+        });
+        if (e != cudaSuccess) return fail(h, TVF_ERR_CUDA, std::string("cudaMemcpyAsync(device to host): ") + cudaGetErrorString(e));
         done += Bc; ++ci;
     }
     for (int i = 0; i < NSLOT; ++i) {
@@ -452,7 +469,7 @@ int pose_host_one(tvf_handle_t h, Method method, const double* corresp, const do
         TVF_CK(cudaStreamSynchronize(h->slot[si].stream));
         if (staged) drain(si);
     }
-    return count_flagged(st_host, B);
+    return count_flagged(c.status(), B);
 }
 
 // contiguous [lo, hi) of B problems for member g of G (remainder to the first members; same rule as sharding.shard_range)
@@ -462,42 +479,29 @@ inline void shard_of(int64_t B, int g, int G, int64_t* lo, int64_t* hi) {
     *hi = *lo + base + (g < rem ? 1 : 0);
 }
 
-int pose_host(tvf_handle_t h, Method method, const double* corresp, const double* calm, int calm_batched, int n,
-              int64_t B, const PoseOut& o) {
-    int rc = check_pose_args(h, corresp, calm, n, B, method);
+// A host-pointer call: checks, page-locking (tvf_set_host_register), then the pipeline, on one device or sharded over the
+// members of a group handle.  Member g solves the contiguous range shard_of(B, g, G) on its own device from its own host
+// thread; problems are independent and a problem's result does not depend on its batch, so the outputs are
+// bit-identical to a single-device call.
+template <class Call> int host_call(tvf_handle_t h, Call c, int64_t B) {
+    int rc = c.check(h, B);
     if (rc != TVF_OK) return rc;
     if (B == 0) return TVF_OK;
     HostPins pins;
     if (h->host_register) {
         TVF_CK(cudaSetDevice(h->device));
-        pins.add(corresp, (size_t)B * 6 * n * 8);
-        if (calm_batched) pins.add(calm, (size_t)B * 27 * 8);
-        pins.add(o.Rt2, (size_t)B * 96); pins.add(o.Rt3, (size_t)B * 96); pins.add(o.reconst, (size_t)B * 3 * n * 8);
-        pins.add(o.T, (size_t)B * 216); pins.add(o.repr_err, (size_t)B * 8); pins.add(o.votes, (size_t)B * 40);
-        pins.add(o.F21, (size_t)B * 72); pins.add(o.F31, (size_t)B * 72); pins.add(o.status, (size_t)B * 4);
+        c.arrays([&](const void* p, const Arr& a) { if (a.per) pins.add(p, (size_t)B * a.per); });
     }
     const int G = 1 + (int)h->peers.size();
-    if (G == 1 || B < G) return pose_host_one(h, method, corresp, calm, calm_batched, n, B, o);
-    // group handle: member g solves the contiguous range shard_of(B, g, G) on its own device from its own host thread;
-    // problems are independent and a problem's result does not depend on its batch, so the outputs are bit-identical
-    // to a single-device call
+    if (G == 1 || B < G) return host_pipeline(h, c, B);
     std::vector<int> rcs((size_t)G, TVF_OK);
     auto run = [&](int g) {
         tvf_handle_t m = (g == 0) ? h : h->peers[(size_t)g - 1];
         int64_t lo, hi; shard_of(B, g, G, &lo, &hi);
-        PoseOut s = o;
-        if (s.Rt2) s.Rt2 += lo * 12;
-        if (s.Rt3) s.Rt3 += lo * 12;
-        if (s.reconst) s.reconst += lo * 3 * n;
-        if (s.T) s.T += lo * 27;
-        if (s.repr_err) s.repr_err += lo;
-        if (s.F21) s.F21 += lo * 9;
-        if (s.F31) s.F31 += lo * 9;
-        if (s.iter) s.iter += lo;
-        if (s.votes) s.votes += lo * 10;
-        if (s.status) s.status += lo;
+        Call s = c;
+        shift(s, lo);
         m->chunk_user = h->chunk_user; m->host_threads = h->host_threads;
-        rcs[(size_t)g] = pose_host_one(m, method, corresp + lo * 6 * n, calm + (calm_batched ? lo * 27 : 0), calm_batched, n, hi - lo, s);
+        rcs[(size_t)g] = host_pipeline(m, s, hi - lo);
     };
     std::vector<std::thread> th;
     for (int g = 1; g < G; ++g) th.emplace_back(run, g);
@@ -515,255 +519,230 @@ int pose_host(tvf_handle_t h, Method method, const double* corresp, const double
     return (int)(flagged > 0x7fffffff ? 0x7fffffff : flagged);
 }
 
-int pose_dev(tvf_handle_t h, Method method, const double* corresp, const double* calm, int calm_batched, int n,
-             int64_t B, const PoseOut& o) {
-    int rc = check_pose_args(h, corresp, calm, n, B, method);
+// outputs of a pose call (any may be null); `votes` = 10 int32 per problem: the 4 + 4 cheirality votes of
+// R_t_from_TFT.m:91-104 in the reference's candidate order for the pairs (1,2) and (1,3), then the two NaN masks
+struct PoseOut {
+    double* Rt2; double* Rt3; double* reconst; double* T; double* repr_err; double* F21; double* F31;
+    int32_t* iter; int32_t* votes; int32_t* status;
+};
+
+// tvf_pose and the per-method pose calls
+struct PoseCall {
+    Method method; const double* corresp; const double* calm; int calm_batched; int n; PoseOut o;
+    ChunkBufs d{};
+    int check(tvf_handle_t h, int64_t B) const { return check_pose_args(h, corresp, calm, n, B, method); }
+    int32_t*& status() { return o.status; }
+    size_t budget(bool host_io) const { return pose_budget(n, host_io, false); }
+    size_t carve(char* base, int64_t C) { return carve_pose(base, n, C, true, calm_batched != 0, false, &d); }
+    template <class F> void arrays(F&& f) {
+        f(corresp, Arr::input(8 * 6 * n, d.in));
+        f(calm, Arr::input(8 * 27, d.calm, !calm_batched));
+        f(o.Rt2, Arr::output(8 * 12, d.Rt2));
+        f(o.Rt3, Arr::output(8 * 12, d.Rt3));
+        f(o.reconst, Arr::output(8 * 3 * n, d.reconst));
+        f(o.T, Arr::output(8 * 27, d.T));
+        f(o.repr_err, Arr::output(8, d.repr));
+        f(o.votes, Arr::output(4 * 10, d.votes));
+        if (method != METHOD_TFT) {
+            f(o.F21, Arr::output(8 * 9, d.F, 8 * 18));
+            f(o.F31, Arr::output(8 * 9, d.F + 9, 8 * 18));
+        }
+        if (method == METHOD_OPTF) f(o.iter, Arr::output(4, d.iter_sum));
+        f(o.status, Arr::output(4, d.status));
+    }
+    int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
+        ChunkBufs k = d;
+        if (method != METHOD_TFT && !o.T) k.T = nullptr;
+        return run_pose_chunk(h, st, method, calm_batched, n, Bc, k);
+    }
+};
+
+int pose_dev(tvf_handle_t h, const PoseCall& c, int64_t B) {
+    int rc = c.check(h, B);
     if (rc != TVF_OK) return rc;
     // the kernels read the correspondences with 128-bit loads and bulk asynchronous copies: 16-byte alignment (every
     // cudaMalloc'ed buffer and every problem boundary inside one satisfies it: a problem is 48 n bytes)
-    if ((reinterpret_cast<uintptr_t>(corresp) & 15u) != 0) return fail(h, TVF_ERR_ARG, "device pointer `corresp` must be 16-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(c.corresp) & 15u) != 0) return fail(h, TVF_ERR_ARG, "device pointer `corresp` must be 16-byte aligned");
     if (B == 0) return TVF_OK;
     TVF_CK(cudaSetDevice(h->device));
     Slot& s = h->slot[0];
     cudaStream_t st = h->use_user_stream ? h->user_stream : s.stream;
-    const int64_t C = pick_chunk(h, n, B, false, false);
+    const int n = c.n;
+    const int64_t C = pick_chunk(h, B, false, c.budget(false));
     // internal buffers only; Rt2/Rt3 are needed internally by the F method's TFT_from_P, so stage them if absent
-    const size_t need = carve(nullptr, n, C, false, false, false, nullptr) + (size_t)(24 * C) * sizeof(double) + 512;
+    const size_t need = carve_pose(nullptr, n, C, false, false, false, nullptr) + (size_t)(24 * C) * sizeof(double) + 512;
     rc = ensure_arena(h, s, need); if (rc) return rc;
-    ChunkBufs b; const size_t used = carve(s.arena, n, C, false, false, false, &b);
+    ChunkBufs b; const size_t used = carve_pose(s.arena, n, C, false, false, false, &b);
     double* tmpRt2 = reinterpret_cast<double*>(s.arena + used);
     double* tmpRt3 = tmpRt2 + 12 * C;
     for (int64_t done = 0; done < B; done += C) {
         const int64_t Bc = (B - done < C) ? (B - done) : C;
-        double* dT = o.T ? o.T + done * 27 : (method == METHOD_TFT ? b.T : nullptr);
-        double* dRt2 = o.Rt2 ? o.Rt2 + done * 12 : tmpRt2;
-        double* dRt3 = o.Rt3 ? o.Rt3 + done * 12 : tmpRt3;
-        rc = run_pose_chunk(h, st, method, corresp + done * 6 * n, calm + (calm_batched ? done * 27 : 0), calm_batched, n,
-                            Bc, dT, b.F, b.core, b.cand, o.votes ? o.votes + done * 10 : b.votes, b.scale, dRt2, dRt3,
-                            o.reconst ? o.reconst + done * 3 * n : nullptr, o.repr_err ? o.repr_err + done : nullptr,
-                            o.status ? o.status + done : b.status, b.iters, o.iter ? o.iter + done : nullptr);
-        if (rc) return rc;
-        if (method != METHOD_TFT && o.F21)
-            TVF_CK(cudaMemcpy2DAsync(o.F21 + done * 9, 72, b.F, 144, 72, (size_t)Bc, cudaMemcpyDeviceToDevice, st));
-        if (method != METHOD_TFT && o.F31)
-            TVF_CK(cudaMemcpy2DAsync(o.F31 + done * 9, 72, b.F + 9, 144, 72, (size_t)Bc, cudaMemcpyDeviceToDevice, st));
+        PoseCall k = c;
+        shift(k, done);
+        const PoseOut& o = k.o;
+        ChunkBufs d = b;                        // the caller's arrays; the work space for those it does not give
+        d.in = k.corresp; d.calm = k.calm; d.reconst = o.reconst; d.repr = o.repr_err; d.iter_sum = o.iter;
+        d.T = o.T ? o.T : (c.method == METHOD_TFT ? b.T : nullptr);
+        d.Rt2 = o.Rt2 ? o.Rt2 : tmpRt2; d.Rt3 = o.Rt3 ? o.Rt3 : tmpRt3;
+        d.votes = o.votes ? o.votes : b.votes; d.status = o.status ? o.status : b.status;
+        rc = run_pose_chunk(h, st, c.method, c.calm_batched, n, Bc, d); if (rc) return rc;
+        if (c.method != METHOD_TFT && o.F21)
+            TVF_CK(cudaMemcpy2DAsync(o.F21, 72, b.F, 144, 72, (size_t)Bc, cudaMemcpyDeviceToDevice, st));
+        if (c.method != METHOD_TFT && o.F31)
+            TVF_CK(cudaMemcpy2DAsync(o.F31, 72, b.F + 9, 144, 72, (size_t)Bc, cudaMemcpyDeviceToDevice, st));
     }
     return TVF_OK;
 }
 
 // ---- bundle adjustment (tvf_bundle_adjust[_dev]) and its covariance (tvf_ba_covariance[_dev]) ------------------------
-// one call's arrays (host or device pointers).  Adjustment: outputs may be null except Rt2 / Rt3.  Covariance (cov):
-// the state is Rt2_0, Rt3_0, X0 (all required) and the outputs cov_cam, cov_pts, sigma2, status may be null.
-struct BaIo {
-    const double* corresp; const double* calm; int calm_batched; int n;
-    const double* Rt2_0; const double* Rt3_0; const double* X0;
-    double* Rt2; double* Rt3; double* X; double* repr; int32_t* iter; int32_t* status;
-    bool cov; double* cov_cam; double* cov_pts; double* sigma2;
-    BaIo shifted(int64_t lo) const {           // problems [lo, ...)
-        BaIo s = *this;
-        s.corresp += lo * 6 * n;
-        if (calm_batched) s.calm += lo * 27;
-        s.Rt2_0 += lo * 12; s.Rt3_0 += lo * 12;
-        if (s.Rt2) s.Rt2 += lo * 12;
-        if (s.Rt3) s.Rt3 += lo * 12;
-        if (s.X0) s.X0 += lo * 3 * n;
-        if (s.X) s.X += lo * 3 * n;
-        if (s.repr) s.repr += lo;
-        if (s.iter) s.iter += lo;
-        if (s.status) s.status += lo;
-        if (s.cov_cam) s.cov_cam += lo * 144;
-        if (s.cov_pts) s.cov_pts += lo * 9 * n;
-        if (s.sigma2) s.sigma2 += lo;
-        return s;
+// `io` holds the caller's arrays (host or device pointers), `d` the chunk's kernel arguments: on the host path device
+// copies carved from a slot arena, on the device path the caller's arrays themselves plus the work space.
+
+// one kernel launch of the adjustment or the covariance: counted, and its launch error reported under the kernel's name
+int ba_launched(tvf_handle_t h, int ok, const char* kernel) {
+    h->launches += 1;
+    if (ok) return TVF_OK;
+    cudaError_t e = cudaGetLastError();
+    return fail(h, TVF_ERR_CUDA, std::string(kernel) + ": " + cudaGetErrorString(e));
+}
+
+int check_ba_size(tvf_handle_t h, int n, int64_t B) {
+    if (B < 0) return fail(h, TVF_ERR_ARG, "bundle_adjust: B >= 0");
+    if (n < 4) return fail(h, TVF_ERR_ARG, "bundle_adjust: needs n >= 4 points (11 + 3n unknowns, 6n residuals)");
+    return TVF_OK;
+}
+
+// outputs may be null except Rt2 / Rt3; X0 null: the kernel triangulates the start points
+struct BundleAdjust {
+    BaArgs io;
+    BaArgs d{};
+    int check(tvf_handle_t h, int64_t B) const {
+        if (!h) return TVF_ERR_ARG;
+        if (!io.corresp || !io.calm || !io.Rt2_0 || !io.Rt3_0 || !io.Rt2 || !io.Rt3)
+            return fail(h, TVF_ERR_ARG, "bundle_adjust: corresp, calm, Rt2_0, Rt3_0, Rt2 and Rt3 must not be NULL");
+        return check_ba_size(h, io.n, B);
+    }
+    int32_t*& status() { return io.status; }
+    // the work space Xc (and X on the device path when the caller wants no points); the host path's inputs and outputs,
+    // counting a batched calm and X0 whether or not the call has them
+    size_t budget(bool host_io) const {
+        const int n = io.n;
+        size_t b = (size_t)2 * 3 * n * sizeof(double);
+        if (host_io) b += (size_t)(6 * n + 27 + 24 + 3 * n + 24 + 1) * sizeof(double) + 2 * sizeof(int32_t);
+        return b;
+    }
+    size_t carve(char* base, int64_t C, bool host_io = true) {
+        const int n = io.n;
+        Carver c(base);
+        d = io;
+        if (host_io) {
+            d.corresp = c.take<double>((size_t)6 * n * C); d.calm = c.take<double>(io.calm_batched ? 27 * C : 27);
+            d.Rt2_0 = c.take<double>(12 * C); d.Rt3_0 = c.take<double>(12 * C);
+            d.X0 = io.X0 ? c.take<double>((size_t)3 * n * C) : nullptr;
+            d.Rt2 = c.take<double>(12 * C); d.Rt3 = c.take<double>(12 * C); d.X = c.take<double>((size_t)3 * n * C);
+            d.repr_err = c.take<double>(C); d.iter = c.take<int>(C); d.status = c.take<int>(C);
+        }
+        if (!d.X) d.X = c.take<double>((size_t)3 * n * C);
+        d.Xc = c.take<double>((size_t)3 * n * C);
+        return c.off;
+    }
+    template <class F> void arrays(F&& f) {
+        const int n = io.n;
+        f(io.corresp, Arr::input(8 * 6 * n, d.corresp));
+        f(io.calm, Arr::input(8 * 27, d.calm, !io.calm_batched));
+        f(io.Rt2_0, Arr::input(8 * 12, d.Rt2_0));
+        f(io.Rt3_0, Arr::input(8 * 12, d.Rt3_0));
+        f(io.X0, Arr::input(8 * 3 * n, d.X0));
+        f(io.Rt2, Arr::output(8 * 12, d.Rt2));
+        f(io.Rt3, Arr::output(8 * 12, d.Rt3));
+        f(io.X, Arr::output(8 * 3 * n, d.X));
+        f(io.repr_err, Arr::output(8, d.repr_err));
+        f(io.iter, Arr::output(4, d.iter));
+        f(io.status, Arr::output(4, d.status));
+    }
+    int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
+        BaArgs a = d; a.B = Bc;
+        return ba_launched(h, launch_bundle_adjust(a, st), "bundle_adjust_kernel");
     }
 };
 
-int check_ba_args(tvf_handle_t h, const BaIo& io, int64_t B) {
-    if (!h) return TVF_ERR_ARG;
-    if (io.cov) {
-        if (!io.corresp || !io.calm || !io.Rt2_0 || !io.Rt3_0 || !io.X0)
+// the state Rt2, Rt3, X is required; every output may be null
+struct Covariance {
+    BaCovArgs io;
+    BaCovArgs d{};
+    int check(tvf_handle_t h, int64_t B) const {
+        if (!h) return TVF_ERR_ARG;
+        if (!io.corresp || !io.calm || !io.Rt2 || !io.Rt3 || !io.X)
             return fail(h, TVF_ERR_ARG, "ba_covariance: corresp, calm, Rt2, Rt3 and reconst must not be NULL");
-    } else if (!io.corresp || !io.calm || !io.Rt2_0 || !io.Rt3_0 || !io.Rt2 || !io.Rt3) {
-        return fail(h, TVF_ERR_ARG, "bundle_adjust: corresp, calm, Rt2_0, Rt3_0, Rt2 and Rt3 must not be NULL");
+        return check_ba_size(h, io.n, B);
     }
-    if (B < 0) return fail(h, TVF_ERR_ARG, "bundle_adjust: B >= 0");
-    if (io.n < 4) return fail(h, TVF_ERR_ARG, "bundle_adjust: needs n >= 4 points (11 + 3n unknowns, 6n residuals)");
-    return TVF_OK;
-}
-
-// per-problem device bytes of a chunk: host_io -> inputs and outputs too; the adjustment always has its two point buffers
-size_t ba_bytes_per_problem(int n, bool host_io, bool cov) {
-    if (cov) return host_io ? (size_t)(6 * n + 27 + 24 + 3 * n + 144 + 9 * n + 1 + 1) * sizeof(double) : 0;
-    size_t b = (size_t)2 * 3 * n * sizeof(double);
-    if (host_io) b += (size_t)(6 * n + 27 + 24 + 3 * n + 24 + 1) * sizeof(double) + 2 * sizeof(int32_t);
-    return b;
-}
-
-int64_t pick_chunk_ba(tvf_handle_t h, int n, int64_t B, bool host_io, bool cov = false) {
-    int64_t c = h->chunk_user > 0 ? h->chunk_user : (host_io ? DEFAULT_CHUNK : DEFAULT_CHUNK_DEV);
-    const size_t per = ba_bytes_per_problem(n, host_io, cov);
-    if (h->chunk_user <= 0 && per > 0) {
-        const int64_t fit = (int64_t)((host_io ? ARENA_BUDGET : 8 * ARENA_BUDGET) / per);
-        if (c > fit) c = fit;
+    int32_t*& status() { return io.status; }
+    // the host path's inputs and outputs, counting a batched calm and cov_pts whether or not the call has them; the
+    // device path needs no work space
+    size_t budget(bool host_io) const {
+        const int n = io.n;
+        return host_io ? (size_t)(6 * n + 27 + 24 + 3 * n + 144 + 9 * n + 1 + 1) * sizeof(double) : 0;
     }
-    if (c < 1) c = 1;
-    if (c > B) c = B;
-    return c;
-}
-
-// device copies of one host chunk of C problems in a slot arena (base = nullptr: size only)
-// (the covariance's chunk: inputs, cov_cam and cov_pts when the caller wants them, sigma2, status)
-size_t carve_ba(char* base, int n, int64_t C, const BaIo& io, BaIo* d, double** Xc) {
-    Carver c(base);
-    *d = BaIo{};
-    d->cov = io.cov;
-    d->corresp = c.take<double>((size_t)6 * n * C); d->calm = c.take<double>(io.calm_batched ? 27 * C : 27);
-    d->calm_batched = io.calm_batched; d->n = n;
-    d->Rt2_0 = c.take<double>(12 * C); d->Rt3_0 = c.take<double>(12 * C); d->X0 = c.take<double>((size_t)3 * n * C);
-    if (io.cov) {
-        d->cov_cam = io.cov_cam ? c.take<double>(144 * C) : nullptr;
-        d->cov_pts = io.cov_pts ? c.take<double>((size_t)9 * n * C) : nullptr;
-        d->sigma2 = c.take<double>(C); d->status = c.take<int32_t>(C);
-        *Xc = nullptr;
+    size_t carve(char* base, int64_t C, bool host_io = true) {
+        const int n = io.n;
+        Carver c(base);
+        d = io;
+        if (host_io) {
+            d.corresp = c.take<double>((size_t)6 * n * C); d.calm = c.take<double>(io.calm_batched ? 27 * C : 27);
+            d.Rt2 = c.take<double>(12 * C); d.Rt3 = c.take<double>(12 * C); d.X = c.take<double>((size_t)3 * n * C);
+            d.cov_cam = io.cov_cam ? c.take<double>(144 * C) : nullptr;
+            d.cov_pts = io.cov_pts ? c.take<double>((size_t)9 * n * C) : nullptr;
+            d.sigma2 = c.take<double>(C); d.status = c.take<int>(C);
+        }
         return c.off;
     }
-    d->Rt2 = c.take<double>(12 * C); d->Rt3 = c.take<double>(12 * C); d->X = c.take<double>((size_t)3 * n * C);
-    *Xc = c.take<double>((size_t)3 * n * C);
-    d->repr = c.take<double>(C); d->iter = c.take<int32_t>(C); d->status = c.take<int32_t>(C);
-    return c.off;
-}
-
-int ba_launch(tvf_handle_t h, cudaStream_t st, const BaIo& d, int64_t Bc, double* Xc) {
-    int ok;
-    if (d.cov) {
-        BaCovArgs a{d.corresp, d.calm, d.calm_batched, d.n, Bc, d.Rt2_0, d.Rt3_0, d.X0, d.cov_cam, d.cov_pts, d.sigma2, d.status};
-        ok = launch_ba_covariance(a, st);
-    } else {
-        BaArgs a{d.corresp, d.calm, d.calm_batched, d.n, Bc, d.Rt2_0, d.Rt3_0, d.X0, d.Rt2, d.Rt3, d.X, Xc, d.repr, d.iter, d.status};
-        ok = launch_bundle_adjust(a, st);
+    template <class F> void arrays(F&& f) {
+        const int n = io.n;
+        f(io.corresp, Arr::input(8 * 6 * n, d.corresp));
+        f(io.calm, Arr::input(8 * 27, d.calm, !io.calm_batched));
+        f(io.Rt2, Arr::input(8 * 12, d.Rt2));
+        f(io.Rt3, Arr::input(8 * 12, d.Rt3));
+        f(io.X, Arr::input(8 * 3 * n, d.X));
+        f(io.cov_cam, Arr::output(8 * 144, d.cov_cam));
+        f(io.cov_pts, Arr::output(8 * 9 * n, d.cov_pts));
+        f(io.sigma2, Arr::output(8, d.sigma2));
+        f(io.status, Arr::output(4, d.status));
     }
-    h->launches += 1;
-    if (!ok) {
-        cudaError_t e = cudaGetLastError();
-        return fail(h, TVF_ERR_CUDA, std::string(d.cov ? "ba_covariance_kernel: " : "bundle_adjust_kernel: ") + cudaGetErrorString(e));
+    int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
+        BaCovArgs a = d; a.B = Bc;
+        return ba_launched(h, launch_ba_covariance(a, st), "ba_covariance_kernel");
     }
-    return TVF_OK;
-}
-
-int ba_host_one(tvf_handle_t h, const BaIo& io, int64_t B) {
-    if (B == 0) return TVF_OK;
-    TVF_CK(cudaSetDevice(h->device));
-    const int n = io.n;
-    const int64_t C = pick_chunk_ba(h, n, B, true, io.cov);
-    std::vector<int32_t> st_tmp;
-    int32_t* st_host = io.status;
-    if (!st_host) { st_tmp.resize((size_t)B); st_host = st_tmp.data(); }
-    TVF_CK(cudaStreamSynchronize(h->slot[0].stream));
-    if (h->use_user_stream) TVF_CK(cudaStreamSynchronize(h->user_stream));
-    int64_t done = 0; int ci = 0; int rc;
-    while (done < B) {
-        const int64_t Bc = (B - done < C) ? (B - done) : C;
-        Slot& s = h->slot[ci % NSLOT];
-        TVF_CK(cudaStreamSynchronize(s.stream));            // the slot's previous chunk (with its copies back) is done
-        BaIo d{}; double* Xc;
-        rc = ensure_arena(h, s, carve_ba(nullptr, n, C, io, &d, &Xc)); if (rc) return rc;
-        carve_ba(s.arena, n, C, io, &d, &Xc);
-        double* x0 = const_cast<double*>(d.X0);
-        if (!io.X0) d.X0 = nullptr;
-        double* in = const_cast<double*>(d.corresp); double* calm = const_cast<double*>(d.calm);
-        double* r2 = const_cast<double*>(d.Rt2_0); double* r3 = const_cast<double*>(d.Rt3_0);
-        const BaIo hio = io.shifted(done);
-        auto up = [&](void* dst, const void* src, size_t bytes) { return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, s.stream); };
-        auto down = [&](void* dst, const void* src, size_t bytes) {
-            return dst ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, s.stream) : cudaSuccess;
-        };
-        TVF_CK(up(in, hio.corresp, (size_t)Bc * 6 * n * sizeof(double)));
-        TVF_CK(up(calm, hio.calm, (size_t)(io.calm_batched ? Bc * 27 : 27) * sizeof(double)));
-        TVF_CK(up(r2, hio.Rt2_0, (size_t)Bc * 12 * sizeof(double)));
-        TVF_CK(up(r3, hio.Rt3_0, (size_t)Bc * 12 * sizeof(double)));
-        if (io.X0) TVF_CK(up(x0, hio.X0, (size_t)Bc * 3 * n * sizeof(double)));
-        rc = ba_launch(h, s.stream, d, Bc, Xc); if (rc) return rc;
-        if (io.cov) {
-            TVF_CK(down(hio.cov_cam, d.cov_cam, (size_t)Bc * 144 * sizeof(double)));
-            TVF_CK(down(hio.cov_pts, d.cov_pts, (size_t)Bc * 9 * n * sizeof(double)));
-            TVF_CK(down(hio.sigma2, d.sigma2, (size_t)Bc * sizeof(double)));
-        } else {
-            TVF_CK(down(hio.Rt2, d.Rt2, (size_t)Bc * 12 * sizeof(double)));
-            TVF_CK(down(hio.Rt3, d.Rt3, (size_t)Bc * 12 * sizeof(double)));
-            TVF_CK(down(hio.X, d.X, (size_t)Bc * 3 * n * sizeof(double)));
-            TVF_CK(down(hio.repr, d.repr, (size_t)Bc * sizeof(double)));
-            TVF_CK(down(hio.iter, d.iter, (size_t)Bc * sizeof(int32_t)));
-        }
-        TVF_CK(down(st_host + done, d.status, (size_t)Bc * sizeof(int32_t)));
-        done += Bc; ++ci;
-    }
-    for (int i = 0; i < NSLOT; ++i) TVF_CK(cudaStreamSynchronize(h->slot[i].stream));
-    return count_flagged(st_host, B);
-}
-
-// host pointers; a group handle shards B exactly as pose_host does (results bit-identical to one device)
-int ba_host(tvf_handle_t h, const BaIo& io, int64_t B) {
-    int rc = check_ba_args(h, io, B);
-    if (rc != TVF_OK) return rc;
-    if (B == 0) return TVF_OK;
-    const int G = 1 + (int)h->peers.size();
-    if (G == 1 || B < G) return ba_host_one(h, io, B);
-    std::vector<int> rcs((size_t)G, TVF_OK);
-    auto run = [&](int g) {
-        tvf_handle_t m = (g == 0) ? h : h->peers[(size_t)g - 1];
-        int64_t lo, hi; shard_of(B, g, G, &lo, &hi);
-        m->chunk_user = h->chunk_user;
-        rcs[(size_t)g] = ba_host_one(m, io.shifted(lo), hi - lo);
-    };
-    std::vector<std::thread> th;
-    for (int g = 1; g < G; ++g) th.emplace_back(run, g);
-    run(0);
-    for (auto& t : th) t.join();
-    int64_t flagged = 0;
-    for (int g = 0; g < G; ++g) {
-        if (rcs[(size_t)g] < 0) {
-            if (g > 0) h->err = "device " + std::to_string(h->peers[(size_t)g - 1]->device) + ": " + h->peers[(size_t)g - 1]->err;
-            return rcs[(size_t)g];
-        }
-        flagged += rcs[(size_t)g];
-    }
-    cudaSetDevice(h->device);
-    return (int)(flagged > 0x7fffffff ? 0x7fffffff : flagged);
-}
+};
 
 // device pointers, asynchronous on the handle's stream
-int ba_dev(tvf_handle_t h, const BaIo& io, int64_t B) {
-    int rc = check_ba_args(h, io, B);
+template <class Call> int ba_dev(tvf_handle_t h, const Call& c, int64_t B) {
+    int rc = c.check(h, B);
     if (rc != TVF_OK) return rc;
-    if ((reinterpret_cast<uintptr_t>(io.corresp) & 15u) != 0) return fail(h, TVF_ERR_ARG, "device pointer `corresp` must be 16-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(c.io.corresp) & 15u) != 0) return fail(h, TVF_ERR_ARG, "device pointer `corresp` must be 16-byte aligned");
     if (B == 0) return TVF_OK;
     TVF_CK(cudaSetDevice(h->device));
     Slot& s = h->slot[0];
     cudaStream_t st = h->use_user_stream ? h->user_stream : s.stream;
-    const int64_t C = pick_chunk_ba(h, io.n, B, false, io.cov);
-    double* Xc = nullptr; double* Xw = nullptr;
-    if (!io.cov) {                                           // the adjustment's work space; the covariance needs none
-        const size_t pts = (size_t)3 * io.n * C;
-        rc = ensure_arena(h, s, 2 * pts * sizeof(double) + 512); if (rc) return rc;
-        Carver c(s.arena);
-        Xc = c.take<double>(pts);
-        Xw = c.take<double>(pts);
-    }
+    const int64_t C = pick_chunk(h, B, false, c.budget(false));
+    Call k = c;
+    rc = ensure_arena(h, s, k.carve(nullptr, C, false)); if (rc) return rc;
     for (int64_t done = 0; done < B; done += C) {
         const int64_t Bc = (B - done < C) ? (B - done) : C;
-        BaIo d = io.shifted(done);
-        if (!io.cov && !io.X) d.X = Xw;
-        rc = ba_launch(h, st, d, Bc, Xc); if (rc) return rc;
+        k = c;
+        shift(k, done);
+        k.carve(s.arena, C, false);
+        rc = k.launch(h, st, Bc); if (rc) return rc;
     }
     return TVF_OK;
 }
 
 // small helper for the stand-alone functions: upload, run, download on slot 0
 struct Up {
-    tvf_handle_t h; cudaStream_t st; int rc = TVF_OK; int next = 1;
+    tvf_handle_t h; cudaStream_t st; int rc = TVF_OK; int next = SCR_UP;
     explicit Up(tvf_handle_t hh) : h(hh), st(hh->slot[0].stream) {}
     template <typename T> T* in(const T* host, size_t count) {
         if (rc) return nullptr;
+        if (next == SCR_UP + UP_SLOTS) { rc = fail(h, TVF_ERR_ARG, "internal: more arrays than UP_SLOTS"); return nullptr; }
         void* p; rc = ensure_scratch(h, next++, count * sizeof(T), &p);
         if (rc) return nullptr;
         if (host && count) {
@@ -1003,7 +982,7 @@ double tvf_fp64_peak_tflops(tvf_handle_t h) {
     if (cudaSetDevice(h->device) != cudaSuccess) return -1.0;
     cudaStream_t st = h->slot[0].stream;
     void* p = nullptr;
-    if (ensure_scratch(h, NSCRATCH - 1, 64, &p) != TVF_OK) return -1.0;
+    if (ensure_scratch(h, SCR_FP64_PEAK, 64, &p) != TVF_OK) return -1.0;
     const int iters = 1 << 15, blocks = h->sm_count * 8;
     cudaEvent_t a, b;
     cudaEventCreate(&a); cudaEventCreate(&b);
@@ -1050,7 +1029,7 @@ int tvf_pose(tvf_handle_t h, int method, const double* corresp, const double* ca
     Method m;
     if (!h) return TVF_ERR_ARG;
     if (!method_of(method, &m)) return fail(h, TVF_ERR_ARG, "method must be 1 (linear TFT), 7 (linear F) or 8 (optimal F)");
-    return pose_host(h, m, corresp, calm, calm_batched, n, B, pose_out_of(out));
+    return host_call(h, PoseCall{m, corresp, calm, calm_batched, n, pose_out_of(out)}, B);
 }
 
 int tvf_pose_dev(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
@@ -1058,43 +1037,43 @@ int tvf_pose_dev(tvf_handle_t h, int method, const double* corresp, const double
     Method m;
     if (!h) return TVF_ERR_ARG;
     if (!method_of(method, &m)) return fail(h, TVF_ERR_ARG, "method must be 1 (linear TFT), 7 (linear F) or 8 (optimal F)");
-    return pose_dev(h, m, corresp, calm, calm_batched, n, B, pose_out_of(out));
+    return pose_dev(h, PoseCall{m, corresp, calm, calm_batched, n, pose_out_of(out)}, B);
 }
 
 int tvf_linear_tft_pose(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                         double* Rt2, double* Rt3, double* reconst, double* T, double* repr_err, int32_t* status) {
-    return pose_host(h, METHOD_TFT, corresp, calm, calm_batched, n, B, PoseOut{Rt2, Rt3, reconst, T, repr_err, nullptr, nullptr, nullptr, nullptr, status});
+    return host_call(h, PoseCall{METHOD_TFT, corresp, calm, calm_batched, n, PoseOut{Rt2, Rt3, reconst, T, repr_err, nullptr, nullptr, nullptr, nullptr, status}}, B);
 }
 
 int tvf_linear_f_pose(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                       double* Rt2, double* Rt3, double* reconst, double* T, double* repr_err, double* F21, double* F31,
                       int32_t* status) {
-    return pose_host(h, METHOD_F, corresp, calm, calm_batched, n, B, PoseOut{Rt2, Rt3, reconst, T, repr_err, F21, F31, nullptr, nullptr, status});
+    return host_call(h, PoseCall{METHOD_F, corresp, calm, calm_batched, n, PoseOut{Rt2, Rt3, reconst, T, repr_err, F21, F31, nullptr, nullptr, status}}, B);
 }
 
 int tvf_optim_f_pose(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                      double* Rt2, double* Rt3, double* reconst, double* T, double* repr_err, double* F21, double* F31,
                      int32_t* iter, int32_t* status) {
-    return pose_host(h, METHOD_OPTF, corresp, calm, calm_batched, n, B, PoseOut{Rt2, Rt3, reconst, T, repr_err, F21, F31, iter, nullptr, status});
+    return host_call(h, PoseCall{METHOD_OPTF, corresp, calm, calm_batched, n, PoseOut{Rt2, Rt3, reconst, T, repr_err, F21, F31, iter, nullptr, status}}, B);
 }
 
 int tvf_optim_f_pose_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                          double* Rt2, double* Rt3, double* reconst, double* T, double* repr_err, double* F21, double* F31,
                          int32_t* iter, int32_t* status) {
-    return pose_dev(h, METHOD_OPTF, corresp, calm, calm_batched, n, B, PoseOut{Rt2, Rt3, reconst, T, repr_err, F21, F31, iter, nullptr, status});
+    return pose_dev(h, PoseCall{METHOD_OPTF, corresp, calm, calm_batched, n, PoseOut{Rt2, Rt3, reconst, T, repr_err, F21, F31, iter, nullptr, status}}, B);
 }
 
 int tvf_optim_f_max_n(void) { return optimf_max_n(); }
 
 int tvf_linear_tft_pose_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                             double* Rt2, double* Rt3, double* reconst, double* T, double* repr_err, int32_t* status) {
-    return pose_dev(h, METHOD_TFT, corresp, calm, calm_batched, n, B, PoseOut{Rt2, Rt3, reconst, T, repr_err, nullptr, nullptr, nullptr, nullptr, status});
+    return pose_dev(h, PoseCall{METHOD_TFT, corresp, calm, calm_batched, n, PoseOut{Rt2, Rt3, reconst, T, repr_err, nullptr, nullptr, nullptr, nullptr, status}}, B);
 }
 
 int tvf_linear_f_pose_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                           double* Rt2, double* Rt3, double* reconst, double* T, double* repr_err, double* F21, double* F31,
                           int32_t* status) {
-    return pose_dev(h, METHOD_F, corresp, calm, calm_batched, n, B, PoseOut{Rt2, Rt3, reconst, T, repr_err, F21, F31, nullptr, nullptr, status});
+    return pose_dev(h, PoseCall{METHOD_F, corresp, calm, calm_batched, n, PoseOut{Rt2, Rt3, reconst, T, repr_err, F21, F31, nullptr, nullptr, status}}, B);
 }
 
 int tvf_linear_tft(tvf_handle_t h, const double* p1, const double* p2, const double* p3, int rows, int n, int64_t B,
@@ -1339,8 +1318,8 @@ int tvf_project3d(tvf_handle_t h, const double* points3d, const double* P, int M
 static int sweep_common(tvf_handle_t h, int64_t first_trial, int64_t B, int n, const double* noise_levels, int L,
                         const double* P, double hi_x, double hi_y, double* d_out, cudaStream_t st) {
     void* p0; void* p1;
-    int rc = ensure_scratch(h, NSCRATCH - 2, (size_t)L * sizeof(double), &p0); if (rc) return rc;
-    rc = ensure_scratch(h, NSCRATCH - 3, 36 * sizeof(double), &p1); if (rc) return rc;
+    int rc = ensure_scratch(h, SCR_SWEEP_NOISE, (size_t)L * sizeof(double), &p0); if (rc) return rc;
+    rc = ensure_scratch(h, SCR_SWEEP_CAMS, 36 * sizeof(double), &p1); if (rc) return rc;
     TVF_CK(cudaMemcpyAsync(p0, noise_levels, (size_t)L * sizeof(double), cudaMemcpyHostToDevice, st));
     TVF_CK(cudaMemcpyAsync(p1, P, 36 * sizeof(double), cudaMemcpyHostToDevice, st));
     launch_sweep_trials(first_trial, B, n, (const double*)p0, L, (const double*)p1, hi_x, hi_y, d_out, st);
@@ -1383,52 +1362,84 @@ int tvf_generate_sweep(tvf_handle_t h, int64_t first_trial, int64_t B, int n, co
     return u.finish();
 }
 
+// What a device-resident sweep keeps over its chunks: trials are generated G at a time into `trials` (the generator
+// shares one pass per seed among its noise levels, one warp per seed, so it wants many seeds per launch) and solved C at
+// a time in `b`.
+struct Sweep {
+    tvf_handle_t h; cudaStream_t st; Method m; double hi_x, hi_y;
+    static constexpr int Q = 512;              // partial sums per level
+    ChunkBufs b; int64_t C, G; double* trials;
+
+    // buffers for chunks of problems of up to n points and `count` trials per generator range; ba: the adjustment's too
+    int init(int n, int64_t count, bool ba) {
+        // nothing crosses the bus, so the solver runs the device path's large chunks; the carve is the host path's because
+        // the evaluation kernels read its per-problem outputs
+        C = pick_chunk(h, count > 0 ? count : 1, false, pose_budget(n, false, ba));
+        Slot& s = h->slot[0];
+        int rc = ensure_arena(h, s, carve_pose(nullptr, n, C, true, false, ba, nullptr)); if (rc) return rc;
+        carve_pose(s.arena, n, C, true, false, ba, &b);
+        G = (count < 4 * C) ? count : 4 * C;
+        void* p;
+        rc = ensure_scratch(h, SCR_SWEEP_TRIALS, (size_t)G * 6 * n * sizeof(double), &p);
+        trials = (double*)p;
+        return rc;
+    }
+
+    // trials [first, first + count) of the L noise levels `noise` with cameras P and n points: generate them, solve them
+    // with `calm` and reduce them against the ground truth `gt` into the partial sums `pp`; with `pb`, also bundle-adjust
+    // each chunk's poses (experiments.m:127-141 with the library's adjustment) and reduce those into `pb`
+    int run(int64_t first, int64_t count, int n, const double* noise, int L, const double* P, const double* calm,
+            const double* gt, double* pp, double* pb) const {
+        for (int64_t gdone = 0; gdone < count; gdone += G) {
+            const int64_t Gc = (count - gdone < G) ? (count - gdone) : G;
+            int rc = sweep_common(h, first + gdone, Gc, n, noise, L, P, hi_x, hi_y, trials, st); if (rc) return rc;
+            for (int64_t off = 0; off < Gc; off += C) {
+                const int64_t Bc = (Gc - off < C) ? (Gc - off) : C;
+                ChunkBufs k = b;
+                k.in = trials + off * 6 * n; k.calm = calm; k.iter_sum = nullptr;
+                rc = run_pose_chunk(h, st, m, 0, n, Bc, k); if (rc) return rc;
+                launch_sweep_eval_accumulate(b.Rt2, b.Rt3, b.repr, b.status, first + gdone + off, Bc, L, Q, gt, pp, st);
+                h->launches += 1;
+                if (!pb) continue;
+                // a trial without a pose starts from NaN: the kernel copies it through with TVF_ST_NONFINITE and iter = 0
+                const BaArgs a{k.in, calm, 0, n, Bc, b.Rt2, b.Rt3, b.reconst, b.ba_Rt2, b.ba_Rt3, b.ba_X, b.ba_Xc, b.ba_repr,
+                               b.ba_iter, b.ba_status};
+                rc = ba_launched(h, launch_bundle_adjust(a, st), "bundle_adjust_kernel"); if (rc) return rc;
+                launch_sweep_eval_accumulate(b.ba_Rt2, b.ba_Rt3, b.ba_repr, b.status, first + gdone + off, Bc, L, Q, gt, pb, st,
+                                             b.ba_status, b.ba_iter);
+                h->launches += 1;
+            }
+        }
+        return TVF_OK;
+    }
+};
+
 // experiments.m:74-124 for one method, device-resident: generate the trials of the sweep, solve them, and
 // reduce ReprError / AngError per noise level.  Only the L x 5 table crosses the bus.
 int tvf_sweep_run(tvf_handle_t h, int method, int64_t first_trial, int64_t B, int n, const double* noise_levels, int L,
                   const double* P, double hi_x, double hi_y, const double* calm, const double* Rt0_2, const double* Rt0_3,
                   double* table) {
     int rc = sweep_check(h, first_trial, B, n, noise_levels, L, P, table); if (rc) return rc;
-    if (!calm || !Rt0_2 || !Rt0_3 || (method != 1 && method != 7 && method != 8))
+    Method m;
+    if (!calm || !Rt0_2 || !Rt0_3 || !method_of(method, &m))
         return fail(h, TVF_ERR_ARG, "method must be 1 (linear TFT), 7 (linear F) or 8 (optimal F); calm/Rt0 required");
-    if (method != 1 && n < 8) return fail(h, TVF_ERR_TOO_FEW_POINTS, TVF_LINEARF_ERRMSG);
+    if (m != METHOD_TFT && n < 8) return fail(h, TVF_ERR_TOO_FEW_POINTS, TVF_LINEARF_ERRMSG);
     TVF_CK(cudaSetDevice(h->device));
-    Slot& s = h->slot[0];
-    cudaStream_t st = s.stream;
-    const int Q = 512;
-    // nothing crosses the bus here, so the solver runs its large device-path launches (the per-problem output buffers of
-    // the host-path layout are still needed: the evaluation kernels read them)
-    const int64_t C = pick_chunk(h, n, B > 0 ? B : 1, false, false);
-    const size_t need = carve(nullptr, n, C, true, false, false, nullptr);
-    rc = ensure_arena(h, s, need); if (rc) return rc;
-    ChunkBufs b; carve(s.arena, n, C, true, false, false, &b);
+    Sweep sw{h, h->slot[0].stream, m, hi_x, hi_y};
+    const cudaStream_t st = sw.st;
+    const int Q = Sweep::Q;
+    rc = sw.init(n, B, false); if (rc) return rc;
     void *pc, *pr, *pp, *pt;
-    rc = ensure_scratch(h, 0, 27 * sizeof(double), &pc); if (rc) return rc;
-    rc = ensure_scratch(h, NSCRATCH - 4, 24 * sizeof(double), &pr); if (rc) return rc;
-    rc = ensure_scratch(h, NSCRATCH - 5, (size_t)L * Q * 5 * sizeof(double), &pp); if (rc) return rc;
-    rc = ensure_scratch(h, NSCRATCH - 6, (size_t)L * 5 * sizeof(double), &pt); if (rc) return rc;
+    rc = ensure_scratch(h, SCR_SWEEP_CALM, 27 * sizeof(double), &pc); if (rc) return rc;
+    rc = ensure_scratch(h, SCR_SWEEP_GT, 24 * sizeof(double), &pr); if (rc) return rc;
+    rc = ensure_scratch(h, SCR_SWEEP_PARTIAL, (size_t)L * Q * 5 * sizeof(double), &pp); if (rc) return rc;
+    rc = ensure_scratch(h, SCR_SWEEP_TABLE, (size_t)L * 5 * sizeof(double), &pt); if (rc) return rc;
     TVF_CK(cudaMemcpyAsync(pc, calm, 27 * sizeof(double), cudaMemcpyHostToDevice, st));
     TVF_CK(cudaMemcpyAsync(pr, Rt0_2, 12 * sizeof(double), cudaMemcpyHostToDevice, st));
     TVF_CK(cudaMemcpyAsync((double*)pr + 12, Rt0_3, 12 * sizeof(double), cudaMemcpyHostToDevice, st));
     TVF_CK(cudaMemsetAsync(pp, 0, (size_t)L * Q * 5 * sizeof(double), st));
-    // The generator shares one pass per seed among its L noise levels (one warp per seed), so it wants many seeds
-    // per launch: trials are generated in super-chunks of up to 4 solver chunks into a staging buffer.
-    const int64_t G = (B < 4 * C) ? B : 4 * C;
-    void* pg;
-    rc = ensure_scratch(h, NSCRATCH - 7, (size_t)G * 6 * n * sizeof(double), &pg); if (rc) return rc;
-    for (int64_t gdone = 0; gdone < B; gdone += G) {
-        const int64_t Gc = (B - gdone < G) ? (B - gdone) : G;
-        rc = sweep_common(h, first_trial + gdone, Gc, n, noise_levels, L, P, hi_x, hi_y, (double*)pg, st); if (rc) return rc;
-        for (int64_t off = 0; off < Gc; off += C) {
-            const int64_t Bc = (Gc - off < C) ? (Gc - off) : C;
-            const double* d_in = (const double*)pg + off * 6 * n;
-            rc = run_pose_chunk(h, st, method == 1 ? METHOD_TFT : (method == 7 ? METHOD_F : METHOD_OPTF), d_in, (const double*)pc, 0, n,
-                                Bc, b.T, b.F, b.core, b.cand, b.votes, b.scale, b.Rt2, b.Rt3, b.reconst, b.repr, b.status, b.iters, nullptr);
-            if (rc) return rc;
-            launch_sweep_eval_accumulate(b.Rt2, b.Rt3, b.repr, b.status, first_trial + gdone + off, Bc, L, Q, (const double*)pr, (double*)pp, st);
-            h->launches += 1;
-        }
-    }
+    rc = sw.run(first_trial, B, n, noise_levels, L, P, (const double*)pc, (const double*)pr, (double*)pp, nullptr);
+    if (rc) return rc;
     launch_sweep_eval_finish((const double*)pp, L, Q, (double*)pt, st);
     h->launches += 1;
     TVF_CK(cudaGetLastError());
@@ -1440,13 +1451,14 @@ int tvf_sweep_run(tvf_handle_t h, int method, int64_t first_trial, int64_t B, in
 // experiments.m:74-124 for any of its four options ('noise', 'focal', 'points', 'angle', :38-47): every level carries its
 // own noise, point count, cameras, calibration and ground truth.  Level by level: the level's trials (one per seed) are
 // generated with its cameras, solved with its n and CalM, and reduced into its row of the table -- all on the device.
-// ba: each chunk's poses are then bundle-adjusted (experiments.m:127-141 with the library's adjustment) and reduced into
-// columns 5-10 of an L x 11 table; without it the table is L x 5 and the chunk size, and so every sum, is unchanged.
+// ba: each chunk's poses are then bundle-adjusted and reduced into columns 5-10 of an L x 11 table; without it the table
+// is L x 5 and the chunk size, and so every sum, is unchanged.
 static int sweep_levels(tvf_handle_t h, int method, int64_t first_trial, int64_t B, const tvf_sweep_level* levels, int L,
                         double hi_x, double hi_y, double* table, bool ba) {
     if (!h) return TVF_ERR_ARG;
     if (!levels || !table || L < 1 || B < 0 || first_trial < 0) return fail(h, TVF_ERR_ARG, "NULL argument or bad size");
-    if (method != 1 && method != 7 && method != 8) return fail(h, TVF_ERR_ARG, "method must be 1 (linear TFT), 7 (linear F) or 8 (optimal F)");
+    Method m;
+    if (!method_of(method, &m)) return fail(h, TVF_ERR_ARG, "method must be 1 (linear TFT), 7 (linear F) or 8 (optimal F)");
     if ((first_trial + B) / L + 1 > 0xffffffffLL) return fail(h, TVF_ERR_ARG, "seed exceeds 32 bits");
     int n_max = 1;
     for (int l = 0; l < L; ++l) {
@@ -1454,24 +1466,17 @@ static int sweep_levels(tvf_handle_t h, int method, int64_t first_trial, int64_t
         if (levels[l].n > n_max) n_max = levels[l].n;
     }
     TVF_CK(cudaSetDevice(h->device));
-    Slot& s = h->slot[0];
-    cudaStream_t st = s.stream;
-    const int Q = 512;
+    Sweep sw{h, h->slot[0].stream, m, hi_x, hi_y};
+    const cudaStream_t st = sw.st;
+    const int Q = Sweep::Q;
     const int W = ba ? 11 : 5;                 // table columns
-    const Method m = method == 1 ? METHOD_TFT : (method == 7 ? METHOD_F : METHOD_OPTF);
-    const int64_t per_level = B / L + 1;
-    const int64_t C = pick_chunk(h, n_max, per_level, false, ba);
-    const size_t need = carve(nullptr, n_max, C, true, false, ba, nullptr);
-    int rc = ensure_arena(h, s, need); if (rc) return rc;
-    ChunkBufs b; carve(s.arena, n_max, C, true, false, ba, &b);
-    void *pc, *pr, *pp, *pt, *pg, *pb = nullptr;
-    rc = ensure_scratch(h, NSCRATCH - 8, (size_t)L * 27 * sizeof(double), &pc); if (rc) return rc;
-    rc = ensure_scratch(h, NSCRATCH - 9, (size_t)L * 24 * sizeof(double), &pr); if (rc) return rc;
-    rc = ensure_scratch(h, NSCRATCH - 5, (size_t)L * Q * 5 * sizeof(double), &pp); if (rc) return rc;
-    rc = ensure_scratch(h, NSCRATCH - 6, (size_t)L * W * sizeof(double), &pt); if (rc) return rc;
-    if (ba) { rc = ensure_scratch(h, NSCRATCH - 10, (size_t)L * Q * 6 * sizeof(double), &pb); if (rc) return rc; }
-    const int64_t G = (per_level < 4 * C) ? per_level : 4 * C;
-    rc = ensure_scratch(h, NSCRATCH - 7, (size_t)G * 6 * n_max * sizeof(double), &pg); if (rc) return rc;
+    int rc = sw.init(n_max, B / L + 1, ba); if (rc) return rc;
+    void *pc, *pr, *pp, *pt, *pb = nullptr;
+    rc = ensure_scratch(h, SCR_SWEEP_CALM, (size_t)L * 27 * sizeof(double), &pc); if (rc) return rc;
+    rc = ensure_scratch(h, SCR_SWEEP_GT, (size_t)L * 24 * sizeof(double), &pr); if (rc) return rc;
+    rc = ensure_scratch(h, SCR_SWEEP_PARTIAL, (size_t)L * Q * 5 * sizeof(double), &pp); if (rc) return rc;
+    rc = ensure_scratch(h, SCR_SWEEP_TABLE, (size_t)L * W * sizeof(double), &pt); if (rc) return rc;
+    if (ba) { rc = ensure_scratch(h, SCR_SWEEP_BA_PARTIAL, (size_t)L * Q * 6 * sizeof(double), &pb); if (rc) return rc; }
     std::vector<double> hc((size_t)L * 27), hr((size_t)L * 24);
     for (int l = 0; l < L; ++l) {
         memcpy(&hc[(size_t)l * 27], levels[l].calm, 27 * sizeof(double));
@@ -1488,34 +1493,12 @@ static int sweep_levels(tvf_handle_t h, int method, int64_t first_trial, int64_t
         // trials j = l + L*q of [first_trial, first_trial + B): 0-based seed index q in [q_lo, q_hi), seed = q + 1
         const int64_t q_lo = (first_trial > l) ? (first_trial - l + L - 1) / L : 0;
         const int64_t q_hi = (first_trial + B > l) ? (first_trial + B - l + L - 1) / L : 0;
-        const int64_t Bl = q_hi - q_lo;
         const int n = levels[l].n;
-        if ((method != 1 && n < 8) || n < 7) { skipped[(size_t)l] = 1; continue; }          // experiments.m:99-104: "not enough matches"
-        if (Bl <= 0) continue;
-        const double* calm_l = (const double*)pc + (size_t)l * 27;
-        const double* gt_l = (const double*)pr + (size_t)l * 24;
-        for (int64_t gdone = 0; gdone < Bl; gdone += G) {
-            const int64_t Gc = (Bl - gdone < G) ? (Bl - gdone) : G;
-            rc = sweep_common(h, q_lo + gdone, Gc, n, &levels[l].noise, 1, levels[l].P, hi_x, hi_y, (double*)pg, st); if (rc) return rc;
-            for (int64_t off = 0; off < Gc; off += C) {
-                const int64_t Bc = (Gc - off < C) ? (Gc - off) : C;
-                const double* d_in = (const double*)pg + off * 6 * n;
-                rc = run_pose_chunk(h, st, m, d_in, calm_l, 0, n, Bc, b.T, b.F, b.core,
-                                    b.cand, b.votes, b.scale, b.Rt2, b.Rt3, b.reconst, b.repr, b.status, b.iters, nullptr);
-                if (rc) return rc;
-                launch_sweep_eval_accumulate(b.Rt2, b.Rt3, b.repr, b.status, q_lo + gdone + off, Bc, 1, Q, gt_l,
-                                             (double*)pp + (size_t)l * Q * 5, st);
-                h->launches += 1;
-                if (!ba) continue;
-                // a trial without a pose starts from NaN: the kernel copies it through with TVF_ST_NONFINITE and iter = 0
-                rc = ba_launch(h, st, BaIo{d_in, calm_l, 0, n, b.Rt2, b.Rt3, b.reconst, b.ba_Rt2, b.ba_Rt3, b.ba_X, b.ba_repr,
-                                           b.ba_iter, b.ba_status}, Bc, b.ba_Xc);
-                if (rc) return rc;
-                launch_sweep_eval_accumulate(b.ba_Rt2, b.ba_Rt3, b.ba_repr, b.status, q_lo + gdone + off, Bc, 1, Q, gt_l,
-                                             (double*)pb + (size_t)l * Q * 6, st, b.ba_status, b.ba_iter);
-                h->launches += 1;
-            }
-        }
+        if ((m != METHOD_TFT && n < 8) || n < 7) { skipped[(size_t)l] = 1; continue; }          // experiments.m:99-104: "not enough matches"
+        if (q_hi <= q_lo) continue;
+        rc = sw.run(q_lo, q_hi - q_lo, n, &levels[l].noise, 1, levels[l].P, (const double*)pc + (size_t)l * 27,
+                    (const double*)pr + (size_t)l * 24, (double*)pp + (size_t)l * Q * 5, ba ? (double*)pb + (size_t)l * Q * 6 : nullptr);
+        if (rc) return rc;
         launch_sweep_eval_finish((const double*)pp + (size_t)l * Q * 5, 1, Q, (double*)pt + (size_t)l * W, st);
         h->launches += 1;
         if (ba) {
@@ -1550,27 +1533,27 @@ int tvf_sweep_run_levels_ba(tvf_handle_t h, int method, int64_t first_trial, int
 int tvf_bundle_adjust(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                       const double* Rt2_0, const double* Rt3_0, const double* reconst0, double* Rt2, double* Rt3,
                       double* reconst, double* repr_err, int32_t* iter, int32_t* status) {
-    return ba_host(h, BaIo{corresp, calm, calm_batched, n, Rt2_0, Rt3_0, reconst0, Rt2, Rt3, reconst, repr_err, iter, status}, B);
+    return host_call(h, BundleAdjust{BaArgs{corresp, calm, calm_batched, n, 0, Rt2_0, Rt3_0, reconst0, Rt2, Rt3, reconst, nullptr,
+                                            repr_err, iter, status}}, B);
 }
 
 int tvf_bundle_adjust_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                           const double* Rt2_0, const double* Rt3_0, const double* reconst0, double* Rt2, double* Rt3,
                           double* reconst, double* repr_err, int32_t* iter, int32_t* status) {
-    return ba_dev(h, BaIo{corresp, calm, calm_batched, n, Rt2_0, Rt3_0, reconst0, Rt2, Rt3, reconst, repr_err, iter, status}, B);
+    return ba_dev(h, BundleAdjust{BaArgs{corresp, calm, calm_batched, n, 0, Rt2_0, Rt3_0, reconst0, Rt2, Rt3, reconst, nullptr,
+                                         repr_err, iter, status}}, B);
 }
 
 int tvf_ba_covariance(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                       const double* Rt2, const double* Rt3, const double* reconst, double* cov_cam, double* cov_pts,
                       double* sigma2, int32_t* status) {
-    return ba_host(h, BaIo{corresp, calm, calm_batched, n, Rt2, Rt3, reconst, nullptr, nullptr, nullptr, nullptr, nullptr,
-                           status, true, cov_cam, cov_pts, sigma2}, B);
+    return host_call(h, Covariance{BaCovArgs{corresp, calm, calm_batched, n, 0, Rt2, Rt3, reconst, cov_cam, cov_pts, sigma2, status}}, B);
 }
 
 int tvf_ba_covariance_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                           const double* Rt2, const double* Rt3, const double* reconst, double* cov_cam, double* cov_pts,
                           double* sigma2, int32_t* status) {
-    return ba_dev(h, BaIo{corresp, calm, calm_batched, n, Rt2, Rt3, reconst, nullptr, nullptr, nullptr, nullptr, nullptr,
-                          status, true, cov_cam, cov_pts, sigma2}, B);
+    return ba_dev(h, Covariance{BaCovArgs{corresp, calm, calm_batched, n, 0, Rt2, Rt3, reconst, cov_cam, cov_pts, sigma2, status}}, B);
 }
 
 int tvf_ang_error(tvf_handle_t h, const double* Rt_true, int true_batched, const double* Rt_est, int64_t B,
