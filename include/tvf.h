@@ -267,6 +267,47 @@ int tvf_ba_covariance_dev(tvf_handle_t h, const double* corresp, const double* c
                           const double* Rt2, const double* Rt3, const double* reconst, double* cov_cam, double* cov_pts,
                           double* sigma2, int32_t* status);
 
+/* ---- robust pose from raw matches: consensus and RANSAC ----------------------------------------------------------
+ * Inlier test of one match x = (x1 y1 x2 y2 x3 y3) under the cameras K1[I|0], K2[R2|t2], K3[R3|t3]: triangulate it as
+ * tvf_triangulate does (triangulation3D.m), dehomogenise X(1:3)/X(4), re-project as tvf_project3d does and subtract x
+ * (experiments_real.m:94-98).  The match is an inlier iff all six residuals are finite and <= threshold in absolute
+ * value.  Unlike the reference, a NaN residual makes the match an outlier.
+ *
+ * tvf_consensus: that test for every match of corresp (6 x n x B) under one pose per problem (Rt2, Rt3 3 x 4 x B);
+ * calm 9 x 3 (calm_batched = 0) or 9 x 3 x B.  inliers (n x B, 0 / 1) and n_inliers (B) may be NULL.  threshold (pixels)
+ * must be finite and > 0.  Chunks and shards like tvf_pose; returns 0 or an error. */
+int tvf_consensus(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
+                  const double* Rt2, const double* Rt3, double threshold, uint8_t* inliers, int32_t* n_inliers);
+
+#define TVF_ST_RANSAC_FAILED 128 /* tvf_ransac_pose: every hypothesis of the problem was flagged: no pose           */
+
+/* Pose of each problem from raw matches with outliers: RANSAC over minimal linear solves and the consensus above.
+ * method 1: hypotheses from LinearTFTPoseEstimation on s = 7 matches; 7: LinearFPoseEstimation on s = 8 (linearF.m:35-37).
+ * Per problem b, with key seeds[b]:
+ *   1. hypothesis h = 0 .. hypotheses-1 draws s distinct match indices (below) and solves the method on those columns;
+ *   2. its score is its consensus count with `threshold`, or -1 when the method flagged it (status != 0);
+ *   3. the best hypothesis has the largest score, ties to the smallest h;
+ *   4. the refit solves the method on the consensus columns of the best hypothesis (index order) and is scored again.
+ * Result rule: if the best score is >= s, the refit's status is 0 and its count is >= the best score, the refit pose
+ * is returned, otherwise the best hypothesis's pose.  inliers (n x B, 0 / 1) and n_inliers (B) are always those of the
+ * returned pose; sample (s x B) holds the best hypothesis's indices.  If every hypothesis is flagged, status gets
+ * TVF_ST_RANSAC_FAILED, Rt2 and Rt3 are NaN, inliers 0 and sample -1; otherwise status is 0.
+ * Sampler (reproducible from NumPy integer for integer): mix64 is splitmix64's output function (z += 0x9E3779B97F4A7C15;
+ * z = (z ^ z >> 30) * 0xBF58476D1CE4E5B9; z = (z ^ z >> 27) * 0x94D049BB133111EB; z ^ z >> 31); draw j of hypothesis h is
+ * r = mix64(seed ^ mix64((h << 8) | j)); uniform(m) = ((r >> 32) * m) >> 32; the indices come from Floyd's algorithm: for
+ * j = 0 .. s-1, m = n - s + j + 1, u = uniform(m), take u, or m - 1 if u was already taken; kept in draw order.
+ * The key is per problem, so a result does not depend on its batch, chunk, shard or form (bit-identical).
+ * Errors: method other than 1 or 7, hypotheses outside 1 .. 2^24, a threshold that is not finite or <= 0, or n < s
+ * (method 7: TVF_ERR_TOO_FEW_POINTS) -> TVF_ERR_ARG.  Outputs may be NULL.  The host form chunks and shards like
+ * tvf_pose.  The _dev form takes device pointers (corresp 16-byte aligned) and, unlike the other _dev forms,
+ * synchronises the handle's stream once per chunk: the refit groups the problems by consensus size, which it reads back. */
+int tvf_ransac_pose(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched, int n,
+                    int64_t B, int hypotheses, double threshold, const uint64_t* seeds, double* Rt2, double* Rt3,
+                    uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* status);
+int tvf_ransac_pose_dev(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched, int n,
+                        int64_t B, int hypotheses, double threshold, const uint64_t* seeds, double* Rt2, double* Rt3,
+                        uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* status);
+
 /* ---- inputs of the measured configurations, generated where they are consumed ------------------------
  * Trials [first_trial, first_trial+B) of experiments.m's sweep: trial j uses noise_levels[j mod L] and
  * seed j div L + 1; each is generateSyntheticScene(n+100, noise, seed, ...) followed by the column

@@ -27,6 +27,7 @@ ST_NO_POSE_3 = 8
 ST_NONFINITE = 16
 ST_BA_NOCONV = 32
 ST_COV_SINGULAR = 64
+ST_RANSAC_FAILED = 128
 
 LINEARF_ERRMSG = ("At least 8 correspondences are necessary to compute the "
                   "fundamental matrix linearly\\n")
@@ -96,6 +97,9 @@ SIGNATURES = {
     "tvf_bundle_adjust_dev": (_I, [_H, C.c_void_p, C.c_void_p, _I, _I, _L] + [C.c_void_p] * 9),
     "tvf_ba_covariance": (_I, [_H, _D, _D, _I, _I, _L, _D, _D, _D, _D, _D, _D, _S]),
     "tvf_ba_covariance_dev": (_I, [_H, C.c_void_p, C.c_void_p, _I, _I, _L] + [C.c_void_p] * 7),
+    "tvf_consensus": (_I, [_H, _D, _D, _I, _I, _L, _D, _D, C.c_double, C.c_void_p, _S]),
+    "tvf_ransac_pose": (_I, [_H, _I, _D, _D, _I, _I, _L, _I, C.c_double, C.c_void_p, _D, _D, C.c_void_p, _S, _S, _S]),
+    "tvf_ransac_pose_dev": (_I, [_H, _I, C.c_void_p, C.c_void_p, _I, _I, _L, _I, C.c_double] + [C.c_void_p] * 7),
     "tvf_launch_count": (_L, [_H]),
     "tvf_profile_enable": (_I, [_H, _I]),
     "tvf_profile_reset": (_I, [_H]),

@@ -370,6 +370,73 @@ def ba_covariance(Corresp, CalM, R_t_2, R_t_3, Reconst, points=False, device=Non
     return out
 
 
+def _pose_pair(R_t_2, R_t_3, B, batched):
+    r2, _, _ = _cm(np.broadcast_to(R_t_2, (B, 3, 4)) if batched else R_t_2, 2)
+    r3, _, _ = _cm(np.broadcast_to(R_t_3, (B, 3, 4)) if batched else R_t_3, 2)
+    if r2.shape != (B, 4, 3) or r3.shape != (B, 4, 3):
+        raise ValueError("R_t_2, R_t_3 must be 3x4 (with the batch axis of Corresp)")
+    return r2, r3
+
+
+def consensus(Corresp, CalM, R_t_2, R_t_3, threshold=1.0, device=None):
+    """Which matches of Corresp (6xN) the pose (R_t_2, R_t_3) explains (tvf_consensus, include/tvf.h): each match is
+    triangulated with K1[I|0], K2*R_t_2, K3*R_t_3, re-projected, and kept iff its six residuals are finite and
+    <= threshold pixels -- the inlier rule of experiments_real.m:94-98 (epfl.inlier_filter), except that a NaN
+    residual makes the match an outlier.  Returns (mask, count): bool (N) and int, or (B,N) and (B,) when batched."""
+    c, batched, B = _cm(Corresp, 2)
+    if c.shape[2] != 6:
+        raise ValueError("Corresp must be 6xN")
+    n = c.shape[1]
+    calm, cb = _calm(CalM, B)
+    r2, r3 = _pose_pair(R_t_2, R_t_3, B, batched)
+    h = _lib.handle(device)
+    mask = np.zeros((B, n), dtype=np.uint8); cnt = np.zeros(B, dtype=np.int32)
+    h.call("tvf_consensus", _p(c), _p(calm), cb, n, B, _p(r2), _p(r3), float(threshold), _vp(mask), cnt.ctypes.data_as(_ip))
+    mask = mask.astype(bool)
+    return (mask, cnt) if batched else (mask[0], int(cnt[0]))
+
+
+class RansacResult(tuple):
+    """(R_t_2, R_t_3, inliers, n_inliers, sample) of ransac_pose, plus .status (0, or TVF_ST_RANSAC_FAILED)."""
+    status = None
+
+
+RANSAC_SAMPLE_SIZE = {1: 7, 7: 8}
+
+
+def ransac_pose(Corresp, CalM, method=1, hypotheses=1024, threshold=1.0, seed=0, device=None):
+    """Pose from raw matches with outliers (tvf_ransac_pose, include/tvf.h): `hypotheses` minimal solves of method 1
+    (LinearTFTPoseEstimation on 7 matches) or 7 (LinearFPoseEstimation on 8), each scored by its consensus (see
+    `consensus`, `threshold` pixels); the method is then run again on the consensus of the best one and that refit is
+    kept if it explains at least as many matches.  seed: int (problem b gets the key seed + b) or an array (B,) of keys.
+    Returns (R_t_2, R_t_3, inliers, n_inliers, sample) -- inliers bool (N), the sample the best hypothesis drew -- with
+    .status; batched inputs give (B,3,4), (B,3,4), (B,N), (B,), (B,s)."""
+    if method not in RANSAC_SAMPLE_SIZE:
+        raise ValueError("ransac_pose: method must be 1 (linear TFT) or 7 (linear F)")
+    s = RANSAC_SAMPLE_SIZE[method]
+    c, batched, B = _cm(Corresp, 2)
+    if c.shape[2] != 6:
+        raise ValueError("Corresp must be 6xN")
+    n = c.shape[1]
+    calm, cb = _calm(CalM, B)
+    if np.ndim(seed) == 0:
+        seeds = (np.uint64(int(seed) % 2 ** 64) + np.arange(B, dtype=np.uint64)).astype(np.uint64)
+    else:
+        seeds = np.ascontiguousarray(seed, dtype=np.uint64)
+        if seeds.shape != (B,):
+            raise ValueError("seed must be an int or an array of B keys")
+    h = _lib.handle(device)
+    Rt2 = np.empty((B, 12)); Rt3 = np.empty((B, 12)); mask = np.zeros((B, n), dtype=np.uint8)
+    cnt = np.zeros(B, dtype=np.int32); smp = np.zeros((B, s), dtype=np.int32); st = np.zeros(B, dtype=np.int32)
+    h.call("tvf_ransac_pose", int(method), _p(c), _p(calm), cb, n, B, int(hypotheses), float(threshold), _vp(seeds),
+           _p(Rt2), _p(Rt3), _vp(mask), cnt.ctypes.data_as(_ip), smp.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
+    mask = mask.astype(bool)
+    out = RansacResult((_from_cm(Rt2, B, (3, 4), batched), _from_cm(Rt3, B, (3, 4), batched),
+                        mask if batched else mask[0], cnt if batched else int(cnt[0]), smp if batched else smp[0]))
+    out.status = st if batched else int(st[0])
+    return out
+
+
 def pose_rms_errors(cov_cam, R_t_2, R_t_3, sigma2=1.0):
     """First-order RMS of the errors AngError measures (auxiliar_functions/AngError.m), in degrees, from a 12x12
     cov_cam of ba_covariance (unit noise) scaled by sigma2: returns (rot_err, t_err), each [view 2, view 3] (shape (2,),

@@ -11,8 +11,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libtvf.so")
 OBJ = os.path.join(HERE, "build")
-SOURCES = ["tvf_core_kernels.cu", "tvf_large_kernels.cu", "tvf_pose_kernels.cu", "tvf_scene_kernels.cu", "tvf_gh_kernels.cu", "tvf_ba_kernels.cu", "tvf_ba_cov_kernels.cu", "tvf_api.cu"]
-HEADERS = ["tvf_math.cuh", "tvf_pose.cuh", "tvf_warp.cuh", "tvf_async.cuh", "tvf_scene.cuh", "tvf_ba.cuh", "tvf_kernels.h", os.path.join("..", "..", "include", "tvf.h")]
+SOURCES = ["tvf_core_kernels.cu", "tvf_large_kernels.cu", "tvf_pose_kernels.cu", "tvf_scene_kernels.cu", "tvf_gh_kernels.cu", "tvf_ba_kernels.cu", "tvf_ba_cov_kernels.cu", "tvf_ransac_kernels.cu", "tvf_api.cu"]
+HEADERS = ["tvf_math.cuh", "tvf_pose.cuh", "tvf_warp.cuh", "tvf_async.cuh", "tvf_scene.cuh", "tvf_ba.cuh", "tvf_ransac.cuh", "tvf_kernels.h", os.path.join("..", "..", "include", "tvf.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xptxas=-v", "-Xcompiler", "-fPIC", "-cudart", "shared"]
 

@@ -7,6 +7,7 @@
 #include <cuda_runtime.h>
 #include <sched.h>
 
+#include <algorithm>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -735,6 +736,174 @@ template <class Call> int ba_dev(tvf_handle_t h, const Call& c, int64_t B) {
     }
     return TVF_OK;
 }
+
+// ---- RANSAC pose (tvf_ransac_pose[_dev]) and consensus (tvf_consensus) ----------------------------------------------
+
+int ransac_launched(tvf_handle_t h) {
+    h->launches += 1;
+    TVF_CK(cudaGetLastError());
+    return TVF_OK;
+}
+
+// outputs may be null: on the device path the work space stands in for them
+struct Ransac {
+    Method method; int s; int H; double th;
+    RansacArgs io;
+    RansacArgs d{};
+    ChunkBufs w{};                       // the pose path's work space, for the B H hypotheses and then the refit
+    int check(tvf_handle_t h, int64_t B) const {
+        if (!h) return TVF_ERR_ARG;
+        if (!io.corresp || !io.calm || !io.seeds) return fail(h, TVF_ERR_ARG, "ransac_pose: corresp, calm and seeds must not be NULL");
+        if (B < 0) return fail(h, TVF_ERR_ARG, "ransac_pose: B >= 0");
+        if (io.n < s) {
+            if (method == METHOD_F) return fail(h, TVF_ERR_TOO_FEW_POINTS, TVF_LINEARF_ERRMSG);
+            return fail(h, TVF_ERR_ARG, "ransac_pose: method 1 needs n >= 7 points");
+        }
+        if (H < 1 || H > (1 << 24)) return fail(h, TVF_ERR_ARG, "ransac_pose: hypotheses must be in 1 .. 2^24");
+        if (!(th > 0.0) || !(th < __builtin_huge_val())) return fail(h, TVF_ERR_ARG, "ransac_pose: threshold must be finite and > 0");
+        return TVF_OK;
+    }
+    int32_t*& status() { return io.status; }
+    // H hypotheses (the pose path's work space at n = s, the minimal problem, its calm, pose and count), the refit's
+    // compacted problem, the best and the refit pose with their masks and counters, and the host path's inputs and
+    // outputs; a batched calm counted either way
+    size_t budget(bool host_io) const {
+        const int n = io.n;
+        size_t b = (size_t)H * (pose_budget(s, false, false) + (size_t)(6 * s + 27 + 24) * 8 + 4);
+        b += (size_t)(6 * n + 27 + 48) * 8 + 2 * (size_t)n + 6 * 4;
+        if (host_io) b += (size_t)(6 * n + 27 + 1 + 24) * 8 + n + 4 * (size_t)(s + 2);
+        return b;
+    }
+    size_t carve(char* base, int64_t C, bool host_io = true) {
+        const int n = io.n;
+        const int64_t Q = C * H;
+        Carver c(base);
+        d = io;
+        if (host_io) {
+            d.corresp = c.take<double>((size_t)6 * n * C); d.calm = c.take<double>(io.calm_batched ? 27 * C : 27);
+            d.seeds = c.take<uint64_t>(C);
+        }
+        if (host_io || !d.Rt2) d.Rt2 = c.take<double>(12 * C);
+        if (host_io || !d.Rt3) d.Rt3 = c.take<double>(12 * C);
+        if (host_io || !d.inliers) d.inliers = c.take<unsigned char>((size_t)n * C);
+        if (host_io || !d.n_inliers) d.n_inliers = c.take<int>(C);
+        if (host_io || !d.sample) d.sample = c.take<int>((size_t)s * C);
+        if (host_io || !d.status) d.status = c.take<int>(C);
+        c.off += carve_pose(base ? base + c.off : nullptr, s, Q, false, false, false, &w);
+        d.gin = c.take<double>((size_t)6 * s * Q); d.gcalm = io.calm_batched ? c.take<double>(27 * Q) : nullptr;
+        d.hRt2 = c.take<double>(12 * Q); d.hRt3 = c.take<double>(12 * Q); d.hstatus = w.status; d.hcount = c.take<int>(Q);
+        d.best_h = c.take<int>(C); d.cnt_best = c.take<int>(C); d.mask_best = c.take<unsigned char>((size_t)n * C);
+        d.bestRt2 = c.take<double>(12 * C); d.bestRt3 = c.take<double>(12 * C);
+        d.refst = c.take<int>(C); d.cnt_refit = c.take<int>(C); d.mask_refit = c.take<unsigned char>((size_t)n * C);
+        d.refRt2 = c.take<double>(12 * C); d.refRt3 = c.take<double>(12 * C);
+        d.rin = c.take<double>((size_t)6 * n * C); d.rcalm = io.calm_batched ? c.take<double>(27 * C) : nullptr;
+        d.plist = c.take<int>(C);
+        return c.off;
+    }
+    template <class F> void arrays(F&& f) {
+        const int n = io.n;
+        f(io.corresp, Arr::input(8 * 6 * n, d.corresp));
+        f(io.calm, Arr::input(8 * 27, d.calm, !io.calm_batched));
+        f(io.seeds, Arr::input(8, d.seeds));
+        f(io.Rt2, Arr::output(8 * 12, d.Rt2));
+        f(io.Rt3, Arr::output(8 * 12, d.Rt3));
+        f(io.inliers, Arr::output(n, d.inliers));
+        f(io.n_inliers, Arr::output(4, d.n_inliers));
+        f(io.sample, Arr::output(4 * s, d.sample));
+        f(io.status, Arr::output(4, d.status));
+    }
+    // sample and solve the hypotheses, score them, select; refit on the consensus of the best, grouped by its size
+    // (the one read-back of the call); rescore; the result rule
+    int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
+        RansacArgs a = d; a.B = Bc;
+        const int n = a.n;
+        const int64_t Q = Bc * H;
+        launch_ransac_sample(a, H, s, st);
+        int rc = ransac_launched(h); if (rc) return rc;
+        ChunkBufs k = w;
+        k.in = a.gin; k.calm = a.calm_batched ? a.gcalm : a.calm; k.Rt2 = a.hRt2; k.Rt3 = a.hRt3;
+        if (method != METHOD_TFT) k.T = nullptr;
+        rc = run_pose_chunk(h, st, method, a.calm_batched, s, Q, k); if (rc) return rc;
+        TVF_CK(cudaMemsetAsync(a.hcount, 0, (size_t)Q * sizeof(int), st));
+        launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, n, Q, H, a.hRt2, a.hRt3, a.hstatus, th, a.hcount, nullptr,
+                                h->sm_count, st);
+        rc = ransac_launched(h); if (rc) return rc;
+        launch_ransac_select(a, H, st);
+        rc = ransac_launched(h); if (rc) return rc;
+        TVF_CK(cudaMemsetAsync(a.cnt_best, 0, (size_t)Bc * sizeof(int), st));
+        launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, n, Bc, 1, a.bestRt2, a.bestRt3, nullptr, th, a.cnt_best,
+                                a.mask_best, h->sm_count, st);
+        rc = ransac_launched(h); if (rc) return rc;
+        std::vector<int> cnt((size_t)Bc);
+        TVF_CK(cudaMemcpyAsync(cnt.data(), a.cnt_best, (size_t)Bc * sizeof(int), cudaMemcpyDeviceToHost, st));
+        TVF_CK(cudaStreamSynchronize(st));
+        TVF_CK(cudaMemsetAsync(a.refst, 0xff, (size_t)Bc * sizeof(int), st));      // -1: no refit
+        std::vector<int> order;
+        for (int64_t b = 0; b < Bc; ++b) if (cnt[(size_t)b] >= s) order.push_back((int)b);
+        std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return cnt[(size_t)x] < cnt[(size_t)y]; });
+        if (!order.empty())
+            TVF_CK(cudaMemcpyAsync(a.plist, order.data(), order.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+        for (size_t g0 = 0; g0 < order.size();) {
+            const int size = cnt[(size_t)order[g0]];
+            size_t g1 = g0;
+            while (g1 < order.size() && cnt[(size_t)order[g1]] == size) ++g1;
+            const int m = (int)(g1 - g0);
+            launch_ransac_gather(a, a.plist + g0, m, size, st);
+            rc = ransac_launched(h); if (rc) return rc;
+            ChunkBufs r = k;                      // the hypotheses' buffers, free again
+            r.in = a.rin; r.calm = a.calm_batched ? a.rcalm : a.calm;
+            rc = run_pose_chunk(h, st, method, a.calm_batched, size, m, r); if (rc) return rc;
+            launch_ransac_scatter(a, a.plist + g0, m, r.Rt2, r.Rt3, r.status, st);
+            rc = ransac_launched(h); if (rc) return rc;
+            g0 = g1;
+        }
+        TVF_CK(cudaMemsetAsync(a.cnt_refit, 0, (size_t)Bc * sizeof(int), st));
+        launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, n, Bc, 1, a.refRt2, a.refRt3, a.refst, th, a.cnt_refit,
+                                a.mask_refit, h->sm_count, st);
+        rc = ransac_launched(h); if (rc) return rc;
+        launch_ransac_finish(a, s, st);
+        return ransac_launched(h);
+    }
+};
+
+// tvf_consensus: no status word, so host_pipeline's temporary one stays zero
+struct Consensus {
+    const double* corresp; const double* calm; int calm_batched; int n; const double* Rt2; const double* Rt3; double th;
+    uint8_t* inliers; int32_t* n_inliers;
+    int32_t* no_status = nullptr;
+    const double *d_corresp = nullptr, *d_calm = nullptr, *d_Rt2 = nullptr, *d_Rt3 = nullptr;
+    uint8_t* d_inliers = nullptr; int32_t* d_count = nullptr;
+    int check(tvf_handle_t h, int64_t B) const {
+        if (!h) return TVF_ERR_ARG;
+        if (!corresp || !calm || !Rt2 || !Rt3) return fail(h, TVF_ERR_ARG, "consensus: corresp, calm, Rt2 and Rt3 must not be NULL");
+        if (B < 0 || n < 1) return fail(h, TVF_ERR_ARG, "consensus: need n >= 1 and B >= 0");
+        if (!(th > 0.0) || !(th < __builtin_huge_val())) return fail(h, TVF_ERR_ARG, "consensus: threshold must be finite and > 0");
+        return TVF_OK;
+    }
+    int32_t*& status() { return no_status; }
+    size_t budget(bool) const { return (size_t)(6 * n + 27 + 24) * 8 + n + 4; }
+    size_t carve(char* base, int64_t C) {
+        Carver c(base);
+        d_corresp = c.take<double>((size_t)6 * n * C); d_calm = c.take<double>(calm_batched ? 27 * C : 27);
+        d_Rt2 = c.take<double>(12 * C); d_Rt3 = c.take<double>(12 * C);
+        d_inliers = c.take<uint8_t>((size_t)n * C); d_count = c.take<int32_t>(C);
+        return c.off;
+    }
+    template <class F> void arrays(F&& f) {
+        f(corresp, Arr::input(8 * 6 * n, d_corresp));
+        f(calm, Arr::input(8 * 27, d_calm, !calm_batched));
+        f(Rt2, Arr::input(8 * 12, d_Rt2));
+        f(Rt3, Arr::input(8 * 12, d_Rt3));
+        f(inliers, Arr::output(n, d_inliers));
+        f(n_inliers, Arr::output(4, d_count));
+    }
+    int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
+        TVF_CK(cudaMemsetAsync(d_count, 0, (size_t)Bc * sizeof(int32_t), st));
+        launch_ransac_consensus(d_corresp, d_calm, calm_batched, n, Bc, 1, d_Rt2, d_Rt3, nullptr, th, d_count, d_inliers,
+                                h->sm_count, st);
+        return ransac_launched(h);
+    }
+};
 
 // small helper for the stand-alone functions: upload, run, download on slot 0
 struct Up {
@@ -1554,6 +1723,37 @@ int tvf_ba_covariance_dev(tvf_handle_t h, const double* corresp, const double* c
                           const double* Rt2, const double* Rt3, const double* reconst, double* cov_cam, double* cov_pts,
                           double* sigma2, int32_t* status) {
     return ba_dev(h, Covariance{BaCovArgs{corresp, calm, calm_batched, n, 0, Rt2, Rt3, reconst, cov_cam, cov_pts, sigma2, status}}, B);
+}
+
+static int ransac_call(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched, int n,
+                       int64_t B, int hypotheses, double threshold, const uint64_t* seeds, double* Rt2, double* Rt3,
+                       uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* status, bool dev) {
+    if (!h) return TVF_ERR_ARG;
+    if (method != 1 && method != 7) return fail(h, TVF_ERR_ARG, "ransac_pose: method must be 1 (linear TFT) or 7 (linear F)");
+    RansacArgs io{};
+    io.corresp = corresp; io.calm = calm; io.calm_batched = calm_batched; io.n = n; io.seeds = seeds;
+    io.Rt2 = Rt2; io.Rt3 = Rt3; io.inliers = inliers; io.n_inliers = n_inliers; io.sample = sample; io.status = status;
+    const Ransac c{method == 1 ? METHOD_TFT : METHOD_F, method == 1 ? 7 : 8, hypotheses, threshold, io};
+    return dev ? ba_dev(h, c, B) : host_call(h, c, B);
+}
+
+int tvf_ransac_pose(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched, int n,
+                    int64_t B, int hypotheses, double threshold, const uint64_t* seeds, double* Rt2, double* Rt3,
+                    uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* status) {
+    return ransac_call(h, method, corresp, calm, calm_batched, n, B, hypotheses, threshold, seeds, Rt2, Rt3, inliers,
+                       n_inliers, sample, status, false);
+}
+
+int tvf_ransac_pose_dev(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched, int n,
+                        int64_t B, int hypotheses, double threshold, const uint64_t* seeds, double* Rt2, double* Rt3,
+                        uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* status) {
+    return ransac_call(h, method, corresp, calm, calm_batched, n, B, hypotheses, threshold, seeds, Rt2, Rt3, inliers,
+                       n_inliers, sample, status, true);
+}
+
+int tvf_consensus(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
+                  const double* Rt2, const double* Rt3, double threshold, uint8_t* inliers, int32_t* n_inliers) {
+    return host_call(h, Consensus{corresp, calm, calm_batched, n, Rt2, Rt3, threshold, inliers, n_inliers}, B);
 }
 
 int tvf_ang_error(tvf_handle_t h, const double* Rt_true, int true_batched, const double* Rt_est, int64_t B,

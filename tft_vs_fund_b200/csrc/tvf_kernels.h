@@ -2,6 +2,7 @@
 // the kernel translation units.  Not installed; the public contract is include/tvf.h.
 #pragma once
 #include <cuda_runtime.h>
+#include <stdint.h>
 
 namespace tvf {
 
@@ -83,6 +84,50 @@ struct BaCovArgs {
     int* status;               // B
 };
 int launch_ba_covariance(const BaCovArgs& a, cudaStream_t stream);
+
+// ---- RANSAC pose (tvf_ransac_kernels.cu).  Device pointers.
+// Consensus of Q poses: pose q (Rt2, Rt3 12 x Q) belongs to problem q / H of corresp (6 x n x B) and calm; hstatus (Q,
+// may be null): a pose with non-zero status scores -1.  count (Q) must be zeroed before; mask (n x Q, may be null)
+// receives the inlier flags.
+void launch_ransac_consensus(const double* corresp, const double* calm, int calm_batched, int n, long long Q, int H,
+                             const double* Rt2, const double* Rt3, const int* hstatus, double th, int* count,
+                             unsigned char* mask, int sm_count, cudaStream_t stream);
+
+// the buffers of one chunk of tvf_ransac_pose: B problems, H hypotheses of s points each
+struct RansacArgs {
+    const double* corresp;     // 6 x n x B, 16-byte aligned
+    const double* calm;        // 9 x 3 (shared) or 9 x 3 x B
+    int calm_batched;
+    int n;
+    long long B;
+    const uint64_t* seeds;     // B
+    // outputs
+    double* Rt2;               // 12 x B
+    double* Rt3;               // 12 x B
+    unsigned char* inliers;    // n x B
+    int* n_inliers;            // B
+    int* sample;               // s x B
+    int* status;               // B
+    // hypotheses (B * H)
+    double* gin;               // 6 x s x (B H): the minimal problems
+    double* gcalm;             // 27 x (B H) when calm_batched
+    double* hRt2; double* hRt3; int* hstatus; int* hcount;
+    // per problem: the best hypothesis and the refit
+    int* best_h; int* cnt_best; unsigned char* mask_best; double* bestRt2; double* bestRt3;
+    int* refst; int* cnt_refit; unsigned char* mask_refit; double* refRt2; double* refRt3;
+    double* rin; double* rcalm; int* plist;   // the refit's compacted problems (6 x n x B, 27 x B) and problem list (B)
+};
+// the s-point minimal problem of every hypothesis (gin, gcalm)
+void launch_ransac_sample(const RansacArgs& a, int H, int s, cudaStream_t stream);
+// per problem the hypothesis of largest hcount (ties: smallest h) -> best_h (-1: all flagged), bestRt2/3 (NaN then)
+void launch_ransac_select(const RansacArgs& a, int H, cudaStream_t stream);
+// problems plist[0..m) of refit size k: their consensus columns (mask_best, index order) -> rin (6 x k x m), rcalm
+void launch_ransac_gather(const RansacArgs& a, const int* plist, int m, int k, cudaStream_t stream);
+// refit results of those problems (Rt2, Rt3, status m each) -> refRt2, refRt3, refst
+void launch_ransac_scatter(const RansacArgs& a, const int* plist, int m, const double* Rt2, const double* Rt3,
+                           const int* st, cudaStream_t stream);
+// the result rule (include/tvf.h, tvf_ransac_pose) -> the outputs
+void launch_ransac_finish(const RansacArgs& a, int s, cudaStream_t stream);
 
 // ---- pose tail -----------------------------------------------------------------------------
 struct PoseTailArgs {

@@ -101,8 +101,17 @@ def prepare_triplet(data, it, repr_err_th=1.0, device=None):
     return dict(triplet=tuple(im), CalM=CalM, R_t0=R_t0, Corresp=Corresp, Corresp_inliers=inl, inlier_mask=mask, REr=REr)
 
 
+def consensus_stats(mask, truth):
+    """A consensus mask against the ground-truth inlier mask: dict(mask, size, precision, recall)."""
+    mask = np.asarray(mask, dtype=bool); truth = np.asarray(truth, dtype=bool)
+    tp = int(np.sum(mask & truth))
+    size = int(np.sum(mask))
+    return dict(mask=mask, size=size, precision=tp / size if size else 0.0,
+                recall=tp / int(np.sum(truth)) if np.any(truth) else 0.0)
+
+
 def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), device=None, details=None,
-             bundle_adjust=False, covariance=False):
+             bundle_adjust=False, covariance=False, raw_matches=False):
     """The linear-method part of experiments_real.m:75-138.  `data`: a Dataset or the path of a dataset directory;
     `triplets_to_test`: rows of indexes_sorted (1-based; the reference uses 1:70 / 1:50, :31-36).  Per loop index `it`:
     pre-filter (:94-101), sample min(100, N) inliers with rng(it) (:103-105; documented stand-in for MATLAB's
@@ -117,7 +126,13 @@ def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), de
     covariance=True (with bundle_adjust): api.ba_covariance is also taken at each adjusted pose, and
     details[k]["ba"][m] gets .sigma2 (the a-posteriori pixel noise variance of the sample) and the predicted RMS
     rotation / translation errors .pred_rot_err, .pred_t_err (degrees, api.pose_rms_errors scaled by sigma2, the mean
-    of the two views as :133-136).  The returned error columns are unchanged."""
+    of the two views as :133-136).  The returned error columns are unchanged.
+    raw_matches=True: the pose comes from api.ransac_pose on ALL N matches of the triplet (1024 hypotheses, threshold
+    1 px, seed = it), so the ground truth is not used for estimation; the evaluation is unchanged (ReprError over the
+    ground-truth inliers, AngError against the ground truth).  details[k]["consensus"][m] holds the consensus mask, its
+    size and its precision and recall against the ground-truth inlier mask; bundle_adjust / covariance run on the
+    consensus columns, starting from the RANSAC pose (the points triangulated from it); a consensus of fewer than 4
+    matches cannot be adjusted and gets +inf in the adjusted columns."""
     from .scene import SceneRNG
     from .experiments import METHODS
     if not isinstance(data, Dataset):
@@ -142,18 +157,29 @@ def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), de
         rec = dict(triplet=d["triplet"], n_inliers=N, REr=d["REr"], sample=sample, res={})
         if bundle_adjust:
             rec["ba"] = {}
+        if raw_matches:
+            rec["consensus"] = {}
+        Nm = d["Corresp"].shape[1] if raw_matches else N
         for m in methods:
-            if (m > 6 and N < 8) or N < 7:                                                              # :117-122
+            if (m > 6 and Nm < 8) or Nm < 7:                                                            # :117-122
                 out[m][row] = np.inf
                 continue
-            res = METHODS[m][1](C0, CalM, device=device)                                                # :126
+            if raw_matches:
+                res = api.ransac_pose(d["Corresp"], CalM, method=m, hypotheses=1024, threshold=1.0, seed=it, device=device)
+                Cm, X0 = d["Corresp"][:, res[2]], None
+                rec["consensus"][m] = consensus_stats(res[2], d["inlier_mask"])
+            else:
+                res = METHODS[m][1](C0, CalM, device=device)                                            # :126
+                Cm, X0 = C0, res[2]
             out[m][row, :3] = errors(res[0], res[1], CalM, inl, d["R_t0"])
             rec["res"][m] = res
-            if bundle_adjust:
-                ba = api.bundle_adjust(C0, CalM, res[0], res[1], res[2], device=device)
+            if bundle_adjust and Cm.shape[1] < 4:                                                       # too few to adjust
+                out[m][row, 3:] = np.inf
+            elif bundle_adjust:
+                ba = api.bundle_adjust(Cm, CalM, res[0], res[1], X0, device=device)
                 out[m][row, 3:] = errors(ba[0], ba[1], CalM, inl, d["R_t0"])
                 if covariance:
-                    cov = api.ba_covariance(C0, CalM, ba[0], ba[1], ba[2], device=device)
+                    cov = api.ba_covariance(Cm, CalM, ba[0], ba[1], ba[2], device=device)
                     rot, tdir = api.pose_rms_errors(cov[0], ba[0], ba[1], sigma2=cov[1])
                     ba.sigma2 = cov[1]
                     ba.pred_rot_err, ba.pred_t_err = float(np.mean(rot)), float(np.mean(tdir))
