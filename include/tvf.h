@@ -308,6 +308,33 @@ int tvf_ransac_pose_dev(tvf_handle_t h, int method, const double* corresp, const
                         int64_t B, int hypotheses, double threshold, const uint64_t* seeds, double* Rt2, double* Rt3,
                         uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* status);
 
+/* RANSAC pose whose hypotheses and result are bundle-adjusted, with local optimisation (LO).  Arguments, checks and
+ * errors as tvf_ransac_pose, plus lo_rounds (0 .. 32, else TVF_ERR_ARG) and lo_done (B, may be NULL): the number of
+ * accepted LO rounds.  Per problem b, with key seeds[b]:
+ *   1. sampling and hypotheses exactly as tvf_ransac_pose (the s indices of hypothesis h are the same);
+ *   2. each hypothesis is adjusted on its own s columns (in draw order) from its pose with the points triangulated,
+ *      i.e. tvf_bundle_adjust(reconst0 = NULL) on those columns, bit for bit;
+ *   3. its score is the consensus count of the adjusted pose, or -1 when the method flagged the hypothesis (status
+ *      != 0) or the adjustment returned TVF_ST_NONFINITE (TVF_ST_BA_NOCONV is scored);
+ *   4. the best hypothesis has the largest score, ties to the smallest h; its adjusted pose, mask and count are current;
+ *   5. LO round r = 1 .. lo_rounds: if the current count is >= 4, tvf_bundle_adjust(reconst0 = NULL) on the current
+ *      consensus columns (index order) from the current pose, and its consensus; the round is accepted, and its pose,
+ *      mask and count become current, iff the adjustment's status has no TVF_ST_NONFINITE and the count is strictly
+ *      larger.  The first round that is not accepted (or a count < 4) ends the rounds.
+ * Result: the current pose with its inliers and n_inliers; sample holds the best hypothesis's indices; status 0, or
+ * TVF_ST_RANSAC_FAILED (Rt2, Rt3 NaN, inliers 0, sample -1, lo_done 0) when every hypothesis scored -1.  A result is
+ * bit-identical whatever its batch, chunk, group-handle shard or form.  The _dev form takes device pointers (corresp
+ * 16-byte aligned) and synchronises the handle's stream at most once per LO round per chunk: each round groups the
+ * problems by consensus size, which it reads back (lo_rounds = 0: no synchronisation). */
+int tvf_ransac_pose_refined(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched, int n,
+                            int64_t B, int hypotheses, double threshold, const uint64_t* seeds, int lo_rounds, double* Rt2,
+                            double* Rt3, uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* lo_done,
+                            int32_t* status);
+int tvf_ransac_pose_refined_dev(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched,
+                                int n, int64_t B, int hypotheses, double threshold, const uint64_t* seeds, int lo_rounds,
+                                double* Rt2, double* Rt3, uint8_t* inliers, int32_t* n_inliers, int32_t* sample,
+                                int32_t* lo_done, int32_t* status);
+
 /* ---- inputs of the measured configurations, generated where they are consumed ------------------------
  * Trials [first_trial, first_trial+B) of experiments.m's sweep: trial j uses noise_levels[j mod L] and
  * seed j div L + 1; each is generateSyntheticScene(n+100, noise, seed, ...) followed by the column

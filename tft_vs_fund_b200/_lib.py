@@ -100,6 +100,10 @@ SIGNATURES = {
     "tvf_consensus": (_I, [_H, _D, _D, _I, _I, _L, _D, _D, C.c_double, C.c_void_p, _S]),
     "tvf_ransac_pose": (_I, [_H, _I, _D, _D, _I, _I, _L, _I, C.c_double, C.c_void_p, _D, _D, C.c_void_p, _S, _S, _S]),
     "tvf_ransac_pose_dev": (_I, [_H, _I, C.c_void_p, C.c_void_p, _I, _I, _L, _I, C.c_double] + [C.c_void_p] * 7),
+    "tvf_ransac_pose_refined": (_I, [_H, _I, _D, _D, _I, _I, _L, _I, C.c_double, C.c_void_p, _I, _D, _D, C.c_void_p,
+                                     _S, _S, _S, _S]),
+    "tvf_ransac_pose_refined_dev": (_I, [_H, _I, C.c_void_p, C.c_void_p, _I, _I, _L, _I, C.c_double, C.c_void_p, _I]
+                                    + [C.c_void_p] * 7),
     "tvf_launch_count": (_L, [_H]),
     "tvf_profile_enable": (_I, [_H, _I]),
     "tvf_profile_reset": (_I, [_H]),

@@ -397,20 +397,25 @@ def consensus(Corresp, CalM, R_t_2, R_t_3, threshold=1.0, device=None):
 
 
 class RansacResult(tuple):
-    """(R_t_2, R_t_3, inliers, n_inliers, sample) of ransac_pose, plus .status (0, or TVF_ST_RANSAC_FAILED)."""
+    """(R_t_2, R_t_3, inliers, n_inliers, sample) of ransac_pose, plus .status (0, or TVF_ST_RANSAC_FAILED) and, with
+    refine=True, .lo_done (the accepted LO rounds)."""
     status = None
+    lo_done = None
 
 
 RANSAC_SAMPLE_SIZE = {1: 7, 7: 8}
 
 
-def ransac_pose(Corresp, CalM, method=1, hypotheses=1024, threshold=1.0, seed=0, device=None):
+def ransac_pose(Corresp, CalM, method=1, hypotheses=1024, threshold=1.0, seed=0, device=None, refine=False, lo_rounds=8):
     """Pose from raw matches with outliers (tvf_ransac_pose, include/tvf.h): `hypotheses` minimal solves of method 1
     (LinearTFTPoseEstimation on 7 matches) or 7 (LinearFPoseEstimation on 8), each scored by its consensus (see
     `consensus`, `threshold` pixels); the method is then run again on the consensus of the best one and that refit is
     kept if it explains at least as many matches.  seed: int (problem b gets the key seed + b) or an array (B,) of keys.
     Returns (R_t_2, R_t_3, inliers, n_inliers, sample) -- inliers bool (N), the sample the best hypothesis drew -- with
-    .status; batched inputs give (B,3,4), (B,3,4), (B,N), (B,), (B,s)."""
+    .status; batched inputs give (B,3,4), (B,3,4), (B,N), (B,), (B,s).
+    refine=True (tvf_ransac_pose_refined): each hypothesis is bundle-adjusted on its own sample before it is scored,
+    and the best one is improved by up to `lo_rounds` (0 .. 32) rounds of bundle adjustment on its consensus, each kept
+    only if it explains strictly more matches; the result also has .lo_done, the number of rounds kept."""
     if method not in RANSAC_SAMPLE_SIZE:
         raise ValueError("ransac_pose: method must be 1 (linear TFT) or 7 (linear F)")
     s = RANSAC_SAMPLE_SIZE[method]
@@ -428,12 +433,20 @@ def ransac_pose(Corresp, CalM, method=1, hypotheses=1024, threshold=1.0, seed=0,
     h = _lib.handle(device)
     Rt2 = np.empty((B, 12)); Rt3 = np.empty((B, 12)); mask = np.zeros((B, n), dtype=np.uint8)
     cnt = np.zeros(B, dtype=np.int32); smp = np.zeros((B, s), dtype=np.int32); st = np.zeros(B, dtype=np.int32)
-    h.call("tvf_ransac_pose", int(method), _p(c), _p(calm), cb, n, B, int(hypotheses), float(threshold), _vp(seeds),
-           _p(Rt2), _p(Rt3), _vp(mask), cnt.ctypes.data_as(_ip), smp.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
+    if refine:
+        lo = np.zeros(B, dtype=np.int32)
+        h.call("tvf_ransac_pose_refined", int(method), _p(c), _p(calm), cb, n, B, int(hypotheses), float(threshold),
+               _vp(seeds), int(lo_rounds), _p(Rt2), _p(Rt3), _vp(mask), cnt.ctypes.data_as(_ip), smp.ctypes.data_as(_ip),
+               lo.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
+    else:
+        h.call("tvf_ransac_pose", int(method), _p(c), _p(calm), cb, n, B, int(hypotheses), float(threshold), _vp(seeds),
+               _p(Rt2), _p(Rt3), _vp(mask), cnt.ctypes.data_as(_ip), smp.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
     mask = mask.astype(bool)
     out = RansacResult((_from_cm(Rt2, B, (3, 4), batched), _from_cm(Rt3, B, (3, 4), batched),
                         mask if batched else mask[0], cnt if batched else int(cnt[0]), smp if batched else smp[0]))
     out.status = st if batched else int(st[0])
+    if refine:
+        out.lo_done = lo if batched else int(lo[0])
     return out
 
 

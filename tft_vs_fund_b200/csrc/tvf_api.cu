@@ -814,16 +814,21 @@ struct Ransac {
     }
     // sample and solve the hypotheses, score them, select; refit on the consensus of the best, grouped by its size
     // (the one read-back of the call); rescore; the result rule
+    // the Q = Bc H minimal problems (gin, gcalm) and their poses (hRt2, hRt3, hstatus); k: the pose path's buffers
+    int hypotheses(tvf_handle_t h, cudaStream_t st, const RansacArgs& a, ChunkBufs& k) const {
+        launch_ransac_sample(a, H, s, st);
+        int rc = ransac_launched(h); if (rc) return rc;
+        k = w;
+        k.in = a.gin; k.calm = a.calm_batched ? a.gcalm : a.calm; k.Rt2 = a.hRt2; k.Rt3 = a.hRt3;
+        if (method != METHOD_TFT) k.T = nullptr;
+        return run_pose_chunk(h, st, method, a.calm_batched, s, a.B * H, k);
+    }
     int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
         RansacArgs a = d; a.B = Bc;
         const int n = a.n;
         const int64_t Q = Bc * H;
-        launch_ransac_sample(a, H, s, st);
-        int rc = ransac_launched(h); if (rc) return rc;
-        ChunkBufs k = w;
-        k.in = a.gin; k.calm = a.calm_batched ? a.gcalm : a.calm; k.Rt2 = a.hRt2; k.Rt3 = a.hRt3;
-        if (method != METHOD_TFT) k.T = nullptr;
-        rc = run_pose_chunk(h, st, method, a.calm_batched, s, Q, k); if (rc) return rc;
+        ChunkBufs k;
+        int rc = hypotheses(h, st, a, k); if (rc) return rc;
         TVF_CK(cudaMemsetAsync(a.hcount, 0, (size_t)Q * sizeof(int), st));
         launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, n, Q, H, a.hRt2, a.hRt3, a.hstatus, th, a.hcount, nullptr,
                                 h->sm_count, st);
@@ -861,6 +866,108 @@ struct Ransac {
         launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, n, Bc, 1, a.refRt2, a.refRt3, a.refst, th, a.cnt_refit,
                                 a.mask_refit, h->sm_count, st);
         rc = ransac_launched(h); if (rc) return rc;
+        launch_ransac_finish(a, s, st);
+        return ransac_launched(h);
+    }
+};
+
+// tvf_ransac_pose_refined: Ransac's layout and hypotheses, each hypothesis adjusted on its own sample (the packed
+// adjustment), and LO rounds of the adjustment on the current consensus
+struct RansacRefined : Ransac {
+    int lo_rounds;
+    double *aRt2 = nullptr, *aRt3 = nullptr, *X = nullptr, *Xc = nullptr;
+    int* ast = nullptr;
+    int check(tvf_handle_t h, int64_t B) const {
+        const int rc = Ransac::check(h, B);
+        if (rc != TVF_OK) return rc;
+        if (lo_rounds < 0 || lo_rounds > 32) return fail(h, TVF_ERR_ARG, "ransac_pose_refined: lo_rounds must be in 0 .. 32");
+        return TVF_OK;
+    }
+    // Ransac's, lo_done, the adjusted hypotheses (pose, status), the adjustment's points and candidates for the larger
+    // of the hypotheses (3 x s each) and an LO round (3 x n), and the LO round's start poses
+    size_t budget(bool host_io) const {
+        const size_t pts = (size_t)3 * (s * (size_t)H > (size_t)io.n ? s * (size_t)H : (size_t)io.n);
+        return Ransac::budget(host_io) + 4 + (size_t)H * (24 * 8 + 4) + 2 * pts * 8 + 24 * 8;
+    }
+    size_t carve(char* base, int64_t C, bool host_io = true) {
+        Carver c(base);
+        c.off = Ransac::carve(base, C, host_io);
+        const int64_t Q = C * H;
+        if (host_io || !d.lo_done) d.lo_done = c.take<int>(C);
+        aRt2 = c.take<double>(12 * Q); aRt3 = c.take<double>(12 * Q); ast = c.take<int>(Q);
+        const size_t pts = (size_t)3 * (s * Q > io.n * C ? s * Q : io.n * C);
+        X = c.take<double>(pts); Xc = c.take<double>(pts);
+        d.gRt2 = c.take<double>(12 * C); d.gRt3 = c.take<double>(12 * C);
+        return c.off;
+    }
+    template <class F> void arrays(F&& f) {
+        Ransac::arrays(f);
+        f(io.lo_done, Arr::output(4, d.lo_done));
+    }
+    // Hypotheses; each adjusted from its pose on its sample (X0 null) and scored (flagged: -1); select; then per LO
+    // round read the counts back (the call's one read-back per round), adjust every problem whose count grew in the
+    // previous round (all in the first) and has >= 4 matches on its consensus, grouped by its size, rescore, accept;
+    // the result rule with no refit.  aRt2, aRt3 and ast hold the hypotheses' adjustments, then an LO round's.
+    int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
+        RansacArgs a = d; a.B = Bc;
+        const int n = a.n;
+        const int64_t Q = Bc * H;
+        ChunkBufs k;
+        int rc = hypotheses(h, st, a, k); if (rc) return rc;
+        const BaArgs hb{a.gin, a.calm_batched ? a.gcalm : a.calm, a.calm_batched, s, Q, a.hRt2, a.hRt3, nullptr, aRt2, aRt3,
+                        X, Xc, nullptr, nullptr, ast};
+        rc = ba_launched(h, launch_bundle_adjust_small(hb, st), "bundle_adjust_small_kernel"); if (rc) return rc;
+        launch_ransac_flag(a.hstatus, ast, Q, st);
+        rc = ransac_launched(h); if (rc) return rc;
+        TVF_CK(cudaMemsetAsync(a.hcount, 0, (size_t)Q * sizeof(int), st));
+        launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, n, Q, H, aRt2, aRt3, ast, th, a.hcount, nullptr,
+                                h->sm_count, st);
+        rc = ransac_launched(h); if (rc) return rc;
+        RansacArgs sel = a; sel.hRt2 = aRt2; sel.hRt3 = aRt3;
+        launch_ransac_select(sel, H, st);
+        rc = ransac_launched(h); if (rc) return rc;
+        TVF_CK(cudaMemsetAsync(a.cnt_best, 0, (size_t)Bc * sizeof(int), st));
+        launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, n, Bc, 1, a.bestRt2, a.bestRt3, nullptr, th, a.cnt_best,
+                                a.mask_best, h->sm_count, st);
+        rc = ransac_launched(h); if (rc) return rc;
+        TVF_CK(cudaMemsetAsync(a.lo_done, 0, (size_t)Bc * sizeof(int), st));
+        std::vector<int> cnt((size_t)Bc), prev;
+        for (int r = 1; r <= lo_rounds; ++r) {
+            TVF_CK(cudaMemcpyAsync(cnt.data(), a.cnt_best, (size_t)Bc * sizeof(int), cudaMemcpyDeviceToHost, st));
+            TVF_CK(cudaStreamSynchronize(st));
+            std::vector<int> order;
+            for (int64_t b = 0; b < Bc; ++b)
+                if (cnt[(size_t)b] >= 4 && (r == 1 || cnt[(size_t)b] > prev[(size_t)b])) order.push_back((int)b);
+            if (order.empty()) break;
+            std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return cnt[(size_t)x] < cnt[(size_t)y]; });
+            TVF_CK(cudaMemcpyAsync(a.plist, order.data(), order.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+            TVF_CK(cudaMemsetAsync(a.refst, 0xff, (size_t)Bc * sizeof(int), st));      // -1: not adjusted this round
+            for (size_t g0 = 0; g0 < order.size();) {
+                const int size = cnt[(size_t)order[g0]];
+                size_t g1 = g0;
+                while (g1 < order.size() && cnt[(size_t)order[g1]] == size) ++g1;
+                const int m = (int)(g1 - g0);
+                launch_ransac_gather(a, a.plist + g0, m, size, st);
+                rc = ransac_launched(h); if (rc) return rc;
+                const BaArgs lb{a.rin, a.calm_batched ? a.rcalm : a.calm, a.calm_batched, size, m, a.gRt2, a.gRt3, nullptr,
+                                aRt2, aRt3, X, Xc, nullptr, nullptr, ast};
+                rc = ba_launched(h, launch_bundle_adjust(lb, st), "bundle_adjust_kernel"); if (rc) return rc;
+                launch_ransac_scatter(a, a.plist + g0, m, aRt2, aRt3, ast, st);
+                rc = ransac_launched(h); if (rc) return rc;
+                g0 = g1;
+            }
+            launch_ransac_flag(nullptr, a.refst, Bc, st);                           // -1 and TVF_ST_NONFINITE: count -1
+            rc = ransac_launched(h); if (rc) return rc;
+            TVF_CK(cudaMemsetAsync(a.cnt_refit, 0, (size_t)Bc * sizeof(int), st));
+            launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, n, Bc, 1, a.refRt2, a.refRt3, a.refst, th, a.cnt_refit,
+                                    a.mask_refit, h->sm_count, st);
+            rc = ransac_launched(h); if (rc) return rc;
+            launch_ransac_lo_accept(a, st);
+            rc = ransac_launched(h); if (rc) return rc;
+            prev.swap(cnt);
+            cnt.resize((size_t)Bc);
+        }
+        TVF_CK(cudaMemsetAsync(a.refst, 0xff, (size_t)Bc * sizeof(int), st));          // the result rule without a refit
         launch_ransac_finish(a, s, st);
         return ransac_launched(h);
     }
@@ -1749,6 +1856,36 @@ int tvf_ransac_pose_dev(tvf_handle_t h, int method, const double* corresp, const
                         uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* status) {
     return ransac_call(h, method, corresp, calm, calm_batched, n, B, hypotheses, threshold, seeds, Rt2, Rt3, inliers,
                        n_inliers, sample, status, true);
+}
+
+static int ransac_refined_call(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched,
+                               int n, int64_t B, int hypotheses, double threshold, const uint64_t* seeds, int lo_rounds,
+                               double* Rt2, double* Rt3, uint8_t* inliers, int32_t* n_inliers, int32_t* sample,
+                               int32_t* lo_done, int32_t* status, bool dev) {
+    if (!h) return TVF_ERR_ARG;
+    if (method != 1 && method != 7) return fail(h, TVF_ERR_ARG, "ransac_pose: method must be 1 (linear TFT) or 7 (linear F)");
+    RansacArgs io{};
+    io.corresp = corresp; io.calm = calm; io.calm_batched = calm_batched; io.n = n; io.seeds = seeds;
+    io.Rt2 = Rt2; io.Rt3 = Rt3; io.inliers = inliers; io.n_inliers = n_inliers; io.sample = sample; io.status = status;
+    io.lo_done = lo_done;
+    const RansacRefined c{Ransac{method == 1 ? METHOD_TFT : METHOD_F, method == 1 ? 7 : 8, hypotheses, threshold, io}, lo_rounds};
+    return dev ? ba_dev(h, c, B) : host_call(h, c, B);
+}
+
+int tvf_ransac_pose_refined(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched, int n,
+                            int64_t B, int hypotheses, double threshold, const uint64_t* seeds, int lo_rounds, double* Rt2,
+                            double* Rt3, uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* lo_done,
+                            int32_t* status) {
+    return ransac_refined_call(h, method, corresp, calm, calm_batched, n, B, hypotheses, threshold, seeds, lo_rounds, Rt2,
+                               Rt3, inliers, n_inliers, sample, lo_done, status, false);
+}
+
+int tvf_ransac_pose_refined_dev(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched,
+                                int n, int64_t B, int hypotheses, double threshold, const uint64_t* seeds, int lo_rounds,
+                                double* Rt2, double* Rt3, uint8_t* inliers, int32_t* n_inliers, int32_t* sample,
+                                int32_t* lo_done, int32_t* status) {
+    return ransac_refined_call(h, method, corresp, calm, calm_batched, n, B, hypotheses, threshold, seeds, lo_rounds, Rt2,
+                               Rt3, inliers, n_inliers, sample, lo_done, status, true);
 }
 
 int tvf_consensus(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,

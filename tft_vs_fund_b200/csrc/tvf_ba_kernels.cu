@@ -1,6 +1,8 @@
 // tvf_ba_kernels.cu -- batched three-view bundle adjustment (tvf_bundle_adjust): Levenberg-Marquardt on the pixel
 // reprojection error with the points eliminated by the Schur complement.  One warp per problem, lanes own points
 // (point i belongs to lane i mod 32), the same mapping as optimf_gh_kernel.  Per-point algebra: tvf_ba.cuh.
+// bundle_adjust_small_kernel runs the same code on groups of 8 lanes, four problems per warp, for n <= 8 (the RANSAC
+// hypotheses of tvf_ransac_pose_refined); "warp" and "lane" below then mean the group and the lane within it.
 //
 // One iteration:
 //   pass A   every lane linearises its points at the current iterate (6 x 3 point and 6 x 11 camera Jacobian),
@@ -21,9 +23,10 @@
 namespace tvf {
 
 constexpr int BA_WARPS = 2;
-constexpr int BA_SLAB = 32 * BA_NSUM;                  // lane-private partial sums (odd stride: conflict-free)
 constexpr int BA_CAMS = (sizeof(BaCams) + 7) / 8;      // doubles per BaCams
-constexpr int BA_PER_WARP = BA_SLAB + BA_NSUM + 1 + 12 + 2 * BA_CAMS;
+// shared doubles of one group of W lanes (one problem): W lane-private rows of partial sums (odd stride: conflict-free),
+// the reduced sums (+1), the camera step with its solve flag, the current and the candidate cameras
+template <int W> constexpr int BA_PER_GROUP = W * BA_NSUM + BA_NSUM + 1 + 12 + 2 * BA_CAMS;
 
 __device__ __forceinline__ bool finite_(double x) { return fabs(x) <= 1.79769313486231570e308; }
 
@@ -33,28 +36,44 @@ __device__ __forceinline__ void load_x6(const double* corresp, long long prob, i
     x6[0] = a.x; x6[1] = a.y; x6[2] = b.x; x6[3] = b.y; x6[4] = c.x; x6[5] = c.y;
 }
 
-__global__ void __launch_bounds__(BA_WARPS * 32)
-bundle_adjust_kernel(const BaArgs a) {
+// sum and max over the W lanes of a group (mask m): warp_sum / warp_max's xor butterfly on the offsets W/2 .. 1
+template <int W> __device__ __forceinline__ double group_sum(double v, unsigned m) {
+#pragma unroll
+    for (int o = W / 2; o > 0; o >>= 1) v += __shfl_xor_sync(m, v, o);
+    return v;
+}
+
+template <int W> __device__ __forceinline__ double group_max(double v, unsigned m) {
+#pragma unroll
+    for (int o = W / 2; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(m, v, o));
+    return v;
+}
+
+// the problems of one group of W lanes (mask gm) in a grid-stride loop; lane = the lane within the group
+template <int W> __device__ __forceinline__ void ba_problems(const BaArgs& a) {
     extern __shared__ __align__(16) double ba_smem[];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    double* slab = ba_smem + (size_t)warp * BA_PER_WARP;
-    double* red = slab + BA_SLAB;                      // BA_NSUM (+1)
+    constexpr int G = BA_WARPS * 32 / W;               // groups (problems in flight) per block
+    const int lane = threadIdx.x & (W - 1), grp = threadIdx.x / W;
+    const unsigned gm = (W == 32) ? FULL : ((1u << W) - 1u) << (threadIdx.x & 31 & ~(W - 1));
+    double* slab = ba_smem + (size_t)grp * BA_PER_GROUP<W>;
+    double* red = slab + W * BA_NSUM;                  // BA_NSUM (+1)
     double* dcs = red + BA_NSUM + 1;                   // 11 camera step entries + solve flag
     BaCams& cur = *reinterpret_cast<BaCams*>(dcs + 12);
     BaCams& cand = *reinterpret_cast<BaCams*>(dcs + 12 + BA_CAMS);
     double* acc = slab + lane * BA_NSUM;
     const int n = a.n;
 
-    for (long long prob = (long long)blockIdx.x * BA_WARPS + warp; prob < a.B; prob += (long long)gridDim.x * BA_WARPS) {
+    for (long long prob = (long long)blockIdx.x * G + grp; prob < a.B; prob += (long long)gridDim.x * G) {
         const double* cm = a.calm + (a.calm_batched ? prob * 27 : 0);
         const double* rt2 = a.Rt2_0 + prob * 12;
         const double* rt3 = a.Rt3_0 + prob * 12;
         double* Xp = a.X + prob * 3 * n;
         double* Xcp = a.Xc + prob * 3 * n;
-        __syncwarp();
+        __syncwarp(gm);
         if (lane == 0) ba_load_cams(cm, rt2, rt3, cur);
-        bool bad_l = (lane < 27 && !finite_(cm[lane])) || (lane < 12 && !(finite_(rt2[lane]) && finite_(rt3[lane])));
-        __syncwarp();
+        bool bad_l = false;
+        for (int e = lane; e < 27; e += W) bad_l = bad_l || !finite_(cm[e]) || (e < 12 && !(finite_(rt2[e]) && finite_(rt3[e])));
+        __syncwarp(gm);
 
         // ---- start points: Reconst0, or triangulation3D({K1[I|0], K2 R_t_2, K3 R_t_3}, Corresp) -----------------
         double cost_l = 0.0;
@@ -72,7 +91,7 @@ bundle_adjust_kernel(const BaArgs a) {
                         P2[r + 3 * col] = s2; P3[r + 3 * col] = s3;
                     }
             }
-            for (int i = lane; i < n; i += 32) {
+            for (int i = lane; i < n; i += W) {
                 double x6[6], X[3];
                 load_x6(a.corresp, prob, n, i, x6);
                 if (a.X0 != nullptr) {
@@ -90,11 +109,11 @@ bundle_adjust_kernel(const BaArgs a) {
                 cost_l += ba_point_cost(cur, X, x6);
             }
         }
-        const double cost0 = warp_sum(cost_l);
+        const double cost0 = group_sum<W>(cost_l, gm);
         const double t2n = sqrt(cur.t2[0] * cur.t2[0] + cur.t2[1] * cur.t2[1] + cur.t2[2] * cur.t2[2]);
-        const bool bad = __any_sync(FULL, bad_l) || !(t2n > 0.0) || !finite_(cost0);
+        const bool bad = __any_sync(gm, bad_l) || !(t2n > 0.0) || !finite_(cost0);
         if (bad) {                                     // inputs copied through (the start points are already in X)
-            if (lane < 12) { a.Rt2[prob * 12 + lane] = rt2[lane]; a.Rt3[prob * 12 + lane] = rt3[lane]; }
+            for (int e = lane; e < 12; e += W) { a.Rt2[prob * 12 + e] = rt2[e]; a.Rt3[prob * 12 + e] = rt3[e]; }
             if (lane == 0) {
                 if (a.repr_err) a.repr_err[prob] = sqrt(cost0 / (3.0 * n));
                 if (a.iter) a.iter[prob] = 0;
@@ -105,22 +124,22 @@ bundle_adjust_kernel(const BaArgs a) {
 
         // ---- gauge |t2| = 1: t2, t3 and the points scaled by 1/|t2| ----------------------------------------------
         const double gs = 1.0 / t2n;
-        __syncwarp();
+        __syncwarp(gm);
         if (lane == 0) {
 #pragma unroll
             for (int k = 0; k < 3; ++k) { cur.t2[k] *= gs; cur.t3[k] *= gs; }
             onb3(cur.t2, cur.u1, cur.u2);
         }
-        __syncwarp();
+        __syncwarp(gm);
         cost_l = 0.0;
-        for (int i = lane; i < n; i += 32) {
+        for (int i = lane; i < n; i += W) {
             double x6[6], X[3];
             load_x6(a.corresp, prob, n, i, x6);
 #pragma unroll
             for (int k = 0; k < 3; ++k) { X[k] = Xp[3 * i + k] * gs; Xp[3 * i + k] = X[k]; }
             cost_l += ba_point_cost(cur, X, x6);
         }
-        double F = 0.5 * warp_sum(cost_l);            // (1/2) sum of squared residuals
+        double F = 0.5 * group_sum<W>(cost_l, gm);           // (1/2) sum of squared residuals
 
         // ---- Levenberg-Marquardt ---------------------------------------------------------------------------------
         double mu = BA_MU0, nu = 2.0, gmax0 = -1.0;
@@ -131,7 +150,7 @@ bundle_adjust_kernel(const BaArgs a) {
             for (int e = 0; e < BA_NSUM; ++e) acc[e] = 0.0;
             bool pd_l = true;
             double gp_l = 0.0;
-            for (int i = lane; i < n; i += 32) {
+            for (int i = lane; i < n; i += W) {
                 double x6[6];
                 load_x6(a.corresp, prob, n, i, x6);
                 const double X[3] = {Xp[3 * i], Xp[3 * i + 1], Xp[3 * i + 2]};
@@ -141,23 +160,23 @@ bundle_adjust_kernel(const BaArgs a) {
                 ba_point_accumulate(p, el, acc);
                 gp_l = fmax(gp_l, fmax(fabs(el.g[0]), fmax(fabs(el.g[1]), fabs(el.g[2]))));
             }
-            __syncwarp();
-            for (int e = lane; e < BA_NSUM; e += 32) {
+            __syncwarp(gm);
+            for (int e = lane; e < BA_NSUM; e += W) {
                 double s = 0.0;
 #pragma unroll 8
-                for (int l = 0; l < 32; ++l) s += slab[l * BA_NSUM + e];
+                for (int l = 0; l < W; ++l) s += slab[l * BA_NSUM + e];
                 red[e] = s;
             }
-            __syncwarp();
-            double gmax = warp_max(gp_l);
+            __syncwarp(gm);
+            double gmax = group_max<W>(gp_l, gm);
 #pragma unroll
             for (int k = 0; k < BA_NC; ++k) gmax = fmax(gmax, fabs(red[BA_GC + k]));
             if (gmax0 < 0.0) gmax0 = gmax;
             if (!(gmax > BA_GTOL * gmax0)) break;                                  // small gradient (or zero)
-            const bool pd = !__any_sync(FULL, !pd_l);
-            __syncwarp();
+            const bool pd = !__any_sync(gm, !pd_l);
+            __syncwarp(gm);
             if (lane == 0) dcs[11] = (pd && ba_solve_reduced(red, mu, dcs)) ? 1.0 : 0.0;
-            __syncwarp();
+            __syncwarp(gm);
             ++solves;
             const bool solved = dcs[11] != 0.0;
             if (solved) {
@@ -165,10 +184,10 @@ bundle_adjust_kernel(const BaArgs a) {
 #pragma unroll
                 for (int k = 0; k < BA_NC; ++k) dc[k] = dcs[k];
                 if (lane == 0) { cand = cur; ba_update_cams(dc, cand); }
-                __syncwarp();
+                __syncwarp(gm);
                 // pass B: back-substitution and the candidate's cost
                 double cn_l = 0.0, pr_l = 0.0, s2_l = 0.0, x2_l = 0.0;
-                for (int i = lane; i < n; i += 32) {
+                for (int i = lane; i < n; i += W) {
                     double x6[6];
                     load_x6(a.corresp, prob, n, i, x6);
                     const double X[3] = {Xp[3 * i], Xp[3 * i + 1], Xp[3 * i + 2]};
@@ -187,8 +206,8 @@ bundle_adjust_kernel(const BaArgs a) {
                     }
                     cn_l += ba_point_cost(cand, Xn, x6);
                 }
-                const double Fn = 0.5 * warp_sum(cn_l);
-                double pred = warp_sum(pr_l), step2 = warp_sum(s2_l), xn2 = warp_sum(x2_l);
+                const double Fn = 0.5 * group_sum<W>(cn_l, gm);
+                double pred = group_sum<W>(pr_l, gm), step2 = group_sum<W>(s2_l, gm), xn2 = group_sum<W>(x2_l, gm);
 #pragma unroll
                 for (int k = 0; k < BA_NC; ++k) {
                     pred += mu * red[BA_DIAG + k] * dc[k] * dc[k] - red[BA_GC + k] * dc[k];
@@ -200,12 +219,12 @@ bundle_adjust_kernel(const BaArgs a) {
                 if (Fn < F) {                          // accept
                     const double rho = (F - Fn) / pred;
                     const bool small_change = !(F - Fn > BA_FTOL * F);
-                    for (int i = lane; i < n; i += 32)
+                    for (int i = lane; i < n; i += W)
 #pragma unroll
                         for (int k = 0; k < 3; ++k) Xp[3 * i + k] = Xcp[3 * i + k];
-                    __syncwarp();
+                    __syncwarp(gm);
                     if (lane == 0) cur = cand;
-                    __syncwarp();
+                    __syncwarp(gm);
                     F = Fn;
                     const double q = 2.0 * rho - 1.0;
                     mu *= fmax(1.0 / 3.0, 1.0 - q * q * q);       // Nielsen
@@ -221,10 +240,10 @@ bundle_adjust_kernel(const BaArgs a) {
             if (solves >= BA_SOLVE_MAX) { st = ST_BA_NOCONV; break; }
         }
 
-        __syncwarp();
-        if (lane < 12) {
-            a.Rt2[prob * 12 + lane] = (lane < 9) ? cur.R2[lane] : cur.t2[lane - 9];
-            a.Rt3[prob * 12 + lane] = (lane < 9) ? cur.R3[lane] : cur.t3[lane - 9];
+        __syncwarp(gm);
+        for (int e = lane; e < 12; e += W) {
+            a.Rt2[prob * 12 + e] = (e < 9) ? cur.R2[e] : cur.t2[e - 9];
+            a.Rt3[prob * 12 + e] = (e < 9) ? cur.R3[e] : cur.t3[e - 9];
         }
         if (lane == 0) {
             if (a.repr_err) a.repr_err[prob] = sqrt(2.0 * F / (3.0 * n));        // ReprError.m:65
@@ -234,18 +253,39 @@ bundle_adjust_kernel(const BaArgs a) {
     }
 }
 
-int launch_bundle_adjust(const BaArgs& a, cudaStream_t stream) {
+__global__ void __launch_bounds__(BA_WARPS * 32) bundle_adjust_kernel(const BaArgs a) { ba_problems<32>(a); }
+
+// Packed variant for n <= 8: groups of 8 lanes, four problems per warp.  Bit-identical to bundle_adjust_kernel on the
+// same problem, because at n <= 8 lanes 8..31 of bundle_adjust_kernel own no point and contribute exact +0.0:
+//   - a lane-private sum (cost, model decrease, step, |X|^2) starts at +0.0 and only adds, so it is never -0.0; the
+//     first two xor steps of warp_sum (offsets 16, 8) add +0.0 to it on lanes 0..7 and change nothing, and the
+//     remaining offsets 4, 2, 1 are group_sum<8>'s butterfly over the same lanes in the same order;
+//   - warp_max of non-negative values: fmax with the +0.0 of the idle lanes changes nothing either;
+//   - the slab sum s = 0.0; s += slab[l] (l ascending) never holds -0.0, so adding the 24 trailing +0.0 rows of the
+//     idle lanes leaves it as group 8's sum over l = 0..7;
+//   - every vote (__any_sync) of the idle lanes is false, and every other step is done by lane 0 or per point.
+__global__ void __launch_bounds__(BA_WARPS * 32) bundle_adjust_small_kernel(const BaArgs a) { ba_problems<BA_SMALL_N>(a); }
+
+template <int W> int launch_groups(void (*kernel)(const BaArgs), const BaArgs& a, cudaStream_t stream) {
     if (a.B <= 0) return 1;
-    const size_t smem = (size_t)BA_WARPS * BA_PER_WARP * sizeof(double);
+    constexpr int G = BA_WARPS * 32 / W;
+    const size_t smem = (size_t)G * BA_PER_GROUP<W> * sizeof(double);
     // the opt-in is a per-device property of the function: set on every launch, as for optimf_gh_kernel
-    if (cudaFuncSetAttribute(bundle_adjust_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
+    if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
         cudaGetLastError();
         return 0;
     }
-    long long blocks = (a.B + BA_WARPS - 1) / BA_WARPS;       // one problem per warp: the block scheduler balances
-    if (blocks > 0x7fffffffLL) blocks = 0x7fffffffLL;         // problems of different iteration counts
-    bundle_adjust_kernel<<<(unsigned)blocks, BA_WARPS * 32, smem, stream>>>(a);
+    long long blocks = (a.B + G - 1) / G;              // one problem per group: the block scheduler balances
+    if (blocks > 0x7fffffffLL) blocks = 0x7fffffffLL;  // problems of different iteration counts
+    kernel<<<(unsigned)blocks, BA_WARPS * 32, smem, stream>>>(a);
     return cudaPeekAtLastError() == cudaSuccess ? 1 : 0;
+}
+
+int launch_bundle_adjust(const BaArgs& a, cudaStream_t stream) { return launch_groups<32>(bundle_adjust_kernel, a, stream); }
+
+int launch_bundle_adjust_small(const BaArgs& a, cudaStream_t stream) {
+    if (a.n > BA_SMALL_N) return 0;
+    return launch_groups<BA_SMALL_N>(bundle_adjust_small_kernel, a, stream);
 }
 
 }  // namespace tvf

@@ -66,6 +66,10 @@ struct BaArgs {
     int* status;               // B
 };
 int launch_bundle_adjust(const BaArgs& a, cudaStream_t stream);
+// the same adjustment, bit for bit, with four problems per warp (groups of 8 lanes) for a.n <= BA_SMALL_N; returns 0
+// for a larger n or a failed launch
+constexpr int BA_SMALL_N = 8;
+int launch_bundle_adjust_small(const BaArgs& a, cudaStream_t stream);
 
 // ---- covariance of the bundle adjustment at a state (tvf_ba_cov_kernels.cu).  Device pointers; cov_cam, cov_pts,
 // sigma2 and status may be null.  Returns 0 if the launch failed.
@@ -116,16 +120,23 @@ struct RansacArgs {
     int* best_h; int* cnt_best; unsigned char* mask_best; double* bestRt2; double* bestRt3;
     int* refst; int* cnt_refit; unsigned char* mask_refit; double* refRt2; double* refRt3;
     double* rin; double* rcalm; int* plist;   // the refit's compacted problems (6 x n x B, 27 x B) and problem list (B)
+    // tvf_ransac_pose_refined: the LO rounds' compacted start poses (12 x B each; null: not gathered) and their count
+    double* gRt2; double* gRt3; int* lo_done;
 };
 // the s-point minimal problem of every hypothesis (gin, gcalm)
 void launch_ransac_sample(const RansacArgs& a, int H, int s, cudaStream_t stream);
 // per problem the hypothesis of largest hcount (ties: smallest h) -> best_h (-1: all flagged), bestRt2/3 (NaN then)
 void launch_ransac_select(const RansacArgs& a, int H, cudaStream_t stream);
-// problems plist[0..m) of refit size k: their consensus columns (mask_best, index order) -> rin (6 x k x m), rcalm
+// problems plist[0..m) of refit size k: their consensus columns (mask_best, index order) -> rin (6 x k x m), rcalm,
+// and bestRt2/3 -> gRt2/3 (12 x m) when gRt2 is not null
 void launch_ransac_gather(const RansacArgs& a, const int* plist, int m, int k, cudaStream_t stream);
 // refit results of those problems (Rt2, Rt3, status m each) -> refRt2, refRt3, refst
 void launch_ransac_scatter(const RansacArgs& a, const int* plist, int m, const double* Rt2, const double* Rt3,
                            const int* st, cudaStream_t stream);
+// st[q] <- 1 if pose_st[q] != 0 (pose_st may be null) or st[q] (an adjustment's status) has ST_NONFINITE, else 0
+void launch_ransac_flag(const int* pose_st, int* st, long long Q, cudaStream_t stream);
+// per problem, if cnt_refit > cnt_best: refRt2/3, mask_refit, cnt_refit -> bestRt2/3, mask_best, cnt_best; ++lo_done
+void launch_ransac_lo_accept(const RansacArgs& a, cudaStream_t stream);
 // the result rule (include/tvf.h, tvf_ransac_pose) -> the outputs
 void launch_ransac_finish(const RansacArgs& a, int s, cudaStream_t stream);
 

@@ -1,6 +1,7 @@
-// tvf_ransac_kernels.cu -- the RANSAC pose estimator's own kernels (tvf_ransac_pose, tvf_consensus): sampling, the
-// three-view consensus (the hot path), selection, the refit's compaction and the result rule.  The hypotheses and the
-// refit themselves are the pose path's kernels (run_pose_chunk in tvf_api.cu).
+// tvf_ransac_kernels.cu -- the RANSAC pose estimator's own kernels (tvf_ransac_pose[_refined], tvf_consensus):
+// sampling, the three-view consensus (the hot path), selection, the refit's compaction, the LO rounds' acceptance and
+// the result rule.  The hypotheses and the refit themselves are the pose path's kernels (run_pose_chunk in tvf_api.cu),
+// their adjustments the bundle adjustment's (tvf_ba_kernels.cu).
 #include "tvf_kernels.h"
 #include "tvf_ransac.cuh"
 
@@ -113,6 +114,7 @@ __global__ void ransac_gather_kernel(RansacArgs a, const int* __restrict__ plist
         base += __popc(bal);
     }
     if (a.calm_batched && lane < 27) a.rcalm[j * 27 + lane] = a.calm[b * 27 + lane];
+    if (a.gRt2 && lane < 12) { a.gRt2[j * 12 + lane] = a.bestRt2[b * 12 + lane]; a.gRt3[j * 12 + lane] = a.bestRt3[b * 12 + lane]; }
 }
 
 __global__ void ransac_scatter_kernel(RansacArgs a, const int* __restrict__ plist, int m, const double* __restrict__ Rt2,
@@ -123,6 +125,25 @@ __global__ void ransac_scatter_kernel(RansacArgs a, const int* __restrict__ plis
     a.refRt2[b * 12 + r] = Rt2[j * 12 + r];
     a.refRt3[b * 12 + r] = Rt3[j * 12 + r];
     if (r == 0) a.refst[b] = st[j];
+}
+
+// st[q] <- 1 if pose_st[q] != 0 (pose_st may be null) or the adjustment's status st[q] has ST_NONFINITE, else 0
+__global__ void ransac_flag_kernel(const int* __restrict__ pose_st, int* st, long long Q) {
+    for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < Q; q += (long long)gridDim.x * blockDim.x)
+        st[q] = ((pose_st && pose_st[q] != 0) || (st[q] & ST_NONFINITE)) ? 1 : 0;
+}
+
+// one warp per problem: an LO round's pose replaces the current one if its count is larger (a flagged one counts -1)
+__global__ void ransac_lo_accept_kernel(RansacArgs a) {
+    const int lane = threadIdx.x & 31;
+    const long long b = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (b >= a.B) return;
+    const int c = a.cnt_refit[b];
+    if (!(c > a.cnt_best[b])) return;
+    for (int i = lane; i < a.n; i += 32) a.mask_best[b * a.n + i] = a.mask_refit[b * a.n + i];
+    if (lane < 12) { a.bestRt2[b * 12 + lane] = a.refRt2[b * 12 + lane]; a.bestRt3[b * 12 + lane] = a.refRt3[b * 12 + lane]; }
+    __syncwarp();
+    if (lane == 0) { a.cnt_best[b] = c; a.lo_done[b] += 1; }
 }
 
 // one warp per problem: the result rule of tvf_ransac_pose
@@ -172,6 +193,15 @@ void launch_ransac_gather(const RansacArgs& a, const int* plist, int m, int k, c
 void launch_ransac_scatter(const RansacArgs& a, const int* plist, int m, const double* Rt2, const double* Rt3,
                            const int* st, cudaStream_t stream) {
     ransac_scatter_kernel<<<blocks_for((long long)m * 12, 128, 1LL << 30), 128, 0, stream>>>(a, plist, m, Rt2, Rt3, st);
+}
+
+void launch_ransac_flag(const int* pose_st, int* st, long long Q, cudaStream_t stream) {
+    if (Q <= 0) return;
+    ransac_flag_kernel<<<blocks_for(Q, 256, 1LL << 20), 256, 0, stream>>>(pose_st, st, Q);
+}
+
+void launch_ransac_lo_accept(const RansacArgs& a, cudaStream_t stream) {
+    ransac_lo_accept_kernel<<<blocks_for(a.B * 32, 128, 1LL << 30), 128, 0, stream>>>(a);
 }
 
 void launch_ransac_finish(const RansacArgs& a, int s, cudaStream_t stream) {

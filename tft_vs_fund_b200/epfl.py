@@ -111,7 +111,7 @@ def consensus_stats(mask, truth):
 
 
 def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), device=None, details=None,
-             bundle_adjust=False, covariance=False, raw_matches=False):
+             bundle_adjust=False, covariance=False, raw_matches=False, ransac_refine=False):
     """The linear-method part of experiments_real.m:75-138.  `data`: a Dataset or the path of a dataset directory;
     `triplets_to_test`: rows of indexes_sorted (1-based; the reference uses 1:70 / 1:50, :31-36).  Per loop index `it`:
     pre-filter (:94-101), sample min(100, N) inliers with rng(it) (:103-105; documented stand-in for MATLAB's
@@ -132,7 +132,9 @@ def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), de
     ground-truth inliers, AngError against the ground truth).  details[k]["consensus"][m] holds the consensus mask, its
     size and its precision and recall against the ground-truth inlier mask; bundle_adjust / covariance run on the
     consensus columns, starting from the RANSAC pose (the points triangulated from it); a consensus of fewer than 4
-    matches cannot be adjusted and gets +inf in the adjusted columns."""
+    matches cannot be adjusted and gets +inf in the adjusted columns.
+    ransac_refine=True (with raw_matches): api.ransac_pose(refine=True) instead, whose hypotheses and result are
+    bundle-adjusted (8 LO rounds); nothing else changes."""
     from .scene import SceneRNG
     from .experiments import METHODS
     if not isinstance(data, Dataset):
@@ -165,7 +167,8 @@ def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), de
                 out[m][row] = np.inf
                 continue
             if raw_matches:
-                res = api.ransac_pose(d["Corresp"], CalM, method=m, hypotheses=1024, threshold=1.0, seed=it, device=device)
+                res = api.ransac_pose(d["Corresp"], CalM, method=m, hypotheses=1024, threshold=1.0, seed=it, device=device,
+                                      refine=ransac_refine)
                 Cm, X0 = d["Corresp"][:, res[2]], None
                 rec["consensus"][m] = consensus_stats(res[2], d["inlier_mask"])
             else:
