@@ -62,9 +62,10 @@ def smallest_eigvec_spd(G, max_iter=80, tol=4e-15):
         newA = A - np.outer(c, rk)
         newA[:, k] = rk; newA[k, k] = -piv
         A = newA
-    # pivot-normalised power iteration (TVF_EIG_PIVOTNORM): the iterate is scaled so that its largest component is 1
+    # pivot-normalised power iteration (tvf_warp.cuh::smallest_eigvec_spd): the iterate is scaled so that its largest component is 1
     # (dividing by the signed pivot also absorbs the sign of -M); one exact 2-norm normalisation at the end
-    # start: M (e_0 + e_{N/2} + e_{N-1}), the sum of three columns of the inverse (TVF_PI_FREE_START): a free first application
+    # start: M (e_0 + e_{N/2} + e_{N-1}), the sum of three columns of the inverse (tvf_warp.cuh::smallest_eigvec_spd_half):
+    # a free first application
     x = A[:, 0] + A[:, N // 2] + A[:, N - 1]
     its = 0
     for its in range(1, max_iter + 1):
@@ -201,7 +202,7 @@ def dlt_null(rows, max_iter=40, tol=1e-15):
         if z @ x < 0:
             z = -z
         d2 = float(np.sum((z - x) ** 2)); x = z
-        # tvf_math.cuh::dlt_null (TVF_DLT_PREDICT): stop on a change below 1e-13, or as soon as the error LEFT,
+        # tvf_math.cuh::dlt_null: stop on a change below 1e-13, or as soon as the error LEFT,
         # |z - x| * rate with rate ~ |z - x| / |previous change|, is below 1e-14
         if not d2 > 1e-26 or not d2 * d2 > 1e-28 * dprev:
             break

@@ -26,9 +26,6 @@ namespace {
 #ifndef TVF_NSLOT
 #define TVF_NSLOT 3
 #endif
-#ifndef TVF_RAMP
-#define TVF_RAMP 0
-#endif
 constexpr int NSLOT = TVF_NSLOT;
 // per-handle device scratch buffers (ensure_scratch): Up's count up from SCR_UP, the named ones lie above them
 constexpr int UP_SLOTS = 12;                    // Up: one buffer per array of a stand-alone call (tvf_rt_from_tft has 9)
@@ -405,27 +402,14 @@ template <class Call> int host_pipeline(tvf_handle_t h, Call c, int64_t B) {
     TVF_CK(cudaStreamSynchronize(h->slot[0].stream));
     if (h->use_user_stream) TVF_CK(cudaStreamSynchronize(h->user_stream));
 
-    // Chunk schedule.  The call is bound by the host link (H2D of chunk i+1, kernels of chunk i and D2H of chunk i-1
-    // overlap).  Quarter- and half-size chunks at both ends, meant to shorten the pipeline's fill and drain, were
-    // measured SLOWER (4.31e7 vs 4.56e7 solves/s end to end at 1 M problems, profiles/r01_variants.md) and are off.
-    const bool ramp = TVF_RAMP && B >= 6 * C && C >= 4096;
+    // Chunk schedule: uniform chunks.  The call is bound by the host link (H2D of chunk i+1, kernels of chunk i and D2H of
+    // chunk i-1 overlap).  Quarter- and half-size chunks at both ends, meant to shorten the pipeline's fill and drain, were
+    // measured SLOWER (4.31e7 vs 4.56e7 solves/s end to end at 1 M problems, profiles/r01_variants.md).
     int64_t done = 0; int ci = 0;
     int rc = TVF_OK;
     while (done < B) {
         const int64_t rem = B - done;
-        int64_t Bc = (rem < C) ? rem : C;
-        if (ramp) {
-            const int64_t tail = C / 2 + C / 4;          // the last two chunks: C/2, then C/4
-            if (rem > tail) {
-                const int64_t body = rem - tail;
-                if (ci == 0) Bc = C / 4;
-                else if (ci == 1) Bc = C / 2;
-                else if (body >= 2 * C) Bc = C;
-                else if (body > C) Bc = (body + 1) / 2;
-                else Bc = body;
-            } else if (rem > C / 4) Bc = rem - C / 4;
-            else Bc = rem;
-        }
+        const int64_t Bc = (rem < C) ? rem : C;
         const int si = ci % NSLOT;
         Slot& s = h->slot[si];
         TVF_CK(cudaStreamSynchronize(s.stream));        // slot reuse: its previous chunk (incl. D2H) is finished

@@ -30,37 +30,6 @@ namespace tvf {
 #ifndef TVF_CORE_MINB
 #define TVF_CORE_MINB 5
 #endif
-// MUFU-seeded square root / reciprocal (full precision, not correctly rounded) in the normalisation statistics of the
-// estimator kernels; the stand-alone Normalize2Ddata kernel keeps the IEEE operations
-#ifndef TVF_FAST_STATS
-#define TVF_FAST_STATS 1
-#endif
-#ifndef TVF_STEP_SYNC
-#define TVF_STEP_SYNC 1
-#endif
-// per-kernel overrides: the stage-2 two-problem kernel runs faster WITHOUT the barrier (26.6 against 27.4 ms per 10 M, its
-// warps' iteration counts differ), the two-problem stage-1 solver faster WITH it (40.8 against 44.3)
-#ifndef TVF_S2_SYNC
-#define TVF_S2_SYNC 0
-#endif
-#ifndef TVF_S1D_SYNC
-#define TVF_S1D_SYNC 1
-#endif
-#if TVF_S2_SYNC
-#define S2_SYNC() __syncthreads()
-#else
-#define S2_SYNC() ((void)0)
-#endif
-#if TVF_S1D_SYNC
-#define S1D_SYNC() __syncthreads()
-#else
-#define S1D_SYNC() ((void)0)
-#endif
-#if TVF_STEP_SYNC
-#define STEP_SYNC() __syncthreads()
-#else
-#define STEP_SYNC() ((void)0)
-#endif
 constexpr int CORE_WARPS = TVF_CORE_WARPS;
 constexpr int CORE_MINB = TVF_CORE_MINB;      // resident CTAs per SM the estimator kernels are compiled for
 constexpr int FEAT_STRIDE = 15;   // 14 features + 1 pad: conflict-free 64-bit lane-strided stores
@@ -102,7 +71,8 @@ __device__ __forceinline__ void load_point(const CoreInput& in, long long prob, 
 }
 
 // Normalize2Ddata.m:34-37 for the three views at once, on points already mapped by
-// x -> s0*x + t0 (identity when there is no outer map).  new = s*x + t.
+// x -> s0*x + t0 (identity when there is no outer map).  new = s*x + t.  The square roots and the reciprocal are the
+// MUFU-seeded ones (full precision, not correctly rounded); the stand-alone Normalize2Ddata kernel keeps the IEEE operations.
 template <bool PACKED>
 __device__ __forceinline__ void view_stats(const CoreInput& in, long long prob, int lane,
                                            const double* s0, const double* t0, double* s, double* t) {
@@ -126,21 +96,13 @@ __device__ __forceinline__ void view_stats(const CoreInput& in, long long prob, 
         for (int v = 0; v < 3; ++v) {
             const double dx = (s0[v] * p[2 * v] + t0[2 * v]) - c[2 * v];
             const double dy = (s0[v] * p[2 * v + 1] + t0[2 * v + 1]) - c[2 * v + 1];
-#if TVF_FAST_STATS
             d[v] += sqrt_(dx * dx + dy * dy);
-#else
-            d[v] += sqrt(dx * dx + dy * dy);
-#endif
         }
     }
 #pragma unroll
     for (int v = 0; v < 3; ++v) {
         const double norm0 = warp_sum(d[v]) * invn;
-#if TVF_FAST_STATS
         s[v] = 1.4142135623730951 * rcp_(norm0);
-#else
-        s[v] = 1.4142135623730951 / norm0;
-#endif
         t[2 * v] = -s[v] * c[2 * v];
         t[2 * v + 1] = -s[v] * c[2 * v + 1];
     }
@@ -245,10 +207,6 @@ __device__ __forceinline__ bool is_diag_moment(int idx) {
     const int a = idx >> 4, bg = idx & 15;
     return (a == 0 || a == 3 || a == 5) && (bg == 0 || bg == 3 || bg == 12 || bg == 15);
 }
-__device__ __forceinline__ double diag_moment_weight(int idx) {       // how many diagonal entries equal this moment
-    const int bg = idx & 15;
-    return (bg == 0) ? 4.0 : ((bg == 15) ? 1.0 : 2.0);
-}
 __device__ __forceinline__ double gram_trace_from_moments(const double* mom) {
     double tr = 0.0;
 #pragma unroll
@@ -279,8 +237,10 @@ __device__ __forceinline__ void solve_from_moments(Stage1Scratch& sc, const unsi
     if (status != nullptr && lane == 0) status[prob] = conv ? 0 : ST_EIG_NOCONV;
 }
 
-template <bool PACKED, bool REFINE>
-__global__ void __launch_bounds__(CORE_WARPS * 32, REFINE ? 3 : CORE_MINB)
+// n < REFINE_N_MAX, one problem per warp: statistics, moments and the solve fused, the null vector refined with the
+// un-squared design rows (larger n takes the split stage 1 below)
+template <bool PACKED>
+__global__ void __launch_bounds__(CORE_WARPS * 32, 3)
 tft_stage1_kernel(CoreInput in, double* __restrict__ ws, int* __restrict__ status) {
     __shared__ Stage1Scratch scratch[CORE_WARPS];
     __shared__ unsigned char gidx[32 * 27];
@@ -291,7 +251,7 @@ tft_stage1_kernel(CoreInput in, double* __restrict__ ws, int* __restrict__ statu
     const int beta = (lane >> 2) & 3, gamma = lane & 3, alpha0 = lane >> 4;
 
     for (long long base = (long long)blockIdx.x * CORE_WARPS; base < in.B; base += (long long)gridDim.x * CORE_WARPS) {
-        STEP_SYNC();                 // keeps the CTA's warps in step: they share instruction-cache lines
+        __syncthreads();             // keeps the CTA's warps in step: they share instruction-cache lines
         const long long prob = base + warp;
         if (prob >= in.B) continue;
         double* rec = ws + prob * CORE_WS_TFT;
@@ -333,40 +293,25 @@ tft_stage1_kernel(CoreInput in, double* __restrict__ ws, int* __restrict__ statu
         if (lane < 3) rec[CW_STATS + lane] = sel3(s, lane);
         if (lane < 6) rec[CW_STATS + 3 + lane] = (lane < 3) ? sel3(t, lane) : sel3(t + 3, lane - 3);
         __syncwarp();
-        if constexpr (REFINE) {
-            solve_from_moments(sc, gidx, rec, lane, status, prob,
-                               [&](const double* xs) { return tft_apply_AtA<PACKED>(in, prob, lane, s, t, xs); }, 2);
-        } else {
-            solve_from_moments(sc, gidx, rec, lane, status, prob, NoRefine(), 0);
-        }
+        solve_from_moments(sc, gidx, rec, lane, status, prob,
+                           [&](const double* xs) { return tft_apply_AtA<PACKED>(in, prob, lane, s, t, xs); }, 2);
     }
 }
 
 // =========================================================================== TFT stage 1, two problems per warp
-// n >= REFINE_N_MAX.  Half h of a warp owns problem 2*pair + h from the first load to the last store: the normalisation
-// statistics (points r, r + 16, ... of the problem on lane r; 4-step half-warp reductions), the 96 moments (lane r owns
-// the view-3 x view-2 product (beta, gamma) = (r >> 2, r & 3) and accumulates it against all six view-1 features: one
-// product, six DFMAs and five shared loads per point for BOTH problems), the unit-trace scaling and diagonal shift
-// applied to the moment table (the 12 moments that make up the diagonal of the Gram occur nowhere else in it, so the
-// shift is added to them), the gather of rows r and r + 14, and the two-rows-per-lane solver above.
-#ifndef TVF_STAGE1_DUAL
-#define TVF_STAGE1_DUAL 1
-#endif
-// solver of the split stage 1 (and of the large-n path): 1 = one problem per warp, one matrix row per lane (96
-// registers, 20 warps per SM), 2 = two problems per warp, two rows per lane (168 registers, 12 warps per SM: 22 % fewer
-// instructions but measured 18 % SLOWER -- the per-sweep reciprocal / publish / read-back chain is exposed with so few warps)
-#ifndef TVF_S1_SOLVER
-#define TVF_S1_SOLVER 2
-#endif
+// n >= REFINE_N_MAX, split in two kernels.  Half h of a warp owns problem 2*pair + h.  The moments kernel computes the
+// normalisation statistics (points r, r + 16, ... of the problem on lane r; 4-step half-warp reductions) and the 96
+// moments (lane r owns the view-3 x view-2 product (beta, gamma) = (r >> 2, r & 3) and accumulates it against all six
+// view-1 features: one product, six DFMAs and five shared loads per point for BOTH problems).  The solve kernel applies
+// the unit-trace scaling and diagonal shift to the moment table (the 12 moments that make up the diagonal of the Gram
+// occur nowhere else in it, so the shift is added to them), gathers rows r and r + 14 and runs the two-rows-per-lane
+// solver.  The fused one-kernel form and the one-row-per-lane solvers measured slower (profiles/r02_variants.md, stage 1).
 // 8-byte asynchronous global -> shared copy (LDGSTS) and the wait for all of this thread's copies
 __device__ __forceinline__ void cp_async8(double* smem_dst, const double* gsrc) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(gsrc) : "memory");
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
-#ifndef TVF_S1D_PREFETCH
-#define TVF_S1D_PREFETCH 1
-#endif
 #ifndef TVF_S1D_MINB
 #define TVF_S1D_MINB 3
 #endif
@@ -395,25 +340,6 @@ __device__ __forceinline__ void solve_pair_scaled(Stage1DualScratch& sc, const u
         if (r < 13) rec[CW_T1 + 14 + r] = x1;
         if (status != nullptr && r == 0) status[prob] = conv ? 0 : ST_EIG_NOCONV;
     }
-}
-
-// moments in sc.mom[h] (raw) -> scaled to unit trace, shifted; then rows r and r + 14 -> null vector -> rec
-// (raw: where the unscaled moments of this half lie -- sc.mom[h] itself, or the prefetch buffer of the solve-only kernel)
-__device__ __forceinline__ void solve_pair_from_moments(Stage1DualScratch& sc, const unsigned char* gidx, int lane, bool live,
-                                                        double* rec, int* status, long long prob, const double* raw) {
-    const int h = lane >> 4, r = lane & 15;
-    double* mom = sc.mom[h];
-    const double tr = gram_trace_from_moments(raw);
-    const double scl = 1.0 / tr;
-    const double delta = 1.0e-13 / 27.0;
-    __syncwarp();
-#pragma unroll
-    for (int q = 0; q < 6; ++q) {
-        const int idx = q * 16 + r;
-        mom[idx] = fma(raw[idx], scl, is_diag_moment(idx) ? delta : 0.0);
-    }
-    __syncwarp();
-    solve_pair_scaled(sc, gidx, lane, live, rec, status, prob);
 }
 
 // Normalisation statistics and the 96 moments of one problem on one half-warp (r = lane & 15).  feat: this half's
@@ -446,21 +372,13 @@ __device__ __forceinline__ void half_stats_moments(const CoreInput& in, long lon
 #pragma unroll
             for (int v = 0; v < 3; ++v) {
                 const double dx = p[2 * v] - c[2 * v], dy = p[2 * v + 1] - c[2 * v + 1];
-#if TVF_FAST_STATS
                 d[v] += sqrt_(dx * dx + dy * dy);
-#else
-                d[v] += sqrt(dx * dx + dy * dy);
-#endif
             }
         }
 #pragma unroll
         for (int v = 0; v < 3; ++v) {
             const double norm0 = half_sum(d[v]) * invn;
-#if TVF_FAST_STATS
             s[v] = 1.4142135623730951 * rcp_(norm0);
-#else
-            s[v] = 1.4142135623730951 / norm0;
-#endif
             t[2 * v] = -s[v] * c[2 * v];
             t[2 * v + 1] = -s[v] * c[2 * v + 1];
         }
@@ -500,43 +418,9 @@ __device__ __forceinline__ void store_moments_stats(double* rec, int r, const do
     if (r < 6) rec[CW_STATS + 3 + r] = (r < 3) ? sel3(t, r) : sel3(t + 3, r - 3);
 }
 
-template <bool PACKED>
-__global__ void __launch_bounds__(CORE_WARPS * 32, TVF_S1D_MINB)
-tft_stage1_dual_kernel(CoreInput in, double* __restrict__ ws, int* __restrict__ status) {
-    __shared__ Stage1DualScratch scratch[CORE_WARPS];
-    __shared__ unsigned char gidx[32 * 27];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    build_gidx(gidx);
-    __syncthreads();
-    Stage1DualScratch& sc = scratch[warp];
-    const int h = lane >> 4, r = lane & 15;
-    const long long npairs = (in.B + 1) / 2;
-
-    for (long long base = (long long)blockIdx.x * CORE_WARPS; base < npairs; base += (long long)gridDim.x * CORE_WARPS) {
-        STEP_SYNC();
-        const long long pair = base + warp;
-        if (pair >= npairs) continue;
-        const bool live = 2 * pair + h < in.B;
-        const long long prob = live ? 2 * pair + h : in.B - 1;          // odd batch: the idle half repeats the last problem
-        double* rec = ws + prob * CORE_WS_TFT;
-        double acc[6], s[3], t[6];
-        half_stats_moments<PACKED>(in, prob, r, sc.feat[h], acc, s, t);
-#pragma unroll
-        for (int q = 0; q < 6; ++q) sc.mom[h][q * 16 + r] = acc[q];
-        if (r < 4) sc.mom[h][96 + r] = 0.0;
-        if (live) store_moments_stats(rec, r, acc, s, t);
-        __syncwarp();
-        solve_pair_from_moments(sc, gidx, lane, live, rec, status, prob, sc.mom[h]);
-    }
-}
-
-// The first half on its own, compiled for many resident warps (it needs few registers and is latency bound: global
-// loads, shuffle reductions, square-root chains): statistics + moments -> work-space record.  The solve then runs as
-// tft_stage1_solve_dual_kernel.  (TVF_STAGE1_SPLIT; the fused kernel above holds 54 matrix doubles per lane, which
-// caps it at 12 warps per SM for its whole run.)
-#ifndef TVF_STAGE1_SPLIT
-#define TVF_STAGE1_SPLIT 1
-#endif
+// The first half, compiled for many resident warps (it needs few registers and is latency bound: global loads, shuffle
+// reductions, square-root chains): statistics + moments -> work-space record.  The solve then runs as
+// tft_stage1_solve_dual_kernel, whose 54 matrix doubles per lane cap it at 12 warps per SM.
 #ifndef TVF_S1M_MINB
 #define TVF_S1M_MINB 10
 #endif
@@ -564,9 +448,6 @@ tft_moments_kernel(CoreInput in, double* __restrict__ ws) {
 // two-stage shared-memory buffer by a bulk asynchronous copy (TMA engine) while the current eight are processed: the three
 // passes over the points (sums, distances, moments) read shared memory, and no warp waits for DRAM (the plain kernel
 // spent most of its stall samples in `long_scoreboard`).  Packed input, n <= MOM_TMA_MAX_N.
-#ifndef TVF_S1M_TMA
-#define TVF_S1M_TMA 1
-#endif
 #ifndef TVF_S1M_TMA_MINB
 #define TVF_S1M_TMA_MINB 6
 #endif
@@ -614,7 +495,8 @@ tft_moments_tma_kernel(CoreInput in, double* __restrict__ ws) {
 #define TVF_S1D_WARPS TVF_CORE_WARPS
 #endif
 constexpr int S1D_WARPS = TVF_S1D_WARPS;
-// Large-n path, two problems per warp: the moments were produced by tft_moments_large_kernel.
+// The second half, two problems per warp: the moments come from tft_moments_kernel, tft_moments_tma_kernel or, at large
+// n, tft_moments_large_kernel.
 __global__ void __launch_bounds__(S1D_WARPS * 32, TVF_S1D_MINB)
 tft_stage1_solve_dual_kernel(long long B, double* __restrict__ ws, int* __restrict__ status) {
     __shared__ Stage1DualScratch scratch[S1D_WARPS];
@@ -625,7 +507,6 @@ tft_stage1_solve_dual_kernel(long long B, double* __restrict__ ws, int* __restri
     Stage1DualScratch& sc = scratch[warp];
     const int h = lane >> 4, r = lane & 15;
     const long long npairs = (B + 1) / 2;
-#if TVF_S1D_PREFETCH
     // The raw moments of the NEXT pair travel global -> shared (cp.async, no registers: the solver leaves none) while this
     // pair is solved; they land in the feature staging buffer, which the solve-only kernel does not use otherwise.
     double* raw = sc.feat[h];
@@ -639,19 +520,17 @@ tft_stage1_solve_dual_kernel(long long B, double* __restrict__ ws, int* __restri
         }
         if (r < 4) sc.mom[h][96 + r] = 0.0;
     }
-#endif
     for (long long base = (long long)blockIdx.x * S1D_WARPS; base < npairs; base += (long long)gridDim.x * S1D_WARPS) {
-        S1D_SYNC();
+        __syncthreads();             // keeps the warps on the same instruction-cache lines: faster than without (profiles/r02_variants.md)
         const long long pair = base + warp;
         if (pair >= npairs) continue;
         const bool live = 2 * pair + h < B;
         const long long prob = live ? 2 * pair + h : B - 1;
         double* rec = ws + prob * CORE_WS_TFT;
-#if TVF_S1D_PREFETCH
         cp_async_wait_all();
         __syncwarp();
-        // scaled table -> sc.mom (two barriers inside); afterwards nobody reads `raw` any more, so the next pair's copy may
-        // start: each lane overwrites only the entries it read itself
+        // scaled table -> sc.mom; afterwards nobody reads `raw` any more, so the next pair's copy may start: each lane
+        // overwrites only the entries it read itself
         const double tr = gram_trace_from_moments(raw);
         const double scl = 1.0 / tr;
         const double delta = 1.0e-13 / 27.0;
@@ -668,115 +547,6 @@ tft_stage1_solve_dual_kernel(long long B, double* __restrict__ ws, int* __restri
         }
         __syncwarp();
         solve_pair_scaled(sc, gidx, lane, live, rec, status, prob);
-#else
-        __syncwarp();
-#pragma unroll
-        for (int q = 0; q < 6; ++q) sc.mom[h][q * 16 + r] = rec[CW_MOM + q * 16 + r];
-        if (r < 4) sc.mom[h][96 + r] = 0.0;
-        __syncwarp();
-        solve_pair_from_moments(sc, gidx, lane, live, rec, status, prob, sc.mom[h]);
-#endif
-    }
-}
-
-// The second half of stage 1 on its own, one problem per warp (27 x 27 Gram from the 96 moments -> null vector).  The
-// moments come from tft_moments_kernel (split stage 1) or from tft_moments_large_kernel (large n).  The unit-trace
-// scaling and the diagonal shift are applied to the moment table (see solve_pair_from_moments).
-#ifndef TVF_S1S_MINB
-#define TVF_S1S_MINB 4
-#endif
-__global__ void __launch_bounds__(CORE_WARPS * 32, TVF_S1S_MINB)
-tft_stage1_solve_kernel(long long B, double* __restrict__ ws, int* __restrict__ status) {
-    __shared__ Stage1Scratch scratch[CORE_WARPS];
-    __shared__ unsigned char gidx[32 * 27];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    build_gidx(gidx);
-    __syncthreads();
-    Stage1Scratch& sc = scratch[warp];
-    const long long stride = (long long)gridDim.x * CORE_WARPS;
-    long long prob = (long long)blockIdx.x * CORE_WARPS + warp;
-    // the three moments of this lane for the NEXT problem are fetched while the current one is being solved
-    double m0 = 0.0, m1 = 0.0, m2 = 0.0;
-    if (prob < B) { const double* rec = ws + prob * CORE_WS_TFT; m0 = rec[CW_MOM + lane]; m1 = rec[CW_MOM + 32 + lane]; m2 = rec[CW_MOM + 64 + lane]; }
-    for (long long base = (long long)blockIdx.x * CORE_WARPS; base < B; base += stride, prob += stride) {
-        STEP_SYNC();
-        if (prob >= B) continue;
-        double* rec = ws + prob * CORE_WS_TFT;
-        // trace = sum of the 12 diagonal moments with multiplicities 4, 2, 2, 1 (gram_trace_from_moments), as one reduction
-        double part = 0.0;
-        part += is_diag_moment(lane) ? diag_moment_weight(lane) * m0 : 0.0;
-        part += is_diag_moment(lane + 32) ? diag_moment_weight(lane + 32) * m1 : 0.0;
-        part += is_diag_moment(lane + 64) ? diag_moment_weight(lane + 64) * m2 : 0.0;
-        const double scl = 1.0 / warp_sum(part);
-        const double delta = 1.0e-13 / 27.0;
-        __syncwarp();
-        sc.mom[lane] = fma(m0, scl, is_diag_moment(lane) ? delta : 0.0);
-        sc.mom[lane + 32] = fma(m1, scl, is_diag_moment(lane + 32) ? delta : 0.0);
-        sc.mom[lane + 64] = fma(m2, scl, is_diag_moment(lane + 64) ? delta : 0.0);
-        if (lane == 0) { sc.mom[96] = 0.0; sc.mom[97] = 0.0; }
-        __syncwarp();
-        if (prob + stride < B) {
-            const double* nrec = ws + (prob + stride) * CORE_WS_TFT;
-            m0 = nrec[CW_MOM + lane]; m1 = nrec[CW_MOM + 32 + lane]; m2 = nrec[CW_MOM + 64 + lane];
-        }
-        double g[27];
-#pragma unroll
-        for (int c = 0; c < 27; ++c) g[c] = sc.mom[gidx[lane * 27 + c]];
-        bool conv;
-        const double tl = smallest_eigvec_spd<27, NoRefine, true>(g, lane, sc.sbuf, &conv);
-        if (lane < 27) rec[CW_T1 + lane] = tl;
-        if (status != nullptr && lane == 0) status[prob] = conv ? 0 : ST_EIG_NOCONV;
-    }
-}
-
-// Solve-only kernel with the row-and-column split layout (smallest_eigvec_spd_cs): TVF_S1_SOLVER = 3.
-#ifndef TVF_S1C_MINB
-#define TVF_S1C_MINB 4
-#endif
-__global__ void __launch_bounds__(CORE_WARPS * 32, TVF_S1C_MINB)
-tft_stage1_solve_cs_kernel(long long B, double* __restrict__ ws, int* __restrict__ status) {
-    __shared__ Stage1Scratch scratch[CORE_WARPS];
-    __shared__ unsigned char gidx[32 * 27];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    build_gidx(gidx);
-    __syncthreads();
-    Stage1Scratch& sc = scratch[warp];
-    const int h = lane >> 4, r = lane & 15;
-    const int row0 = (r < 14) ? r : 31, row1 = (r < 13) ? r + 14 : 31;          // rows >= 27 gather the zero sentinel
-    for (long long base = (long long)blockIdx.x * CORE_WARPS; base < B; base += (long long)gridDim.x * CORE_WARPS) {
-        STEP_SYNC();
-        const long long prob = base + warp;
-        if (prob >= B) continue;
-        double* rec = ws + prob * CORE_WS_TFT;
-        const double m0 = rec[CW_MOM + lane], m1 = rec[CW_MOM + 32 + lane], m2 = rec[CW_MOM + 64 + lane];
-        double part = 0.0;
-        part += is_diag_moment(lane) ? diag_moment_weight(lane) * m0 : 0.0;
-        part += is_diag_moment(lane + 32) ? diag_moment_weight(lane + 32) * m1 : 0.0;
-        part += is_diag_moment(lane + 64) ? diag_moment_weight(lane + 64) * m2 : 0.0;
-        const double scl = 1.0 / warp_sum(part);
-        const double delta = 1.0e-13 / 27.0;
-        __syncwarp();
-        sc.mom[lane] = fma(m0, scl, is_diag_moment(lane) ? delta : 0.0);
-        sc.mom[lane + 32] = fma(m1, scl, is_diag_moment(lane + 32) ? delta : 0.0);
-        sc.mom[lane + 64] = fma(m2, scl, is_diag_moment(lane + 64) ? delta : 0.0);
-        if (lane == 0) { sc.mom[96] = 0.0; sc.mom[97] = 0.0; }
-        __syncwarp();
-        double g0[14], g1[14];
-#pragma unroll
-        for (int c = 0; c < 14; ++c) {
-            const int col = 14 * h + c;                     // column 27 (h = 1, c = 13) is padding
-            const bool pad = (h == 1) && (c == 13);
-            g0[c] = pad ? 0.0 : sc.mom[gidx[row0 * 27 + (pad ? 0 : col)]];
-            g1[c] = pad ? 0.0 : sc.mom[gidx[row1 * 27 + (pad ? 0 : col)]];
-        }
-        double x0, x1;
-        bool conv;
-        smallest_eigvec_spd_cs<27>(g0, g1, lane, sc.sbuf, &x0, &x1, &conv);
-        if (h == 0) {
-            if (r < 14) rec[CW_T1 + r] = x0;
-            if (r < 13) rec[CW_T1 + 14 + r] = x1;
-        }
-        if (status != nullptr && lane == 0) status[prob] = conv ? 0 : ST_EIG_NOCONV;
     }
 }
 
@@ -862,8 +632,10 @@ struct __align__(16) Stage2Scratch {
     double Nm[28];                   // N1, inv(N2), inv(N3)
 };
 
-template <bool PACKED, bool REFINE>
-__global__ void __launch_bounds__(CORE_WARPS * 32, REFINE ? 3 : CORE_MINB)
+// n < REFINE_N_MAX, one problem per warp: the projected null vector is refined with the design rows (larger n takes
+// tft_stage2_dual_kernel below)
+template <bool PACKED>
+__global__ void __launch_bounds__(CORE_WARPS * 32, 3)
 tft_stage2_kernel(CoreInput in, const double* __restrict__ ws, double* __restrict__ Tout,
                   double* __restrict__ P2out, double* __restrict__ P3out, int* __restrict__ status) {
     const int normalize = in.normalize;
@@ -874,7 +646,7 @@ tft_stage2_kernel(CoreInput in, const double* __restrict__ ws, double* __restric
     const int jr = lane % 3, kr = (lane / 3) % 3, ir = (lane < 27) ? lane / 9 : 0;
 
     for (long long base = (long long)blockIdx.x * CORE_WARPS; base < B; base += (long long)gridDim.x * CORE_WARPS) {
-        STEP_SYNC();
+        __syncthreads();
         const long long prob = base + warp;
         if (prob >= B) continue;
         const double* rec = ws + prob * CORE_WS_TFT;
@@ -913,7 +685,7 @@ tft_stage2_kernel(CoreInput in, const double* __restrict__ ws, double* __restric
             const double st_s[3] = {rec[CW_STATS], rec[CW_STATS + 1], rec[CW_STATS + 2]};
             const double st_t[6] = {rec[CW_STATS + 3], rec[CW_STATS + 4], rec[CW_STATS + 5], rec[CW_STATS + 6],
                                     rec[CW_STATS + 7], rec[CW_STATS + 8]};
-            // Up' A'A Up tp from the design rows (refinement of the projected problem, small n only)
+            // Up' A'A Up tp from the design rows (refinement of the projected problem)
             auto resid15 = [&](const double* xs) {
                 double a27 = 0.0;
                 if (lane < 27) {
@@ -935,9 +707,7 @@ tft_stage2_kernel(CoreInput in, const double* __restrict__ ws, double* __restric
                 return (lane < 15) ? r : 0.0;
             };
             bool conv2;
-            double tpl;
-            if constexpr (REFINE) tpl = smallest_eigvec_spd<15>(g15, lane, sc.sbuf, &conv2, resid15, 1);
-            else tpl = smallest_eigvec_spd<15>(g15, lane, sc.sbuf, &conv2);
+            const double tpl = smallest_eigvec_spd<15>(g15, lane, sc.sbuf, &conv2, resid15, 1);
             if (!conv2) st |= ST_EIG_NOCONV;
             __syncwarp();
             if (lane < 15) sc.tp[lane] = tpl;
@@ -1009,25 +779,14 @@ tft_stage2_kernel(CoreInput in, const double* __restrict__ ws, double* __restric
 // The pair's two work-space records are adjacent in global memory (2 x 1120 bytes): lane 0 fetches the NEXT pair's with one
 // bulk asynchronous copy per warp (own mbarrier) as soon as the current pair's moments have been consumed (the epipoles
 // and statistics are copied aside first), so no pair waits for its loads.
-#ifndef TVF_S2_TMA
-#define TVF_S2_TMA 1
-#endif
 struct __align__(16) Stage2DualScratch {
     double sbuf[64];
     double H[2][15 * H15_LD];            // Up' G Up of the two problems
-#if TVF_S2_TMA
     double rec2[2 * CORE_WS_TFT];        // the two work-space records as they lie in global memory (one bulk copy)
-#else
-    double mom2[2][96];                  // moments of the two problems
-#endif
     double es[2][28];                    // e21, u1, u2 (0..8), e31, v1, v2 (9..17), normalisation statistics (18..26)
     double T[2][28];
     double tp[2][16];
 };
-
-#ifndef TVF_STAGE2_DUAL
-#define TVF_STAGE2_DUAL 1
-#endif
 
 // resident CTAs per SM the kernel is compiled for: 5 (96 registers, 12 bytes spilled) measured 14.7 ms per 10 M against 15.1 at 4
 // (128 registers, 4 bytes spilled) and 16.2 at 3 (profiles/r03_stage2_factored_h.md)
@@ -1045,7 +804,6 @@ tft_stage2_dual_kernel(int normalize, long long B, const double* __restrict__ ws
     const bool has1 = r15 < 11;
     const int e0 = r15, e1 = has1 ? r15 + 16 : 26;
     const long long npairs = (B + 1) / 2;
-#if TVF_S2_TMA
     __shared__ unsigned long long wbar[CORE_WARPS];
     const long long pstride = (long long)gridDim.x * CORE_WARPS;
     auto fetch = [&](long long pr) {                        // lane 0 only: records of pair pr -> sc.rec2
@@ -1058,10 +816,10 @@ tft_stage2_dual_kernel(int normalize, long long B, const double* __restrict__ ws
     __syncthreads();
     if (lane == 0 && (long long)blockIdx.x * CORE_WARPS + warp < npairs) fetch((long long)blockIdx.x * CORE_WARPS + warp);
     unsigned parity = 0;
-#endif
 
+    // no CTA barrier per pair: the warps' iteration counts differ, and the kernel measured faster without it
+    // (profiles/r02_variants.md)
     for (long long base = (long long)blockIdx.x * CORE_WARPS; base < npairs; base += (long long)gridDim.x * CORE_WARPS) {
-        S2_SYNC();
         const long long pair = base + warp;
         if (pair >= npairs) continue;
         const long long prob0 = 2 * pair;
@@ -1070,7 +828,6 @@ tft_stage2_dual_kernel(int normalize, long long B, const double* __restrict__ ws
         const int hp = live ? h : 0;
         // lane 16 p + q: epipoles (q < 6) and normalisation statistics (6 <= q < 15) of problem p, set aside
         const int es_slot = (r15 < 3) ? r15 : ((r15 < 6) ? r15 + 6 : r15 + 12);
-#if TVF_S2_TMA
         mbar_wait(&wbar[warp], parity);
         parity ^= 1u;
         const double* mom = sc.rec2 + hp * CORE_WS_TFT + CW_MOM;
@@ -1078,26 +835,6 @@ tft_stage2_dual_kernel(int normalize, long long B, const double* __restrict__ ws
             const double* recq = sc.rec2 + hp * CORE_WS_TFT;
             if (r15 < 15) sc.es[h][es_slot] = (r15 < 6) ? recq[CW_EPI + r15] : recq[CW_STATS + r15 - 6];
         }
-#else
-        // every global load of the pair is issued up front (moments, epipoles, normalisation statistics): one exposed memory
-        // latency per pair
-        const double* mom = sc.mom2[hp];
-        {
-            double mm[2][3];
-#pragma unroll
-            for (int p = 0; p < 2; ++p) {
-                const double* rec = ws + (prob0 + ((p < nprob) ? p : 0)) * CORE_WS_TFT;
-                mm[p][0] = rec[CW_MOM + lane]; mm[p][1] = rec[CW_MOM + 32 + lane]; mm[p][2] = rec[CW_MOM + 64 + lane];
-            }
-            const double* recq = ws + (prob0 + hp) * CORE_WS_TFT;
-            const double ev = (r15 < 6) ? recq[CW_EPI + r15] : ((r15 < 15) ? recq[CW_STATS + r15 - 6] : 0.0);
-#pragma unroll
-            for (int p = 0; p < 2; ++p) {
-                sc.mom2[p][lane] = mm[p][0]; sc.mom2[p][lane + 32] = mm[p][1]; sc.mom2[p][lane + 64] = mm[p][2];
-            }
-            if (r15 < 15) sc.es[h][es_slot] = ev;
-        }
-#endif
         __syncwarp();
         {
             // orthonormal completions, once per problem: lane 0 of the half -> u1, u2; lane 1 -> v1, v2
@@ -1113,9 +850,7 @@ tft_stage2_dual_kernel(int normalize, long long B, const double* __restrict__ ws
         const double* bh = sc.es[h];
         form_h15(mom, bh, bh + 9, r15, sc.H[h]);
         __syncwarp();
-#if TVF_S2_TMA
         if (lane == 0 && pair + pstride < npairs) fetch(pair + pstride);       // every lane is done with sc.rec2
-#endif
         // ---- the smallest eigenvector of H (linearTFT.m:84), both problems at once
         {
             double g15[15];
@@ -1223,7 +958,7 @@ f_stage1_kernel(CoreInput in, double* __restrict__ ws, int* __restrict__ status)
     const int ar = (lane < 9) ? lane / 3 : 0, br = (lane < 9) ? lane % 3 : 0;
 
     for (long long base = (long long)blockIdx.x * CORE_WARPS; base < in.B; base += (long long)gridDim.x * CORE_WARPS) {
-        STEP_SYNC();
+        __syncthreads();
         const long long prob = base + warp;
         if (prob >= in.B) continue;
         double* rec = ws + prob * CORE_WS_F;
@@ -1359,53 +1094,31 @@ static inline unsigned core_grid_minb(long long units, int sm_count, int minb) {
 
 int launch_tft_stage1(const CoreInput& in, double* ws, int* status, int sm_count, cudaStream_t stream) {
     if (in.B <= 0) return 0;
-    const unsigned g = core_grid(in.B, sm_count);
-    const bool refine = in.n < REFINE_N_MAX;       // barely determined systems: polish with the un-squared rows
-#if TVF_STAGE1_DUAL
-    if (!refine) {
-#if TVF_STAGE1_SPLIT
-        const unsigned gm = core_grid_minb((in.B + 1) / 2, sm_count, TVF_S1M_MINB);
-#if TVF_S1M_TMA
-        if (in.packed && in.n <= MOM_TMA_MAX_N) {
-            const size_t dyn = 2 * (size_t)(2 * CORE_WARPS) * in.n * 48;
-            cudaFuncSetAttribute(tft_moments_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);   // per launch: per device
-            const unsigned gt = core_grid_minb((in.B + 1) / 2, sm_count, TVF_S1M_TMA_MINB);
-            tft_moments_tma_kernel<<<gt, CORE_WARPS * 32, dyn, stream>>>(in, ws);
-            return 1;
-        }
-#endif
-        if (in.packed) tft_moments_kernel<true><<<gm, CORE_WARPS * 32, 0, stream>>>(in, ws);
-        else tft_moments_kernel<false><<<gm, CORE_WARPS * 32, 0, stream>>>(in, ws);
-        return 1;                 // the caller follows up with launch_tft_stage1_solve
-#else
-        const unsigned gd = core_grid_minb((in.B + 1) / 2, sm_count, TVF_S1D_MINB);
-        if (in.packed) tft_stage1_dual_kernel<true><<<gd, CORE_WARPS * 32, 0, stream>>>(in, ws, status);
-        else tft_stage1_dual_kernel<false><<<gd, CORE_WARPS * 32, 0, stream>>>(in, ws, status);
+    if (in.n < REFINE_N_MAX) {       // barely determined systems: polish with the un-squared rows
+        const unsigned g = core_grid(in.B, sm_count);
+        if (in.packed) tft_stage1_kernel<true><<<g, CORE_WARPS * 32, 0, stream>>>(in, ws, status);
+        else tft_stage1_kernel<false><<<g, CORE_WARPS * 32, 0, stream>>>(in, ws, status);
         return 0;
-#endif
     }
-#endif
-    if (in.packed && refine) tft_stage1_kernel<true, true><<<g, CORE_WARPS * 32, 0, stream>>>(in, ws, status);
-    else if (in.packed) tft_stage1_kernel<true, false><<<g, CORE_WARPS * 32, 0, stream>>>(in, ws, status);
-    else if (refine) tft_stage1_kernel<false, true><<<g, CORE_WARPS * 32, 0, stream>>>(in, ws, status);
-    else tft_stage1_kernel<false, false><<<g, CORE_WARPS * 32, 0, stream>>>(in, ws, status);
-    return 0;
+    if (in.packed && in.n <= MOM_TMA_MAX_N) {
+        const size_t dyn = 2 * (size_t)(2 * CORE_WARPS) * in.n * 48;
+        cudaFuncSetAttribute(tft_moments_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);   // per launch: per device
+        const unsigned gt = core_grid_minb((in.B + 1) / 2, sm_count, TVF_S1M_TMA_MINB);
+        tft_moments_tma_kernel<<<gt, CORE_WARPS * 32, dyn, stream>>>(in, ws);
+        return 1;
+    }
+    const unsigned gm = core_grid_minb((in.B + 1) / 2, sm_count, TVF_S1M_MINB);
+    if (in.packed) tft_moments_kernel<true><<<gm, CORE_WARPS * 32, 0, stream>>>(in, ws);
+    else tft_moments_kernel<false><<<gm, CORE_WARPS * 32, 0, stream>>>(in, ws);
+    return 1;                 // the caller follows up with launch_tft_stage1_solve
 }
 
 void launch_tft_stage1_solve(long long B, double* ws, int* status, int sm_count, cudaStream_t stream) {
     if (B <= 0) return;
-#if TVF_S1_SOLVER == 2
-    {
-        long long blocks = ((B + 1) / 2 + S1D_WARPS - 1) / S1D_WARPS;
-        const long long cap = (long long)sm_count * TVF_S1D_MINB * 4;
-        if (blocks > cap) blocks = cap;
-        tft_stage1_solve_dual_kernel<<<(unsigned)(blocks < 1 ? 1 : blocks), S1D_WARPS * 32, 0, stream>>>(B, ws, status);
-    }
-#elif TVF_S1_SOLVER == 3
-    tft_stage1_solve_cs_kernel<<<core_grid_minb(B, sm_count, TVF_S1C_MINB), CORE_WARPS * 32, 0, stream>>>(B, ws, status);
-#else
-    tft_stage1_solve_kernel<<<core_grid_minb(B, sm_count, TVF_S1S_MINB), CORE_WARPS * 32, 0, stream>>>(B, ws, status);
-#endif
+    long long blocks = ((B + 1) / 2 + S1D_WARPS - 1) / S1D_WARPS;
+    const long long cap = (long long)sm_count * TVF_S1D_MINB * 4;
+    if (blocks > cap) blocks = cap;
+    tft_stage1_solve_dual_kernel<<<(unsigned)(blocks < 1 ? 1 : blocks), S1D_WARPS * 32, 0, stream>>>(B, ws, status);
 }
 
 void launch_tft_epipoles(double* ws, long long B, cudaStream_t stream) {
@@ -1416,18 +1129,13 @@ void launch_tft_epipoles(double* ws, long long B, cudaStream_t stream) {
 void launch_tft_stage2(const CoreInput& in, const double* ws, double* T, double* P2, double* P3, int* status,
                        int sm_count, cudaStream_t stream) {
     if (in.B <= 0) return;
-    const unsigned g = core_grid(in.B, sm_count);
-    const bool refine = in.n < REFINE_N_MAX;
-#if TVF_STAGE2_DUAL
-    if (!refine) {          // the un-refined step never touches the points again: two problems per warp
+    if (in.n >= REFINE_N_MAX) {     // the un-refined step never touches the points again: two problems per warp
         tft_stage2_dual_kernel<<<core_grid_minb((in.B + 1) / 2, sm_count, TVF_S2D_MINB), CORE_WARPS * 32, 0, stream>>>(in.normalize, in.B, ws, T, P2, P3, status);
         return;
     }
-#endif
-    if (in.packed && refine) tft_stage2_kernel<true, true><<<g, CORE_WARPS * 32, 0, stream>>>(in, ws, T, P2, P3, status);
-    else if (in.packed) tft_stage2_kernel<true, false><<<g, CORE_WARPS * 32, 0, stream>>>(in, ws, T, P2, P3, status);
-    else if (refine) tft_stage2_kernel<false, true><<<g, CORE_WARPS * 32, 0, stream>>>(in, ws, T, P2, P3, status);
-    else tft_stage2_kernel<false, false><<<g, CORE_WARPS * 32, 0, stream>>>(in, ws, T, P2, P3, status);
+    const unsigned g = core_grid(in.B, sm_count);
+    if (in.packed) tft_stage2_kernel<true><<<g, CORE_WARPS * 32, 0, stream>>>(in, ws, T, P2, P3, status);
+    else tft_stage2_kernel<false><<<g, CORE_WARPS * 32, 0, stream>>>(in, ws, T, P2, P3, status);
 }
 
 void launch_f_stage1(const CoreInput& in, double* ws, int* status, int sm_count, cudaStream_t stream) {

@@ -42,9 +42,6 @@ namespace tvf {
 #ifndef TVF_LG_MINB
 #define TVF_LG_MINB 3
 #endif
-#ifndef TVF_LG_SQRT5
-#define TVF_LG_SQRT5 1
-#endif
 constexpr int LG_CLUSTER = TVF_LG_CLUSTER;
 constexpr int LG_THREADS = 128;
 constexpr int LG_WARPS = LG_THREADS / 32;
@@ -94,28 +91,19 @@ __device__ __forceinline__ double warp_reduce_transposed(double (&v)[NV], int la
 
 // sqrt(x) for x >= 0 without the ~15 FP64 issue slots of the IEEE sequence: MUFU.RSQ64H seed (relative error ~2^-20, it
 // only looks at the high word), one Goldschmidt step (-> ~2^-39) and a residual correction (-> below 1 ulp; not
-// correctly rounded).  TVF_LG_SQRT5 (default): the half reciprocal h is taken from the seed by an exponent decrement on
+// correctly rounded).  The half reciprocal h is taken from the seed by an exponent decrement on
 // the integer pipe and is NOT refined -- it only scales the last correction, whose own size is 2^-39 of the result, so
 // its 2^-20 error enters at 2^-59: 5 FP64 issue slots instead of 7 (+1.4 % on the kernel).  x below 1e-300 (incl. 0)
 // returns 0.
 __device__ __forceinline__ double sqrt_fast(double x) {
     double y;
     asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(x));
-#if TVF_LG_SQRT5
     const double h = __hiloint2double(__double2hiint(y) - 0x00100000, __double2loint(y));     // y / 2 (y is normal here)
     double g = x * y;
     const double r = fma(-g, h, 0.5);
     g = fma(g, r, g);
     const double d = fma(-g, g, x);
     g = fma(d, h, g);
-#else
-    double g = x * y, h = 0.5 * y;
-    const double r = fma(-g, h, 0.5);
-    g = fma(g, r, g);
-    h = fma(h, r, h);
-    const double d = fma(-g, g, x);
-    g = fma(d, h, g);
-#endif
     return (__double2hiint(x) > 0x01a00000) ? g : 0.0;      // x > ~1e-300 (x >= 0), without touching the FP64 pipe
 }
 

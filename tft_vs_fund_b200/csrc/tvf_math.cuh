@@ -18,19 +18,11 @@
 
 namespace tvf {
 
-#ifndef TVF_FAST_RSQRT
-#define TVF_FAST_RSQRT 1
-#endif
-#ifndef TVF_DLT_PREDICT
-#define TVF_DLT_PREDICT 1
-#endif
-
 // 1/sqrt(x) for normal positive x.  Device: MUFU.RSQ64H seed (~20 bits) + two Newton steps (full double precision,
 // not correctly rounded, no special-case path: 8 instructions instead of the ~16 of CUDA's rsqrt()).  x = 0 gives
 // NaN (CUDA: +inf); every caller multiplies the result into a vector that is then 0*inf = NaN as well, or guards x > 0.
 TVF_HD double rsqrt_(double x) {
 #if defined(__CUDA_ARCH__)
-#if TVF_FAST_RSQRT
     double y;
     asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(x));
     const double h = 0.5 * x;
@@ -38,9 +30,6 @@ TVF_HD double rsqrt_(double x) {
     y = fma(y, e, y);
     e = fma(-h * y, y, 0.5);
     return fma(y, e, y);
-#else
-    return rsqrt(x);
-#endif
 #else
     return 1.0 / sqrt(x);
 #endif
@@ -196,9 +185,6 @@ TVF_HD void jacobi_svd3(double* A, double* V, double* s, int* sweeps = nullptr) 
 // linear TFT estimate at 3 px noise, 0 for a valid (calibrated, constrained) tensor -- two to five steps.  Returns false
 // when it has not converged in NULL3_MAX_IT steps (two nearly equal smallest singular values); the caller then takes
 // the Jacobi route, which does not care.
-#ifndef TVF_NULL3_QR
-#define TVF_NULL3_QR 1
-#endif
 constexpr int NULL3_MAX_IT = 12;
 TVF_HD bool null3_qr(const double* M, bool transpose, double* v) {
     double a[3][3];
@@ -271,9 +257,7 @@ TVF_HD bool null3_qr(const double* M, bool transpose, double* v) {
 
 // V(:,end) of svd(M) for a 3x3 M (column-major); M is not modified.
 TVF_HD void null3(const double* M, double* v) {
-#if TVF_NULL3_QR
     if (null3_qr(M, false, v)) return;
-#endif
     double A[9], V[9], s[3];
 #pragma unroll
     for (int i = 0; i < 9; ++i) A[i] = M[i];
@@ -282,9 +266,7 @@ TVF_HD void null3(const double* M, double* v) {
 }
 // same for M.' without forming the transpose in memory
 TVF_HD void null3_t(const double* M, double* v) {
-#if TVF_NULL3_QR
     if (null3_qr(M, true, v)) return;
-#endif
     double A[9], V[9], s[3];
 #pragma unroll
     for (int c = 0; c < 3; ++c)
@@ -459,9 +441,7 @@ TVF_HD void dlt_null(double (&a)[M][4], double* x, int* iters = nullptr) {
     double inv = rsqrt_(x0 * x0 + x1 * x1 + x2 * x2 + x3 * x3);
     x0 *= inv; x1 *= inv; x2 *= inv; x3 *= inv;
     int it = 0;
-#if TVF_DLT_PREDICT
     double dprev = 0.0;               // squared change of the previous step (0: no rate estimate yet)
-#endif
     for (; it < 40; ++it) {
         const double y0 = x0 * d[0];
         const double y1 = (x1 - r[0][1] * y0) * d[1];
@@ -473,7 +453,6 @@ TVF_HD void dlt_null(double (&a)[M][4], double* x, int* iters = nullptr) {
         double z0 = (y0 - r[0][1] * z1 - r[0][2] * z2 - r[0][3] * z3) * d[0];
         inv = rsqrt_(z0 * z0 + z1 * z1 + z2 * z2 + z3 * z3);
         z0 *= inv; z1 *= inv; z2 *= inv; z3 *= inv;
-#if TVF_DLT_PREDICT
         // squared change d2 = |z - x|^2.  Inverse iteration converges linearly with rate rho = (s4/s3)^2 ~ d2/dprev
         // (in squares: rho^2), so the error LEFT in z is ~ |z - x| * rho: stop as soon as that product is below 1e-14
         // instead of running one more step only to see a change below 1e-13.  (All terms are squares: sign symmetric.)
@@ -482,11 +461,6 @@ TVF_HD void dlt_null(double (&a)[M][4], double* x, int* iters = nullptr) {
         x0 = z0; x1 = z1; x2 = z2; x3 = z3;
         if (!(d2 > 1e-26) || !(d2 * d2 > 1e-28 * dprev)) { ++it; break; }
         dprev = d2;
-#else
-        const double diff = fmax(fmax(fabs(z0 - x0), fabs(z1 - x1)), fmax(fabs(z2 - x2), fabs(z3 - x3)));
-        x0 = z0; x1 = z1; x2 = z2; x3 = z3;
-        if (!(diff > 1e-13)) { ++it; break; }   // linear rate <= ~1e-3: the error left is far below 1e-13
-#endif
     }
     x[0] = x0; x[1] = x1; x[2] = x2; x[3] = x3;
     if (iters) *iters = it;

@@ -5,26 +5,10 @@
 #pragma once
 #include "tvf_math.cuh"
 
-#ifndef TVF_CHEIR_UNROLL
-#define TVF_CHEIR_UNROLL 1
-#endif
-// votes from certified depth signs (dlt4_depth_signs) wherever the DLT solution itself is not needed
-#ifndef TVF_VOTE_FAST_SIGNS
-#define TVF_VOTE_FAST_SIGNS 1
-#endif
 // second-chance certificate from the 4 x 4 normal equations (dlt4_depth_signs, round 2 first half) between the ray test
 // and the accurate route: off -- what the ray test declines it mostly declines too
 #ifndef TVF_VOTE_GRAM_SIGNS
 #define TVF_VOTE_GRAM_SIGNS 0
-#endif
-// certified ray / plane test (dlt4_depth_signs_ray) first; 0 with TVF_VOTE_GRAM_SIGNS=1 and TVF_TAIL_REUSE_X=1 is the tail of
-// the first half of round 2
-#ifndef TVF_VOTE_RAY_SIGNS
-#define TVF_VOTE_RAY_SIGNS 1
-#endif
-// the accurate route behind the ray test as an out-of-line device function (it runs for 0.1 % of the vote DLTs)
-#ifndef TVF_CHEIR_NOINLINE
-#define TVF_CHEIR_NOINLINE 0
 #endif
 
 namespace tvf {
@@ -154,18 +138,14 @@ TVF_HD void triangulate3(const double* Pa, const double* Pb, const double* Pc, c
 // come from the certified ray/plane test (dlt4_depth_signs_ray, ~45 FP64 operations) and only the DLTs it declines
 // (0.1 % of the sweep's, none at n = 10 000) take the accurate route.
 // AFF: m7 comes from dlt_row_minors<true> (view-1 camera K1*[I | 0]).
-#if defined(__CUDACC__) && TVF_CHEIR_NOINLINE
-#define TVF_COLD_DEV __host__ __device__ __noinline__ static
-#else
-#define TVF_COLD_DEV TVF_HD
-#endif
-// the accurate route of one candidate: Householder DLT, the two depth signs (or the NaN flag), optionally the solution
-TVF_COLD_DEV void cheirality_accurate(const double* ra, const double* rb, const double* rc, const double* rd, const double* r3,
+// the accurate route of one candidate: Householder DLT, the two depth signs (or the NaN flag), optionally the solution.
+// Inlined: as an out-of-line function it measured slower (profiles/r02_variants.md).
+TVF_HD void cheirality_accurate(const double* ra, const double* rb, const double* rc, const double* rd, const double* r3,
                                       double tz, int q, int* v, int* nanmask, double* dst) {
     double a[4][4];
 #pragma unroll
     for (int e = 0; e < 4; ++e) { a[0][e] = ra[e]; a[1][e] = rb[e]; a[2][e] = rc[e]; a[3][e] = rd[e]; }
-#if TVF_VOTE_FAST_SIGNS && TVF_VOTE_GRAM_SIGNS
+#if TVF_VOTE_GRAM_SIGNS
     if (dst == nullptr) {
         int sx, sz;
         if (dlt4_depth_signs(a, r3, tz, &sx, &sz)) { v[q] += sx + sz; return; }
@@ -188,20 +168,17 @@ TVF_COLD_DEV void cheirality_accurate(const double* ra, const double* rb, const 
 template <bool AFF = false>
 TVF_HD void cheirality_point(const double* ra, const double* rb, const double* m7, const double* c, double x2, double y2,
                              int* v, int* nanmask, double* Xa, double* Xb) {
-    constexpr int kUnroll = TVF_CHEIR_UNROLL;
-#pragma unroll(kUnroll)
+#pragma unroll 1
     for (int q = 0; q < 2; ++q) {
         double P[12], r3[3], tz;
         candidate_camera(c, q == 0 ? 0 : 3, P, r3, &tz);
         double rc[4], rd[4];
         dlt_rows(P, x2, y2, rc, rd);
         double* dst = (q == 0) ? Xa : Xb;
-#if TVF_VOTE_FAST_SIGNS && TVF_VOTE_RAY_SIGNS
         if (dst == nullptr) {          // only the two depth signs are needed: certified shortcut, else the accurate route
             int sx, sz;
             if (m7 != nullptr && dlt4_depth_signs_ray<AFF>(m7, rc, rd, r3, tz, &sx, &sz)) { v[q] += sx + sz; continue; }
         }
-#endif
         cheirality_accurate(ra, rb, rc, rd, r3, tz, q, v, nanmask, dst);
     }
 }

@@ -29,15 +29,10 @@ struct PointMap {
     }
 };
 
-#ifndef TVF_TAIL_SERIAL_SUM
-#define TVF_TAIL_SERIAL_SUM 1
-#endif
-
 // Sums of the tpp partials of each problem in TWO arrays at once, result at lpt==0.  Up to 32 points per problem the
 // owner thread adds them in index order after ONE barrier (a fixed order, so still bit-reproducible); the log-depth
 // tree of seg_reduce costs a CTA barrier per level, which is what the fused tail was waiting on.
 __device__ __forceinline__ void seg_reduce2(double* ra, double* rb, const PointMap& m) {
-#if TVF_TAIL_SERIAL_SUM
     if (m.tpp <= 32) {
         __syncthreads();
         if (m.lp < m.ppb && m.lpt == 0) {
@@ -48,7 +43,6 @@ __device__ __forceinline__ void seg_reduce2(double* ra, double* rb, const PointM
         __syncthreads();
         return;
     }
-#endif
     int s = 1;
     while (s < m.tpp) s <<= 1;
     for (s >>= 1; s >= 1; s >>= 1) {
@@ -77,9 +71,6 @@ __device__ __forceinline__ const double* calm_of(const PoseTailArgs& a, long lon
 }
 
 // ------------------------------------------------------------------ candidates
-#ifndef TVF_CAND_STORE128
-#define TVF_CAND_STORE128 1
-#endif
 #ifndef TVF_CAND_THREADS
 #define TVF_CAND_THREADS 128
 #endif
@@ -109,24 +100,16 @@ candidates_kernel(int mode, const double* __restrict__ model, PoseTailArgs a) {
         for (int i = 0; i < 18; ++i) F[i] = model[b * 18 + i];
         st = candidates_from_f(F, F + 9, calm, cand);
     }
-#if TVF_CAND_STORE128
     {   // the record is 672 bytes and the arena 256-byte aligned: 42 128-bit stores instead of 84 64-bit ones
         double2* dst = reinterpret_cast<double2*>(a.cand + b * CAND_SIZE);
 #pragma unroll
         for (int i = 0; i < CAND_SIZE / 2; ++i) dst[i] = make_double2(cand[2 * i], cand[2 * i + 1]);
     }
-#else
-#pragma unroll
-    for (int i = 0; i < CAND_SIZE; ++i) a.cand[b * CAND_SIZE + i] = cand[i];
-#endif
     if (a.status != nullptr && st != 0) a.status[b] |= st;
 }
 
 // ------------------------------------------------------------------------ votes
-// the ray test in its form for a view-1 camera K1*[I | 0] (three cofactors are single products)
-#ifndef TVF_RAY_AFF
-#define TVF_RAY_AFF true
-#endif
+// The ray test runs in its form for a view-1 camera K1*[I | 0] (three cofactors are single products).
 #ifndef TVF_VOTES_MINB
 #define TVF_VOTES_MINB 2
 #endif
@@ -148,9 +131,9 @@ votes_kernel(PoseTailArgs a) {
                 const double2 p1 = __ldg(q), p2 = __ldg(q + 1), p3 = __ldg(q + 2);
                 double ra[4], rb[4], m7[7];
                 dlt_rows(P1, p1.x, p1.y, ra, rb);
-                dlt_row_minors<TVF_RAY_AFF>(ra, rb, m7);               // P1 = K1*[I | 0]
-                cheirality_point<TVF_RAY_AFF>(ra, rb, m7, cand, p2.x, p2.y, v2, &n2, nullptr, nullptr);
-                cheirality_point<TVF_RAY_AFF>(ra, rb, m7, cand + CAND_PAIR, p3.x, p3.y, v3, &n3, nullptr, nullptr);
+                dlt_row_minors<true>(ra, rb, m7);               // P1 = K1*[I | 0]
+                cheirality_point<true>(ra, rb, m7, cand, p2.x, p2.y, v2, &n2, nullptr, nullptr);
+                cheirality_point<true>(ra, rb, m7, cand + CAND_PAIR, p3.x, p3.y, v3, &n3, nullptr, nullptr);
             }
             int vote[8], nan2, nan3;
             expand_votes(v2, n2, vote, &nan2);
@@ -371,21 +354,12 @@ final_large_kernel(PoseTailArgs a) {
 // ------------------------------------------------------------- fused tail (7 <= n <= 256)
 // votes + t3 scale + final triangulation/ReprError in one launch: each CTA owns whole problems (one
 // thread per point), so every per-problem reduction is CTA-local and the three phases are separated by
-// __syncthreads only.  The two-view solutions found during the cheirality test are reused for the scale
-// (the selected candidate's DLT is the one R_t_from_TFT.m:69 computes again).  The selected cameras live
-// in shared memory (36 doubles per problem), not in registers, between the phases.
+// __syncthreads only.  The votes come from the certified ray test; the scale phase runs ONE accurate two-view
+// DLT per point, of the selected pose (R_t_from_TFT.m:69).  The selected cameras live in shared memory
+// (36 doubles per problem), not in registers, between the phases.
 
 #ifndef TVF_TAIL_MINB
 #define TVF_TAIL_MINB 2
-#endif
-// 1 = round-2 form: both pair-2 candidates are triangulated accurately during the votes and the selected solution is
-// reused for the scale (3 accurate DLTs per point); 0 = all four votes by the certified ray test, ONE accurate two-view
-// DLT of the selected pose in the scale phase
-#ifndef TVF_TAIL_REUSE_X
-#define TVF_TAIL_REUSE_X 0
-#endif
-#ifndef TVF_TAIL_TMA
-#define TVF_TAIL_TMA 1
 #endif
 // entry i (0..35) of the three cameras P1 | P2 | P3 of a problem for the selected candidates k2, k3
 __device__ __forceinline__ double camera_entry(const double* calm, const double* cand, int k2, int k3, int i) {
@@ -446,7 +420,6 @@ pose_tail_fused_kernel(PoseTailArgs a) {
     const PointMap m(a.n, THREADS);
     const int own = threadIdx.x - m.lpt;        // first thread of this thread's problem
     const double qnan = __longlong_as_double(0x7ff8000000000000LL);
-#if TVF_TAIL_TMA
     // The correspondences and the candidate records of the CTA's NEXT group of problems (two contiguous ranges of global
     // memory: ppb*n*48 and ppb*672 bytes) are brought into the other half of a two-stage shared-memory buffer by two bulk
     // asynchronous copies (TMA engine) that one thread issues at the top of the iteration; every phase reads shared memory.
@@ -467,54 +440,35 @@ pose_tail_fused_kernel(PoseTailArgs a) {
         mbar_init(&tbar[0], 1); mbar_init(&tbar[1], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-#endif
     for (int e = threadIdx.x; e < m.ppb * 4; e += PT_THREADS) sv[e] = 0;
     for (int e = threadIdx.x; e < m.ppb; e += PT_THREADS) snan[e] = 0;
     __syncthreads();
-#if TVF_TAIL_TMA
     if (threadIdx.x == 0 && (long long)blockIdx.x * m.ppb < a.B) issue((long long)blockIdx.x * m.ppb, 0);
     int iter = 0;
-#endif
     for (long long b0 = (long long)blockIdx.x * m.ppb; b0 < a.B; b0 += (long long)gridDim.x * m.ppb) {
         const long long b = b0 + m.lp;
         const bool live = (m.lp < m.ppb && b < a.B);
-#if TVF_TAIL_TMA
         // the other stage was last read before the final barrier of the previous iteration: free to be refilled
         if (threadIdx.x == 0 && b0 + bstep < a.B) issue(b0 + bstep, (iter + 1) & 1);
         const unsigned char* stg = tail_dsm + (size_t)(iter & 1) * stage_bytes;
         mbar_wait(&tbar[iter & 1], (unsigned)(iter >> 1) & 1u);
         ++iter;
         const double* cand = reinterpret_cast<const double*>(stg + pts_bytes) + (live ? m.lp : 0) * CAND_SIZE;
-#else
-        const double* cand = a.cand + (live ? b : 0) * CAND_SIZE;
-#endif
         double* Ps = sP + (live ? m.lp : 0) * 36;
         double p6[6] = {0, 0, 0, 0, 0, 0};
-#if TVF_TAIL_REUSE_X
-        double Xa[4] = {0, 0, 0, 1}, Xb[4] = {0, 0, 0, 1};
-#endif
         // ---- phase 1: cheirality votes (R_t_from_TFT.m:91-104) --------------------------------
         if (live) {
             double P1[12];
             load_K1_as_P1(calm_of(a, b), P1);
-#if TVF_TAIL_TMA
             const double2* q = reinterpret_cast<const double2*>(stg) + (m.lp * a.n + m.lpt) * 3;
             const double2 q1 = q[0], q2 = q[1], q3 = q[2];
-#else
-            const double2* q = reinterpret_cast<const double2*>(a.corresp + (b * a.n + m.lpt) * 6);
-            const double2 q1 = __ldg(q), q2 = __ldg(q + 1), q3 = __ldg(q + 2);
-#endif
             p6[0] = q1.x; p6[1] = q1.y; p6[2] = q2.x; p6[3] = q2.y; p6[4] = q3.x; p6[5] = q3.y;
             double ra[4], rb[4], m7[7];
             dlt_rows(P1, p6[0], p6[1], ra, rb);
-            dlt_row_minors<TVF_RAY_AFF>(ra, rb, m7);                   // P1 = K1*[I | 0]
+            dlt_row_minors<true>(ra, rb, m7);                   // P1 = K1*[I | 0]
             int v2[2] = {0, 0}, v3[2] = {0, 0}, n2 = 0, n3 = 0;
-#if TVF_TAIL_REUSE_X
-            cheirality_point<TVF_RAY_AFF>(ra, rb, m7, cand, p6[2], p6[3], v2, &n2, Xa, Xb);
-#else
-            cheirality_point<TVF_RAY_AFF>(ra, rb, m7, cand, p6[2], p6[3], v2, &n2, nullptr, nullptr);
-#endif
-            cheirality_point<TVF_RAY_AFF>(ra, rb, m7, cand + CAND_PAIR, p6[4], p6[5], v3, &n3, nullptr, nullptr);
+            cheirality_point<true>(ra, rb, m7, cand, p6[2], p6[3], v2, &n2, nullptr, nullptr);
+            cheirality_point<true>(ra, rb, m7, cand + CAND_PAIR, p6[4], p6[5], v3, &n3, nullptr, nullptr);
             int* dst = sv + m.lp * 4;
             if (v2[0]) atomicAdd(dst + 0, v2[0]);
             if (v2[1]) atomicAdd(dst + 1, v2[1]);
@@ -546,23 +500,8 @@ pose_tail_fused_kernel(PoseTailArgs a) {
         // ---- phase 2: t3 scale (R_t_from_TFT.m:68-74) ----------------------------------------------
         double num = 0.0, den = 0.0;
         if (live) {
-#if TVF_TAIL_REUSE_X
-            // X of the selected pair-2 candidate: (R,t)->Xa, (R,-t)->(Xa, -w), (Rp,-t)->(Xb, -w), (Rp,t)->Xb
-            const bool useA = (k2 == 0 || k2 == 1 || k2 == 15);
-            const double w = ((k2 == 1 || k2 == 2) ? -1.0 : 1.0) * (useA ? Xa[3] : Xb[3]);
-            const double iw = 1.0 / w;
-            const double Xc[3] = {(useA ? Xa[0] : Xb[0]) * iw, (useA ? Xa[1] : Xb[1]) * iw, (useA ? Xa[2] : Xb[2]) * iw};
-            double X3[3], c1[3], c2[3];
-            mat3_vec(Ps + 24, Xc, X3);
-            const double p3[3] = {p6[4], p6[5], 1.0};
-            cross3(p3, X3, c1);
-            cross3(p3, Ps + 33, c2);
-            num = c1[0] * c2[0] + c1[1] * c2[1] + c1[2] * c2[2];
-            den = c2[0] * c2[0] + c2[1] * c2[1] + c2[2] * c2[2];
-#else
             // the ONE accurate two-view DLT of the point: cameras 1 and 2 of the selected pose (R_t_from_TFT.m:69)
             scale_point(Ps, Ps + 12, Ps + 24, Ps + 33, p6, &num, &den);
-#endif
         }
         red0[threadIdx.x] = num; red1[threadIdx.x] = den;
         seg_reduce2_split(red0, red1, m);
@@ -882,16 +821,11 @@ static inline unsigned tail_grid(const PoseTailArgs& a, int sm_count) {
 
 // CTA size of the fused tail: 128 threads (four resident CTAs per SM: the five barriers of an iteration wait for four warps
 // instead of eight) unless 256 threads pack whole problems noticeably better (n = 48: 5 x 48 of 256 against 2 x 48 of 128)
-#ifndef TVF_TAIL_SMALL_CTA
-#define TVF_TAIL_SMALL_CTA 1
-#endif
 static inline int fused_tail_threads(int n) {
-#if TVF_TAIL_SMALL_CTA
     if (n <= TVF_TAIL_CTA) {
         const int live_s = (TVF_TAIL_CTA / n) * n * (256 / TVF_TAIL_CTA), live256 = (256 / n) * n;      // live threads per 256
         if (live_s * 16 >= live256 * 15) return TVF_TAIL_CTA;
     }
-#endif
     return 256;
 }
 
@@ -900,14 +834,10 @@ static void launch_fused_t(const PoseTailArgs& a, int sm_count, cudaStream_t str
     const int tpp = (a.n <= THREADS) ? a.n : THREADS;
     const int ppb = THREADS / tpp;
     const unsigned grid = grid_for(a.B, ppb, (long long)sm_count * 16 * (THREADS == PT_THREADS ? TVF_TAIL_MINB : TVF_TAIL_MINB_SMALL));
-#if TVF_TAIL_TMA
     const size_t dyn = 2 * (size_t)ppb * ((size_t)a.n * 48 + CAND_SIZE * 8);      // two stages of points + candidate records
     // (set on every launch: the attribute is per device and per context, a process-wide flag would miss the second GPU)
     cudaFuncSetAttribute(pose_tail_fused_kernel<THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
     pose_tail_fused_kernel<THREADS><<<grid, THREADS, dyn, stream>>>(a);
-#else
-    pose_tail_fused_kernel<THREADS><<<grid, THREADS, 0, stream>>>(a);
-#endif
 }
 
 void launch_pose_tail_fused(const PoseTailArgs& a, int sm_count, cudaStream_t stream) {

@@ -1,6 +1,6 @@
 // tvf_scene_kernels.cu -- batched trials of the synthetic sweep generated on the device (SURVEY.md 8 f1).
 // One thread per trial; the MT19937 state and the 6 x (n+100) coordinate scratch live in local memory.
-#include <cstdlib>
+#include <cstdint>
 
 #include "tvf_kernels.h"
 #include "tvf_scene.cuh"
@@ -372,10 +372,8 @@ sweep_seeds_warp_kernel(long long first_trial, long long B, int n, const double*
 void launch_sweep_trials(long long first_trial, long long B, int n, const double* d_noise_levels, int L, const double* d_P,
                          double hi_x, double hi_y, double* d_out, cudaStream_t stream) {
     if (B <= 0) return;
-    // development switch for A/B timing: TVF_SCENE_THREAD_PER_SEED=1 selects the thread-per-seed / per-trial kernels
-    static const bool per_thread = [] { const char* e = getenv("TVF_SCENE_THREAD_PER_SEED"); return e && e[0] == '1'; }();
     const long long seeds = (first_trial + B - 1) / L - first_trial / L + 1;
-    if (!per_thread && (reinterpret_cast<uintptr_t>(d_out) & 15) == 0) {
+    if ((reinterpret_cast<uintptr_t>(d_out) & 15) == 0) {
         const size_t smem = 288 + SW_WARPS * sw_warp_bytes(n + 100);
         const unsigned grid = (unsigned)((seeds + SW_WARPS - 1) / SW_WARPS);
         if (n + 100 <= 128)
