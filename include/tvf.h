@@ -50,6 +50,21 @@ typedef struct tvf_context* tvf_handle_t;
 #define TVF_ST_BA_NOCONV 32    /* tvf_bundle_adjust: iteration cap reached before the stopping rule held          */
 #define TVF_ST_COV_SINGULAR 64 /* tvf_ba_covariance: reduced camera system or a point block not positive definite:
                                   covariance undefined                                                            */
+#define TVF_ST_TOO_FEW_MATCHES 256 /* a problem of a ragged batch has fewer matches than the method needs (below)   */
+
+/* Ragged batches (the *_ragged entry points): problems with different numbers of matches in one call.
+ *   offsets: int64 [B + 1] in HOST memory, for the host and the _dev forms alike (the library cuts its chunks by them);
+ *            offsets[0] = 0 and the values never decrease, else TVF_ERR_ARG.  Problem b owns matches offsets[b] ..
+ *            offsets[b+1]-1, so n_b = offsets[b+1] - offsets[b]; n_b = 0 is allowed.
+ *   corresp: 6 x offsets[B], the matches of all problems concatenated (48 bytes per match: every problem boundary keeps
+ *            the 16-byte alignment of the base pointer, which the _dev forms check).  Per-match arrays are packed the
+ *            same way: reconst0 / reconst 3 x offsets[B], cov_pts 3 x 3 x offsets[B], inliers offsets[B] bytes.
+ *   Per-problem arrays keep the shapes of the uniform call: calm (shared or batched), poses, seeds, sample, counts,
+ *   status, iter, lo_done, repr_err, sigma2, cov_cam.
+ * A uniform call rejects an n below the method's minimum; a ragged call flags that problem TVF_ST_TOO_FEW_MATCHES
+ * instead, with the outputs its entry point lists, and goes on.  Every other problem's outputs are bit-identical to the
+ * uniform call on that problem alone (B = 1, n = n_b, the same calm, start and seed key), whatever the batch, chunk
+ * (tvf_set_chunk), group-handle shard (contiguous ranges of about equal match counts) or form. */
 
 /* the message linearF.m:36 raises; gateways re-raise it verbatim */
 #define TVF_LINEARF_ERRMSG \
@@ -236,6 +251,16 @@ int tvf_bundle_adjust(tvf_handle_t h, const double* corresp, const double* calm,
 int tvf_bundle_adjust_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                           const double* Rt2_0, const double* Rt3_0, const double* reconst0, double* Rt2, double* Rt3,
                           double* reconst, double* repr_err, int32_t* iter, int32_t* status);
+/* tvf_bundle_adjust over a ragged batch (n replaced by offsets; layout above).  A problem of n_b < 4 matches:
+ * TVF_ST_TOO_FEW_MATCHES, Rt2 / Rt3 = the start copied through, its reconst and repr_err NaN, iter 0.  The _dev form is
+ * asynchronous apart from the copy of each chunk's offsets. */
+int tvf_bundle_adjust_ragged(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, const int64_t* offsets,
+                             int64_t B, const double* Rt2_0, const double* Rt3_0, const double* reconst0, double* Rt2,
+                             double* Rt3, double* reconst, double* repr_err, int32_t* iter, int32_t* status);
+int tvf_bundle_adjust_ragged_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched,
+                                 const int64_t* offsets, int64_t B, const double* Rt2_0, const double* Rt3_0,
+                                 const double* reconst0, double* Rt2, double* Rt3, double* reconst, double* repr_err,
+                                 int32_t* iter, int32_t* status);
 
 /* ---- first-order covariance of the bundle adjustment at a state ------------------------------------------------
  * The uncertainty of tvf_bundle_adjust's result: the inverse of the Gauss-Newton matrix H = J'J of the adjustment's
@@ -266,6 +291,15 @@ int tvf_ba_covariance(tvf_handle_t h, const double* corresp, const double* calm,
 int tvf_ba_covariance_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                           const double* Rt2, const double* Rt3, const double* reconst, double* cov_cam, double* cov_pts,
                           double* sigma2, int32_t* status);
+/* tvf_ba_covariance over a ragged batch (n replaced by offsets; layout above).  A problem of n_b < 4 matches:
+ * TVF_ST_TOO_FEW_MATCHES and every output of it NaN.  The _dev form is asynchronous apart from the copy of each chunk's
+ * offsets. */
+int tvf_ba_covariance_ragged(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, const int64_t* offsets,
+                             int64_t B, const double* Rt2, const double* Rt3, const double* reconst, double* cov_cam,
+                             double* cov_pts, double* sigma2, int32_t* status);
+int tvf_ba_covariance_ragged_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched,
+                                 const int64_t* offsets, int64_t B, const double* Rt2, const double* Rt3,
+                                 const double* reconst, double* cov_cam, double* cov_pts, double* sigma2, int32_t* status);
 
 /* ---- robust pose from raw matches: consensus and RANSAC ----------------------------------------------------------
  * Inlier test of one match x = (x1 y1 x2 y2 x3 y3) under the cameras K1[I|0], K2[R2|t2], K3[R3|t3]: triangulate it as
@@ -278,6 +312,10 @@ int tvf_ba_covariance_dev(tvf_handle_t h, const double* corresp, const double* c
  * must be finite and > 0.  Chunks and shards like tvf_pose; returns 0 or an error. */
 int tvf_consensus(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                   const double* Rt2, const double* Rt3, double threshold, uint8_t* inliers, int32_t* n_inliers);
+/* tvf_consensus over a ragged batch (n replaced by offsets; layout above); n_b = 0 gives the count 0. */
+int tvf_consensus_ragged(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, const int64_t* offsets,
+                         int64_t B, const double* Rt2, const double* Rt3, double threshold, uint8_t* inliers,
+                         int32_t* n_inliers);
 
 #define TVF_ST_RANSAC_FAILED 128 /* tvf_ransac_pose: every hypothesis of the problem was flagged: no pose           */
 
@@ -307,6 +345,16 @@ int tvf_ransac_pose(tvf_handle_t h, int method, const double* corresp, const dou
 int tvf_ransac_pose_dev(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched, int n,
                         int64_t B, int hypotheses, double threshold, const uint64_t* seeds, double* Rt2, double* Rt3,
                         uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* status);
+/* tvf_ransac_pose over a ragged batch (n replaced by offsets; layout above), `hypotheses` per problem; the sampler's rule
+ * uses n_b in place of n.  A problem of n_b < s matches: TVF_ST_TOO_FEW_MATCHES, Rt2 / Rt3 NaN, inliers 0, n_inliers 0,
+ * sample -1.  The _dev form synchronises once per chunk, as tvf_ransac_pose_dev does. */
+int tvf_ransac_pose_ragged(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched,
+                           const int64_t* offsets, int64_t B, int hypotheses, double threshold, const uint64_t* seeds,
+                           double* Rt2, double* Rt3, uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* status);
+int tvf_ransac_pose_ragged_dev(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched,
+                               const int64_t* offsets, int64_t B, int hypotheses, double threshold, const uint64_t* seeds,
+                               double* Rt2, double* Rt3, uint8_t* inliers, int32_t* n_inliers, int32_t* sample,
+                               int32_t* status);
 
 /* RANSAC pose whose hypotheses and result are bundle-adjusted, with local optimisation (LO).  Arguments, checks and
  * errors as tvf_ransac_pose, plus lo_rounds (0 .. 32, else TVF_ERR_ARG) and lo_done (B, may be NULL): the number of
@@ -334,6 +382,16 @@ int tvf_ransac_pose_refined_dev(tvf_handle_t h, int method, const double* corres
                                 int n, int64_t B, int hypotheses, double threshold, const uint64_t* seeds, int lo_rounds,
                                 double* Rt2, double* Rt3, uint8_t* inliers, int32_t* n_inliers, int32_t* sample,
                                 int32_t* lo_done, int32_t* status);
+/* tvf_ransac_pose_refined over a ragged batch, as tvf_ransac_pose_ragged; a problem of n_b < s matches also gets
+ * lo_done 0.  The _dev form synchronises as tvf_ransac_pose_refined_dev does. */
+int tvf_ransac_pose_refined_ragged(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched,
+                                   const int64_t* offsets, int64_t B, int hypotheses, double threshold, const uint64_t* seeds,
+                                   int lo_rounds, double* Rt2, double* Rt3, uint8_t* inliers, int32_t* n_inliers,
+                                   int32_t* sample, int32_t* lo_done, int32_t* status);
+int tvf_ransac_pose_refined_ragged_dev(tvf_handle_t h, int method, const double* corresp, const double* calm,
+                                       int calm_batched, const int64_t* offsets, int64_t B, int hypotheses, double threshold,
+                                       const uint64_t* seeds, int lo_rounds, double* Rt2, double* Rt3, uint8_t* inliers,
+                                       int32_t* n_inliers, int32_t* sample, int32_t* lo_done, int32_t* status);
 
 /* ---- inputs of the measured configurations, generated where they are consumed ------------------------
  * Trials [first_trial, first_trial+B) of experiments.m's sweep: trial j uses noise_levels[j mod L] and

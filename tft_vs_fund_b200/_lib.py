@@ -28,6 +28,7 @@ ST_NONFINITE = 16
 ST_BA_NOCONV = 32
 ST_COV_SINGULAR = 64
 ST_RANSAC_FAILED = 128
+ST_TOO_FEW_MATCHES = 256
 
 LINEARF_ERRMSG = ("At least 8 correspondences are necessary to compute the "
                   "fundamental matrix linearly\\n")
@@ -104,6 +105,19 @@ SIGNATURES = {
                                      _S, _S, _S, _S]),
     "tvf_ransac_pose_refined_dev": (_I, [_H, _I, C.c_void_p, C.c_void_p, _I, _I, _L, _I, C.c_double, C.c_void_p, _I]
                                     + [C.c_void_p] * 7),
+    "tvf_consensus_ragged": (_I, [_H, _D, _D, _I, C.c_void_p, _L, _D, _D, C.c_double, C.c_void_p, _S]),
+    "tvf_bundle_adjust_ragged": (_I, [_H, _D, _D, _I, C.c_void_p, _L, _D, _D, _D, _D, _D, _D, _D, _S, _S]),
+    "tvf_bundle_adjust_ragged_dev": (_I, [_H, C.c_void_p, C.c_void_p, _I, C.c_void_p, _L] + [C.c_void_p] * 9),
+    "tvf_ba_covariance_ragged": (_I, [_H, _D, _D, _I, C.c_void_p, _L, _D, _D, _D, _D, _D, _D, _S]),
+    "tvf_ba_covariance_ragged_dev": (_I, [_H, C.c_void_p, C.c_void_p, _I, C.c_void_p, _L] + [C.c_void_p] * 7),
+    "tvf_ransac_pose_ragged": (_I, [_H, _I, _D, _D, _I, C.c_void_p, _L, _I, C.c_double, C.c_void_p, _D, _D, C.c_void_p,
+                                    _S, _S, _S]),
+    "tvf_ransac_pose_ragged_dev": (_I, [_H, _I, C.c_void_p, C.c_void_p, _I, C.c_void_p, _L, _I, C.c_double]
+                                   + [C.c_void_p] * 7),
+    "tvf_ransac_pose_refined_ragged": (_I, [_H, _I, _D, _D, _I, C.c_void_p, _L, _I, C.c_double, C.c_void_p, _I, _D, _D,
+                                            C.c_void_p, _S, _S, _S, _S]),
+    "tvf_ransac_pose_refined_ragged_dev": (_I, [_H, _I, C.c_void_p, C.c_void_p, _I, C.c_void_p, _L, _I, C.c_double,
+                                                C.c_void_p, _I] + [C.c_void_p] * 7),
     "tvf_launch_count": (_L, [_H]),
     "tvf_profile_enable": (_I, [_H, _I]),
     "tvf_profile_reset": (_I, [_H]),

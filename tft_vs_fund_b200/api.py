@@ -6,7 +6,11 @@ tests read like calls of the reference.  Arrays use the MATLAB shapes:
 ``Corresp`` 6xN, ``CalM`` 9x3, poses 3x4, ``T`` 3x3x3 with ``T[:, :, i]`` the
 i-th slice, ``Reconst`` 3xN.  Every function also takes a leading batch axis
 (``Corresp`` (B,6,N), ``CalM`` (9,3) or (B,9,3)) and then returns batched
-arrays ((B,3,4), (B,3,N), (B,3,3,3), ...).
+arrays ((B,3,4), (B,3,N), (B,3,3,3), ...).  ransac_pose, bundle_adjust,
+ba_covariance and consensus also take a list of B matrices ``Corresp`` 6xN_b
+with their own N_b (a ragged batch, include/tvf.h); per-problem outputs then
+come back stacked (B,...) and per-match outputs (inliers, Reconst, cov_pts) as
+lists.
 
 All arithmetic happens in libtvf.so on the GPU; this module only reshapes
 between NumPy (row-major) and the library's MATLAB column-major layout.
@@ -49,6 +53,47 @@ def _from_cm(buf, B, dims, batched):
     nd = len(dims)
     a = buf.reshape((B,) + tuple(reversed(dims))).transpose((0,) + tuple(range(nd, 0, -1)))
     return a if batched else a[0]
+
+
+def _check_offsets(offsets, B):
+    """Offsets of a ragged batch of B problems as int64 (B+1,): start at 0, never decrease."""
+    o = np.ascontiguousarray(offsets, dtype=np.int64)
+    if o.shape != (B + 1,):
+        raise ValueError("offsets must have B + 1 = %d entries, got shape %s" % (B + 1, o.shape))
+    if o[0] != 0:
+        raise ValueError("offsets[0] must be 0")
+    if np.any(np.diff(o) < 0):
+        raise ValueError("offsets must not decrease")
+    return o
+
+
+def _pack(arrays, rows):
+    """list of B matrices rows x N_b -> (the ragged layout of include/tvf.h: buffer (N, rows), matches concatenated,
+    column-major per problem; offsets int64 (B+1,))."""
+    mats = [np.asarray(a, dtype=np.float64) for a in arrays]
+    for a in mats:
+        if a.ndim != 2 or a.shape[0] != rows:
+            raise ValueError("expected a list of %d x N_b arrays, got shape %s" % (rows, a.shape))
+    offsets = np.concatenate([[0], np.cumsum([a.shape[1] for a in mats], dtype=np.int64)]).astype(np.int64)
+    buf = np.concatenate([a.T for a in mats]) if mats else np.zeros((0, rows))
+    return np.ascontiguousarray(buf), offsets
+
+
+def _unpack(buf, offsets, dims):
+    """the inverse of _pack for per-match outputs of `dims` per match (e.g. (3,) for Reconst, (3, 3) for cov_pts; () for a
+    flag): list of (dims..., N_b) arrays."""
+    offsets = _check_offsets(offsets, len(offsets) - 1)
+    k = int(np.prod(dims, dtype=np.int64))
+    buf = np.asarray(buf).reshape(-1)
+    if buf.size != offsets[-1] * k:
+        raise ValueError("buffer holds %d values, offsets describe %d" % (buf.size, offsets[-1] * k))
+    return [_from_cm(buf[offsets[b] * k:offsets[b + 1] * k], 1, tuple(dims) + (int(offsets[b + 1] - offsets[b]),), False)
+            for b in range(len(offsets) - 1)]
+
+
+def _ragged(Corresp):
+    """Corresp is a ragged batch: a list (or tuple) of 6 x N_b matrices."""
+    return isinstance(Corresp, (list, tuple))
 
 
 def _calm(CalM, B):
@@ -304,7 +349,11 @@ def bundle_adjust(Corresp, CalM, R_t_2, R_t_3, Reconst=None, device=None):
     over R2, t2 (|t2| = 1), R3, t3 and the points, camera 1 fixed at K1[I|0], from the start (R_t_2, R_t_3, Reconst).
     Reconst None: the start points are triangulated from the start poses.  Not the reference's BundleAdjustment.m (which
     normalises the image data first; DESIGN.md section 8).  Returns (R_t_2, R_t_3, Reconst, iter) with .repr_err (the
-    result's ReprError) and .status (TVF_ST_* bits: NONFINITE, BA_NOCONV)."""
+    result's ReprError) and .status (TVF_ST_* bits: NONFINITE, BA_NOCONV).
+    Corresp a list of 6xN_b (a ragged batch): R_t_2, R_t_3 (B,3,4), Reconst None or a list of 3xN_b; returns stacked
+    poses, Reconst as a list and (B,) iter; a problem of N_b < 4 gets TVF_ST_TOO_FEW_MATCHES (start poses, NaN points)."""
+    if _ragged(Corresp):
+        return _bundle_adjust_ragged(Corresp, CalM, R_t_2, R_t_3, Reconst, device)
     c, batched, B = _cm(Corresp, 2)
     if c.shape[2] != 6:
         raise ValueError("Corresp must be 6xN")
@@ -331,6 +380,27 @@ def bundle_adjust(Corresp, CalM, R_t_2, R_t_3, Reconst=None, device=None):
     return out
 
 
+def _bundle_adjust_ragged(Corresp, CalM, R_t_2, R_t_3, Reconst, device):
+    c, offs = _pack(Corresp, 6)
+    B = len(Corresp)
+    calm, cb = _calm(CalM, B)
+    r2, r3 = _pose_pair(R_t_2, R_t_3, B, True)
+    x0 = None
+    if Reconst is not None:
+        x0, ox = _pack(Reconst, 3)
+        if not np.array_equal(ox, offs):
+            raise ValueError("Reconst must be a list of 3xN_b with the N_b of Corresp")
+    h = _lib.handle(device)
+    Rt2 = np.empty((B, 12)); Rt3 = np.empty((B, 12)); Rec = np.empty(3 * offs[-1]); rep = np.empty(B)
+    its = np.zeros(B, dtype=np.int32); st = np.zeros(B, dtype=np.int32)
+    h.call("tvf_bundle_adjust_ragged", _p(c), _p(calm), cb, _vp(offs), B, _p(r2), _p(r3), _p(x0), _p(Rt2), _p(Rt3), _p(Rec),
+           _p(rep), its.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
+    out = BundleAdjustResult((_from_cm(Rt2, B, (3, 4), True), _from_cm(Rt3, B, (3, 4), True), _unpack(Rec, offs, (3,)), its))
+    out.repr_err = rep
+    out.status = st
+    return out
+
+
 class CovarianceResult(tuple):
     """(cov_cam, sigma2) of ba_covariance, plus .cov_pts (None unless points=True) and .status."""
     cov_pts = None
@@ -345,7 +415,10 @@ def ba_covariance(Corresp, CalM, R_t_2, R_t_3, Reconst, points=False, device=Non
     noise variance sum r^2 / (3N - 11), or by any other sigma^2.  points=True also fills .cov_pts, 3x3xN (the marginal
     covariance of each point in the gauge-normalised frame, unit noise).  .status: TVF_ST_* bits (NONFINITE,
     COV_SINGULAR); a flagged problem's outputs are NaN.  Batched like bundle_adjust: cov_cam (B,12,12), sigma2 (B,),
-    cov_pts (B,3,3,N)."""
+    cov_pts (B,3,3,N).  Corresp a list of 6xN_b (a ragged batch, Reconst then a list of 3xN_b): .cov_pts is a list of
+    3x3xN_b; a problem of N_b < 4 gets TVF_ST_TOO_FEW_MATCHES and NaN outputs."""
+    if _ragged(Corresp):
+        return _ba_covariance_ragged(Corresp, CalM, R_t_2, R_t_3, Reconst, points, device)
     c, batched, B = _cm(Corresp, 2)
     if c.shape[2] != 6:
         raise ValueError("Corresp must be 6xN")
@@ -370,6 +443,26 @@ def ba_covariance(Corresp, CalM, R_t_2, R_t_3, Reconst, points=False, device=Non
     return out
 
 
+def _ba_covariance_ragged(Corresp, CalM, R_t_2, R_t_3, Reconst, points, device):
+    c, offs = _pack(Corresp, 6)
+    B = len(Corresp)
+    calm, cb = _calm(CalM, B)
+    r2, r3 = _pose_pair(R_t_2, R_t_3, B, True)
+    x, ox = _pack(Reconst, 3)
+    if not np.array_equal(ox, offs):
+        raise ValueError("Reconst must be a list of 3xN_b with the N_b of Corresp")
+    h = _lib.handle(device)
+    cc = np.empty((B, 144)); s2 = np.empty(B); st = np.zeros(B, dtype=np.int32)
+    cp = np.empty(9 * offs[-1]) if points else None
+    h.call("tvf_ba_covariance_ragged", _p(c), _p(calm), cb, _vp(offs), B, _p(r2), _p(r3), _p(x), _p(cc), _p(cp), _p(s2),
+           st.ctypes.data_as(_ip))
+    out = CovarianceResult((_from_cm(cc, B, (12, 12), True), s2))
+    if points:
+        out.cov_pts = _unpack(cp, offs, (3, 3))
+    out.status = st
+    return out
+
+
 def _pose_pair(R_t_2, R_t_3, B, batched):
     r2, _, _ = _cm(np.broadcast_to(R_t_2, (B, 3, 4)) if batched else R_t_2, 2)
     r3, _, _ = _cm(np.broadcast_to(R_t_3, (B, 3, 4)) if batched else R_t_3, 2)
@@ -382,7 +475,17 @@ def consensus(Corresp, CalM, R_t_2, R_t_3, threshold=1.0, device=None):
     """Which matches of Corresp (6xN) the pose (R_t_2, R_t_3) explains (tvf_consensus, include/tvf.h): each match is
     triangulated with K1[I|0], K2*R_t_2, K3*R_t_3, re-projected, and kept iff its six residuals are finite and
     <= threshold pixels -- the inlier rule of experiments_real.m:94-98 (epfl.inlier_filter), except that a NaN
-    residual makes the match an outlier.  Returns (mask, count): bool (N) and int, or (B,N) and (B,) when batched."""
+    residual makes the match an outlier.  Returns (mask, count): bool (N) and int, or (B,N) and (B,) when batched, or a
+    list of bool (N_b) and (B,) for a list of 6xN_b (a ragged batch)."""
+    if _ragged(Corresp):
+        c, offs = _pack(Corresp, 6)
+        B = len(Corresp)
+        calm, cb = _calm(CalM, B)
+        r2, r3 = _pose_pair(R_t_2, R_t_3, B, True)
+        mask = np.zeros(offs[-1], dtype=np.uint8); cnt = np.zeros(B, dtype=np.int32)
+        _lib.handle(device).call("tvf_consensus_ragged", _p(c), _p(calm), cb, _vp(offs), B, _p(r2), _p(r3), float(threshold),
+                                 _vp(mask), cnt.ctypes.data_as(_ip))
+        return [m.astype(bool) for m in _unpack(mask, offs, ())], cnt
     c, batched, B = _cm(Corresp, 2)
     if c.shape[2] != 6:
         raise ValueError("Corresp must be 6xN")
@@ -415,14 +518,21 @@ def ransac_pose(Corresp, CalM, method=1, hypotheses=1024, threshold=1.0, seed=0,
     .status; batched inputs give (B,3,4), (B,3,4), (B,N), (B,), (B,s).
     refine=True (tvf_ransac_pose_refined): each hypothesis is bundle-adjusted on its own sample before it is scored,
     and the best one is improved by up to `lo_rounds` (0 .. 32) rounds of bundle adjustment on its consensus, each kept
-    only if it explains strictly more matches; the result also has .lo_done, the number of rounds kept."""
+    only if it explains strictly more matches; the result also has .lo_done, the number of rounds kept.
+    Corresp a list of 6xN_b (a ragged batch): every output is batched, inliers a list of bool (N_b); a problem with
+    N_b < s gets TVF_ST_TOO_FEW_MATCHES (NaN poses, no inliers, sample -1) instead of an error."""
     if method not in RANSAC_SAMPLE_SIZE:
         raise ValueError("ransac_pose: method must be 1 (linear TFT) or 7 (linear F)")
     s = RANSAC_SAMPLE_SIZE[method]
-    c, batched, B = _cm(Corresp, 2)
-    if c.shape[2] != 6:
-        raise ValueError("Corresp must be 6xN")
-    n = c.shape[1]
+    ragged = _ragged(Corresp)
+    if ragged:
+        c, offs = _pack(Corresp, 6)
+        batched, B, n = True, len(Corresp), 0
+    else:
+        c, batched, B = _cm(Corresp, 2)
+        if c.shape[2] != 6:
+            raise ValueError("Corresp must be 6xN")
+        n = c.shape[1]
     calm, cb = _calm(CalM, B)
     if np.ndim(seed) == 0:
         seeds = (np.uint64(int(seed) % 2 ** 64) + np.arange(B, dtype=np.uint64)).astype(np.uint64)
@@ -431,17 +541,21 @@ def ransac_pose(Corresp, CalM, method=1, hypotheses=1024, threshold=1.0, seed=0,
         if seeds.shape != (B,):
             raise ValueError("seed must be an int or an array of B keys")
     h = _lib.handle(device)
-    Rt2 = np.empty((B, 12)); Rt3 = np.empty((B, 12)); mask = np.zeros((B, n), dtype=np.uint8)
+    Rt2 = np.empty((B, 12)); Rt3 = np.empty((B, 12)); mask = np.zeros(offs[-1] if ragged else (B, n), dtype=np.uint8)
     cnt = np.zeros(B, dtype=np.int32); smp = np.zeros((B, s), dtype=np.int32); st = np.zeros(B, dtype=np.int32)
+    # the ragged entry points take the offsets where the uniform ones take n
+    name, size = ("tvf_ransac_pose_refined" if refine else "tvf_ransac_pose"), n
+    if ragged:
+        name, size = name + "_ragged", _vp(offs)
     if refine:
         lo = np.zeros(B, dtype=np.int32)
-        h.call("tvf_ransac_pose_refined", int(method), _p(c), _p(calm), cb, n, B, int(hypotheses), float(threshold),
+        h.call(name, int(method), _p(c), _p(calm), cb, size, B, int(hypotheses), float(threshold),
                _vp(seeds), int(lo_rounds), _p(Rt2), _p(Rt3), _vp(mask), cnt.ctypes.data_as(_ip), smp.ctypes.data_as(_ip),
                lo.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
     else:
-        h.call("tvf_ransac_pose", int(method), _p(c), _p(calm), cb, n, B, int(hypotheses), float(threshold), _vp(seeds),
+        h.call(name, int(method), _p(c), _p(calm), cb, size, B, int(hypotheses), float(threshold), _vp(seeds),
                _p(Rt2), _p(Rt3), _vp(mask), cnt.ctypes.data_as(_ip), smp.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
-    mask = mask.astype(bool)
+    mask = [m.astype(bool) for m in _unpack(mask, offs, ())] if ragged else mask.astype(bool)
     out = RansacResult((_from_cm(Rt2, B, (3, 4), batched), _from_cm(Rt3, B, (3, 4), batched),
                         mask if batched else mask[0], cnt if batched else int(cnt[0]), smp if batched else smp[0]))
     out.status = st if batched else int(st[0])

@@ -344,25 +344,101 @@ inline size_t align256(size_t bytes) { return (bytes + 255) & ~size_t(255); }
 // ---- host-pointer calls -------------------------------------------------------------------------------------------
 // A host-pointer entry point is a Call: its caller arrays, the device buffers of the chunk in flight (`d`), and
 //   size_t budget(bool host_io)          per-problem bytes of a chunk, for pick_chunk
-//   size_t carve(char* base, int64_t C)  lays `d` out in a slot arena (base = nullptr: size only)
+//   size_t budget_match(bool host_io)    per-match bytes of a chunk of a ragged call, for its match budget
+//   size_t carve(char* base, int64_t C, int64_t M)   lays `d` out in a slot arena for C problems and, ragged, M matches
+//                                        (base = nullptr: size only)
 //   void arrays(F f)                     f(caller pointer, Arr) for every caller array: the one place their layout is written
 //   int launch(h, stream, Bc)            the kernels of one chunk on `d`
 //   int check(h, B), int32_t*& status()  argument checks; the per-problem status array
+//   Ragged rg                            the offsets of a ragged call (uniform: none)
+
+// A ragged call (include/tvf.h: problem b owns matches offs[b] .. offs[b+1]-1): its offsets in host memory from the
+// call's first problem on, the chunk's offsets rebased to 0 on the device (carved with the chunk's buffers) and the
+// chunk's match count
+struct Ragged {
+    const int64_t* offs = nullptr;     // null: a uniform call
+    long long* d_offs = nullptr;
+    int64_t m = 0;
+};
+
+int check_offsets(tvf_handle_t h, const char* what, const int64_t* offs, int64_t B) {
+    if (B < 0) return fail(h, TVF_ERR_ARG, std::string(what) + ": B >= 0");
+    if (!offs) return fail(h, TVF_ERR_ARG, std::string(what) + ": offsets must not be NULL");
+    if (offs[0] != 0) return fail(h, TVF_ERR_ARG, std::string(what) + ": offsets[0] must be 0");
+    for (int64_t b = 0; b < B; ++b) {
+        const int64_t nb = offs[b + 1] - offs[b];
+        if (nb < 0) return fail(h, TVF_ERR_ARG, std::string(what) + ": offsets must not decrease");
+        if (nb > 0x7fffffffLL) return fail(h, TVF_ERR_ARG, std::string(what) + ": a problem has more than 2^31 - 1 matches");
+    }
+    return TVF_OK;
+}
 
 // One caller array beside its device buffer in the chunk's arena
 struct Arr {
     bool out;         // false: host -> device before the chunk's kernels; true: device -> host after them
-    size_t per;       // bytes per problem; 0: one copy of `pitch` bytes that every problem shares (a 9 x 3 calm)
+    size_t per;       // bytes per problem (per match when `match`); 0: one copy of `pitch` bytes that every problem
+                      // shares (a 9 x 3 calm)
     const void* dev;  // the chunk's device buffer
     size_t pitch;     // bytes per problem in `dev` (F21 / F31: 72 bytes out of each 144-byte F record)
-    size_t bytes(int64_t k) const { return per ? (size_t)k * per : pitch; }   // of k problems
+    bool match = false;   // a per-match array of a ragged call (corresp, reconst, inliers, ...)
     static Arr input(size_t per, const void* dev, bool shared = false) { return Arr{false, shared ? 0 : per, dev, per}; }
     static Arr output(size_t per, const void* dev, size_t pitch = 0) { return Arr{true, per, dev, pitch ? pitch : per}; }
+    // `bytes` per match: per problem n x bytes (uniform), or per match (ragged)
+    static Arr points(const Ragged& rg, int n, size_t bytes, const void* dev, bool out) {
+        Arr a = out ? output(rg.offs ? bytes : n * bytes, dev) : input(rg.offs ? bytes : n * bytes, dev);
+        a.match = rg.offs != nullptr;
+        return a;
+    }
+    // byte offset of problem b in the caller's array (offs: the call's offsets, for a per-match array)
+    size_t at(const int64_t* offs, int64_t b) const { return (size_t)(match ? offs[b] - offs[0] : b) * per; }
+    // bytes of problems [lo, hi)
+    size_t bytes(const int64_t* offs, int64_t lo, int64_t hi) const { return per ? at(offs, hi) - at(offs, lo) : pitch; }
 };
 
 // the caller arrays of `c` from problem `lo` on
 template <class Call> void shift(Call& c, int64_t lo) {
-    c.arrays([&](auto& p, const Arr& a) { if (p) p += lo * (int64_t)(a.per / sizeof(*p)); });
+    c.arrays([&](auto& p, const Arr& a) { if (p) p += (int64_t)(a.at(c.rg.offs, lo) / sizeof(*p)); });
+    if (c.rg.offs) c.rg.offs += lo;
+}
+
+// The chunks of a call over B problems, as their ends.  Uniform: every C problems, C = pick_chunk.  Ragged: contiguous
+// ranges cut greedily at C problems or at the match budget M (per-match bytes against the arena budget, the same budget
+// pick_chunk uses), whichever comes first; a problem larger than M gets a chunk of its own.  *C, *M: the most problems
+// and matches of one chunk, the shape its buffers are carved for.
+template <class Call> std::vector<int64_t> plan_chunks(tvf_handle_t h, const Call& c, int64_t B, bool host_io, int64_t* C,
+                                                       int64_t* M) {
+    *C = pick_chunk(h, B, host_io, c.budget(host_io));
+    *M = 0;
+    std::vector<int64_t> ends;
+    const int64_t* o = c.rg.offs;
+    if (!o) {
+        for (int64_t e = *C; e < B + *C; e += *C) ends.push_back(e < B ? e : B);
+        return ends;
+    }
+    const size_t pm = c.budget_match(host_io);
+    const int64_t cap = pm ? (int64_t)((host_io ? ARENA_BUDGET : 8 * ARENA_BUDGET) / pm) : INT64_MAX;
+    int64_t most = 0;
+    for (int64_t lo = 0; lo < B;) {
+        int64_t hi = lo + 1;
+        while (hi < B && hi - lo < *C && o[hi + 1] - o[lo] <= cap) ++hi;
+        ends.push_back(hi);
+        *M = std::max(*M, o[hi] - o[lo]);
+        most = std::max(most, hi - lo);
+        lo = hi;
+    }
+    *C = most;
+    return ends;
+}
+
+// A ragged call's chunk [lo, hi): its offsets rebased to 0 to the chunk's device copy (ordered on `st` before the
+// chunk's kernels; pageable, so the runtime stages them before it returns) and rg.m.  Uniform: nothing.
+template <class Call> int put_offsets(tvf_handle_t h, Call& c, int64_t lo, int64_t hi, cudaStream_t st) {
+    if (!c.rg.offs) return TVF_OK;
+    std::vector<long long> v((size_t)(hi - lo + 1));
+    for (int64_t b = lo; b <= hi; ++b) v[(size_t)(b - lo)] = c.rg.offs[b] - c.rg.offs[lo];
+    c.rg.m = v.back();
+    TVF_CK(cudaMemcpyAsync(c.rg.d_offs, v.data(), v.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+    return TVF_OK;
 }
 
 // One host-pointer call on one device.  Chunk i runs on slot i mod NSLOT (stream + arena), so its H2D, kernels and D2H
@@ -370,8 +446,12 @@ template <class Call> void shift(Call& c, int64_t lo) {
 template <class Call> int host_pipeline(tvf_handle_t h, Call c, int64_t B) {
     if (B == 0) return TVF_OK;
     TVF_CK(cudaSetDevice(h->device));
-    const int64_t C = pick_chunk(h, B, true, c.budget(true));
-    const size_t need = c.carve(nullptr, C);
+    int64_t C, M;
+    const std::vector<int64_t> ends = plan_chunks(h, c, B, true, &C, &M);
+    const size_t need = c.carve(nullptr, C, M);
+    const int64_t* offs = c.rg.offs;
+    // the staging buffer of one chunk holds C problems and M matches of each array
+    auto cap = [&](const Arr& a) { return a.per ? (size_t)(a.match ? M : C) * a.per : a.pitch; };
     // Pageable caller memory (what a MEX gateway receives): cudaMemcpyAsync would fall back to synchronous copies through
     // the runtime's own bounce buffer and serialise the pipeline (measured 6.6e6 solves/s against 4.5e7 with pinned
     // buffers).  Instead every chunk goes through a pinned per-slot staging buffer that a few host threads fill and drain.
@@ -379,13 +459,13 @@ template <class Call> int host_pipeline(tvf_handle_t h, Call c, int64_t B) {
     size_t moved = 0;
     bool pageable = false;
     c.arrays([&](const void* p, const Arr& a) {
-        if (p && a.per) { moved += a.bytes(B); pageable = pageable || is_pageable(p); }
+        if (p && a.per) { moved += a.bytes(offs, 0, B); pageable = pageable || is_pageable(p); }
     });
     const bool staged = pageable && !h->host_register && moved >= (size_t(4) << 20);
     std::vector<int32_t> st_tmp;
     if (!c.status()) { st_tmp.resize((size_t)B); c.status() = st_tmp.data(); }
     size_t stage_bytes = 0;
-    c.arrays([&](const void* p, const Arr& a) { if (p && a.per) stage_bytes += align256(a.bytes(C)); });
+    c.arrays([&](const void* p, const Arr& a) { if (p && a.per) stage_bytes += align256(cap(a)); });
     int nthreads = h->host_threads;
     if (nthreads <= 0) {
         const int hw = (int)std::thread::hardware_concurrency();
@@ -407,14 +487,14 @@ template <class Call> int host_pipeline(tvf_handle_t h, Call c, int64_t B) {
     // measured SLOWER (4.31e7 vs 4.56e7 solves/s end to end at 1 M problems, profiles/r01_variants.md).
     int64_t done = 0; int ci = 0;
     int rc = TVF_OK;
-    while (done < B) {
-        const int64_t rem = B - done;
-        const int64_t Bc = (rem < C) ? rem : C;
+    for (const int64_t end : ends) {
+        const int64_t Bc = end - done;
         const int si = ci % NSLOT;
         Slot& s = h->slot[si];
         TVF_CK(cudaStreamSynchronize(s.stream));        // slot reuse: its previous chunk (incl. D2H) is finished
         rc = ensure_arena(h, s, need); if (rc) return rc;
-        c.carve(s.arena, C);
+        c.carve(s.arena, C, M);
+        rc = put_offsets(h, c, done, end, s.stream); if (rc) return rc;
         char* stage = nullptr;
         if (staged) {
             drain(si);                                   // the slot's previous outputs leave the staging buffer first
@@ -425,25 +505,25 @@ template <class Call> int host_pipeline(tvf_handle_t h, Call c, int64_t B) {
         cudaError_t e = cudaSuccess;
         c.arrays([&](const void* p, const Arr& a) {
             if (!p || a.out || e != cudaSuccess) return;
-            const char* src = (const char*)p + (size_t)done * a.per;
+            const char* src = (const char*)p + a.at(offs, done);
             if (staged && a.per) {
-                par_memcpy(stage, src, a.bytes(Bc), nthreads);
+                par_memcpy(stage, src, a.bytes(offs, done, end), nthreads);
                 src = stage;
-                stage += align256(a.bytes(C));
+                stage += align256(cap(a));
             }
-            e = cudaMemcpyAsync(const_cast<void*>(a.dev), src, a.bytes(Bc), cudaMemcpyHostToDevice, s.stream);
+            e = cudaMemcpyAsync(const_cast<void*>(a.dev), src, a.bytes(offs, done, end), cudaMemcpyHostToDevice, s.stream);
         });
         if (e != cudaSuccess) return fail(h, TVF_ERR_CUDA, std::string("cudaMemcpyAsync(host to device): ") + cudaGetErrorString(e));
         rc = c.launch(h, s.stream, Bc); if (rc) return rc;
         c.arrays([&](const void* p, const Arr& a) {
             if (!p || !a.out || e != cudaSuccess) return;
-            char* dst = (char*)const_cast<void*>(p) + (size_t)done * a.per;
+            char* dst = (char*)const_cast<void*>(p) + a.at(offs, done);
             if (staged) {
-                pending[si].push_back(Drain{dst, stage, a.bytes(Bc)});
+                pending[si].push_back(Drain{dst, stage, a.bytes(offs, done, end)});
                 dst = stage;
-                stage += align256(a.bytes(C));
+                stage += align256(cap(a));
             }
-            e = (a.pitch == a.per) ? cudaMemcpyAsync(dst, a.dev, a.bytes(Bc), cudaMemcpyDeviceToHost, s.stream)
+            e = (a.pitch == a.per) ? cudaMemcpyAsync(dst, a.dev, a.bytes(offs, done, end), cudaMemcpyDeviceToHost, s.stream)
                                    : cudaMemcpy2DAsync(dst, a.per, a.dev, a.pitch, a.per, (size_t)Bc, cudaMemcpyDeviceToHost, s.stream);
         });
         if (e != cudaSuccess) return fail(h, TVF_ERR_CUDA, std::string("cudaMemcpyAsync(device to host): ") + cudaGetErrorString(e));
@@ -464,6 +544,18 @@ inline void shard_of(int64_t B, int g, int G, int64_t* lo, int64_t* hi) {
     *hi = *lo + base + (g < rem ? 1 : 0);
 }
 
+// the same for a ragged call (offs: B + 1 offsets from 0): member g starts at the first problem whose matches start at or
+// after g / G of all matches, so the ranges hold about equal match counts
+inline void shard_of_matches(const int64_t* offs, int64_t B, int g, int G, int64_t* lo, int64_t* hi) {
+    auto start = [&](int k) -> int64_t {
+        if (k == G) return B;
+        const int64_t t = (int64_t)((__int128)offs[B] * k / G);
+        return std::lower_bound(offs, offs + B, t) - offs;
+    };
+    *lo = start(g);
+    *hi = start(g + 1);
+}
+
 // A host-pointer call: checks, page-locking (tvf_set_host_register), then the pipeline, on one device or sharded over the
 // members of a group handle.  Member g solves the contiguous range shard_of(B, g, G) on its own device from its own host
 // thread; problems are independent and a problem's result does not depend on its batch, so the outputs are
@@ -475,14 +567,15 @@ template <class Call> int host_call(tvf_handle_t h, Call c, int64_t B) {
     HostPins pins;
     if (h->host_register) {
         TVF_CK(cudaSetDevice(h->device));
-        c.arrays([&](const void* p, const Arr& a) { if (a.per) pins.add(p, (size_t)B * a.per); });
+        c.arrays([&](const void* p, const Arr& a) { if (a.per) pins.add(p, a.bytes(c.rg.offs, 0, B)); });
     }
     const int G = 1 + (int)h->peers.size();
     if (G == 1 || B < G) return host_pipeline(h, c, B);
     std::vector<int> rcs((size_t)G, TVF_OK);
     auto run = [&](int g) {
         tvf_handle_t m = (g == 0) ? h : h->peers[(size_t)g - 1];
-        int64_t lo, hi; shard_of(B, g, G, &lo, &hi);
+        int64_t lo, hi;
+        if (c.rg.offs) shard_of_matches(c.rg.offs, B, g, G, &lo, &hi); else shard_of(B, g, G, &lo, &hi);
         Call s = c;
         shift(s, lo);
         m->chunk_user = h->chunk_user; m->host_threads = h->host_threads;
@@ -515,10 +608,12 @@ struct PoseOut {
 struct PoseCall {
     Method method; const double* corresp; const double* calm; int calm_batched; int n; PoseOut o;
     ChunkBufs d{};
+    Ragged rg{};                          // always uniform
     int check(tvf_handle_t h, int64_t B) const { return check_pose_args(h, corresp, calm, n, B, method); }
     int32_t*& status() { return o.status; }
     size_t budget(bool host_io) const { return pose_budget(n, host_io, false); }
-    size_t carve(char* base, int64_t C) { return carve_pose(base, n, C, true, calm_batched != 0, false, &d); }
+    size_t budget_match(bool) const { return 0; }
+    size_t carve(char* base, int64_t C, int64_t) { return carve_pose(base, n, C, true, calm_batched != 0, false, &d); }
     template <class F> void arrays(F&& f) {
         f(corresp, Arr::input(8 * 6 * n, d.in));
         f(calm, Arr::input(8 * 27, d.calm, !calm_batched));
@@ -601,11 +696,12 @@ int check_ba_size(tvf_handle_t h, int n, int64_t B) {
 struct BundleAdjust {
     BaArgs io;
     BaArgs d{};
+    Ragged rg{};                          // ragged: io.n = 0, every per-point array per match
     int check(tvf_handle_t h, int64_t B) const {
         if (!h) return TVF_ERR_ARG;
         if (!io.corresp || !io.calm || !io.Rt2_0 || !io.Rt3_0 || !io.Rt2 || !io.Rt3)
             return fail(h, TVF_ERR_ARG, "bundle_adjust: corresp, calm, Rt2_0, Rt3_0, Rt2 and Rt3 must not be NULL");
-        return check_ba_size(h, io.n, B);
+        return rg.offs ? check_offsets(h, "bundle_adjust", rg.offs, B) : check_ba_size(h, io.n, B);
     }
     int32_t*& status() { return io.status; }
     // the work space Xc (and X on the device path when the caller wants no points); the host path's inputs and outputs,
@@ -614,40 +710,42 @@ struct BundleAdjust {
         const int n = io.n;
         size_t b = (size_t)2 * 3 * n * sizeof(double);
         if (host_io) b += (size_t)(6 * n + 27 + 24 + 3 * n + 24 + 1) * sizeof(double) + 2 * sizeof(int32_t);
-        return b;
+        return b + (rg.offs ? sizeof(long long) : 0);
     }
-    size_t carve(char* base, int64_t C, bool host_io = true) {
-        const int n = io.n;
+    size_t budget_match(bool host_io) const { return (size_t)(2 * 3 + (host_io ? 9 : 0)) * sizeof(double); }
+    size_t carve(char* base, int64_t C, int64_t M, bool host_io = true) {
+        const int64_t P = rg.offs ? M : (int64_t)io.n * C;      // points of the chunk
         Carver c(base);
         d = io;
         if (host_io) {
-            d.corresp = c.take<double>((size_t)6 * n * C); d.calm = c.take<double>(io.calm_batched ? 27 * C : 27);
+            d.corresp = c.take<double>((size_t)6 * P); d.calm = c.take<double>(io.calm_batched ? 27 * C : 27);
             d.Rt2_0 = c.take<double>(12 * C); d.Rt3_0 = c.take<double>(12 * C);
-            d.X0 = io.X0 ? c.take<double>((size_t)3 * n * C) : nullptr;
-            d.Rt2 = c.take<double>(12 * C); d.Rt3 = c.take<double>(12 * C); d.X = c.take<double>((size_t)3 * n * C);
+            d.X0 = io.X0 ? c.take<double>((size_t)3 * P) : nullptr;
+            d.Rt2 = c.take<double>(12 * C); d.Rt3 = c.take<double>(12 * C); d.X = c.take<double>((size_t)3 * P);
             d.repr_err = c.take<double>(C); d.iter = c.take<int>(C); d.status = c.take<int>(C);
         }
-        if (!d.X) d.X = c.take<double>((size_t)3 * n * C);
-        d.Xc = c.take<double>((size_t)3 * n * C);
+        if (!d.X) d.X = c.take<double>((size_t)3 * P);
+        d.Xc = c.take<double>((size_t)3 * P);
+        if (rg.offs) d.offs = rg.d_offs = c.take<long long>(C + 1);
         return c.off;
     }
     template <class F> void arrays(F&& f) {
         const int n = io.n;
-        f(io.corresp, Arr::input(8 * 6 * n, d.corresp));
+        f(io.corresp, Arr::points(rg, n, 8 * 6, d.corresp, false));
         f(io.calm, Arr::input(8 * 27, d.calm, !io.calm_batched));
         f(io.Rt2_0, Arr::input(8 * 12, d.Rt2_0));
         f(io.Rt3_0, Arr::input(8 * 12, d.Rt3_0));
-        f(io.X0, Arr::input(8 * 3 * n, d.X0));
+        f(io.X0, Arr::points(rg, n, 8 * 3, d.X0, false));
         f(io.Rt2, Arr::output(8 * 12, d.Rt2));
         f(io.Rt3, Arr::output(8 * 12, d.Rt3));
-        f(io.X, Arr::output(8 * 3 * n, d.X));
+        f(io.X, Arr::points(rg, n, 8 * 3, d.X, true));
         f(io.repr_err, Arr::output(8, d.repr_err));
         f(io.iter, Arr::output(4, d.iter));
         f(io.status, Arr::output(4, d.status));
     }
     int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
         BaArgs a = d; a.B = Bc;
-        return ba_launched(h, launch_bundle_adjust(a, st), "bundle_adjust_kernel");
+        return ba_launched(h, launch_bundle_adjust(a, st), rg.offs ? "bundle_adjust_ragged_kernel" : "bundle_adjust_kernel");
     }
 };
 
@@ -655,47 +753,51 @@ struct BundleAdjust {
 struct Covariance {
     BaCovArgs io;
     BaCovArgs d{};
+    Ragged rg{};                          // ragged: io.n = 0, every per-point array per match
     int check(tvf_handle_t h, int64_t B) const {
         if (!h) return TVF_ERR_ARG;
         if (!io.corresp || !io.calm || !io.Rt2 || !io.Rt3 || !io.X)
             return fail(h, TVF_ERR_ARG, "ba_covariance: corresp, calm, Rt2, Rt3 and reconst must not be NULL");
-        return check_ba_size(h, io.n, B);
+        return rg.offs ? check_offsets(h, "ba_covariance", rg.offs, B) : check_ba_size(h, io.n, B);
     }
     int32_t*& status() { return io.status; }
     // the host path's inputs and outputs, counting a batched calm and cov_pts whether or not the call has them; the
     // device path needs no work space
     size_t budget(bool host_io) const {
         const int n = io.n;
-        return host_io ? (size_t)(6 * n + 27 + 24 + 3 * n + 144 + 9 * n + 1 + 1) * sizeof(double) : 0;
+        return (host_io ? (size_t)(6 * n + 27 + 24 + 3 * n + 144 + 9 * n + 1 + 1) * sizeof(double) : 0) +
+               (rg.offs ? sizeof(long long) : 0);
     }
-    size_t carve(char* base, int64_t C, bool host_io = true) {
-        const int n = io.n;
+    size_t budget_match(bool host_io) const { return host_io ? (size_t)(6 + 3 + 9) * sizeof(double) : 0; }
+    size_t carve(char* base, int64_t C, int64_t M, bool host_io = true) {
+        const int64_t P = rg.offs ? M : (int64_t)io.n * C;      // points of the chunk
         Carver c(base);
         d = io;
         if (host_io) {
-            d.corresp = c.take<double>((size_t)6 * n * C); d.calm = c.take<double>(io.calm_batched ? 27 * C : 27);
-            d.Rt2 = c.take<double>(12 * C); d.Rt3 = c.take<double>(12 * C); d.X = c.take<double>((size_t)3 * n * C);
+            d.corresp = c.take<double>((size_t)6 * P); d.calm = c.take<double>(io.calm_batched ? 27 * C : 27);
+            d.Rt2 = c.take<double>(12 * C); d.Rt3 = c.take<double>(12 * C); d.X = c.take<double>((size_t)3 * P);
             d.cov_cam = io.cov_cam ? c.take<double>(144 * C) : nullptr;
-            d.cov_pts = io.cov_pts ? c.take<double>((size_t)9 * n * C) : nullptr;
+            d.cov_pts = io.cov_pts ? c.take<double>((size_t)9 * P) : nullptr;
             d.sigma2 = c.take<double>(C); d.status = c.take<int>(C);
         }
+        if (rg.offs) d.offs = rg.d_offs = c.take<long long>(C + 1);
         return c.off;
     }
     template <class F> void arrays(F&& f) {
         const int n = io.n;
-        f(io.corresp, Arr::input(8 * 6 * n, d.corresp));
+        f(io.corresp, Arr::points(rg, n, 8 * 6, d.corresp, false));
         f(io.calm, Arr::input(8 * 27, d.calm, !io.calm_batched));
         f(io.Rt2, Arr::input(8 * 12, d.Rt2));
         f(io.Rt3, Arr::input(8 * 12, d.Rt3));
-        f(io.X, Arr::input(8 * 3 * n, d.X));
+        f(io.X, Arr::points(rg, n, 8 * 3, d.X, false));
         f(io.cov_cam, Arr::output(8 * 144, d.cov_cam));
-        f(io.cov_pts, Arr::output(8 * 9 * n, d.cov_pts));
+        f(io.cov_pts, Arr::points(rg, n, 8 * 9, d.cov_pts, true));
         f(io.sigma2, Arr::output(8, d.sigma2));
         f(io.status, Arr::output(4, d.status));
     }
     int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
         BaCovArgs a = d; a.B = Bc;
-        return ba_launched(h, launch_ba_covariance(a, st), "ba_covariance_kernel");
+        return ba_launched(h, launch_ba_covariance(a, st), rg.offs ? "ba_covariance_ragged_kernel" : "ba_covariance_kernel");
     }
 };
 
@@ -708,15 +810,18 @@ template <class Call> int ba_dev(tvf_handle_t h, const Call& c, int64_t B) {
     TVF_CK(cudaSetDevice(h->device));
     Slot& s = h->slot[0];
     cudaStream_t st = h->use_user_stream ? h->user_stream : s.stream;
-    const int64_t C = pick_chunk(h, B, false, c.budget(false));
+    int64_t C, M;
+    const std::vector<int64_t> ends = plan_chunks(h, c, B, false, &C, &M);
     Call k = c;
-    rc = ensure_arena(h, s, k.carve(nullptr, C, false)); if (rc) return rc;
-    for (int64_t done = 0; done < B; done += C) {
-        const int64_t Bc = (B - done < C) ? (B - done) : C;
+    rc = ensure_arena(h, s, k.carve(nullptr, C, M, false)); if (rc) return rc;
+    int64_t done = 0;
+    for (const int64_t end : ends) {
         k = c;
         shift(k, done);
-        k.carve(s.arena, C, false);
-        rc = k.launch(h, st, Bc); if (rc) return rc;
+        k.carve(s.arena, C, M, false);
+        rc = put_offsets(h, k, 0, end - done, st); if (rc) return rc;
+        rc = k.launch(h, st, end - done); if (rc) return rc;
+        done = end;
     }
     return TVF_OK;
 }
@@ -735,11 +840,15 @@ struct Ransac {
     RansacArgs io;
     RansacArgs d{};
     ChunkBufs w{};                       // the pose path's work space, for the B H hypotheses and then the refit
+    Ragged rg{};                         // ragged: io.n = 0, corresp and inliers per match
     int check(tvf_handle_t h, int64_t B) const {
         if (!h) return TVF_ERR_ARG;
         if (!io.corresp || !io.calm || !io.seeds) return fail(h, TVF_ERR_ARG, "ransac_pose: corresp, calm and seeds must not be NULL");
         if (B < 0) return fail(h, TVF_ERR_ARG, "ransac_pose: B >= 0");
-        if (io.n < s) {
+        if (rg.offs) {                   // a problem of fewer than s matches is flagged, not an error
+            const int rc = check_offsets(h, "ransac_pose", rg.offs, B);
+            if (rc != TVF_OK) return rc;
+        } else if (io.n < s) {
             if (method == METHOD_F) return fail(h, TVF_ERR_TOO_FEW_POINTS, TVF_LINEARF_ERRMSG);
             return fail(h, TVF_ERR_ARG, "ransac_pose: method 1 needs n >= 7 points");
         }
@@ -756,51 +865,63 @@ struct Ransac {
         size_t b = (size_t)H * (pose_budget(s, false, false) + (size_t)(6 * s + 27 + 24) * 8 + 4);
         b += (size_t)(6 * n + 27 + 48) * 8 + 2 * (size_t)n + 6 * 4;
         if (host_io) b += (size_t)(6 * n + 27 + 1 + 24) * 8 + n + 4 * (size_t)(s + 2);
-        return b;
+        return b + (rg.offs ? sizeof(long long) : 0);
     }
-    size_t carve(char* base, int64_t C, bool host_io = true) {
-        const int n = io.n;
+    size_t budget_match(bool host_io) const { return (size_t)6 * 8 + 2 + (host_io ? 6 * 8 + 1 : 0); }
+    size_t carve(char* base, int64_t C, int64_t M, bool host_io = true) {
+        const int64_t P = rg.offs ? M : (int64_t)io.n * C;      // matches of the chunk
         const int64_t Q = C * H;
         Carver c(base);
         d = io;
         if (host_io) {
-            d.corresp = c.take<double>((size_t)6 * n * C); d.calm = c.take<double>(io.calm_batched ? 27 * C : 27);
+            d.corresp = c.take<double>((size_t)6 * P); d.calm = c.take<double>(io.calm_batched ? 27 * C : 27);
             d.seeds = c.take<uint64_t>(C);
         }
         if (host_io || !d.Rt2) d.Rt2 = c.take<double>(12 * C);
         if (host_io || !d.Rt3) d.Rt3 = c.take<double>(12 * C);
-        if (host_io || !d.inliers) d.inliers = c.take<unsigned char>((size_t)n * C);
+        if (host_io || !d.inliers) d.inliers = c.take<unsigned char>((size_t)P);
         if (host_io || !d.n_inliers) d.n_inliers = c.take<int>(C);
         if (host_io || !d.sample) d.sample = c.take<int>((size_t)s * C);
         if (host_io || !d.status) d.status = c.take<int>(C);
         c.off += carve_pose(base ? base + c.off : nullptr, s, Q, false, false, false, &w);
         d.gin = c.take<double>((size_t)6 * s * Q); d.gcalm = io.calm_batched ? c.take<double>(27 * Q) : nullptr;
         d.hRt2 = c.take<double>(12 * Q); d.hRt3 = c.take<double>(12 * Q); d.hstatus = w.status; d.hcount = c.take<int>(Q);
-        d.best_h = c.take<int>(C); d.cnt_best = c.take<int>(C); d.mask_best = c.take<unsigned char>((size_t)n * C);
+        d.best_h = c.take<int>(C); d.cnt_best = c.take<int>(C); d.mask_best = c.take<unsigned char>((size_t)P);
         d.bestRt2 = c.take<double>(12 * C); d.bestRt3 = c.take<double>(12 * C);
-        d.refst = c.take<int>(C); d.cnt_refit = c.take<int>(C); d.mask_refit = c.take<unsigned char>((size_t)n * C);
+        d.refst = c.take<int>(C); d.cnt_refit = c.take<int>(C); d.mask_refit = c.take<unsigned char>((size_t)P);
         d.refRt2 = c.take<double>(12 * C); d.refRt3 = c.take<double>(12 * C);
-        d.rin = c.take<double>((size_t)6 * n * C); d.rcalm = io.calm_batched ? c.take<double>(27 * C) : nullptr;
+        d.rin = c.take<double>((size_t)6 * P); d.rcalm = io.calm_batched ? c.take<double>(27 * C) : nullptr;
         d.plist = c.take<int>(C);
+        if (rg.offs) rg.d_offs = c.take<long long>(C + 1);
         return c.off;
     }
     template <class F> void arrays(F&& f) {
         const int n = io.n;
-        f(io.corresp, Arr::input(8 * 6 * n, d.corresp));
+        f(io.corresp, Arr::points(rg, n, 8 * 6, d.corresp, false));
         f(io.calm, Arr::input(8 * 27, d.calm, !io.calm_batched));
         f(io.seeds, Arr::input(8, d.seeds));
         f(io.Rt2, Arr::output(8 * 12, d.Rt2));
         f(io.Rt3, Arr::output(8 * 12, d.Rt3));
-        f(io.inliers, Arr::output(n, d.inliers));
+        f(io.inliers, Arr::points(rg, n, 1, d.inliers, true));
         f(io.n_inliers, Arr::output(4, d.n_inliers));
         f(io.sample, Arr::output(4 * s, d.sample));
         f(io.status, Arr::output(4, d.status));
+    }
+    // consensus counts of the poses of a.B problems, hyp per problem (into count, zeroed before; mask may be null)
+    void consensus(tvf_handle_t h, cudaStream_t st, const RansacArgs& a, int hyp, const double* Rt2, const double* Rt3,
+                   const int* hst, int* count, unsigned char* mask) const {
+        if (rg.offs)
+            launch_ransac_consensus_ragged(a.corresp, a.calm, a.calm_batched, rg.d_offs, a.B, rg.m, hyp, Rt2, Rt3, hst, th,
+                                           count, mask, h->sm_count, st);
+        else
+            launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, a.n, a.B * hyp, hyp, Rt2, Rt3, hst, th, count, mask,
+                                    h->sm_count, st);
     }
     // sample and solve the hypotheses, score them, select; refit on the consensus of the best, grouped by its size
     // (the one read-back of the call); rescore; the result rule
     // the Q = Bc H minimal problems (gin, gcalm) and their poses (hRt2, hRt3, hstatus); k: the pose path's buffers
     int hypotheses(tvf_handle_t h, cudaStream_t st, const RansacArgs& a, ChunkBufs& k) const {
-        launch_ransac_sample(a, H, s, st);
+        launch_ransac_sample(a, H, s, st, rg.d_offs);
         int rc = ransac_launched(h); if (rc) return rc;
         k = w;
         k.in = a.gin; k.calm = a.calm_batched ? a.gcalm : a.calm; k.Rt2 = a.hRt2; k.Rt3 = a.hRt3;
@@ -809,19 +930,16 @@ struct Ransac {
     }
     int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
         RansacArgs a = d; a.B = Bc;
-        const int n = a.n;
         const int64_t Q = Bc * H;
         ChunkBufs k;
         int rc = hypotheses(h, st, a, k); if (rc) return rc;
         TVF_CK(cudaMemsetAsync(a.hcount, 0, (size_t)Q * sizeof(int), st));
-        launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, n, Q, H, a.hRt2, a.hRt3, a.hstatus, th, a.hcount, nullptr,
-                                h->sm_count, st);
+        consensus(h, st, a, H, a.hRt2, a.hRt3, a.hstatus, a.hcount, nullptr);
         rc = ransac_launched(h); if (rc) return rc;
         launch_ransac_select(a, H, st);
         rc = ransac_launched(h); if (rc) return rc;
         TVF_CK(cudaMemsetAsync(a.cnt_best, 0, (size_t)Bc * sizeof(int), st));
-        launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, n, Bc, 1, a.bestRt2, a.bestRt3, nullptr, th, a.cnt_best,
-                                a.mask_best, h->sm_count, st);
+        consensus(h, st, a, 1, a.bestRt2, a.bestRt3, nullptr, a.cnt_best, a.mask_best);
         rc = ransac_launched(h); if (rc) return rc;
         std::vector<int> cnt((size_t)Bc);
         TVF_CK(cudaMemcpyAsync(cnt.data(), a.cnt_best, (size_t)Bc * sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -837,7 +955,7 @@ struct Ransac {
             size_t g1 = g0;
             while (g1 < order.size() && cnt[(size_t)order[g1]] == size) ++g1;
             const int m = (int)(g1 - g0);
-            launch_ransac_gather(a, a.plist + g0, m, size, st);
+            launch_ransac_gather(a, a.plist + g0, m, size, st, rg.d_offs);
             rc = ransac_launched(h); if (rc) return rc;
             ChunkBufs r = k;                      // the hypotheses' buffers, free again
             r.in = a.rin; r.calm = a.calm_batched ? a.rcalm : a.calm;
@@ -847,10 +965,9 @@ struct Ransac {
             g0 = g1;
         }
         TVF_CK(cudaMemsetAsync(a.cnt_refit, 0, (size_t)Bc * sizeof(int), st));
-        launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, n, Bc, 1, a.refRt2, a.refRt3, a.refst, th, a.cnt_refit,
-                                a.mask_refit, h->sm_count, st);
+        consensus(h, st, a, 1, a.refRt2, a.refRt3, a.refst, a.cnt_refit, a.mask_refit);
         rc = ransac_launched(h); if (rc) return rc;
-        launch_ransac_finish(a, s, st);
+        launch_ransac_finish(a, s, st, rg.d_offs);
         return ransac_launched(h);
     }
 };
@@ -873,13 +990,16 @@ struct RansacRefined : Ransac {
         const size_t pts = (size_t)3 * (s * (size_t)H > (size_t)io.n ? s * (size_t)H : (size_t)io.n);
         return Ransac::budget(host_io) + 4 + (size_t)H * (24 * 8 + 4) + 2 * pts * 8 + 24 * 8;
     }
-    size_t carve(char* base, int64_t C, bool host_io = true) {
+    // an LO round's points (3 per match), counted beside the hypotheses' rather than overlapping them
+    size_t budget_match(bool host_io) const { return Ransac::budget_match(host_io) + 2 * 3 * 8; }
+    size_t carve(char* base, int64_t C, int64_t M, bool host_io = true) {
         Carver c(base);
-        c.off = Ransac::carve(base, C, host_io);
+        c.off = Ransac::carve(base, C, M, host_io);
         const int64_t Q = C * H;
+        const int64_t P = rg.offs ? M : (int64_t)io.n * C;      // matches of the chunk
         if (host_io || !d.lo_done) d.lo_done = c.take<int>(C);
         aRt2 = c.take<double>(12 * Q); aRt3 = c.take<double>(12 * Q); ast = c.take<int>(Q);
-        const size_t pts = (size_t)3 * (s * Q > io.n * C ? s * Q : io.n * C);
+        const size_t pts = (size_t)3 * (s * Q > P ? s * Q : P);
         X = c.take<double>(pts); Xc = c.take<double>(pts);
         d.gRt2 = c.take<double>(12 * C); d.gRt3 = c.take<double>(12 * C);
         return c.off;
@@ -894,7 +1014,6 @@ struct RansacRefined : Ransac {
     // the result rule with no refit.  aRt2, aRt3 and ast hold the hypotheses' adjustments, then an LO round's.
     int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
         RansacArgs a = d; a.B = Bc;
-        const int n = a.n;
         const int64_t Q = Bc * H;
         ChunkBufs k;
         int rc = hypotheses(h, st, a, k); if (rc) return rc;
@@ -904,15 +1023,13 @@ struct RansacRefined : Ransac {
         launch_ransac_flag(a.hstatus, ast, Q, st);
         rc = ransac_launched(h); if (rc) return rc;
         TVF_CK(cudaMemsetAsync(a.hcount, 0, (size_t)Q * sizeof(int), st));
-        launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, n, Q, H, aRt2, aRt3, ast, th, a.hcount, nullptr,
-                                h->sm_count, st);
+        consensus(h, st, a, H, aRt2, aRt3, ast, a.hcount, nullptr);
         rc = ransac_launched(h); if (rc) return rc;
         RansacArgs sel = a; sel.hRt2 = aRt2; sel.hRt3 = aRt3;
         launch_ransac_select(sel, H, st);
         rc = ransac_launched(h); if (rc) return rc;
         TVF_CK(cudaMemsetAsync(a.cnt_best, 0, (size_t)Bc * sizeof(int), st));
-        launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, n, Bc, 1, a.bestRt2, a.bestRt3, nullptr, th, a.cnt_best,
-                                a.mask_best, h->sm_count, st);
+        consensus(h, st, a, 1, a.bestRt2, a.bestRt3, nullptr, a.cnt_best, a.mask_best);
         rc = ransac_launched(h); if (rc) return rc;
         TVF_CK(cudaMemsetAsync(a.lo_done, 0, (size_t)Bc * sizeof(int), st));
         std::vector<int> cnt((size_t)Bc), prev;
@@ -931,7 +1048,7 @@ struct RansacRefined : Ransac {
                 size_t g1 = g0;
                 while (g1 < order.size() && cnt[(size_t)order[g1]] == size) ++g1;
                 const int m = (int)(g1 - g0);
-                launch_ransac_gather(a, a.plist + g0, m, size, st);
+                launch_ransac_gather(a, a.plist + g0, m, size, st, rg.d_offs);
                 rc = ransac_launched(h); if (rc) return rc;
                 const BaArgs lb{a.rin, a.calm_batched ? a.rcalm : a.calm, a.calm_batched, size, m, a.gRt2, a.gRt3, nullptr,
                                 aRt2, aRt3, X, Xc, nullptr, nullptr, ast};
@@ -943,16 +1060,15 @@ struct RansacRefined : Ransac {
             launch_ransac_flag(nullptr, a.refst, Bc, st);                           // -1 and TVF_ST_NONFINITE: count -1
             rc = ransac_launched(h); if (rc) return rc;
             TVF_CK(cudaMemsetAsync(a.cnt_refit, 0, (size_t)Bc * sizeof(int), st));
-            launch_ransac_consensus(a.corresp, a.calm, a.calm_batched, n, Bc, 1, a.refRt2, a.refRt3, a.refst, th, a.cnt_refit,
-                                    a.mask_refit, h->sm_count, st);
+            consensus(h, st, a, 1, a.refRt2, a.refRt3, a.refst, a.cnt_refit, a.mask_refit);
             rc = ransac_launched(h); if (rc) return rc;
-            launch_ransac_lo_accept(a, st);
+            launch_ransac_lo_accept(a, st, rg.d_offs);
             rc = ransac_launched(h); if (rc) return rc;
             prev.swap(cnt);
             cnt.resize((size_t)Bc);
         }
         TVF_CK(cudaMemsetAsync(a.refst, 0xff, (size_t)Bc * sizeof(int), st));          // the result rule without a refit
-        launch_ransac_finish(a, s, st);
+        launch_ransac_finish(a, s, st, rg.d_offs);
         return ransac_launched(h);
     }
 };
@@ -964,34 +1080,45 @@ struct Consensus {
     int32_t* no_status = nullptr;
     const double *d_corresp = nullptr, *d_calm = nullptr, *d_Rt2 = nullptr, *d_Rt3 = nullptr;
     uint8_t* d_inliers = nullptr; int32_t* d_count = nullptr;
+    Ragged rg{};                          // ragged: n = 0, corresp and inliers per match
     int check(tvf_handle_t h, int64_t B) const {
         if (!h) return TVF_ERR_ARG;
         if (!corresp || !calm || !Rt2 || !Rt3) return fail(h, TVF_ERR_ARG, "consensus: corresp, calm, Rt2 and Rt3 must not be NULL");
-        if (B < 0 || n < 1) return fail(h, TVF_ERR_ARG, "consensus: need n >= 1 and B >= 0");
+        if (rg.offs) {
+            const int rc = check_offsets(h, "consensus", rg.offs, B);
+            if (rc != TVF_OK) return rc;
+        } else if (B < 0 || n < 1) return fail(h, TVF_ERR_ARG, "consensus: need n >= 1 and B >= 0");
         if (!(th > 0.0) || !(th < __builtin_huge_val())) return fail(h, TVF_ERR_ARG, "consensus: threshold must be finite and > 0");
         return TVF_OK;
     }
     int32_t*& status() { return no_status; }
-    size_t budget(bool) const { return (size_t)(6 * n + 27 + 24) * 8 + n + 4; }
-    size_t carve(char* base, int64_t C) {
+    size_t budget(bool) const { return (size_t)(6 * n + 27 + 24) * 8 + n + 4 + (rg.offs ? 8 : 0); }
+    size_t budget_match(bool) const { return (size_t)6 * 8 + 1; }
+    size_t carve(char* base, int64_t C, int64_t M) {
+        const int64_t P = rg.offs ? M : (int64_t)n * C;      // matches of the chunk
         Carver c(base);
-        d_corresp = c.take<double>((size_t)6 * n * C); d_calm = c.take<double>(calm_batched ? 27 * C : 27);
+        d_corresp = c.take<double>((size_t)6 * P); d_calm = c.take<double>(calm_batched ? 27 * C : 27);
         d_Rt2 = c.take<double>(12 * C); d_Rt3 = c.take<double>(12 * C);
-        d_inliers = c.take<uint8_t>((size_t)n * C); d_count = c.take<int32_t>(C);
+        d_inliers = c.take<uint8_t>((size_t)P); d_count = c.take<int32_t>(C);
+        if (rg.offs) rg.d_offs = c.take<long long>(C + 1);
         return c.off;
     }
     template <class F> void arrays(F&& f) {
-        f(corresp, Arr::input(8 * 6 * n, d_corresp));
+        f(corresp, Arr::points(rg, n, 8 * 6, d_corresp, false));
         f(calm, Arr::input(8 * 27, d_calm, !calm_batched));
         f(Rt2, Arr::input(8 * 12, d_Rt2));
         f(Rt3, Arr::input(8 * 12, d_Rt3));
-        f(inliers, Arr::output(n, d_inliers));
+        f(inliers, Arr::points(rg, n, 1, d_inliers, true));
         f(n_inliers, Arr::output(4, d_count));
     }
     int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
         TVF_CK(cudaMemsetAsync(d_count, 0, (size_t)Bc * sizeof(int32_t), st));
-        launch_ransac_consensus(d_corresp, d_calm, calm_batched, n, Bc, 1, d_Rt2, d_Rt3, nullptr, th, d_count, d_inliers,
-                                h->sm_count, st);
+        if (rg.offs)
+            launch_ransac_consensus_ragged(d_corresp, d_calm, calm_batched, rg.d_offs, Bc, rg.m, 1, d_Rt2, d_Rt3, nullptr, th,
+                                           d_count, d_inliers, h->sm_count, st);
+        else
+            launch_ransac_consensus(d_corresp, d_calm, calm_batched, n, Bc, 1, d_Rt2, d_Rt3, nullptr, th, d_count, d_inliers,
+                                    h->sm_count, st);
         return ransac_launched(h);
     }
 };
@@ -1816,15 +1943,52 @@ int tvf_ba_covariance_dev(tvf_handle_t h, const double* corresp, const double* c
     return ba_dev(h, Covariance{BaCovArgs{corresp, calm, calm_batched, n, 0, Rt2, Rt3, reconst, cov_cam, cov_pts, sigma2, status}}, B);
 }
 
+int tvf_bundle_adjust_ragged(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, const int64_t* offsets,
+                             int64_t B, const double* Rt2_0, const double* Rt3_0, const double* reconst0, double* Rt2,
+                             double* Rt3, double* reconst, double* repr_err, int32_t* iter, int32_t* status) {
+    BundleAdjust c{BaArgs{corresp, calm, calm_batched, 0, 0, Rt2_0, Rt3_0, reconst0, Rt2, Rt3, reconst, nullptr, repr_err, iter,
+                          status}};
+    c.rg.offs = offsets;
+    return host_call(h, c, B);
+}
+
+int tvf_bundle_adjust_ragged_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched,
+                                 const int64_t* offsets, int64_t B, const double* Rt2_0, const double* Rt3_0,
+                                 const double* reconst0, double* Rt2, double* Rt3, double* reconst, double* repr_err,
+                                 int32_t* iter, int32_t* status) {
+    BundleAdjust c{BaArgs{corresp, calm, calm_batched, 0, 0, Rt2_0, Rt3_0, reconst0, Rt2, Rt3, reconst, nullptr, repr_err, iter,
+                          status}};
+    c.rg.offs = offsets;
+    return ba_dev(h, c, B);
+}
+
+int tvf_ba_covariance_ragged(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, const int64_t* offsets,
+                             int64_t B, const double* Rt2, const double* Rt3, const double* reconst, double* cov_cam,
+                             double* cov_pts, double* sigma2, int32_t* status) {
+    Covariance c{BaCovArgs{corresp, calm, calm_batched, 0, 0, Rt2, Rt3, reconst, cov_cam, cov_pts, sigma2, status}};
+    c.rg.offs = offsets;
+    return host_call(h, c, B);
+}
+
+int tvf_ba_covariance_ragged_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched,
+                                 const int64_t* offsets, int64_t B, const double* Rt2, const double* Rt3,
+                                 const double* reconst, double* cov_cam, double* cov_pts, double* sigma2, int32_t* status) {
+    Covariance c{BaCovArgs{corresp, calm, calm_batched, 0, 0, Rt2, Rt3, reconst, cov_cam, cov_pts, sigma2, status}};
+    c.rg.offs = offsets;
+    return ba_dev(h, c, B);
+}
+
 static int ransac_call(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched, int n,
                        int64_t B, int hypotheses, double threshold, const uint64_t* seeds, double* Rt2, double* Rt3,
-                       uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* status, bool dev) {
+                       uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* status, bool dev,
+                       const int64_t* offsets = nullptr) {
     if (!h) return TVF_ERR_ARG;
     if (method != 1 && method != 7) return fail(h, TVF_ERR_ARG, "ransac_pose: method must be 1 (linear TFT) or 7 (linear F)");
     RansacArgs io{};
     io.corresp = corresp; io.calm = calm; io.calm_batched = calm_batched; io.n = n; io.seeds = seeds;
     io.Rt2 = Rt2; io.Rt3 = Rt3; io.inliers = inliers; io.n_inliers = n_inliers; io.sample = sample; io.status = status;
-    const Ransac c{method == 1 ? METHOD_TFT : METHOD_F, method == 1 ? 7 : 8, hypotheses, threshold, io};
+    Ransac c{method == 1 ? METHOD_TFT : METHOD_F, method == 1 ? 7 : 8, hypotheses, threshold, io};
+    c.rg.offs = offsets;
     return dev ? ba_dev(h, c, B) : host_call(h, c, B);
 }
 
@@ -1845,14 +2009,15 @@ int tvf_ransac_pose_dev(tvf_handle_t h, int method, const double* corresp, const
 static int ransac_refined_call(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched,
                                int n, int64_t B, int hypotheses, double threshold, const uint64_t* seeds, int lo_rounds,
                                double* Rt2, double* Rt3, uint8_t* inliers, int32_t* n_inliers, int32_t* sample,
-                               int32_t* lo_done, int32_t* status, bool dev) {
+                               int32_t* lo_done, int32_t* status, bool dev, const int64_t* offsets = nullptr) {
     if (!h) return TVF_ERR_ARG;
     if (method != 1 && method != 7) return fail(h, TVF_ERR_ARG, "ransac_pose: method must be 1 (linear TFT) or 7 (linear F)");
     RansacArgs io{};
     io.corresp = corresp; io.calm = calm; io.calm_batched = calm_batched; io.n = n; io.seeds = seeds;
     io.Rt2 = Rt2; io.Rt3 = Rt3; io.inliers = inliers; io.n_inliers = n_inliers; io.sample = sample; io.status = status;
     io.lo_done = lo_done;
-    const RansacRefined c{Ransac{method == 1 ? METHOD_TFT : METHOD_F, method == 1 ? 7 : 8, hypotheses, threshold, io}, lo_rounds};
+    RansacRefined c{Ransac{method == 1 ? METHOD_TFT : METHOD_F, method == 1 ? 7 : 8, hypotheses, threshold, io}, lo_rounds};
+    c.rg.offs = offsets;
     return dev ? ba_dev(h, c, B) : host_call(h, c, B);
 }
 
@@ -1872,9 +2037,48 @@ int tvf_ransac_pose_refined_dev(tvf_handle_t h, int method, const double* corres
                                Rt3, inliers, n_inliers, sample, lo_done, status, true);
 }
 
+int tvf_ransac_pose_ragged(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched,
+                           const int64_t* offsets, int64_t B, int hypotheses, double threshold, const uint64_t* seeds,
+                           double* Rt2, double* Rt3, uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* status) {
+    return ransac_call(h, method, corresp, calm, calm_batched, 0, B, hypotheses, threshold, seeds, Rt2, Rt3, inliers,
+                       n_inliers, sample, status, false, offsets);
+}
+
+int tvf_ransac_pose_ragged_dev(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched,
+                               const int64_t* offsets, int64_t B, int hypotheses, double threshold, const uint64_t* seeds,
+                               double* Rt2, double* Rt3, uint8_t* inliers, int32_t* n_inliers, int32_t* sample,
+                               int32_t* status) {
+    return ransac_call(h, method, corresp, calm, calm_batched, 0, B, hypotheses, threshold, seeds, Rt2, Rt3, inliers,
+                       n_inliers, sample, status, true, offsets);
+}
+
+int tvf_ransac_pose_refined_ragged(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched,
+                                   const int64_t* offsets, int64_t B, int hypotheses, double threshold, const uint64_t* seeds,
+                                   int lo_rounds, double* Rt2, double* Rt3, uint8_t* inliers, int32_t* n_inliers,
+                                   int32_t* sample, int32_t* lo_done, int32_t* status) {
+    return ransac_refined_call(h, method, corresp, calm, calm_batched, 0, B, hypotheses, threshold, seeds, lo_rounds, Rt2,
+                               Rt3, inliers, n_inliers, sample, lo_done, status, false, offsets);
+}
+
+int tvf_ransac_pose_refined_ragged_dev(tvf_handle_t h, int method, const double* corresp, const double* calm,
+                                       int calm_batched, const int64_t* offsets, int64_t B, int hypotheses, double threshold,
+                                       const uint64_t* seeds, int lo_rounds, double* Rt2, double* Rt3, uint8_t* inliers,
+                                       int32_t* n_inliers, int32_t* sample, int32_t* lo_done, int32_t* status) {
+    return ransac_refined_call(h, method, corresp, calm, calm_batched, 0, B, hypotheses, threshold, seeds, lo_rounds, Rt2,
+                               Rt3, inliers, n_inliers, sample, lo_done, status, true, offsets);
+}
+
 int tvf_consensus(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
                   const double* Rt2, const double* Rt3, double threshold, uint8_t* inliers, int32_t* n_inliers) {
     return host_call(h, Consensus{corresp, calm, calm_batched, n, Rt2, Rt3, threshold, inliers, n_inliers}, B);
+}
+
+int tvf_consensus_ragged(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, const int64_t* offsets,
+                         int64_t B, const double* Rt2, const double* Rt3, double threshold, uint8_t* inliers,
+                         int32_t* n_inliers) {
+    Consensus c{corresp, calm, calm_batched, 0, Rt2, Rt3, threshold, inliers, n_inliers};
+    c.rg.offs = offsets;
+    return host_call(h, c, B);
 }
 
 int tvf_ang_error(tvf_handle_t h, const double* Rt_true, int true_batched, const double* Rt_est, int64_t B,

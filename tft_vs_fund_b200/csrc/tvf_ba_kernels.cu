@@ -49,8 +49,9 @@ template <int W> __device__ __forceinline__ double group_max(double v, unsigned 
     return v;
 }
 
-// the problems of one group of W lanes (mask gm) in a grid-stride loop; lane = the lane within the group
-template <int W> __device__ __forceinline__ void ba_problems(const BaArgs& a) {
+// the problems of one group of W lanes (mask gm) in a grid-stride loop; lane = the lane within the group.  Ragged: problem
+// prob owns matches a.offs[prob] .. a.offs[prob+1]-1 (n varies per problem); the uniform form indexes by prob * a.n
+template <int W, bool Ragged> __device__ __forceinline__ void ba_problems(const BaArgs& a) {
     extern __shared__ __align__(16) double ba_smem[];
     constexpr int G = BA_WARPS * 32 / W;               // groups (problems in flight) per block
     const int lane = threadIdx.x & (W - 1), grp = threadIdx.x / W;
@@ -61,14 +62,30 @@ template <int W> __device__ __forceinline__ void ba_problems(const BaArgs& a) {
     BaCams& cur = *reinterpret_cast<BaCams*>(dcs + 12);
     BaCams& cand = *reinterpret_cast<BaCams*>(dcs + 12 + BA_CAMS);
     double* acc = slab + lane * BA_NSUM;
-    const int n = a.n;
+    const int n_all = a.n;
 
     for (long long prob = (long long)blockIdx.x * G + grp; prob < a.B; prob += (long long)gridDim.x * G) {
+        // ragged: the problem's matches as problem 0 of a batch of n = n_b
+        const long long off = Ragged ? a.offs[prob] : 0;
+        const int n = Ragged ? (int)(a.offs[prob + 1] - off) : n_all;
+        const long long pi = Ragged ? 0 : prob;        // the problem index the point loads use
+        const double* corresp = a.corresp + off * 6;
         const double* cm = a.calm + (a.calm_batched ? prob * 27 : 0);
         const double* rt2 = a.Rt2_0 + prob * 12;
         const double* rt3 = a.Rt3_0 + prob * 12;
-        double* Xp = a.X + prob * 3 * n;
-        double* Xcp = a.Xc + prob * 3 * n;
+        double* Xp = Ragged ? a.X + off * 3 : a.X + prob * 3 * n;
+        double* Xcp = Ragged ? a.Xc + off * 3 : a.Xc + prob * 3 * n;
+        if (Ragged && n < 4) {                         // too few: start poses copied through, points and error NaN
+            const double qnan = __longlong_as_double(0x7ff8000000000000LL);
+            for (int e = lane; e < 12; e += W) { a.Rt2[prob * 12 + e] = rt2[e]; a.Rt3[prob * 12 + e] = rt3[e]; }
+            for (int e = lane; e < 3 * n; e += W) Xp[e] = qnan;
+            if (lane == 0) {
+                if (a.repr_err) a.repr_err[prob] = qnan;
+                if (a.iter) a.iter[prob] = 0;
+                if (a.status) a.status[prob] = ST_TOO_FEW_MATCHES;
+            }
+            continue;
+        }
         __syncwarp(gm);
         if (lane == 0) ba_load_cams(cm, rt2, rt3, cur);
         bool bad_l = false;
@@ -93,9 +110,9 @@ template <int W> __device__ __forceinline__ void ba_problems(const BaArgs& a) {
             }
             for (int i = lane; i < n; i += W) {
                 double x6[6], X[3];
-                load_x6(a.corresp, prob, n, i, x6);
+                load_x6(corresp, pi, n, i, x6);
                 if (a.X0 != nullptr) {
-                    const double* q = a.X0 + (prob * n + i) * 3;
+                    const double* q = a.X0 + (Ragged ? off + i : prob * n + i) * 3;
                     X[0] = q[0]; X[1] = q[1]; X[2] = q[2];
                 } else {
                     double Xh[4];
@@ -134,7 +151,7 @@ template <int W> __device__ __forceinline__ void ba_problems(const BaArgs& a) {
         cost_l = 0.0;
         for (int i = lane; i < n; i += W) {
             double x6[6], X[3];
-            load_x6(a.corresp, prob, n, i, x6);
+            load_x6(corresp, pi, n, i, x6);
 #pragma unroll
             for (int k = 0; k < 3; ++k) { X[k] = Xp[3 * i + k] * gs; Xp[3 * i + k] = X[k]; }
             cost_l += ba_point_cost(cur, X, x6);
@@ -152,7 +169,7 @@ template <int W> __device__ __forceinline__ void ba_problems(const BaArgs& a) {
             double gp_l = 0.0;
             for (int i = lane; i < n; i += W) {
                 double x6[6];
-                load_x6(a.corresp, prob, n, i, x6);
+                load_x6(corresp, pi, n, i, x6);
                 const double X[3] = {Xp[3 * i], Xp[3 * i + 1], Xp[3 * i + 2]};
                 BaPoint p; BaElim el;
                 ba_point_jac(cur, X, x6, p);
@@ -189,7 +206,7 @@ template <int W> __device__ __forceinline__ void ba_problems(const BaArgs& a) {
                 double cn_l = 0.0, pr_l = 0.0, s2_l = 0.0, x2_l = 0.0;
                 for (int i = lane; i < n; i += W) {
                     double x6[6];
-                    load_x6(a.corresp, prob, n, i, x6);
+                    load_x6(corresp, pi, n, i, x6);
                     const double X[3] = {Xp[3 * i], Xp[3 * i + 1], Xp[3 * i + 2]};
                     BaPoint p; BaElim el;
                     ba_point_jac(cur, X, x6, p);
@@ -253,7 +270,9 @@ template <int W> __device__ __forceinline__ void ba_problems(const BaArgs& a) {
     }
 }
 
-__global__ void __launch_bounds__(BA_WARPS * 32) bundle_adjust_kernel(const BaArgs a) { ba_problems<32>(a); }
+__global__ void __launch_bounds__(BA_WARPS * 32) bundle_adjust_kernel(const BaArgs a) { ba_problems<32, false>(a); }
+// the ragged batch (a.offs): the same code per problem at n = n_b, so bit-identical to bundle_adjust_kernel on it alone
+__global__ void __launch_bounds__(BA_WARPS * 32) bundle_adjust_ragged_kernel(const BaArgs a) { ba_problems<32, true>(a); }
 
 // Packed variant for n <= 8: groups of 8 lanes, four problems per warp.  Bit-identical to bundle_adjust_kernel on the
 // same problem, because at n <= 8 lanes 8..31 of bundle_adjust_kernel own no point and contribute exact +0.0:
@@ -264,7 +283,7 @@ __global__ void __launch_bounds__(BA_WARPS * 32) bundle_adjust_kernel(const BaAr
 //   - the slab sum s = 0.0; s += slab[l] (l ascending) never holds -0.0, so adding the 24 trailing +0.0 rows of the
 //     idle lanes leaves it as group 8's sum over l = 0..7;
 //   - every vote (__any_sync) of the idle lanes is false, and every other step is done by lane 0 or per point.
-__global__ void __launch_bounds__(BA_WARPS * 32) bundle_adjust_small_kernel(const BaArgs a) { ba_problems<BA_SMALL_N>(a); }
+__global__ void __launch_bounds__(BA_WARPS * 32) bundle_adjust_small_kernel(const BaArgs a) { ba_problems<BA_SMALL_N, false>(a); }
 
 template <int W> int launch_groups(void (*kernel)(const BaArgs), const BaArgs& a, cudaStream_t stream) {
     if (a.B <= 0) return 1;
@@ -281,7 +300,9 @@ template <int W> int launch_groups(void (*kernel)(const BaArgs), const BaArgs& a
     return cudaPeekAtLastError() == cudaSuccess ? 1 : 0;
 }
 
-int launch_bundle_adjust(const BaArgs& a, cudaStream_t stream) { return launch_groups<32>(bundle_adjust_kernel, a, stream); }
+int launch_bundle_adjust(const BaArgs& a, cudaStream_t stream) {
+    return launch_groups<32>(a.offs ? bundle_adjust_ragged_kernel : bundle_adjust_kernel, a, stream);
+}
 
 int launch_bundle_adjust_small(const BaArgs& a, cudaStream_t stream) {
     if (a.n > BA_SMALL_N) return 0;

@@ -64,7 +64,11 @@ struct BaArgs {
     double* repr_err;          // B
     int* iter;                 // B
     int* status;               // B
+    // ragged batch (null: uniform n): problem b owns matches offs[b] .. offs[b+1]-1 of corresp (6 x offs[B]), X0, X and
+    // Xc (3 x offs[B]); n is unused.  Last member: the kernel parameters before it keep their offsets.
+    const long long* offs;
 };
+// offs != null: bundle_adjust_ragged_kernel, which gives a problem of fewer than 4 matches TVF_ST_TOO_FEW_MATCHES
 int launch_bundle_adjust(const BaArgs& a, cudaStream_t stream);
 // the same adjustment, bit for bit, with four problems per warp (groups of 8 lanes) for a.n <= BA_SMALL_N; returns 0
 // for a larger n or a failed launch
@@ -86,6 +90,7 @@ struct BaCovArgs {
     double* cov_pts;           // 9 x n x B
     double* sigma2;            // B
     int* status;               // B
+    const long long* offs;     // ragged batch as BaArgs::offs (cov_pts 9 x offs[B]); null: uniform n
 };
 int launch_ba_covariance(const BaCovArgs& a, cudaStream_t stream);
 
@@ -96,6 +101,12 @@ int launch_ba_covariance(const BaCovArgs& a, cudaStream_t stream);
 void launch_ransac_consensus(const double* corresp, const double* calm, int calm_batched, int n, long long Q, int H,
                              const double* Rt2, const double* Rt3, const int* hstatus, double th, int* count,
                              unsigned char* mask, int sm_count, cudaStream_t stream);
+// the same over a ragged batch: problem b owns matches offs[b] .. offs[b+1]-1 (m = offs[B] in all) and poses
+// b H .. b H + H-1; mask (H m, may be null): problem b's H x n_b flags start at H offs[b]
+void launch_ransac_consensus_ragged(const double* corresp, const double* calm, int calm_batched, const long long* offs,
+                                    long long B, long long m, int H, const double* Rt2, const double* Rt3,
+                                    const int* hstatus, double th, int* count, unsigned char* mask, int sm_count,
+                                    cudaStream_t stream);
 
 // the buffers of one chunk of tvf_ransac_pose: B problems, H hypotheses of s points each
 struct RansacArgs {
@@ -123,22 +134,27 @@ struct RansacArgs {
     // tvf_ransac_pose_refined: the LO rounds' compacted start poses (12 x B each; null: not gathered) and their count
     double* gRt2; double* gRt3; int* lo_done;
 };
+// The launchers below take `offs`, a ragged batch as BaArgs::offs (corresp, inliers, mask_best and mask_refit per match;
+// null: uniform n), and then run the *_ragged_kernel forms, where a problem of fewer than s matches samples NaN columns
+// and finishes with TVF_ST_TOO_FEW_MATCHES.  offs is a kernel parameter of its own, not a member of RansacArgs: kernel
+// parameters follow the struct, and a larger struct would move them in the uniform kernels' machine code.
 // the s-point minimal problem of every hypothesis (gin, gcalm)
-void launch_ransac_sample(const RansacArgs& a, int H, int s, cudaStream_t stream);
+void launch_ransac_sample(const RansacArgs& a, int H, int s, cudaStream_t stream, const long long* offs = nullptr);
 // per problem the hypothesis of largest hcount (ties: smallest h) -> best_h (-1: all flagged), bestRt2/3 (NaN then)
 void launch_ransac_select(const RansacArgs& a, int H, cudaStream_t stream);
 // problems plist[0..m) of refit size k: their consensus columns (mask_best, index order) -> rin (6 x k x m), rcalm,
 // and bestRt2/3 -> gRt2/3 (12 x m) when gRt2 is not null
-void launch_ransac_gather(const RansacArgs& a, const int* plist, int m, int k, cudaStream_t stream);
+void launch_ransac_gather(const RansacArgs& a, const int* plist, int m, int k, cudaStream_t stream,
+                          const long long* offs = nullptr);
 // refit results of those problems (Rt2, Rt3, status m each) -> refRt2, refRt3, refst
 void launch_ransac_scatter(const RansacArgs& a, const int* plist, int m, const double* Rt2, const double* Rt3,
                            const int* st, cudaStream_t stream);
 // st[q] <- 1 if pose_st[q] != 0 (pose_st may be null) or st[q] (an adjustment's status) has ST_NONFINITE, else 0
 void launch_ransac_flag(const int* pose_st, int* st, long long Q, cudaStream_t stream);
 // per problem, if cnt_refit > cnt_best: refRt2/3, mask_refit, cnt_refit -> bestRt2/3, mask_best, cnt_best; ++lo_done
-void launch_ransac_lo_accept(const RansacArgs& a, cudaStream_t stream);
+void launch_ransac_lo_accept(const RansacArgs& a, cudaStream_t stream, const long long* offs = nullptr);
 // the result rule (include/tvf.h, tvf_ransac_pose) -> the outputs
-void launch_ransac_finish(const RansacArgs& a, int s, cudaStream_t stream);
+void launch_ransac_finish(const RansacArgs& a, int s, cudaStream_t stream, const long long* offs = nullptr);
 
 // ---- pose tail -----------------------------------------------------------------------------
 struct PoseTailArgs {

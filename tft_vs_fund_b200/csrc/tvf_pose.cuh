@@ -28,6 +28,7 @@ constexpr int ST_EPIPOLE_ZERO = 2;   // sign(V(end))==0 at R_t_from_TFT.m:50/55
 constexpr int ST_NO_POSE_2 = 4;      // all four cheirality votes negative/NaN: MATLAB leaves R_f undefined
 constexpr int ST_NO_POSE_3 = 8;
 constexpr int ST_NONFINITE = 16;     // non-finite value in the outputs
+constexpr int ST_TOO_FEW_MATCHES = 256;  // a problem of a ragged batch has fewer matches than the method needs
 
 TVF_HD void fill_pair_(const double* E, const double* K, double* c) {
     decompose_essential(E, c + OFF_R, c + OFF_RP, c + OFF_T);

@@ -110,8 +110,43 @@ def consensus_stats(mask, truth):
                 recall=tp / int(np.sum(truth)) if np.any(truth) else 0.0)
 
 
+def _raw_batched(preps, methods, ransac_refine, bundle_adjust, covariance, device):
+    """The estimates of run_real(raw_matches=True) for all triplets at once: per method one ragged api.ransac_pose over
+    the triplets it can run (seed = loop index, CalM per triplet), then one ragged api.bundle_adjust and api.ba_covariance
+    over the consensus sets of >= 4 matches.  Returns {method: {row: (res, ba, cov)}}, each entry what the per-triplet
+    loop computes for that row (ba, cov None where it computes none); every problem is bit-identical to its B = 1 call."""
+    out = {}
+    for m in methods:
+        rows = [r for r, d in enumerate(preps) if not ((m > 6 and d["Corresp"].shape[1] < 8) or d["Corresp"].shape[1] < 7)]
+        out[m] = {}
+        if not rows:
+            continue
+        res = api.ransac_pose([preps[r]["Corresp"] for r in rows], np.stack([preps[r]["CalM"] for r in rows]), method=m,
+                              hypotheses=1024, threshold=1.0, seed=np.array([r + 1 for r in rows], dtype=np.uint64),
+                              device=device, refine=ransac_refine)
+        for k, r in enumerate(rows):
+            one = api.RansacResult((res[0][k], res[1][k], res[2][k], int(res[3][k]), res[4][k]))
+            one.status = int(res.status[k])
+            one.lo_done = int(res.lo_done[k]) if ransac_refine else None
+            out[m][r] = [one, None, None]
+        adj = [k for k, r in enumerate(rows) if res[3][k] >= 4] if bundle_adjust else []
+        if not adj:
+            continue
+        Cm = [preps[rows[k]]["Corresp"][:, res[2][k]] for k in adj]
+        CalM = np.stack([preps[rows[k]]["CalM"] for k in adj])
+        ba = api.bundle_adjust(Cm, CalM, res[0][adj], res[1][adj], None, device=device)
+        cov = api.ba_covariance(Cm, CalM, ba[0], ba[1], ba[2], device=device) if covariance else None
+        for j, k in enumerate(adj):
+            one = api.BundleAdjustResult((ba[0][j], ba[1][j], ba[2][j], int(ba[3][j])))
+            one.repr_err, one.status = float(ba.repr_err[j]), int(ba.status[j])
+            out[m][rows[k]][1] = one
+            if covariance:
+                out[m][rows[k]][2] = api.CovarianceResult((cov[0][j], float(cov[1][j])))
+    return out
+
+
 def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), device=None, details=None,
-             bundle_adjust=False, covariance=False, raw_matches=False, ransac_refine=False):
+             bundle_adjust=False, covariance=False, raw_matches=False, ransac_refine=False, batched=False):
     """The linear-method part of experiments_real.m:75-138.  `data`: a Dataset or the path of a dataset directory;
     `triplets_to_test`: rows of indexes_sorted (1-based; the reference uses 1:70 / 1:50, :31-36).  Per loop index `it`:
     pre-filter (:94-101), sample min(100, N) inliers with rng(it) (:103-105; documented stand-in for MATLAB's
@@ -134,11 +169,16 @@ def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), de
     consensus columns, starting from the RANSAC pose (the points triangulated from it); a consensus of fewer than 4
     matches cannot be adjusted and gets +inf in the adjusted columns.
     ransac_refine=True (with raw_matches): api.ransac_pose(refine=True) instead, whose hypotheses and result are
-    bundle-adjusted (8 LO rounds); nothing else changes."""
+    bundle-adjusted (8 LO rounds); nothing else changes.
+    batched=True (with raw_matches): the triplets are prepared first, then RANSAC runs over all of them in one ragged
+    call per method, and the adjustment and covariance in one ragged call each; the return value and `details` equal
+    the per-triplet loop's exactly."""
     from .scene import SceneRNG
     from .experiments import METHODS
     if not isinstance(data, Dataset):
         data = load_dataset(data)
+    if batched and not raw_matches:
+        raise ValueError("run_real: batched=True needs raw_matches=True")
     out = {m: np.zeros((len(triplets_to_test), 6 if bundle_adjust else 3)) for m in methods}
 
     def errors(R2, R3, CalM, inl, R_t0):
@@ -148,9 +188,10 @@ def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), de
         r3, t3 = api.AngError(R_t0[1], R3, device=device)
         return [rep, (r2 + r3) / 2, (t2 + t3) / 2]                                                      # :133-136
 
-    for row, trip in enumerate(triplets_to_test):
+    preps = [prepare_triplet(data, trip, device=device) for trip in triplets_to_test]
+    est = _raw_batched(preps, methods, ransac_refine, bundle_adjust, covariance, device) if batched else None
+    for row, d in enumerate(preps):
         it = row + 1                                                                                    # :75 loop index
-        d = prepare_triplet(data, trip, device=device)
         inl = d["Corresp_inliers"]
         N = inl.shape[1]
         sample = SceneRNG(it).randsample(N, min(initial_sample_size, N))                               # :103-105
@@ -166,7 +207,11 @@ def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), de
             if (m > 6 and Nm < 8) or Nm < 7:                                                            # :117-122
                 out[m][row] = np.inf
                 continue
-            if raw_matches:
+            if batched:
+                res = est[m][row][0]
+                Cm, X0 = d["Corresp"][:, res[2]], None
+                rec["consensus"][m] = consensus_stats(res[2], d["inlier_mask"])
+            elif raw_matches:
                 res = api.ransac_pose(d["Corresp"], CalM, method=m, hypotheses=1024, threshold=1.0, seed=it, device=device,
                                       refine=ransac_refine)
                 Cm, X0 = d["Corresp"][:, res[2]], None
@@ -179,10 +224,10 @@ def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), de
             if bundle_adjust and Cm.shape[1] < 4:                                                       # too few to adjust
                 out[m][row, 3:] = np.inf
             elif bundle_adjust:
-                ba = api.bundle_adjust(Cm, CalM, res[0], res[1], X0, device=device)
+                ba = est[m][row][1] if batched else api.bundle_adjust(Cm, CalM, res[0], res[1], X0, device=device)
                 out[m][row, 3:] = errors(ba[0], ba[1], CalM, inl, d["R_t0"])
                 if covariance:
-                    cov = api.ba_covariance(Cm, CalM, ba[0], ba[1], ba[2], device=device)
+                    cov = est[m][row][2] if batched else api.ba_covariance(Cm, CalM, ba[0], ba[1], ba[2], device=device)
                     rot, tdir = api.pose_rms_errors(cov[0], ba[0], ba[1], sigma2=cov[1])
                     ba.sigma2 = cov[1]
                     ba.pred_rot_err, ba.pred_t_err = float(np.mean(rot)), float(np.mean(tdir))
