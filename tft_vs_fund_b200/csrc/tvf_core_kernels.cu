@@ -1102,7 +1102,7 @@ int launch_tft_stage1(const CoreInput& in, double* ws, int* status, int sm_count
     }
     if (in.packed && in.n <= MOM_TMA_MAX_N) {
         const size_t dyn = 2 * (size_t)(2 * CORE_WARPS) * in.n * 48;
-        cudaFuncSetAttribute(tft_moments_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);   // per launch: per device
+        allow_max_dynamic_smem(tft_moments_tma_kernel);                                                      // per launch: per device
         const unsigned gt = core_grid_minb((in.B + 1) / 2, sm_count, TVF_S1M_TMA_MINB);
         tft_moments_tma_kernel<<<gt, CORE_WARPS * 32, dyn, stream>>>(in, ws);
         return 1;

@@ -215,4 +215,17 @@ constexpr int SWEEP_MAX_N = 60;      // n + 100 points per scene must fit the pe
 void launch_sweep_trials(long long first_trial, long long B, int n, const double* d_noise_levels, int L, const double* d_P,
                          double hi_x, double hi_y, double* d_out, cudaStream_t stream);
 
+// Opts `kernel` in to all the dynamic shared memory the current device allows, for a kernel whose size depends on n.  The
+// attribute belongs to the function and the device, not to the calling thread: the members of a group handle on one
+// device launch concurrently with different n, and setting each launch's own size let one member lower the limit just
+// before another's larger launch (cudaErrorInvalidValue, or outputs left unwritten).  Every caller sets the same value.
+template <class Kernel> inline void allow_max_dynamic_smem(Kernel kernel) {
+    int dev = 0, optin = 0;
+    cudaFuncAttributes fa{};
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    cudaFuncGetAttributes(&fa, kernel);
+    cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)fa.sharedSizeBytes);
+}
+
 }  // namespace tvf

@@ -836,7 +836,7 @@ static void launch_fused_t(const PoseTailArgs& a, int sm_count, cudaStream_t str
     const unsigned grid = grid_for(a.B, ppb, (long long)sm_count * 16 * (THREADS == PT_THREADS ? TVF_TAIL_MINB : TVF_TAIL_MINB_SMALL));
     const size_t dyn = 2 * (size_t)ppb * ((size_t)a.n * 48 + CAND_SIZE * 8);      // two stages of points + candidate records
     // (set on every launch: the attribute is per device and per context, a process-wide flag would miss the second GPU)
-    cudaFuncSetAttribute(pose_tail_fused_kernel<THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+    allow_max_dynamic_smem(pose_tail_fused_kernel<THREADS>);
     pose_tail_fused_kernel<THREADS><<<grid, THREADS, dyn, stream>>>(a);
 }
 
