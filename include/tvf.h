@@ -262,6 +262,58 @@ int tvf_bundle_adjust_ragged_dev(tvf_handle_t h, const double* corresp, const do
                                  const double* reconst0, double* Rt2, double* Rt3, double* reconst, double* repr_err,
                                  int32_t* iter, int32_t* status);
 
+/* ---- robust-loss bundle adjustment (M-estimation) -------------------------------------------------------------------
+ * The model of tvf_bundle_adjust (camera 1 = K1[I|0], |t2| = 1, unknowns R2, t2, R3, t3 and the points, the same gauge
+ * normalisation of the start, n >= 4), with one loss per match.  With s_i the sum of the six squared pixel residuals of
+ * match i, it minimises
+ *     cost = sum_i c^2 rho(s_i / c^2),     c = scale > 0 in pixels (the scale of a match's 6-residual norm),
+ * so a match is one unit, as in the inlier test of tvf_consensus.  The losses are SciPy's least_squares definitions:
+ *     TVF_LOSS_HUBER    rho(z) = z for z <= 1, 2 sqrt(z) - 1 otherwise    rho'(z) = min(1, 1 / sqrt(z))
+ *     TVF_LOSS_SOFT_L1  rho(z) = 2 (sqrt(1 + z) - 1)                      rho'(z) = 1 / sqrt(1 + z)
+ *     TVF_LOSS_CAUCHY   rho(z) = ln(1 + z)                                rho'(z) = 1 / (1 + z)
+ * Huber's match with s_i <= c^2 contributes exactly s_i with weight exactly 1.  There is no plain loss: that is
+ * tvf_bundle_adjust.
+ *
+ * Solver: tvf_bundle_adjust's Levenberg-Marquardt with an IRLS-weighted Gauss-Newton model.  At each linearisation
+ * every match gets w_i = rho'(s_i / c^2) at the current iterate and its residuals and Jacobian rows are scaled by
+ * sqrt(w_i) (w_i > 0: every point block stays positive definite).  The weighted g = sum_i w_i J_i' r_i is the exact
+ * gradient of (1/2) cost, so the damping schedule, the stopping rule and its constants are those of tvf_bundle_adjust,
+ * with (1/2) cost in place of (1/2) sum r^2; a step is accepted only if it lowers the cost, so the cost never exceeds
+ * the start's; a rejected step keeps the weights of its linearisation.  The model has no second-order rho'' term
+ * (Triggs' correction): that changes the path to a stationary point, not the stationary points.
+ *
+ * loss: TVF_LOSS_*; scale: finite, > 0 and with a normal c^2 (1e-154 < c < 1e154); otherwise TVF_ERR_ARG before any
+ * device work, as is n < 4.  Inputs and Rt2, Rt3, reconst, iter, status as tvf_bundle_adjust; every output except Rt2
+ * and Rt3 may be NULL.  repr_err (B) is the plain ReprError of the result over all n matches (tvf_bundle_adjust's
+ * definition); cost (B) the objective at the result; weights (n x B) rho'(s_i / c^2) at the result.  Statuses are
+ * tvf_bundle_adjust's: TVF_ST_NONFINITE copies the inputs through and sets that problem's cost and weights NaN;
+ * TVF_ST_BA_NOCONV.  Results are bit-identical whatever the batch, chunk, group-handle shard, form or the outputs
+ * requested.  The _dev form takes device pointers (corresp 16-byte aligned) and is asynchronous on the handle's
+ * stream. */
+#define TVF_LOSS_HUBER 1
+#define TVF_LOSS_SOFT_L1 2
+#define TVF_LOSS_CAUCHY 3
+int tvf_bundle_adjust_robust(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
+                             int loss, double scale, const double* Rt2_0, const double* Rt3_0, const double* reconst0,
+                             double* Rt2, double* Rt3, double* reconst, double* repr_err, double* cost, double* weights,
+                             int32_t* iter, int32_t* status);
+int tvf_bundle_adjust_robust_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n,
+                                 int64_t B, int loss, double scale, const double* Rt2_0, const double* Rt3_0,
+                                 const double* reconst0, double* Rt2, double* Rt3, double* reconst, double* repr_err,
+                                 double* cost, double* weights, int32_t* iter, int32_t* status);
+/* tvf_bundle_adjust_robust over a ragged batch (n replaced by offsets; weights 1 x offsets[B]).  A problem of n_b < 4
+ * matches: TVF_ST_TOO_FEW_MATCHES as in tvf_bundle_adjust_ragged, its cost and weights NaN.  Every other problem's
+ * results equal the uniform call's on it alone, bit for bit. */
+int tvf_bundle_adjust_robust_ragged(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched,
+                                    const int64_t* offsets, int64_t B, int loss, double scale, const double* Rt2_0,
+                                    const double* Rt3_0, const double* reconst0, double* Rt2, double* Rt3, double* reconst,
+                                    double* repr_err, double* cost, double* weights, int32_t* iter, int32_t* status);
+int tvf_bundle_adjust_robust_ragged_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched,
+                                        const int64_t* offsets, int64_t B, int loss, double scale, const double* Rt2_0,
+                                        const double* Rt3_0, const double* reconst0, double* Rt2, double* Rt3,
+                                        double* reconst, double* repr_err, double* cost, double* weights, int32_t* iter,
+                                        int32_t* status);
+
 /* ---- first-order covariance of the bundle adjustment at a state ------------------------------------------------
  * The uncertainty of tvf_bundle_adjust's result: the inverse of the Gauss-Newton matrix H = J'J of the adjustment's
  * model (pixel residuals, camera 1 = K1[I|0], |t2| = 1), taken at the given state without damping.  The state (Rt2, Rt3

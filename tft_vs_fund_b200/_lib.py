@@ -45,6 +45,7 @@ class SweepLevel(C.Structure):
 
 
 METHOD_IDS = {"tft": 1, "f": 7, "optf": 8}      # numbering of experiments.m:51-59
+LOSS_IDS = {"huber": 1, "soft_l1": 2, "cauchy": 3}   # TVF_LOSS_*: SciPy least_squares' names
 
 # name -> (restype, argtypes); mirrors include/tvf.h one to one
 _H = C.c_void_p
@@ -96,6 +97,11 @@ SIGNATURES = {
     "tvf_linear_f_pose_dev": (_I, [_H, C.c_void_p, C.c_void_p, _I, _I, _L] + [C.c_void_p] * 8),
     "tvf_bundle_adjust": (_I, [_H, _D, _D, _I, _I, _L, _D, _D, _D, _D, _D, _D, _D, _S, _S]),
     "tvf_bundle_adjust_dev": (_I, [_H, C.c_void_p, C.c_void_p, _I, _I, _L] + [C.c_void_p] * 9),
+    "tvf_bundle_adjust_robust": (_I, [_H, _D, _D, _I, _I, _L, _I, C.c_double] + [_D] * 9 + [_S, _S]),
+    "tvf_bundle_adjust_robust_dev": (_I, [_H, C.c_void_p, C.c_void_p, _I, _I, _L, _I, C.c_double] + [C.c_void_p] * 11),
+    "tvf_bundle_adjust_robust_ragged": (_I, [_H, _D, _D, _I, C.c_void_p, _L, _I, C.c_double] + [_D] * 9 + [_S, _S]),
+    "tvf_bundle_adjust_robust_ragged_dev": (_I, [_H, C.c_void_p, C.c_void_p, _I, C.c_void_p, _L, _I, C.c_double]
+                                            + [C.c_void_p] * 11),
     "tvf_ba_covariance": (_I, [_H, _D, _D, _I, _I, _L, _D, _D, _D, _D, _D, _D, _S]),
     "tvf_ba_covariance_dev": (_I, [_H, C.c_void_p, C.c_void_p, _I, _I, _L] + [C.c_void_p] * 7),
     "tvf_consensus": (_I, [_H, _D, _D, _I, _I, _L, _D, _D, C.c_double, C.c_void_p, _S]),

@@ -335,25 +335,41 @@ def AngError(R_t_true, R_t_est, device=None):
 
 
 class BundleAdjustResult(tuple):
-    """(R_t_2, R_t_3, Reconst, iter) of bundle_adjust, plus .repr_err and .status.  epfl.run_real(covariance=True) also
-    sets .sigma2 and the predicted RMS errors .pred_rot_err, .pred_t_err (degrees, mean of views 2 and 3)."""
+    """(R_t_2, R_t_3, Reconst, iter) of bundle_adjust, plus .repr_err and .status (and, with a loss, .cost and
+    .weights).  epfl.run_real(covariance=True) also sets .sigma2 and the predicted RMS errors .pred_rot_err, .pred_t_err
+    (degrees, mean of views 2 and 3)."""
     repr_err = None
     status = None
+    cost = None
+    weights = None
     sigma2 = None
     pred_rot_err = None
     pred_t_err = None
 
 
-def bundle_adjust(Corresp, CalM, R_t_2, R_t_3, Reconst=None, device=None):
+def _loss_id(loss, scale):
+    if loss not in _lib.LOSS_IDS:
+        raise ValueError("loss must be one of %s, got %r" % (sorted(_lib.LOSS_IDS), loss))
+    if scale is None:
+        raise ValueError("a robust loss needs its scale (pixels)")
+    return _lib.LOSS_IDS[loss], float(scale)
+
+
+def bundle_adjust(Corresp, CalM, R_t_2, R_t_3, Reconst=None, device=None, loss=None, scale=None):
     """Three-view bundle adjustment of a pose (tvf_bundle_adjust, include/tvf.h): minimises the pixel reprojection error
     over R2, t2 (|t2| = 1), R3, t3 and the points, camera 1 fixed at K1[I|0], from the start (R_t_2, R_t_3, Reconst).
     Reconst None: the start points are triangulated from the start poses.  Not the reference's BundleAdjustment.m (which
     normalises the image data first; DESIGN.md section 8).  Returns (R_t_2, R_t_3, Reconst, iter) with .repr_err (the
     result's ReprError) and .status (TVF_ST_* bits: NONFINITE, BA_NOCONV).
     Corresp a list of 6xN_b (a ragged batch): R_t_2, R_t_3 (B,3,4), Reconst None or a list of 3xN_b; returns stacked
-    poses, Reconst as a list and (B,) iter; a problem of N_b < 4 gets TVF_ST_TOO_FEW_MATCHES (start poses, NaN points)."""
+    poses, Reconst as a list and (B,) iter; a problem of N_b < 4 gets TVF_ST_TOO_FEW_MATCHES (start poses, NaN points).
+    loss = "huber" | "soft_l1" | "cauchy" with scale c (pixels): the robust adjustment (tvf_bundle_adjust_robust), which
+    minimises sum_i c^2 rho(s_i / c^2), s_i the six squared residuals of match i, with SciPy least_squares' rho.  The
+    result then also has .cost (the objective; (B,) when batched) and .weights (rho'(s_i / c^2) per match: (N,), (B,N),
+    or a list of (N_b,) for a ragged batch); .repr_err stays the plain ReprError over all matches."""
+    robust = None if loss is None else _loss_id(loss, scale)
     if _ragged(Corresp):
-        return _bundle_adjust_ragged(Corresp, CalM, R_t_2, R_t_3, Reconst, device)
+        return _bundle_adjust_ragged(Corresp, CalM, R_t_2, R_t_3, Reconst, device, robust)
     c, batched, B = _cm(Corresp, 2)
     if c.shape[2] != 6:
         raise ValueError("Corresp must be 6xN")
@@ -371,16 +387,24 @@ def bundle_adjust(Corresp, CalM, R_t_2, R_t_3, Reconst=None, device=None):
     h = _lib.handle(device)
     Rt2 = np.empty((B, 12)); Rt3 = np.empty((B, 12)); Rec = np.empty((B, 3 * n)); rep = np.empty(B)
     its = np.zeros(B, dtype=np.int32); st = np.zeros(B, dtype=np.int32)
-    h.call("tvf_bundle_adjust", _p(c), _p(calm), cb, n, B, _p(r2), _p(r3), _p(x0), _p(Rt2), _p(Rt3), _p(Rec), _p(rep),
-           its.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
+    if robust is None:
+        h.call("tvf_bundle_adjust", _p(c), _p(calm), cb, n, B, _p(r2), _p(r3), _p(x0), _p(Rt2), _p(Rt3), _p(Rec), _p(rep),
+               its.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
+    else:
+        cost = np.empty(B); w = np.empty((B, n))
+        h.call("tvf_bundle_adjust_robust", _p(c), _p(calm), cb, n, B, robust[0], robust[1], _p(r2), _p(r3), _p(x0), _p(Rt2),
+               _p(Rt3), _p(Rec), _p(rep), _p(cost), _p(w), its.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
     out = BundleAdjustResult((_from_cm(Rt2, B, (3, 4), batched), _from_cm(Rt3, B, (3, 4), batched),
                               _from_cm(Rec, B, (3, n), batched), its if batched else int(its[0])))
     out.repr_err = rep if batched else float(rep[0])
     out.status = st if batched else int(st[0])
+    if robust is not None:
+        out.cost = cost if batched else float(cost[0])
+        out.weights = w if batched else w[0]
     return out
 
 
-def _bundle_adjust_ragged(Corresp, CalM, R_t_2, R_t_3, Reconst, device):
+def _bundle_adjust_ragged(Corresp, CalM, R_t_2, R_t_3, Reconst, device, robust=None):
     c, offs = _pack(Corresp, 6)
     B = len(Corresp)
     calm, cb = _calm(CalM, B)
@@ -393,11 +417,19 @@ def _bundle_adjust_ragged(Corresp, CalM, R_t_2, R_t_3, Reconst, device):
     h = _lib.handle(device)
     Rt2 = np.empty((B, 12)); Rt3 = np.empty((B, 12)); Rec = np.empty(3 * offs[-1]); rep = np.empty(B)
     its = np.zeros(B, dtype=np.int32); st = np.zeros(B, dtype=np.int32)
-    h.call("tvf_bundle_adjust_ragged", _p(c), _p(calm), cb, _vp(offs), B, _p(r2), _p(r3), _p(x0), _p(Rt2), _p(Rt3), _p(Rec),
-           _p(rep), its.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
+    if robust is None:
+        h.call("tvf_bundle_adjust_ragged", _p(c), _p(calm), cb, _vp(offs), B, _p(r2), _p(r3), _p(x0), _p(Rt2), _p(Rt3),
+               _p(Rec), _p(rep), its.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
+    else:
+        cost = np.empty(B); w = np.empty(offs[-1])
+        h.call("tvf_bundle_adjust_robust_ragged", _p(c), _p(calm), cb, _vp(offs), B, robust[0], robust[1], _p(r2), _p(r3),
+               _p(x0), _p(Rt2), _p(Rt3), _p(Rec), _p(rep), _p(cost), _p(w), its.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
     out = BundleAdjustResult((_from_cm(Rt2, B, (3, 4), True), _from_cm(Rt3, B, (3, 4), True), _unpack(Rec, offs, (3,)), its))
     out.repr_err = rep
     out.status = st
+    if robust is not None:
+        out.cost = cost
+        out.weights = [w[offs[b]:offs[b + 1]].copy() for b in range(B)]
     return out
 
 

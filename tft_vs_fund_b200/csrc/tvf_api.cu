@@ -749,6 +749,46 @@ struct BundleAdjust {
     }
 };
 
+// the robust-loss adjustment: BundleAdjust's arrays, work space and checks, plus the loss and two outputs that may be
+// null, cost (per problem) and weights (per match).  BundleAdjust's own chunk budget is left as it is.
+struct BundleAdjustRobust : BundleAdjust {
+    BaRobustArgs rio;
+    BaRobustArgs rd{};
+    int check(tvf_handle_t h, int64_t B) const {
+        if (!h) return TVF_ERR_ARG;
+        if (rio.loss < TVF_LOSS_HUBER || rio.loss > TVF_LOSS_CAUCHY)
+            return fail(h, TVF_ERR_ARG, "bundle_adjust_robust: loss must be TVF_LOSS_HUBER, TVF_LOSS_SOFT_L1 or TVF_LOSS_CAUCHY");
+        const double c2 = rio.scale * rio.scale;       // the kernel divides by c^2: a normal number, so z = s / c^2 is exact
+        if (!(rio.scale > 0.0) || !(c2 >= 2.2250738585072014e-308 && c2 <= 1.79769313486231570e308))
+            return fail(h, TVF_ERR_ARG, "bundle_adjust_robust: scale must be finite and > 0 (1e-154 < scale < 1e154)");
+        return BundleAdjust::check(h, B);
+    }
+    size_t budget(bool host_io) const {
+        return BundleAdjust::budget(host_io) + (host_io ? (size_t)(1 + io.n) * sizeof(double) : 0);
+    }
+    size_t budget_match(bool host_io) const { return BundleAdjust::budget_match(host_io) + (host_io ? sizeof(double) : 0); }
+    size_t carve(char* base, int64_t C, int64_t M, bool host_io = true) {
+        Carver c(base);
+        c.off = BundleAdjust::carve(base, C, M, host_io);
+        rd = rio;
+        if (host_io) {
+            rd.cost = c.take<double>(C);
+            rd.weights = rio.weights ? c.take<double>((size_t)(rg.offs ? M : (int64_t)io.n * C)) : nullptr;
+        }
+        return c.off;
+    }
+    template <class F> void arrays(F&& f) {
+        BundleAdjust::arrays(f);
+        f(rio.cost, Arr::output(8, rd.cost));
+        f(rio.weights, Arr::points(rg, io.n, 8, rd.weights, true));
+    }
+    int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
+        BaArgs a = d; a.B = Bc;
+        return ba_launched(h, launch_bundle_adjust_robust(a, rd, st),
+                           rg.offs ? "bundle_adjust_robust_ragged_kernel" : "bundle_adjust_robust_kernel");
+    }
+};
+
 // the state Rt2, Rt3, X is required; every output may be null
 struct Covariance {
     BaCovArgs io;
@@ -1960,6 +2000,51 @@ int tvf_bundle_adjust_ragged_dev(tvf_handle_t h, const double* corresp, const do
                           status}};
     c.rg.offs = offsets;
     return ba_dev(h, c, B);
+}
+
+static int ba_robust_call(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
+                          int loss, double scale, const double* Rt2_0, const double* Rt3_0, const double* reconst0,
+                          double* Rt2, double* Rt3, double* reconst, double* repr_err, double* cost, double* weights,
+                          int32_t* iter, int32_t* status, bool dev, const int64_t* offsets = nullptr) {
+    BundleAdjustRobust c{};
+    c.io = BaArgs{corresp, calm, calm_batched, n, 0, Rt2_0, Rt3_0, reconst0, Rt2, Rt3, reconst, nullptr, repr_err, iter,
+                  status};
+    c.rio = BaRobustArgs{loss, scale, cost, weights};
+    c.rg.offs = offsets;
+    return dev ? ba_dev(h, c, B) : host_call(h, c, B);
+}
+
+int tvf_bundle_adjust_robust(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,
+                             int loss, double scale, const double* Rt2_0, const double* Rt3_0, const double* reconst0,
+                             double* Rt2, double* Rt3, double* reconst, double* repr_err, double* cost, double* weights,
+                             int32_t* iter, int32_t* status) {
+    return ba_robust_call(h, corresp, calm, calm_batched, n, B, loss, scale, Rt2_0, Rt3_0, reconst0, Rt2, Rt3, reconst,
+                          repr_err, cost, weights, iter, status, false);
+}
+
+int tvf_bundle_adjust_robust_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n,
+                                 int64_t B, int loss, double scale, const double* Rt2_0, const double* Rt3_0,
+                                 const double* reconst0, double* Rt2, double* Rt3, double* reconst, double* repr_err,
+                                 double* cost, double* weights, int32_t* iter, int32_t* status) {
+    return ba_robust_call(h, corresp, calm, calm_batched, n, B, loss, scale, Rt2_0, Rt3_0, reconst0, Rt2, Rt3, reconst,
+                          repr_err, cost, weights, iter, status, true);
+}
+
+int tvf_bundle_adjust_robust_ragged(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched,
+                                    const int64_t* offsets, int64_t B, int loss, double scale, const double* Rt2_0,
+                                    const double* Rt3_0, const double* reconst0, double* Rt2, double* Rt3, double* reconst,
+                                    double* repr_err, double* cost, double* weights, int32_t* iter, int32_t* status) {
+    return ba_robust_call(h, corresp, calm, calm_batched, 0, B, loss, scale, Rt2_0, Rt3_0, reconst0, Rt2, Rt3, reconst,
+                          repr_err, cost, weights, iter, status, false, offsets);
+}
+
+int tvf_bundle_adjust_robust_ragged_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched,
+                                        const int64_t* offsets, int64_t B, int loss, double scale, const double* Rt2_0,
+                                        const double* Rt3_0, const double* reconst0, double* Rt2, double* Rt3,
+                                        double* reconst, double* repr_err, double* cost, double* weights, int32_t* iter,
+                                        int32_t* status) {
+    return ba_robust_call(h, corresp, calm, calm_batched, 0, B, loss, scale, Rt2_0, Rt3_0, reconst0, Rt2, Rt3, reconst,
+                          repr_err, cost, weights, iter, status, true, offsets);
 }
 
 int tvf_ba_covariance_ragged(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, const int64_t* offsets,

@@ -305,6 +305,51 @@ TVF_HD bool ba_solve_reduced(double* red, double mu, double* dc) {
     return finite;
 }
 
+// ---- robust losses (tvf_bundle_adjust_robust) --------------------------------------------------------------------
+// One loss per match: the match's cost is c^2 rho(s / c^2), s = ba_point_cost (its six squared residuals), with SciPy's
+// least_squares definitions of rho.  The IRLS weight w = rho'(s / c^2) scales the match's residuals and Jacobian rows by
+// sqrt(w) (ba_point_weigh), so every sum of the elimination is w times the plain one and g is the gradient of (1/2) cost.
+constexpr int BA_LOSS_HUBER = 1, BA_LOSS_SOFT_L1 = 2, BA_LOSS_CAUCHY = 3;     // TVF_LOSS_*
+
+// c^2 rho(s / c^2); Huber's quadratic branch returns s itself
+TVF_HD double ba_loss_cost(int loss, double s, double c2) {
+    const double z = s / c2;
+    if (loss == BA_LOSS_HUBER) return (s <= c2) ? s : c2 * (2.0 * sqrt(z) - 1.0);
+    if (loss == BA_LOSS_SOFT_L1) return c2 * (2.0 * (sqrt(1.0 + z) - 1.0));
+    return c2 * log1p(z);
+}
+
+// rho'(s / c^2); Huber's quadratic branch returns exactly 1
+TVF_HD double ba_loss_weight(int loss, double s, double c2) {
+    const double z = s / c2;
+    if (loss == BA_LOSS_HUBER) return (s <= c2) ? 1.0 : 1.0 / sqrt(z);
+    if (loss == BA_LOSS_SOFT_L1) return 1.0 / sqrt(1.0 + z);
+    return 1.0 / (1.0 + z);
+}
+
+// the match's weight at its residuals p.r; p's residuals and Jacobian blocks are scaled by sqrt(w) in place
+TVF_HD double ba_point_weigh(BaPoint& p, int loss, double c2) {
+    double s = 0.0;                       // summed view by view, as ba_point_cost does
+#pragma unroll
+    for (int k = 0; k < 6; k += 2) s += p.r[k] * p.r[k] + p.r[k + 1] * p.r[k + 1];
+    const double w = ba_loss_weight(loss, s, c2);
+    const double q = sqrt(w);
+#pragma unroll
+    for (int k = 0; k < 6; ++k) {
+        p.r[k] *= q;
+#pragma unroll
+        for (int j = 0; j < 3; ++j) p.Jp[k][j] *= q;
+    }
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+#pragma unroll
+        for (int j = 0; j < 5; ++j) p.J2[k][j] *= q;
+#pragma unroll
+        for (int j = 0; j < 6; ++j) p.J3[k][j] *= q;
+    }
+    return w;
+}
+
 // ---- first-order covariance at a state (tvf_ba_covariance, tvf_ba_cov_kernels.cu) -------------------------------
 // H = J'J at mu = 0.  The camera block of H^-1 is S^-1 (S = the reduced matrix of ba_point_accumulate); point i's block
 // is V_i^-1 + V_i^-1 H_pc,i S^-1 H_cp,i V_i^-1 = L^-T (I + W S^-1 W') L^-1 with V_i = L L' and W = L^-1 H_pc,i.

@@ -49,9 +49,22 @@ template <int W> __device__ __forceinline__ double group_max(double v, unsigned 
     return v;
 }
 
+// a match's share of the objective: its six squared residuals, or c^2 rho(s / c^2) for the robust adjustment
+template <bool Robust> __device__ __forceinline__ double match_cost(const BaCams& c, const double* X, const double* x6,
+                                                                   const BaRobustArgs& rob) {
+    const double s = ba_point_cost(c, X, x6);
+    if constexpr (Robust) return ba_loss_cost(rob.loss, s, rob.scale * rob.scale);
+    else return s;
+}
+
 // the problems of one group of W lanes (mask gm) in a grid-stride loop; lane = the lane within the group.  Ragged: problem
-// prob owns matches a.offs[prob] .. a.offs[prob+1]-1 (n varies per problem); the uniform form indexes by prob * a.n
-template <int W, bool Ragged> __device__ __forceinline__ void ba_problems(const BaArgs& a) {
+// prob owns matches a.offs[prob] .. a.offs[prob+1]-1 (n varies per problem); the uniform form indexes by prob * a.n.
+// Robust: the objective is sum c^2 rho(s_i / c^2) (rob.loss, rob.scale); each linearisation weighs every match's residuals
+// and Jacobian rows by sqrt(rho'(s_i / c^2)) at the current iterate (IRLS), in pass A and pass B alike, so both passes
+// form the same elimination from the same inputs.  F is (1/2) cost and the weighted g its gradient, so the schedule and
+// the stopping rule are the plain adjustment's.
+template <int W, bool Ragged, bool Robust = false>
+__device__ __forceinline__ void ba_problems(const BaArgs& a, const BaRobustArgs& rob = BaRobustArgs{}) {
     extern __shared__ __align__(16) double ba_smem[];
     constexpr int G = BA_WARPS * 32 / W;               // groups (problems in flight) per block
     const int lane = threadIdx.x & (W - 1), grp = threadIdx.x / W;
@@ -79,6 +92,10 @@ template <int W, bool Ragged> __device__ __forceinline__ void ba_problems(const 
             const double qnan = __longlong_as_double(0x7ff8000000000000LL);
             for (int e = lane; e < 12; e += W) { a.Rt2[prob * 12 + e] = rt2[e]; a.Rt3[prob * 12 + e] = rt3[e]; }
             for (int e = lane; e < 3 * n; e += W) Xp[e] = qnan;
+            if constexpr (Robust) {
+                if (rob.weights) for (int e = lane; e < n; e += W) rob.weights[off + e] = qnan;
+                if (lane == 0 && rob.cost) rob.cost[prob] = qnan;
+            }
             if (lane == 0) {
                 if (a.repr_err) a.repr_err[prob] = qnan;
                 if (a.iter) a.iter[prob] = 0;
@@ -131,6 +148,11 @@ template <int W, bool Ragged> __device__ __forceinline__ void ba_problems(const 
         const bool bad = __any_sync(gm, bad_l) || !(t2n > 0.0) || !finite_(cost0);
         if (bad) {                                     // inputs copied through (the start points are already in X)
             for (int e = lane; e < 12; e += W) { a.Rt2[prob * 12 + e] = rt2[e]; a.Rt3[prob * 12 + e] = rt3[e]; }
+            if constexpr (Robust) {                    // cost and weights NaN
+                const double qnan = __longlong_as_double(0x7ff8000000000000LL);
+                if (rob.weights) for (int e = lane; e < n; e += W) rob.weights[(Ragged ? off : prob * n) + e] = qnan;
+                if (lane == 0 && rob.cost) rob.cost[prob] = qnan;
+            }
             if (lane == 0) {
                 if (a.repr_err) a.repr_err[prob] = sqrt(cost0 / (3.0 * n));
                 if (a.iter) a.iter[prob] = 0;
@@ -154,9 +176,9 @@ template <int W, bool Ragged> __device__ __forceinline__ void ba_problems(const 
             load_x6(corresp, pi, n, i, x6);
 #pragma unroll
             for (int k = 0; k < 3; ++k) { X[k] = Xp[3 * i + k] * gs; Xp[3 * i + k] = X[k]; }
-            cost_l += ba_point_cost(cur, X, x6);
+            cost_l += match_cost<Robust>(cur, X, x6, rob);
         }
-        double F = 0.5 * group_sum<W>(cost_l, gm);           // (1/2) sum of squared residuals
+        double F = 0.5 * group_sum<W>(cost_l, gm);           // (1/2) sum of squared residuals (robust: (1/2) cost)
 
         // ---- Levenberg-Marquardt ---------------------------------------------------------------------------------
         double mu = BA_MU0, nu = 2.0, gmax0 = -1.0;
@@ -173,6 +195,7 @@ template <int W, bool Ragged> __device__ __forceinline__ void ba_problems(const 
                 const double X[3] = {Xp[3 * i], Xp[3 * i + 1], Xp[3 * i + 2]};
                 BaPoint p; BaElim el;
                 ba_point_jac(cur, X, x6, p);
+                if constexpr (Robust) ba_point_weigh(p, rob.loss, rob.scale * rob.scale);
                 pd_l = ba_point_eliminate(p, mu, el) && pd_l;
                 ba_point_accumulate(p, el, acc);
                 gp_l = fmax(gp_l, fmax(fabs(el.g[0]), fmax(fabs(el.g[1]), fabs(el.g[2]))));
@@ -210,6 +233,7 @@ template <int W, bool Ragged> __device__ __forceinline__ void ba_problems(const 
                     const double X[3] = {Xp[3 * i], Xp[3 * i + 1], Xp[3 * i + 2]};
                     BaPoint p; BaElim el;
                     ba_point_jac(cur, X, x6, p);
+                    if constexpr (Robust) ba_point_weigh(p, rob.loss, rob.scale * rob.scale);
                     ba_point_eliminate(p, mu, el);
                     double dX[3], Xn[3];
                     ba_point_step(el, dc, dX);
@@ -221,7 +245,7 @@ template <int W, bool Ragged> __device__ __forceinline__ void ba_problems(const 
                         s2_l += dX[k] * dX[k];
                         x2_l += X[k] * X[k];
                     }
-                    cn_l += ba_point_cost(cand, Xn, x6);
+                    cn_l += match_cost<Robust>(cand, Xn, x6, rob);
                 }
                 const double Fn = 0.5 * group_sum<W>(cn_l, gm);
                 double pred = group_sum<W>(pr_l, gm), step2 = group_sum<W>(s2_l, gm), xn2 = group_sum<W>(x2_l, gm);
@@ -262,7 +286,24 @@ template <int W, bool Ragged> __device__ __forceinline__ void ba_problems(const 
             a.Rt2[prob * 12 + e] = (e < 9) ? cur.R2[e] : cur.t2[e - 9];
             a.Rt3[prob * 12 + e] = (e < 9) ? cur.R3[e] : cur.t3[e - 9];
         }
-        if (lane == 0) {
+        if constexpr (Robust) {                        // the weights and the plain ReprError at the result
+            double s_l = 0.0;
+            for (int i = lane; i < n; i += W) {
+                double x6[6];
+                load_x6(corresp, pi, n, i, x6);
+                const double X[3] = {Xp[3 * i], Xp[3 * i + 1], Xp[3 * i + 2]};
+                const double s = ba_point_cost(cur, X, x6);
+                if (rob.weights) rob.weights[(Ragged ? off : prob * n) + i] = ba_loss_weight(rob.loss, s, rob.scale * rob.scale);
+                s_l += s;
+            }
+            const double s_all = group_sum<W>(s_l, gm);
+            if (lane == 0) {
+                if (a.repr_err) a.repr_err[prob] = sqrt(s_all / (3.0 * n));
+                if (rob.cost) rob.cost[prob] = 2.0 * F;
+                if (a.iter) a.iter[prob] = lin;
+                if (a.status) a.status[prob] = st;
+            }
+        } else if (lane == 0) {
             if (a.repr_err) a.repr_err[prob] = sqrt(2.0 * F / (3.0 * n));        // ReprError.m:65
             if (a.iter) a.iter[prob] = lin;
             if (a.status) a.status[prob] = st;
@@ -285,7 +326,16 @@ __global__ void __launch_bounds__(BA_WARPS * 32) bundle_adjust_ragged_kernel(con
 //   - every vote (__any_sync) of the idle lanes is false, and every other step is done by lane 0 or per point.
 __global__ void __launch_bounds__(BA_WARPS * 32) bundle_adjust_small_kernel(const BaArgs a) { ba_problems<BA_SMALL_N, false>(a); }
 
-template <int W> int launch_groups(void (*kernel)(const BaArgs), const BaArgs& a, cudaStream_t stream) {
+// the robust-loss adjustment (tvf_bundle_adjust_robust), uniform and ragged; the loss id is warp-uniform
+__global__ void __launch_bounds__(BA_WARPS * 32) bundle_adjust_robust_kernel(const BaArgs a, const BaRobustArgs rob) {
+    ba_problems<32, false, true>(a, rob);
+}
+__global__ void __launch_bounds__(BA_WARPS * 32) bundle_adjust_robust_ragged_kernel(const BaArgs a, const BaRobustArgs rob) {
+    ba_problems<32, true, true>(a, rob);
+}
+
+template <int W, class Kernel, class... Extra>
+int launch_groups(Kernel kernel, const BaArgs& a, cudaStream_t stream, const Extra&... extra) {
     if (a.B <= 0) return 1;
     constexpr int G = BA_WARPS * 32 / W;
     const size_t smem = (size_t)G * BA_PER_GROUP<W> * sizeof(double);
@@ -296,7 +346,7 @@ template <int W> int launch_groups(void (*kernel)(const BaArgs), const BaArgs& a
     }
     long long blocks = (a.B + G - 1) / G;              // one problem per group: the block scheduler balances
     if (blocks > 0x7fffffffLL) blocks = 0x7fffffffLL;  // problems of different iteration counts
-    kernel<<<(unsigned)blocks, BA_WARPS * 32, smem, stream>>>(a);
+    kernel<<<(unsigned)blocks, BA_WARPS * 32, smem, stream>>>(a, extra...);
     return cudaPeekAtLastError() == cudaSuccess ? 1 : 0;
 }
 
@@ -307,6 +357,10 @@ int launch_bundle_adjust(const BaArgs& a, cudaStream_t stream) {
 int launch_bundle_adjust_small(const BaArgs& a, cudaStream_t stream) {
     if (a.n > BA_SMALL_N) return 0;
     return launch_groups<BA_SMALL_N>(bundle_adjust_small_kernel, a, stream);
+}
+
+int launch_bundle_adjust_robust(const BaArgs& a, const BaRobustArgs& r, cudaStream_t stream) {
+    return launch_groups<32>(a.offs ? bundle_adjust_robust_ragged_kernel : bundle_adjust_robust_kernel, a, stream, r);
 }
 
 }  // namespace tvf

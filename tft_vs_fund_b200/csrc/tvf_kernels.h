@@ -74,6 +74,16 @@ int launch_bundle_adjust(const BaArgs& a, cudaStream_t stream);
 // for a larger n or a failed launch
 constexpr int BA_SMALL_N = 8;
 int launch_bundle_adjust_small(const BaArgs& a, cudaStream_t stream);
+// the robust-loss adjustment (tvf_bundle_adjust_robust): the loss and the extra outputs are a kernel parameter of their
+// own, so BaArgs, and with it the plain kernels' parameters, stay as they are
+struct BaRobustArgs {
+    int loss;                  // BA_LOSS_* of tvf_ba.cuh (= TVF_LOSS_*)
+    double scale;              // c > 0, pixels
+    double* cost;              // B: sum of c^2 rho(s_i / c^2) at the result; may be null
+    double* weights;           // n x B (ragged: offs[B]): rho'(s_i / c^2) at the result; may be null
+};
+// offs != null: bundle_adjust_robust_ragged_kernel
+int launch_bundle_adjust_robust(const BaArgs& a, const BaRobustArgs& r, cudaStream_t stream);
 
 // ---- covariance of the bundle adjustment at a state (tvf_ba_cov_kernels.cu).  Device pointers; cov_cam, cov_pts,
 // sigma2 and status may be null.  Returns 0 if the launch failed.
