@@ -372,7 +372,9 @@ int tvf_consensus_ragged(tvf_handle_t h, const double* corresp, const double* ca
 #define TVF_ST_RANSAC_FAILED 128 /* tvf_ransac_pose: every hypothesis of the problem was flagged: no pose           */
 
 /* Pose of each problem from raw matches with outliers: RANSAC over minimal linear solves and the consensus above.
- * method 1: hypotheses from LinearTFTPoseEstimation on s = 7 matches; 7: LinearFPoseEstimation on s = 8 (linearF.m:35-37).
+ * method 1: hypotheses from LinearTFTPoseEstimation on s = 7 matches; 7: LinearFPoseEstimation on s = 8 (linearF.m:35-37);
+ * 9: tvf_five_point_pose on s = 5 (below), whose refit is LinearFPoseEstimation and runs only on a consensus of >= 8
+ * matches (otherwise the best hypothesis is returned).
  * Per problem b, with key seeds[b]:
  *   1. hypothesis h = 0 .. hypotheses-1 draws s distinct match indices (below) and solves the method on those columns;
  *   2. its score is its consensus count with `threshold`, or -1 when the method flagged it (status != 0);
@@ -387,7 +389,7 @@ int tvf_consensus_ragged(tvf_handle_t h, const double* corresp, const double* ca
  * r = mix64(seed ^ mix64((h << 8) | j)); uniform(m) = ((r >> 32) * m) >> 32; the indices come from Floyd's algorithm: for
  * j = 0 .. s-1, m = n - s + j + 1, u = uniform(m), take u, or m - 1 if u was already taken; kept in draw order.
  * The key is per problem, so a result does not depend on its batch, chunk, shard or form (bit-identical).
- * Errors: method other than 1 or 7, hypotheses outside 1 .. 2^24, a threshold that is not finite or <= 0, or n < s
+ * Errors: method other than 1, 7 or 9, hypotheses outside 1 .. 2^24, a threshold that is not finite or <= 0, or n < s
  * (method 7: TVF_ERR_TOO_FEW_POINTS) -> TVF_ERR_ARG.  Outputs may be NULL.  The host form chunks and shards like
  * tvf_pose.  The _dev form takes device pointers (corresp 16-byte aligned) and, unlike the other _dev forms,
  * synchronises the handle's stream once per chunk: the refit groups the problems by consensus size, which it reads back. */
@@ -407,6 +409,35 @@ int tvf_ransac_pose_ragged_dev(tvf_handle_t h, int method, const double* corresp
                                const int64_t* offsets, int64_t B, int hypotheses, double threshold, const uint64_t* seeds,
                                double* Rt2, double* Rt3, uint8_t* inliers, int32_t* n_inliers, int32_t* sample,
                                int32_t* status);
+
+/* Calibrated five-point minimal three-view pose (Nistér 2004; Stewénius et al. 2006), the hypotheses of RANSAC method 9.
+ * corresp 6 x 5 x B (one sample of 5 matches per problem, in the sampler's draw order); calm 9 x 3 or 9 x 3 x B.  Per
+ * problem, with view 1 = K1[I|0]:
+ *   1. rays q = K^-1 [x y 1]' in every view;
+ *   2. the 4-dimensional null space {X, Y, Z, W} of the 5 x 9 epipolar system q2' E q1 = 0 of views 1, 2 (Householder
+ *      QR of its transpose);
+ *   3. E = x X + y Y + z Z + W: det E = 0 and 2 E E' E - tr(E E') E = 0 give ten cubics, a 10 x 20 matrix reduced by
+ *      Gauss-Jordan with partial pivoting (a zero pivot: TVF_ST_NO_POSE_2, n_E 0);
+ *   4. Nistér's 3 x 3 polynomial matrix in z gives a degree-10 polynomial whose real roots (Sturm sequences, bisection
+ *      and Newton) are taken in ascending z; n_E (0 .. 10) is their count;
+ *   5. one E per root, unit Frobenius norm, its largest-magnitude entry positive (the first of equal ones); E holds
+ *      them in root order, NaN after the n_E-th;
+ *   6. view 2: each E is decomposed as the linear F method does; the first of (R, t), (R, -t), (Rp, -t), (Rp, t) that
+ *      puts all 5 points (two-view DLT, unit-norm X) in front of views 1 and 2 is kept, |t2| = 1; a point with
+ *      |X(4)| <= 1e-12 (at infinity: no parallax) is in front of neither view; an E without such a candidate is dropped;
+ *   7. view 3: P3P (Lambda Twist) on columns 0, 1, 2 of the triangulated points, up to 4 roots; a root that puts any of
+ *      the 5 points behind view 3 is dropped; t3 is in the scale of t2;
+ *   8. the pose is the surviving (E, P3P root) pair with the smallest largest view-3 reprojection error (Euclidean,
+ *      pixels) of columns 3 and 4; ties to the earlier E, then the earlier root.
+ * status: 0; TVF_ST_NO_POSE_2 when no E survives step 6; TVF_ST_NO_POSE_3 when no P3P root survives; TVF_ST_NONFINITE
+ * for a non-finite pose.  The pose (Rt2, Rt3 3 x 4 x B) is NaN whenever status != 0.  Every output may be NULL.  E is
+ * 3 x 3 x 10 x B, n_E B.  A result is bit-identical whatever its batch, chunk, group-handle shard or form, and equals
+ * RANSAC method 9's hypothesis on the same columns.  Returns the number of flagged problems or an error; the _dev form
+ * takes device pointers (corresp 16-byte aligned) and is asynchronous on the handle's stream. */
+int tvf_five_point_pose(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int64_t B, double* Rt2,
+                        double* Rt3, double* E, int32_t* n_E, int32_t* status);
+int tvf_five_point_pose_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int64_t B,
+                            double* Rt2, double* Rt3, double* E, int32_t* n_E, int32_t* status);
 
 /* RANSAC pose whose hypotheses and result are bundle-adjusted, with local optimisation (LO).  Arguments, checks and
  * errors as tvf_ransac_pose, plus lo_rounds (0 .. 32, else TVF_ERR_ARG) and lo_done (B, may be NULL): the number of

@@ -10,6 +10,7 @@ from .api import (  # noqa: F401
     Normalize2Ddata, transform_TFT, R_t_from_TFT, TFT_from_P, triangulation3D,
     ReprError, AngError, crossM, project3Dpoints, PoseResult, bundle_adjust, BundleAdjustResult,
     ba_covariance, CovarianceResult, pose_rms_errors, consensus, ransac_pose, RansacResult,
+    five_point_pose, FivePointResult,
 )
 from ._lib import TvfError, Handle, handle, load, LIB_PATH  # noqa: F401
 from .scene import generateSyntheticScene, sweep_batch, SceneRNG  # noqa: F401
@@ -19,6 +20,6 @@ __all__ = [
     "LinearTFTPoseEstimation", "LinearFPoseEstimation", "OptimFPoseEstimation", "linearTFT", "linearF", "optimF",
     "Normalize2Ddata", "transform_TFT", "R_t_from_TFT", "TFT_from_P",
     "triangulation3D", "ReprError", "AngError", "crossM", "project3Dpoints", "bundle_adjust",
-    "ba_covariance", "pose_rms_errors", "consensus", "ransac_pose",
+    "ba_covariance", "pose_rms_errors", "consensus", "ransac_pose", "five_point_pose",
     "generateSyntheticScene", "sweep_batch", "Handle", "handle", "TvfError",
 ]

@@ -124,6 +124,8 @@ SIGNATURES = {
                                             C.c_void_p, _S, _S, _S, _S]),
     "tvf_ransac_pose_refined_ragged_dev": (_I, [_H, _I, C.c_void_p, C.c_void_p, _I, C.c_void_p, _L, _I, C.c_double,
                                                 C.c_void_p, _I] + [C.c_void_p] * 7),
+    "tvf_five_point_pose": (_I, [_H, _D, _D, _I, _L, _D, _D, _D, _S, _S]),
+    "tvf_five_point_pose_dev": (_I, [_H, C.c_void_p, C.c_void_p, _I, _L] + [C.c_void_p] * 5),
     "tvf_launch_count": (_L, [_H]),
     "tvf_profile_enable": (_I, [_H, _I]),
     "tvf_profile_reset": (_I, [_H]),

@@ -538,14 +538,43 @@ class RansacResult(tuple):
     lo_done = None
 
 
-RANSAC_SAMPLE_SIZE = {1: 7, 7: 8}
+RANSAC_SAMPLE_SIZE = {1: 7, 7: 8, 9: 5}
+
+
+class FivePointResult(tuple):
+    """(R_t_2, R_t_3) of five_point_pose, plus .E (3x3x10, NaN after the n_E-th), .n_E and .status."""
+    E = None
+    n_E = None
+    status = None
+
+
+def five_point_pose(Corresp, CalM, device=None):
+    """Calibrated five-point minimal pose of 5 matches (tvf_five_point_pose, include/tvf.h): the essential matrices of
+    views 1-2 (Nistér), the pose of view 2 that puts the 5 points in front of both views, view 3 by P3P on matches 0-2,
+    and the (E, P3P) pair with the smallest view-3 error on matches 3-4.  Corresp 6x5 (or (B,6,5)); returns
+    (R_t_2, R_t_3) with .E (3,3,10) (or (B,3,3,10)), .n_E and .status; a flagged problem's pose is NaN.  These are RANSAC
+    method 9's hypotheses."""
+    c, batched, B = _cm(Corresp, 2)
+    if c.shape[1:] != (5, 6):
+        raise ValueError("Corresp must be 6x5")
+    calm, cb = _calm(CalM, B)
+    Rt2 = np.empty((B, 12)); Rt3 = np.empty((B, 12)); E = np.empty((B, 90))
+    nE = np.zeros(B, dtype=np.int32); st = np.zeros(B, dtype=np.int32)
+    _lib.handle(device).call("tvf_five_point_pose", _p(c), _p(calm), cb, B, _p(Rt2), _p(Rt3), _p(E),
+                             nE.ctypes.data_as(_ip), st.ctypes.data_as(_ip))
+    out = FivePointResult((_from_cm(Rt2, B, (3, 4), batched), _from_cm(Rt3, B, (3, 4), batched)))
+    out.E = _from_cm(E, B, (3, 3, 10), batched)
+    out.n_E = nE if batched else int(nE[0])
+    out.status = st if batched else int(st[0])
+    return out
 
 
 def ransac_pose(Corresp, CalM, method=1, hypotheses=1024, threshold=1.0, seed=0, device=None, refine=False, lo_rounds=8):
     """Pose from raw matches with outliers (tvf_ransac_pose, include/tvf.h): `hypotheses` minimal solves of method 1
-    (LinearTFTPoseEstimation on 7 matches) or 7 (LinearFPoseEstimation on 8), each scored by its consensus (see
-    `consensus`, `threshold` pixels); the method is then run again on the consensus of the best one and that refit is
-    kept if it explains at least as many matches.  seed: int (problem b gets the key seed + b) or an array (B,) of keys.
+    (LinearTFTPoseEstimation on 7 matches), 7 (LinearFPoseEstimation on 8) or 9 (five_point_pose on 5), each scored by
+    its consensus (see `consensus`, `threshold` pixels); the method (method 9: LinearFPoseEstimation, on a consensus of
+    at least 8) is then run again on the consensus of the best one and that refit is kept if it explains at least as
+    many matches.  seed: int (problem b gets the key seed + b) or an array (B,) of keys.
     Returns (R_t_2, R_t_3, inliers, n_inliers, sample) -- inliers bool (N), the sample the best hypothesis drew -- with
     .status; batched inputs give (B,3,4), (B,3,4), (B,N), (B,), (B,s).
     refine=True (tvf_ransac_pose_refined): each hypothesis is bundle-adjusted on its own sample before it is scored,
@@ -554,7 +583,7 @@ def ransac_pose(Corresp, CalM, method=1, hypotheses=1024, threshold=1.0, seed=0,
     Corresp a list of 6xN_b (a ragged batch): every output is batched, inliers a list of bool (N_b); a problem with
     N_b < s gets TVF_ST_TOO_FEW_MATCHES (NaN poses, no inliers, sample -1) instead of an error."""
     if method not in RANSAC_SAMPLE_SIZE:
-        raise ValueError("ransac_pose: method must be 1 (linear TFT) or 7 (linear F)")
+        raise ValueError("ransac_pose: method must be 1 (linear TFT), 7 (linear F) or 9 (five-point)")
     s = RANSAC_SAMPLE_SIZE[method]
     ragged = _ragged(Corresp)
     if ragged:

@@ -195,7 +195,7 @@ int64_t pick_chunk(tvf_handle_t h, int64_t B, bool host_io, size_t per) {
     return c;
 }
 
-enum Method { METHOD_TFT = 0, METHOD_F = 1, METHOD_OPTF = 2 };
+enum Method { METHOD_TFT = 0, METHOD_F = 1, METHOD_OPTF = 2, METHOD_FIVEPT = 3 };   // FIVEPT: RANSAC hypotheses only
 
 cudaEvent_t get_event(tvf_handle_t h) {
     if (!h->free_events.empty()) { cudaEvent_t e = h->free_events.back(); h->free_events.pop_back(); return e; }
@@ -890,6 +890,7 @@ struct Ransac {
             if (rc != TVF_OK) return rc;
         } else if (io.n < s) {
             if (method == METHOD_F) return fail(h, TVF_ERR_TOO_FEW_POINTS, TVF_LINEARF_ERRMSG);
+            if (method == METHOD_FIVEPT) return fail(h, TVF_ERR_ARG, "ransac_pose: method 9 needs n >= 5 points");
             return fail(h, TVF_ERR_ARG, "ransac_pose: method 1 needs n >= 7 points");
         }
         if (H < 1 || H > (1 << 24)) return fail(h, TVF_ERR_ARG, "ransac_pose: hypotheses must be in 1 .. 2^24");
@@ -965,9 +966,16 @@ struct Ransac {
         int rc = ransac_launched(h); if (rc) return rc;
         k = w;
         k.in = a.gin; k.calm = a.calm_batched ? a.gcalm : a.calm; k.Rt2 = a.hRt2; k.Rt3 = a.hRt3;
+        if (method == METHOD_FIVEPT) {
+            launch_five_point_pose(k.in, k.calm, a.calm_batched, a.B * H, a.hRt2, a.hRt3, nullptr, nullptr, a.hstatus, st);
+            return ransac_launched(h);
+        }
         if (method != METHOD_TFT) k.T = nullptr;
         return run_pose_chunk(h, st, method, a.calm_batched, s, a.B * H, k);
     }
+    // the refit's method and the least consensus it needs: method 9 refits with linear F on >= 8 columns
+    Method refit_method() const { return method == METHOD_FIVEPT ? METHOD_F : method; }
+    int refit_min() const { return method == METHOD_FIVEPT ? 8 : s; }
     int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
         RansacArgs a = d; a.B = Bc;
         const int64_t Q = Bc * H;
@@ -986,7 +994,7 @@ struct Ransac {
         TVF_CK(cudaStreamSynchronize(st));
         TVF_CK(cudaMemsetAsync(a.refst, 0xff, (size_t)Bc * sizeof(int), st));      // -1: no refit
         std::vector<int> order;
-        for (int64_t b = 0; b < Bc; ++b) if (cnt[(size_t)b] >= s) order.push_back((int)b);
+        for (int64_t b = 0; b < Bc; ++b) if (cnt[(size_t)b] >= refit_min()) order.push_back((int)b);
         std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return cnt[(size_t)x] < cnt[(size_t)y]; });
         if (!order.empty())
             TVF_CK(cudaMemcpyAsync(a.plist, order.data(), order.size() * sizeof(int), cudaMemcpyHostToDevice, st));
@@ -999,7 +1007,7 @@ struct Ransac {
             rc = ransac_launched(h); if (rc) return rc;
             ChunkBufs r = k;                      // the hypotheses' buffers, free again
             r.in = a.rin; r.calm = a.calm_batched ? a.rcalm : a.calm;
-            rc = run_pose_chunk(h, st, method, a.calm_batched, size, m, r); if (rc) return rc;
+            rc = run_pose_chunk(h, st, refit_method(), a.calm_batched, size, m, r); if (rc) return rc;
             launch_ransac_scatter(a, a.plist + g0, m, r.Rt2, r.Rt3, r.status, st);
             rc = ransac_launched(h); if (rc) return rc;
             g0 = g1;
@@ -1109,6 +1117,49 @@ struct RansacRefined : Ransac {
         }
         TVF_CK(cudaMemsetAsync(a.refst, 0xff, (size_t)Bc * sizeof(int), st));          // the result rule without a refit
         launch_ransac_finish(a, s, st, rg.d_offs);
+        return ransac_launched(h);
+    }
+};
+
+// tvf_five_point_pose: the minimal pose of each problem, the kernel RANSAC method 9 runs on its hypotheses
+struct FivePoint {
+    struct Io {
+        const double* corresp; const double* calm; int calm_batched;
+        double* Rt2; double* Rt3; double* E; int32_t* n_E; int32_t* status;
+    } io;
+    Io d{};
+    Ragged rg{};                          // always uniform
+    int check(tvf_handle_t h, int64_t B) const {
+        if (!h) return TVF_ERR_ARG;
+        if (!io.corresp || !io.calm) return fail(h, TVF_ERR_ARG, "five_point_pose: corresp and calm must not be NULL");
+        if (B < 0) return fail(h, TVF_ERR_ARG, "five_point_pose: B >= 0");
+        return TVF_OK;
+    }
+    int32_t*& status() { return io.status; }
+    size_t budget(bool host_io) const { return host_io ? (size_t)(30 + 27 + 24 + 9 * 10) * 8 + 2 * 4 : 0; }
+    size_t budget_match(bool) const { return 0; }
+    size_t carve(char* base, int64_t C, int64_t, bool host_io = true) {
+        Carver c(base);
+        d = io;
+        if (host_io) {
+            d.corresp = c.take<double>(30 * C); d.calm = c.take<double>(io.calm_batched ? 27 * C : 27);
+            d.Rt2 = io.Rt2 ? c.take<double>(12 * C) : nullptr; d.Rt3 = io.Rt3 ? c.take<double>(12 * C) : nullptr;
+            d.E = io.E ? c.take<double>(90 * C) : nullptr; d.n_E = io.n_E ? c.take<int32_t>(C) : nullptr;
+            d.status = c.take<int32_t>(C);
+        }
+        return c.off;
+    }
+    template <class F> void arrays(F&& f) {
+        f(io.corresp, Arr::input(8 * 30, d.corresp));
+        f(io.calm, Arr::input(8 * 27, d.calm, !io.calm_batched));
+        f(io.Rt2, Arr::output(8 * 12, d.Rt2));
+        f(io.Rt3, Arr::output(8 * 12, d.Rt3));
+        f(io.E, Arr::output(8 * 90, d.E));
+        f(io.n_E, Arr::output(4, d.n_E));
+        f(io.status, Arr::output(4, d.status));
+    }
+    int launch(tvf_handle_t h, cudaStream_t st, int64_t Bc) {
+        launch_five_point_pose(d.corresp, d.calm, d.calm_batched, Bc, d.Rt2, d.Rt3, d.E, d.n_E, d.status, st);
         return ransac_launched(h);
     }
 };
@@ -2063,16 +2114,20 @@ int tvf_ba_covariance_ragged_dev(tvf_handle_t h, const double* corresp, const do
     return ba_dev(h, c, B);
 }
 
+static Method ransac_method(int method) { return method == 1 ? METHOD_TFT : (method == 7 ? METHOD_F : METHOD_FIVEPT); }
+static int ransac_sample_size(int method) { return method == 1 ? 7 : (method == 7 ? 8 : 5); }
+
 static int ransac_call(tvf_handle_t h, int method, const double* corresp, const double* calm, int calm_batched, int n,
                        int64_t B, int hypotheses, double threshold, const uint64_t* seeds, double* Rt2, double* Rt3,
                        uint8_t* inliers, int32_t* n_inliers, int32_t* sample, int32_t* status, bool dev,
                        const int64_t* offsets = nullptr) {
     if (!h) return TVF_ERR_ARG;
-    if (method != 1 && method != 7) return fail(h, TVF_ERR_ARG, "ransac_pose: method must be 1 (linear TFT) or 7 (linear F)");
+    if (method != 1 && method != 7 && method != 9)
+        return fail(h, TVF_ERR_ARG, "ransac_pose: method must be 1 (linear TFT), 7 (linear F) or 9 (five-point)");
     RansacArgs io{};
     io.corresp = corresp; io.calm = calm; io.calm_batched = calm_batched; io.n = n; io.seeds = seeds;
     io.Rt2 = Rt2; io.Rt3 = Rt3; io.inliers = inliers; io.n_inliers = n_inliers; io.sample = sample; io.status = status;
-    Ransac c{method == 1 ? METHOD_TFT : METHOD_F, method == 1 ? 7 : 8, hypotheses, threshold, io};
+    Ransac c{ransac_method(method), ransac_sample_size(method), hypotheses, threshold, io};
     c.rg.offs = offsets;
     return dev ? ba_dev(h, c, B) : host_call(h, c, B);
 }
@@ -2096,12 +2151,13 @@ static int ransac_refined_call(tvf_handle_t h, int method, const double* corresp
                                double* Rt2, double* Rt3, uint8_t* inliers, int32_t* n_inliers, int32_t* sample,
                                int32_t* lo_done, int32_t* status, bool dev, const int64_t* offsets = nullptr) {
     if (!h) return TVF_ERR_ARG;
-    if (method != 1 && method != 7) return fail(h, TVF_ERR_ARG, "ransac_pose: method must be 1 (linear TFT) or 7 (linear F)");
+    if (method != 1 && method != 7 && method != 9)
+        return fail(h, TVF_ERR_ARG, "ransac_pose: method must be 1 (linear TFT), 7 (linear F) or 9 (five-point)");
     RansacArgs io{};
     io.corresp = corresp; io.calm = calm; io.calm_batched = calm_batched; io.n = n; io.seeds = seeds;
     io.Rt2 = Rt2; io.Rt3 = Rt3; io.inliers = inliers; io.n_inliers = n_inliers; io.sample = sample; io.status = status;
     io.lo_done = lo_done;
-    RansacRefined c{Ransac{method == 1 ? METHOD_TFT : METHOD_F, method == 1 ? 7 : 8, hypotheses, threshold, io}, lo_rounds};
+    RansacRefined c{Ransac{ransac_method(method), ransac_sample_size(method), hypotheses, threshold, io}, lo_rounds};
     c.rg.offs = offsets;
     return dev ? ba_dev(h, c, B) : host_call(h, c, B);
 }
@@ -2151,6 +2207,16 @@ int tvf_ransac_pose_refined_ragged_dev(tvf_handle_t h, int method, const double*
                                        int32_t* n_inliers, int32_t* sample, int32_t* lo_done, int32_t* status) {
     return ransac_refined_call(h, method, corresp, calm, calm_batched, 0, B, hypotheses, threshold, seeds, lo_rounds, Rt2,
                                Rt3, inliers, n_inliers, sample, lo_done, status, true, offsets);
+}
+
+int tvf_five_point_pose(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int64_t B, double* Rt2,
+                        double* Rt3, double* E, int32_t* n_E, int32_t* status) {
+    return host_call(h, FivePoint{{corresp, calm, calm_batched, Rt2, Rt3, E, n_E, status}}, B);
+}
+
+int tvf_five_point_pose_dev(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int64_t B,
+                            double* Rt2, double* Rt3, double* E, int32_t* n_E, int32_t* status) {
+    return ba_dev(h, FivePoint{{corresp, calm, calm_batched, Rt2, Rt3, E, n_E, status}}, B);
 }
 
 int tvf_consensus(tvf_handle_t h, const double* corresp, const double* calm, int calm_batched, int n, int64_t B,

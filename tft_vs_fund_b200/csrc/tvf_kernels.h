@@ -166,6 +166,12 @@ void launch_ransac_lo_accept(const RansacArgs& a, cudaStream_t stream, const lon
 // the result rule (include/tvf.h, tvf_ransac_pose) -> the outputs
 void launch_ransac_finish(const RansacArgs& a, int s, cudaStream_t stream, const long long* offs = nullptr);
 
+// ---- calibrated five-point minimal pose (tvf_fivept_kernels.cu) -----------------------------
+// five_point_pose_kernel: B problems of 5 columns (in 6 x 5 x B), calm 9 x 3 (x B when calm_batched); Rt2, Rt3 3 x 4 x B,
+// E 9 x 10 x B, nE and status B, each may be null
+void launch_five_point_pose(const double* in, const double* calm, int calm_batched, long long B, double* Rt2, double* Rt3,
+                            double* E, int* nE, int* status, cudaStream_t stream);
+
 // ---- pose tail -----------------------------------------------------------------------------
 struct PoseTailArgs {
     const double* corresp;     // 6 x n x B

@@ -110,6 +110,11 @@ def consensus_stats(mask, truth):
                 recall=tp / int(np.sum(truth)) if np.any(truth) else 0.0)
 
 
+def _too_few(m, n):
+    """Method m cannot run on n matches: methods 1 / 7 as experiments_real.m:117-122, method 9 (RANSAC only) below 5."""
+    return n < 5 if m == 9 else ((m > 6 and n < 8) or n < 7)
+
+
 def _raw_batched(preps, methods, ransac_refine, bundle_adjust, covariance, device):
     """The estimates of run_real(raw_matches=True) for all triplets at once: per method one ragged api.ransac_pose over
     the triplets it can run (seed = loop index, CalM per triplet), then one ragged api.bundle_adjust and api.ba_covariance
@@ -117,7 +122,7 @@ def _raw_batched(preps, methods, ransac_refine, bundle_adjust, covariance, devic
     loop computes for that row (ba, cov None where it computes none); every problem is bit-identical to its B = 1 call."""
     out = {}
     for m in methods:
-        rows = [r for r, d in enumerate(preps) if not ((m > 6 and d["Corresp"].shape[1] < 8) or d["Corresp"].shape[1] < 7)]
+        rows = [r for r, d in enumerate(preps) if not _too_few(m, d["Corresp"].shape[1])]
         out[m] = {}
         if not rows:
             continue
@@ -168,6 +173,7 @@ def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), de
     size and its precision and recall against the ground-truth inlier mask; bundle_adjust / covariance run on the
     consensus columns, starting from the RANSAC pose (the points triangulated from it); a consensus of fewer than 4
     matches cannot be adjusted and gets +inf in the adjusted columns.
+    Method 9 (raw_matches only): RANSAC over five-point hypotheses (api.five_point_pose).
     ransac_refine=True (with raw_matches): api.ransac_pose(refine=True) instead, whose hypotheses and result are
     bundle-adjusted (8 LO rounds); nothing else changes.
     batched=True (with raw_matches): the triplets are prepared first, then RANSAC runs over all of them in one ragged
@@ -179,6 +185,8 @@ def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), de
         data = load_dataset(data)
     if batched and not raw_matches:
         raise ValueError("run_real: batched=True needs raw_matches=True")
+    if 9 in methods and not raw_matches:
+        raise ValueError("run_real: method 9 (five-point RANSAC) needs raw_matches=True")
     out = {m: np.zeros((len(triplets_to_test), 6 if bundle_adjust else 3)) for m in methods}
 
     def errors(R2, R3, CalM, inl, R_t0):
@@ -204,7 +212,7 @@ def run_real(data, triplets_to_test, initial_sample_size=100, methods=(1, 7), de
             rec["consensus"] = {}
         Nm = d["Corresp"].shape[1] if raw_matches else N
         for m in methods:
-            if (m > 6 and Nm < 8) or Nm < 7:                                                            # :117-122
+            if _too_few(m, Nm):                                                                          # :117-122
                 out[m][row] = np.inf
                 continue
             if batched:
